@@ -18,6 +18,9 @@ cores/4 concurrent processes of 4 threads, one ensemble member each.  /root/refe
 present on the GPU box, so that arm runs the oracle port (oracle/drvae_oracle.py: the same torch
 CPU ops, autograd and torch.optim.Adam the reference calls; pinned to the reference in
 oracle/make_golden.py).
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0's models) as .npy files, so that two builds can
+be compared output for output: every input is seeded, so the same arguments give the same inputs in every run.
 """
 import argparse
 import json
@@ -40,6 +43,7 @@ FIELDS = {"drvae": ("x1", "x2", "y", "has_x2", "has_y"), "pvae": ("x1", "x2", "h
 METRIC = "DrVAE train samples/sec (fwd+bwd+Adam)"
 UNIT = "samples/s"
 DATASET_ROWS = 600  # synthetic device-resident dataset per ensemble member (end-to-end loop)
+DUMP_PARAMS = 1 << 22  # parameters written by --dump-outputs (16 MB of float32); a larger model is sampled
 
 
 _STDOUT_FD = None
@@ -69,6 +73,21 @@ def measured_peaks():
         return dict(hbm=p["hbm_gbs"], bf16=p["bf16_tflops"], bf16_sustained=p["bf16_tflops_sustained"], which="measured")
     except Exception:
         return dict(hbm=6650.0, bf16=1590.0, bf16_sustained=1400.0, which="fallback")
+
+
+def dump_outputs(out_dir, losses, params):
+    """losses.npy: the [models, 8] loss terms the step returned.  params.npy: the flat [models, parameters] buffer the
+    step updated, or, when it holds more than DUMP_PARAMS values, those at DUMP_PARAMS indices drawn with seed 0 and
+    sorted, the same for every run of the same workload.  Both float32."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = params.reshape(-1)
+    if flat.numel() > DUMP_PARAMS:
+        idx = torch.randint(flat.numel(), (DUMP_PARAMS,), generator=torch.Generator().manual_seed(0)).sort().values
+        flat = flat[idx.to(flat.device)]
+    np.save(os.path.join(out_dir, "losses.npy"), losses.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "params.npy"), flat.detach().float().cpu().numpy())
 
 
 def ncu_traffic(kernel_tag):
@@ -364,7 +383,7 @@ def parity_check():
             "tolerance": 1e-3, "ELBO": float(got[5]), "ELBO_oracle": float(want["ELBO"])}
 
 
-def dp8192_result(ranks, steps, warmup):
+def dp8192_result(ranks, steps, warmup, dump_dir=None):
     """BASELINE configs[3]: DrVAE README architecture, ONE model, global minibatch 8192, rows sharded over the ranks
     (drvae_b200.dp).  Strong scaling: the global batch is fixed."""
     import torch
@@ -399,6 +418,8 @@ def dp8192_result(ranks, steps, warmup):
         losses = runner.step(devb, seed=1, row_offset=lo, host_flags=host)
     e1.record()
     ranks.barrier()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, losses, plan.params)
     ms = ranks.max(e0.elapsed_time(e1))
     launches = plan.launch_count() - l0
     peaks = measured_peaks()
@@ -421,18 +442,18 @@ def other_workloads(ranks, steps):
     out = {}
     for kind in ("drvae", "pvae", "vfae"):
         plan, host, devb, _ = build_ensemble(kind, 1, 0, ranks.dev)
-        ms, launches, _ = time_steps(plan, devb, max(steps, 50), 5, seed=1)
-        per = ms / max(steps, 50)
+        ms, launches, _ = time_steps(plan, devb, steps, 5, seed=1)
+        per = ms / steps
         floor_us = max(24.0 * N_PARAMS[kind] / (peaks["hbm"] * 1e9), FLOP_PER_SAMPLE[kind] * BATCH / (peaks["bf16_sustained"] * 1e12)) * 1e6
         out["%s150" % kind] = {"workload": "%s README config, ONE model, batch 150 (BASELINE configs[%d])" % (kind, ("drvae", "pvae", "vfae").index(kind)),
-                               "ms_per_step": per, "value": BATCH / (per * 1e-3), "unit": UNIT, "launches_per_step": launches / max(steps, 50),
+                               "ms_per_step": per, "value": BATCH / (per * 1e-3), "unit": UNIT, "launches_per_step": launches / steps,
                                "floor_us": floor_us, "frac_of_floor": floor_us / (per * 1e3),
                                "floor": "max(24 B x parameters / measured HBM GB/s, GEMM FLOPs / sustained bf16): launch/latency-bound (SURVEY 8(d))"}
         # the same step through the persistent step kernel (one cooperative launch for the whole forward + dX chain,
         # grid barriers between dependent stages): measured next to the default graph of launches, not the default
         plan.set_step_kernel(True)
-        ms2, launches2, _ = time_steps(plan, devb, max(steps, 50), 5, seed=1)
-        out["%s150" % kind]["persistent_step_kernel"] = {"ms_per_step": ms2 / max(steps, 50), "launches_per_step": launches2 / max(steps, 50)}
+        ms2, launches2, _ = time_steps(plan, devb, steps, 5, seed=1)
+        out["%s150" % kind]["persistent_step_kernel"] = {"ms_per_step": ms2 / steps, "launches_per_step": launches2 / steps}
         del plan
     M = 32
     for kind in ("pvae", "vfae"):
@@ -460,7 +481,13 @@ def main():
     ap.add_argument("--cpu-baseline-steps", type=int, default=12)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip other_workloads / dp8192 / parity (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's loss terms and "
+                                                          "updated parameters (a seeded sample of them) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU step (--impl b200)")
     if args.warmup < 3:
         args.warmup = 3
     quiet_stdout()
@@ -472,7 +499,7 @@ def main():
     ranks = Ranks()
     rank, world, dev = ranks.rank, ranks.world, ranks.dev
     if args.workload == "dp8192":
-        r = dp8192_result(ranks, args.steps, args.warmup)
+        r = dp8192_result(ranks, args.steps, args.warmup, dump_dir=args.dump_outputs)
         line = {"metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "bf16",
                 "data": "synthetic", "config": {"workload": r["workload"], "global_batch": 8192, "parallelism": "dp%d" % world},
@@ -495,6 +522,8 @@ def main():
     sampler.start()
     time.sleep(0.25)
     ms, launches, step_no = time_steps(plan, devb, args.steps, 0, seed=rank, ranks=ranks, step0=step_no)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, plan.losses, plan.params)  # train_step's result buffer still holds the last step
     ms = ranks.max(ms)
     samples = world * M * BATCH * args.steps
     value = samples / (ms / 1e3)

@@ -79,7 +79,8 @@ def main():
                     r = fw[key].detach().numpy()
                     o = fo[key].numpy()
                     assert np.allclose(r, o, rtol=1e-4, atol=1e-5), (cname, kind, key)
-                    rec["fwd/" + key] = r if (full or key in ("pred", "proba")) else r[:, :8]
+                    # README shapes: the first 1024 rows x 8 columns (keeps the 8192-row fixture under 1 MB)
+                    rec["fwd/" + key] = r if (full or key in ("pred", "proba")) else r[:1024, :8]
             # eval-mode loss (no noise draws, no update)
             le, draws_e = rh.reference_step(model, kind, batch, SEED_TAPE + 100, train=False)
             lo = om.loss(batch, orc.Tape(recorded=draws_e), train=False)

@@ -1,10 +1,12 @@
 """CPU: the oracle (oracle/drvae_oracle.py) against the golden vectors recorded from the
 reference itself (tests/golden/*.npz, written by oracle/make_golden.py)."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from helpers import ARCH, KINDS, L, NROWS, SEED_MODEL, SEED_TAPE, golden, orc
+from helpers import ARCH, GOLDEN, KINDS, L, NROWS, SEED_MODEL, SEED_TAPE, golden, orc
 
 from drvae_b200.init import init_state_dict
 
@@ -62,6 +64,11 @@ def test_oracle_forward_matches_reference_golden(kind):
     for key in ("pred", "proba", "z1", "z2", "x1_rec", "x2_pert"):
         if "fwd/" + key in g.files:
             assert np.allclose(fo[key].numpy(), g["fwd/" + key], rtol=1e-4, atol=1e-5), key
+
+
+def test_golden_files_stay_small():
+    for f in os.listdir(GOLDEN):
+        assert os.path.getsize(os.path.join(GOLDEN, f)) <= 1 << 20, f
 
 
 def test_bf16_emulation_is_close_to_fp32():
