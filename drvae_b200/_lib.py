@@ -48,6 +48,11 @@ class HParams(ctypes.Structure):
                 ("log_prior_y", c_float * 8), ("global_counts_dev", c_void_p)]
 
 
+class MemberHParams(ctypes.Structure):
+    _fields_ = [("yloss_rate", c_float), ("pertloss_rate", c_float), ("kl_qz2pz2_rate", c_float), ("noise_std", c_float),
+                ("lr", c_float), ("weight_decay", c_float), ("log_prior_y", c_float * 8)]
+
+
 class EpsLayout(ctypes.Structure):
     _fields_ = [("off_x1", c_ll), ("off_x2", c_ll), ("off_z1", c_ll), ("off_z2", c_ll), ("off_z2f", c_ll),
                 ("off_z3", c_ll), ("total", c_ll)]
@@ -72,7 +77,7 @@ EXPORTS = ["drvae_last_error", "drvae_plan_create", "drvae_plan_destroy", "drvae
            "drvae_profile_end", "drvae_plan_num_buckets", "drvae_plan_bucket_info", "drvae_stream_wait_bucket", "drvae_set_graph", "drvae_plan_graph_replays", "drvae_debug_wait_stats",
            "drvae_push_scalars", "drvae_set_external_scalars", "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_set_chains", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
            "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_adam_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
-           "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction"]
+           "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams"]
 
 
 def load():
@@ -138,6 +143,8 @@ def load():
     lib.drvae_infer.argtypes = [c_void_p, c_void_p, c_int, P(InferOut), c_void_p]
     lib.drvae_push_scalars.restype = c_int
     lib.drvae_push_scalars.argtypes = [c_void_p, P(Noise), P(HParams), c_int, c_void_p]
+    lib.drvae_set_member_hparams.restype = c_int
+    lib.drvae_set_member_hparams.argtypes = [c_void_p, P(MemberHParams), c_int, c_void_p]
     lib.drvae_set_external_scalars.restype = c_int
     lib.drvae_set_external_scalars.argtypes = [c_void_p, c_int]
     lib.drvae_debug_wait_stats.restype = c_int

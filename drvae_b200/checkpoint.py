@@ -22,17 +22,19 @@ def _host_views(plan, flat_cpu, model):
     return out
 
 
-def state_dicts(plan):
-    """-> [state_dict of member 0, ..., n_models - 1] (CPU tensors, reference layout); one device->host copy."""
-    flat = plan.params.detach().cpu()
+def state_dicts(plan, params=None):
+    """-> [state_dict of member 0, ..., n_models - 1] (CPU tensors, reference layout); one device->host copy.
+    params: an [n_models, param_count] buffer in the plan's layout to read instead of plan.params (e.g. snapshots)."""
+    flat = (plan.params if params is None else params).detach().cpu()
     return [_host_views(plan, flat, m) for m in range(plan.E)]
 
 
-def save_ensemble(plan, pattern):
-    """One reference-compatible .pth per member: pattern.format(i), e.g. 'models/drug{:03d}.pth'.  Returns the paths."""
+def save_ensemble(plan, pattern, params=None):
+    """One reference-compatible .pth per member: pattern.format(i), e.g. 'models/drug{:03d}.pth', or the i-th entry of
+    a list of paths.  params: as in state_dicts.  Returns the paths."""
     paths = []
-    for m, sd in enumerate(state_dicts(plan)):
-        path = pattern.format(m)
+    for m, sd in enumerate(state_dicts(plan, params)):
+        path = pattern[m] if isinstance(pattern, (list, tuple)) else pattern.format(m)
         d = os.path.dirname(path)
         if d:
             os.makedirs(d, exist_ok=True)

@@ -112,6 +112,8 @@ def split(d, fold, n_folds=5):
 
 def main(argv=None):
     argv = list(sys.argv[1:] if argv is None else argv)
+    if argv and argv[0] == "sweep":
+        return sweep_main(argv[1:])
     if not argv or argv[0] not in ("drvae", "pvae", "vfae"):
         raise SystemExit("usage: python -m drvae_b200.cli {drvae|pvae|vfae} --modelid ID --datafile FILE [flags]")
     kind = argv.pop(0)
@@ -123,18 +125,7 @@ def main(argv=None):
     torch.manual_seed(args.rseed)
     np.random.seed(args.rseed)
     sing, pair = load_data(args.datafile, args.rseed)
-    s_tr, s_va, s_te = split(sing, args.fold)
-    p_tr, p_va, p_te = split(pair, args.fold)
-    if kind == 'vfae':
-        mode = 'both' if args.alldata else 'sing_only'
-        wrap = lambda s_, p_, **kw: wrap_in_VFAEDataset(s_, p_, concat=mode, **kw)
-    else:
-        mode = 'pair_only' if args.pair_data_only else 'both'
-        wrap = lambda s_, p_, **kw: wrap_in_DrVAEDataset(s_, p_, concat=mode, **kw)
-    train_ds, _ = wrap(s_tr, p_tr, downlabel_to=args.downlabel_to,
-                       remove_unlabeled=(kind != 'pvae' and not args.semi_supervised))
-    valid_ds, _ = wrap(s_va, p_va)
-    test_ds, _ = wrap(s_te, p_te)
+    train_ds, valid_ds, test_ds = fold_datasets(kind, args, sing, pair, args.fold)
     dim_x = train_ds.x1.shape[1]
     modelid = args.modelid
     if modelid == 'auto':
@@ -190,6 +181,117 @@ def main(argv=None):
     with open(out, 'w') as f:
         json.dump({args.drug: results}, f, indent=1)
     print('wrote', out)
+    return results
+
+
+# ------------------------------------------------------------------------------------------------
+# sweep: the reference's job grid (src/scripts/submitVAE.sh) as one ensemble plan (drvae_b200/sweep.py)
+# ------------------------------------------------------------------------------------------------
+def build_sweep_parser(kind):
+    """The flags of `kind`'s driver plus the grid axes.  --modelid, --rseed and --fold do not apply: members are named
+    per grid point as the reference's driver names them with --modelid auto."""
+    p = build_parser(kind)
+    p.prog = "drvae_b200.cli sweep " + kind
+    for act in p._actions:
+        if act.dest == 'modelid':
+            act.required, act.default = False, 'auto'
+    a = p.add_argument
+    a('--rseeds', type=int, nargs='+', required=True, help='random seeds of the grid')
+    a('--folds', type=int, nargs='+', required=True, help='data folds of the grid (1 to 5)')
+    if kind in ('drvae', 'vfae'):
+        a('--yloss-rates', type=float, nargs='+', default=None, help='y-loss rates of the grid (default: --yloss-rate)')
+    return p
+
+
+def sweep_grid(kind, args):
+    """-> [(seed, rate, fold, modelid)] in the order seeds x rates x folds; rate is 0 for PVAE (no y loss)."""
+    rates = (args.yloss_rates or [args.yloss_rate]) if kind != 'pvae' else [0]
+    return [(s, r, f, 'RS{}_L{}_YR{}_FOLD{}'.format(s, args.L, r, f)) for s in args.rseeds for r in rates for f in args.folds]
+
+
+def fold_datasets(kind, args, sing, pair, fold):
+    """(train, valid, test) datasets of one fold, as the single-model driver builds them."""
+    s_tr, s_va, s_te = split(sing, fold)
+    p_tr, p_va, p_te = split(pair, fold)
+    if kind == 'vfae':
+        mode = 'both' if args.alldata else 'sing_only'
+        wrap = lambda s_, p_, **kw: wrap_in_VFAEDataset(s_, p_, concat=mode, **kw)
+    else:
+        mode = 'pair_only' if args.pair_data_only else 'both'
+        wrap = lambda s_, p_, **kw: wrap_in_DrVAEDataset(s_, p_, concat=mode, **kw)
+    train_ds, _ = wrap(s_tr, p_tr, downlabel_to=args.downlabel_to,
+                       remove_unlabeled=(kind != 'pvae' and not args.semi_supervised))
+    return train_ds, wrap(s_va, p_va)[0], wrap(s_te, p_te)[0]
+
+
+def class_prior(kind, args, train_ds, dim_y=2):
+    """--clf-dataprior: class frequencies of the fold's labeled training rows; else uniform."""
+    if kind == 'pvae' or not args.clf_dataprior:
+        return [1.0 / dim_y] * dim_y
+    lab = train_ds.y[train_ds.has_y != 0].long()
+    prior = np.bincount(lab.numpy(), minlength=dim_y).astype(float)
+    return list(prior / prior.sum())
+
+
+def sweep_main(argv):
+    from . import checkpoint
+    from .sweep import evaluate_members, fit_sweep, pad_members
+    if not argv or argv[0] not in ("drvae", "pvae", "vfae"):
+        raise SystemExit("usage: python -m drvae_b200.cli sweep {drvae|pvae|vfae} --datafile FILE --rseeds S... --folds F... "
+                         "[--yloss-rates R...] [flags]")
+    kind = argv.pop(0)
+    args = build_sweep_parser(kind).parse_args(argv)
+    print(args)
+    assert args.data_mode in ['strictC2C'], 'Unsupported data mode'
+    assert args.type_y == 'discrete', 'sweep: only type-y discrete is supported'
+    assert args.useMF is False, 'use of mol.features not supported'
+    assert not (args.useS or args.useMMD or getattr(args, 'class_y', [])), 'sweep: use-s, use-mmd and class-y are not supported'
+    grid = sweep_grid(kind, args)
+    data = {}  # the single-model driver loads the data with its --rseed
+    for seed in args.rseeds:
+        data[seed] = load_data(args.datafile, seed)
+    folds = {(s, f): fold_datasets(kind, args, *data[s], f) for s in args.rseeds for f in args.folds}
+    members, datasets = [], []
+    for seed, rate, fold, _ in grid:
+        train_ds, valid_ds, _ = folds[(seed, fold)]
+        hp = dict(yloss_rate=rate, pertloss_rate=0.05 if kind != 'vfae' else 0.,
+                  kl_qz2pz2_rate=args.kl_z2_rate if kind == 'pvae' else 1., noise_std=args.noise_var, lr=0.0005,
+                  weight_decay=0.05, prior_y=class_prior(kind, args, train_ds))
+        members.append(dict(seed=seed, hparams=hp))
+        datasets.append((train_ds, valid_ds))
+    dim_x = datasets[0][0].x1.shape[1]
+    if kind == 'drvae':
+        arch = dict(dim_z3=args.dim_z3, enc_z3=args.enc_z3, dec_z1=args.dec_z1)
+    elif kind == 'vfae':
+        arch = dict(dim_z3=args.dim_z2, enc_z3=args.enc_z2, dec_z1=args.dec_z1)
+    else:
+        arch = dict(dim_z3=0, enc_z3=[], dec_z1=[])
+    arch.update(dim_x=dim_x, dim_y=2, dim_z1=args.dim_z1, enc_z1=args.enc_z1, dec_x=args.dec_x)
+    epochs = args.epochs or (300 if kind == 'drvae' else 1000)
+    out = fit_sweep(kind, arch, members, datasets, batch_size=args.batch_size, L=args.L, epochs=epochs,
+                    early_stop=args.stopearly, add_noise=args.train_w_noise,
+                    anneal_perturb=(1, 0) if kind != 'vfae' else None, sample_seed=args.rseeds[0], log=print)
+    plan = out['plan']
+    outdir = args.outdir or '.'
+    os.makedirs(os.path.join(outdir, 'models'), exist_ok=True)
+    os.makedirs(os.path.join(outdir, 'results'), exist_ok=True)
+    cls = {'drvae': 'DrVAE', 'pvae': 'PVAE', 'vfae': 'VFAE'}[kind]
+    paths = [os.path.join(outdir, 'models', '{}_SD_{}_{}.pth'.format(cls, g[3], args.drug)) for g in grid]
+    checkpoint.save_ensemble(plan, paths, out['best'])
+    # eval-mode losses are not computed: loss_forward normalises by one N for all members, and padding rows would
+    # enter the normalisers of every member with a smaller split
+    perfs = {}
+    for name, which in (('train', 0), ('valid', 1), ('test', 2)):
+        fields, mask, _ = pad_members(kind, [folds[(g[0], g[2])][which] for g in grid])
+        perfs[name] = evaluate_members(plan, kind, {k: v.to(plan.device) for k, v in fields.items()}, mask.to(plan.device))
+    results = []
+    for m, (seed, rate, fold, modelid) in enumerate(grid):
+        res = {name: dict(perfs[name][m]) for name in perfs}
+        path = os.path.join(outdir, 'results', '{}_SD_all_{}.json'.format(cls, modelid))
+        with open(path, 'w') as f:
+            json.dump({args.drug: res}, f, indent=1)
+        print('wrote', path, '(snapshot at epoch {})'.format(out['snapshot_epoch'][m]))
+        results.append(res)
     return results
 
 

@@ -374,6 +374,10 @@ __device__ __forceinline__ float sigmoid_sp(float x) { return x > 20.f ? 1.f : 1
 struct AdamHyper {
   float lr_bc1, beta1, beta2, eps, wd, inv_sqrt_bc2;
 };
+// Adam scalars of global model `model`: `ms` bytes between models (0: one copy shared by the ensemble).
+__device__ __forceinline__ AdamHyper adam_of(const AdamHyper* h, int ms, int model) {
+  return *reinterpret_cast<const AdamHyper*>(reinterpret_cast<const char*>(h) + (long long)model * ms);
+}
 __device__ __forceinline__ void adam_update(float g, float& p, float& m, float& v, const AdamHyper& h) {
   const float gr = g + h.wd * p;
   m = h.beta1 * m + (1.f - h.beta1) * gr;

@@ -95,6 +95,7 @@ struct DwaParams {
   bf16* shadow;             // shadow arena (direct-store variant)
   long long shadow_ms;
   const AdamHyper* adam;
+  int adam_ms;              // bytes between the Adam scalars of consecutive models (0: shared)
   DebugWord* dbg;
   unsigned long long* trace;
   int trace_id;
@@ -394,12 +395,12 @@ __global__ void __launch_bounds__(DWA_THREADS, DWA_MIN_BLOCKS) dwadam_kernel(con
     const int w = warp - 4, q = w & 3, g = w >> 2;
     const int kl = q * 32 + lane;          // tile-local input feature = TMEM lane
     const int et = threadIdx.x - 128;      // 0 .. 511
-    const AdamHyper h = *p.adam;
     uint32_t it = 0, j = 0;
     for (int tile = p.tile_begin + blockIdx.x; tile < p.tile_end; tile += gridDim.x) {
       const DwaTile t = dwa_tile(p, L, tile);
       if (!t.active) continue;
       const DwaLayer& y = L[t.layer];
+      const AdamHyper h = adam_of(p.adam, p.adam_ms, t.model);
       const uint32_t a = j & 1, aph = (j >> 1) & 1;
       const int kk = t.m0 + kl;  // D row
       const bool is_w = kk < y.kin, is_b = kk == y.kin, is_c = kk > y.kin && kk < y.kaug;

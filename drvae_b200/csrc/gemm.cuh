@@ -183,7 +183,8 @@ struct EpiParams {
   long long drv_bias_off;
   long long drv_clsb_off;
   int drv_clsb_ld;
-  const AdamHyper* adam;  // device memory (StepDyn): changes every step
+  const AdamHyper* adam;  // device memory (StepDyn or the member table): changes every step
+  int adam_ms;            // bytes between the Adam scalars of consecutive models (0: shared)
   // EPI_DECLOSS / EPI_DECOUT
   const float4* tgt4;  // fp32 targets, chunk4 layout [Xc/4][tgt_rcap] float4
   long long tgt_ms;    // float4 elements between models
@@ -377,7 +378,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
       float* P = e.adam_p + rc.model * e.grad_ms + kofs;
       float* M1 = e.adam_m + rc.model * e.grad_ms + kofs;
       float* V2 = e.adam_v + rc.model * e.grad_ms + kofs;
-      const AdamHyper h = *e.adam;
+      const AdamHyper h = adam_of(e.adam, e.adam_ms, rc.model);
       float pv[16], mv[16], vv[16];
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
@@ -768,7 +769,7 @@ __device__ __forceinline__ void adam_pipe_apply(const EpiParams& e, int model, i
     for (int i = 0; i < 8; ++i) acc[i] = 0.f;
   }
   if (k >= e.g_kaug) return;
-  const AdamHyper h = *e.adam;
+  const AdamHyper h = adam_of(e.adam, e.adam_ms, model);
 #pragma unroll
   for (int i = 0; i < 8; ++i) adam_update(acc[i], b.p[i], b.m[i], b.v[i], h);
   float* P = e.adam_p + model * e.grad_ms + kofs;
@@ -960,7 +961,7 @@ __device__ __forceinline__ void adam_vec_apply(const EpiParams& e, int model, in
     quad_transpose4(x1, g[1], lane);
   }
   if (k4 >= e.g_kaug) return;
-  const AdamHyper h = *e.adam;
+  const AdamHyper h = adam_of(e.adam, e.adam_ms, model);
 #pragma unroll
   for (int j = 0; j < 2; ++j) {
     adam_update(g[j][0], b.p[j].x, b.m[j].x, b.v[j].x, h);

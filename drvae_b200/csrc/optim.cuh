@@ -47,7 +47,8 @@ struct AdamArgs {
   const Seg* segs;
   int nseg;
   int P;  // parameters per model
-  const AdamHyper* h;  // device memory (StepDyn)
+  const AdamHyper* h;  // device memory (StepDyn or the member table)
+  int h_ms;            // bytes between the Adam scalars of consecutive models (0: shared)
   int update;  // 0: only refresh the derived copies from the current parameters
   // parameters [skip_lo, skip_hi) are left untouched when the batch (global counts if given) has no pair rows
   int skip_lo, skip_hi;
@@ -67,7 +68,7 @@ __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
   float* dv = a.derived.at(mdl);
   const int base = blockIdx.x * 1024 + threadIdx.x;
   AdamHyper hyper{};
-  if (a.update) hyper = *a.h;
+  if (a.update) hyper = adam_of(a.h, a.h_ms, mdl);
   bool skip_range = false;
   if (a.update && a.skip_hi > a.skip_lo) {
     const int np = a.dyn->s.gN > 0 ? a.dyn->s.gNp : a.counts[(long long)mdl * a.counts_stride + CNT_NP];
@@ -157,16 +158,34 @@ __global__ void spin_kernel(long long cycles) {
   while (clock64() - t0 < cycles) __nanosleep(64);
 }
 
-// writes the per-step scalars; the only kernel whose arguments differ between two steps of the same shape
-__global__ void set_dyn_kernel(StepDyn value, StepDyn* dst) {
+// writes the per-step scalars; the only kernel whose arguments differ between two steps of the same shape.  With a
+// member table it also expands the table into this step's per-member scalars: lr / bc1 rounds like the host's float
+// division of adam_scalars(), so a member gets exactly the update of a table-less plan run with its lr.
+__global__ void set_dyn_kernel(StepDyn value, StepDyn* dst, MemberExpand mx) {
   pdl_launch_dependents();
   pdl_wait();
-  if (value.counts_dev) {  // batch-global normalisers left in device memory by the caller's all-reduce
-    value.s.gN = (int)value.counts_dev[0];
-    value.s.gNp = (int)value.counts_dev[1];
-    value.s.gNlab = (int)value.counts_dev[2];
+  if (threadIdx.x == 0) {
+    if (value.counts_dev) {  // batch-global normalisers left in device memory by the caller's all-reduce
+      value.s.gN = (int)value.counts_dev[0];
+      value.s.gNp = (int)value.counts_dev[1];
+      value.s.gNlab = (int)value.counts_dev[2];
+    }
+    *dst = value;
   }
-  *dst = value;
+  for (int k = threadIdx.x; k < mx.n; k += blockDim.x) {
+    const drvae_member_hparams_t h = mx.table[k];
+    MemberScalars s;
+    s.noise_std = h.noise_std;
+    s.pertloss_rate = h.pertloss_rate;
+    s.kl_qz2pz2_rate = h.kl_qz2pz2_rate;
+    s.yloss_rate = h.yloss_rate;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) s.log_prior[j] = h.log_prior_y[j];
+    s.adam = value.s.mem.adam;
+    s.adam.lr_bc1 = __fdiv_rn(h.lr, value.bc1);
+    s.adam.wd = h.weight_decay;
+    mx.out[k] = s;
+  }
 }
 
 // ε block generator.  Every normal is keyed by (seed, step, model, segment, MC sample, GLOBAL row,

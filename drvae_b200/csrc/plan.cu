@@ -94,6 +94,13 @@ struct drvae_plan {
   bool shadows_valid = false;
   // per-step scalars in device memory + CUDA-graph replay of the launch sequence (see step_entry)
   StepDyn* d_dyn = nullptr;
+  // member table (drvae_set_member_hparams): device copy of the caller's table, its per-step expansion, and the pinned
+  // staging the copy is made from (member_ev: the last copy out of it)
+  bool member_table = false;
+  drvae_member_hparams_t* d_member_hp = nullptr;
+  MemberScalars* d_member = nullptr;
+  drvae_member_hparams_t* h_member_stage = nullptr;
+  cudaEvent_t member_ev = nullptr;
   bool graph_enabled = true;
   bool external_dyn = false;  // the caller pushes the per-step scalars (drvae_push_scalars) and captures the sequence itself
   struct GraphEntry {
@@ -718,6 +725,10 @@ extern "C" int drvae_plan_destroy(drvae_plan_t* pl) {
   if (pl->d_dwa_stats) cudaFree(pl->d_dwa_stats);
   if (pl->d_stepk_bar) cudaFree(pl->d_stepk_bar);
   if (pl->d_sview) cudaFree(pl->d_sview);
+  if (pl->d_member_hp) cudaFree(pl->d_member_hp);
+  if (pl->d_member) cudaFree(pl->d_member);
+  if (pl->h_member_stage) cudaFreeHost(pl->h_member_stage);
+  if (pl->member_ev) cudaEventDestroy(pl->member_ev);
   for (auto& ev : pl->bucket_ev) cudaEventDestroy(ev);
   for (auto& ch : pl->chain) {
     for (int i = 0; i < drvae_plan::Chain::N_EVENTS; ++i)
@@ -937,6 +948,16 @@ void prof_post(drvae_plan* pl, cudaStream_t st) {
   cudaEventRecord(pl->prof_ev[pl->prof_used++], st);
 }
 
+// Where the readers of per-member scalars look (MemberScalars in plan.h): the shared copy in the per-step block with
+// stride 0, or the member table's per-step expansion.
+const MemberScalars* member_base(const drvae_plan* pl) { return pl->member_table ? pl->d_member : &pl->d_dyn->s.mem; }
+const AdamHyper* member_adam(const drvae_plan* pl) { return &member_base(pl)->adam; }
+int member_adam_ms(const drvae_plan* pl) { return pl->member_table ? (int)sizeof(MemberScalars) : 0; }
+MemberExpand member_expand(const drvae_plan* pl) {
+  return pl->member_table ? MemberExpand{pl->d_member_hp, pl->d_member, pl->E} : MemberExpand{nullptr, nullptr, 0};
+}
+int set_dyn_threads(const MemberExpand& mx) { return mx.n > 0 ? std::min(256, (mx.n + 31) / 32 * 32) : 1; }
+
 struct Exec {
   drvae_plan* pl;
   cudaStream_t st;
@@ -1132,7 +1153,8 @@ struct Exec {
       e.drv_bias_off = W.bias_off;
       e.drv_clsb_off = W.clsb_off;
       e.drv_clsb_ld = W.rcap;
-      e.adam = &pl->d_dyn->s.adam;
+      e.adam = member_adam(pl);
+      e.adam_ms = member_adam_ms(pl);
     }
     const bool aside = dw_stream && !fused && dw_stream != st;
     cudaStream_t chain_st = st;
@@ -1229,11 +1251,12 @@ struct Exec {
 };
 
 // Step-dependent Adam scalars, computed once on the host so that the fused epilogue and the
-// stand-alone kernel apply bit-identical updates.
-AdamHyper adam_scalars(const drvae_hparams_t* hp) {
+// stand-alone kernel apply bit-identical updates.  bc1_out: the bias correction lr is divided by (member tables).
+AdamHyper adam_scalars(const drvae_hparams_t* hp, float* bc1_out) {
   const double t = (double)hp->step + 1.0;
   const float bc1 = (float)(1.0 - pow((double)hp->beta1, t));
   const float bc2 = (float)(1.0 - pow((double)hp->beta2, t));
+  *bc1_out = bc1;
   AdamHyper a;
   a.lr_bc1 = hp->lr / bc1;
   a.inv_sqrt_bc2 = 1.0f / sqrtf(bc2);
@@ -1277,6 +1300,8 @@ int fill_view(drvae_plan* pl, Exec& ex, const drvae_batch_t* b, const drvae_nois
   v.eps_z3 = MBuf<const float>{eps + pl->epsl.off_z3, ems};
   v.own_noise = (nz && nz->eps) ? 0 : 1;
   v.dyn = pl->d_dyn;
+  v.mem = member_base(pl);
+  v.mem_stride = pl->member_table ? 1 : 0;
   v.sview_dev = nullptr;
   v.params = MBuf<float>{pl->params, pl->P};
   v.clf_w = pl->wn ? MBuf<const float>{pl->derived.p + pl->clf_eff_off, pl->derived.ms}
@@ -1292,18 +1317,18 @@ StepDyn make_dyn(const drvae_noise_t* nz, const drvae_hparams_t* hp, bool fused_
   StepDyn d{};
   StepScalars& s = d.s;
   s.kl_min = hp->kl_min;
-  s.noise_std = hp->noise_std;
+  s.mem.noise_std = hp->noise_std;
   s.beta_pert = hp->beta_pert;
-  s.pertloss_rate = hp->pertloss_rate;
-  s.kl_qz2pz2_rate = hp->kl_qz2pz2_rate;
-  s.yloss_rate = hp->yloss_rate;
+  s.mem.pertloss_rate = hp->pertloss_rate;
+  s.mem.kl_qz2pz2_rate = hp->kl_qz2pz2_rate;
+  s.mem.yloss_rate = hp->yloss_rate;
   s.training = hp->training;
   s.add_noise = hp->add_noise;
   s.gN = hp->global_N;
   s.gNp = hp->global_Np;
   s.gNlab = hp->global_Nlab;
-  for (int j = 0; j < 8; ++j) s.log_prior[j] = hp->log_prior_y[j];
-  s.adam = adam_scalars(hp);
+  for (int j = 0; j < 8; ++j) s.mem.log_prior[j] = hp->log_prior_y[j];
+  s.mem.adam = adam_scalars(hp, &d.bc1);
   s.fused_adam = fused_adam ? 1 : 0;
   d.noise_step = (unsigned)hp->step;
   d.noise_seed = nz ? nz->seed : 0ULL;
@@ -1314,7 +1339,8 @@ StepDyn make_dyn(const drvae_noise_t* nz, const drvae_hparams_t* hp, bool fused_
 
 int push_dyn(drvae_plan* pl, const StepDyn& d, cudaStream_t st) {
   prof_pre(pl, st, ":set_dyn");
-  launch_k(set_dyn_kernel, dim3(1), dim3(1), 0, st, 2, d, pl->d_dyn);
+  const MemberExpand mx = member_expand(pl);
+  launch_k(set_dyn_kernel, dim3(1), dim3(set_dyn_threads(mx)), 0, st, 2, d, pl->d_dyn, mx);
   prof_post(pl, st);
   pl->launches++;
   cudaError_t err = cudaGetLastError();
@@ -1336,7 +1362,8 @@ int run_adam(drvae_plan* pl, const drvae_hparams_t* hp, int update, cudaStream_t
   a.nseg = (int)pl->segs.size();
   a.P = pl->P;
   a.update = update;
-  a.h = &pl->d_dyn->s.adam;  // the caller has pushed this step's scalars
+  a.h = member_adam(pl);  // the caller has pushed this step's scalars
+  a.h_ms = member_adam_ms(pl);
   // PVAE: p(z2|z1) takes part in the loss only through pair rows (PVAE.py:313-330); without pairs the reference's
   // gradient is None and torch.optim.Adam leaves the tensors (and their moments) untouched
   a.skip_lo = a.skip_hi = 0;
@@ -1463,7 +1490,8 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
     dp.drv_ms = pl->derived.ms;
     dp.shadow = pl->shadow.p;
     dp.shadow_ms = pl->shadow.ms;
-    dp.adam = &pl->d_dyn->s.adam;
+    dp.adam = member_adam(pl);
+    dp.adam_ms = member_adam_ms(pl);
     dp.dbg = pl->dbg;
     cudaStream_t keep = ex.st;
     ex.st = stream;
@@ -1992,7 +2020,8 @@ int step_entry(drvae_plan* pl, int seq, const drvae_batch_t* b, const drvae_nois
     if (ge.exec) {
       StepDyn value = dyn;
       StepDyn* dst = pl->d_dyn;
-      void* args[2] = {&value, &dst};
+      MemberExpand mx = member_expand(pl);
+      void* args[3] = {&value, &dst, &mx};
       cudaKernelNodeParams np = ge.dyn_params;
       np.kernelParams = args;
       np.extra = nullptr;
@@ -2052,6 +2081,7 @@ extern "C" int drvae_dp_attach(drvae_plan_t* pl, const drvae_dp_peers_t* peers) 
   if (peers->world < 1 || peers->world > DP_MAX_RANKS || peers->rank < 0 || peers->rank >= peers->world)
     return set_error("drvae_dp_attach: bad rank / world size");
   if (!pl->params || !pl->adam_m || !pl->adam_v) return set_error("drvae_dp_attach: bind parameters and Adam moments first");
+  if (pl->member_table) return set_error("drvae_dp_attach: a plan with a member table cannot be data-parallel");
   DpPeers d{};
   d.rank = peers->rank;
   d.world = peers->world;
@@ -2103,7 +2133,7 @@ extern "C" int drvae_dp_adam_step(drvae_plan_t* pl, const drvae_hparams_t* hp, f
   a.nseg = (int)pl->segs.size();
   a.P = pl->P;
   a.update = 1;
-  a.h = &pl->d_dyn->s.adam;
+  a.h = &pl->d_dyn->s.mem.adam;
   a.skip_lo = a.skip_hi = 0;
   if (pl->arch.kind == DRVAE_KIND_PVAE && pl->has_T) a.skip_lo = (int)pl->T_range[0], a.skip_hi = (int)(pl->T_range[0] + pl->T_range[1]);
   a.dyn = pl->d_dyn;
@@ -2131,6 +2161,44 @@ extern "C" int drvae_push_scalars(drvae_plan_t* pl, const drvae_noise_t* nz, con
                                   void* stream) {
   if (!pl || !hp) return set_error("drvae_push_scalars: null argument");
   return push_dyn(pl, make_dyn(nz, hp, fused_adam != 0), (cudaStream_t)stream);
+}
+extern "C" int drvae_set_member_hparams(drvae_plan_t* pl, const drvae_member_hparams_t* members, int count, void* stream) {
+  if (!pl) return set_error("drvae_set_member_hparams: null plan");
+  if (pl->dp_on) return set_error("drvae_set_member_hparams: a data-parallel plan cannot take a member table");
+  if (count == 0 && !members) {
+    if (pl->member_table) drop_graphs(pl);  // captured sequences read the table's expansion
+    pl->member_table = false;
+    return 0;
+  }
+  if (!members || count != pl->E) return set_error("drvae_set_member_hparams: need n_models entries (or NULL and 0 to clear)");
+  for (int k = 0; k < count; ++k) {
+    const drvae_member_hparams_t& h = members[k];
+    const float nonneg[] = {h.yloss_rate, h.pertloss_rate, h.kl_qz2pz2_rate, h.noise_std, h.lr, h.weight_decay};
+    for (float r : nonneg)
+      if (!isfinite(r) || r < 0.f)
+        return set_error("drvae_set_member_hparams: rates, noise_std, lr and weight_decay must be finite and >= 0");
+    for (int j = 0; j < 8; ++j)
+      if (!isfinite(h.log_prior_y[j])) return set_error("drvae_set_member_hparams: log_prior_y must be finite");
+  }
+  cudaError_t err = cudaSuccess;
+  if (!pl->d_member_hp) {
+    err = cudaMalloc(&pl->d_member_hp, sizeof(drvae_member_hparams_t) * pl->E);
+    if (err == cudaSuccess) err = cudaMalloc(&pl->d_member, sizeof(MemberScalars) * pl->E);
+    if (err == cudaSuccess) err = cudaMallocHost(&pl->h_member_stage, sizeof(drvae_member_hparams_t) * pl->E);
+    if (err == cudaSuccess) err = cudaEventCreateWithFlags(&pl->member_ev, cudaEventDisableTiming);
+    if (err != cudaSuccess) return set_cuda_error("drvae_set_member_hparams", err);
+  } else {
+    err = cudaEventSynchronize(pl->member_ev);  // the previous table may still be on its way out of the staging buffer
+    if (err != cudaSuccess) return set_cuda_error("drvae_set_member_hparams", err);
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  memcpy(pl->h_member_stage, members, sizeof(drvae_member_hparams_t) * pl->E);
+  err = cudaMemcpyAsync(pl->d_member_hp, pl->h_member_stage, sizeof(drvae_member_hparams_t) * pl->E, cudaMemcpyHostToDevice, st);
+  if (err == cudaSuccess) err = cudaEventRecord(pl->member_ev, st);
+  if (err != cudaSuccess) return set_cuda_error("drvae_set_member_hparams", err);
+  if (!pl->member_table) drop_graphs(pl);  // the kernels' per-member pointers and strides change
+  pl->member_table = true;
+  return 0;
 }
 extern "C" int drvae_set_external_scalars(drvae_plan_t* pl, int enable) {
   if (!pl) return set_error("drvae_set_external_scalars: null plan");
@@ -2288,6 +2356,8 @@ extern "C" int drvae_infer(drvae_plan_t* pl, const float* x1, int N, const drvae
   v.clf_w = pl->wn ? MBuf<const float>{pl->derived.p + pl->clf_eff_off, pl->derived.ms}
                    : MBuf<const float>{pl->params + pl->clf_w_off, pl->P};
   v.dyn = pl->d_dyn;
+  v.mem = member_base(pl);
+  v.mem_stride = pl->member_table ? 1 : 0;
   v.sview_dev = nullptr;
   v.own_noise = 0;
   {

@@ -113,14 +113,24 @@ struct MlpBlock {
 // ---------------------------------------------------------------------------------------------
 // Device-visible view used by the row kernels
 // ---------------------------------------------------------------------------------------------
+// Scalars that may differ between ensemble members (drvae_set_member_hparams).  Every reader takes a base pointer and a
+// model stride (DevView::member, EpiParams / DwaParams / AdamArgs adam + adam_ms): without a member table the stride
+// is 0 and the base is the shared copy in StepDyn, so a table-less plan reads the same values as one without the
+// feature; with a table the base is the plan's per-member array, expanded by set_dyn_kernel at the head of each step.
+struct MemberScalars {
+  float noise_std;
+  float pertloss_rate, kl_qz2pz2_rate, yloss_rate;
+  float log_prior[8];  // log prior_y
+  AdamHyper adam;
+};
+
 struct StepScalars {
-  float kl_min, noise_std;
-  float beta_pert, pertloss_rate, kl_qz2pz2_rate, yloss_rate;
+  float kl_min;
+  float beta_pert;
   int training, add_noise;
   int gN, gNp, gNlab;  // global normalisers (0 = use local counts)
-  AdamHyper adam;
   int fused_adam;  // 1: the optimizer update happens inside the gradient kernels (drvae_train_step)
-  float log_prior[8];  // log prior_y
+  MemberScalars mem;  // shared values of the per-member scalars
 };
 
 // Everything that changes from step to step.  Lives in device memory (one block per plan), written by
@@ -129,10 +139,19 @@ struct StepScalars {
 // replayed as a CUDA graph with only that one kernel node's arguments updated.
 struct StepDyn {
   StepScalars s;
+  float bc1;  // Adam bias correction 1 - beta1^t: a member's lr_bc1 is its lr / bc1 (set_dyn_kernel)
   unsigned int noise_step;
   unsigned long long noise_seed;
   long long row_offset;
   const long long* counts_dev;  // optional device {N, Np, Nlab} summed over the shards: overrides s.gN / gNp / gNlab
+};
+
+// Member table of a plan (drvae_set_member_hparams): set_dyn_kernel expands `table` (n entries, device) into `out`.
+// n = 0: no table.
+struct MemberExpand {
+  const drvae_member_hparams_t* table;
+  MemberScalars* out;
+  int n;
 };
 
 struct DevView {
@@ -206,6 +225,9 @@ struct DevView {
                             // effective (weight-normalised) copy in the derived arena
   MBuf<float> losses;  // [8]
   const StepDyn* dyn;  // per-step scalars (device memory)
+  const MemberScalars* mem;  // per-member scalars of global model m: mem[m * mem_stride] (stride 0: the copy in dyn)
+  int mem_stride;
+  __host__ __device__ __forceinline__ const MemberScalars& member(int m) const { return mem[(long long)m * mem_stride]; }
   SampleView* sview_dev;  // device copy of the sampling epilogue's view (written by rowmap_kernel; null: not used)
   unsigned long long* trace;  // kernel trace buffer (null: off) and this launch's slot
   int trace_id;

@@ -150,10 +150,10 @@ __global__ void __launch_bounds__(ROWMAP_THREADS) rowmap_kernel(DevView v) {
     const float Lf = v.L;
     float* cf = v.coefs.at(m);
     cf[COEF_RECL] = 1.f / (Lf * gN);
-    cf[COEF_PERT] = v.dyn->s.beta_pert * v.dyn->s.pertloss_rate / (Lf * gNp);
-    cf[COEF_KLZ2] = v.dyn->s.beta_pert * v.dyn->s.kl_qz2pz2_rate / (Lf * gN);
+    cf[COEF_PERT] = v.dyn->s.beta_pert * v.member(m).pertloss_rate / (Lf * gNp);
+    cf[COEF_KLZ2] = v.dyn->s.beta_pert * v.member(m).kl_qz2pz2_rate / (Lf * gN);
     cf[COEF_KLD] = 1.f / (Lf * gN);
-    cf[COEF_YL] = v.dyn->s.yloss_rate / (Lf * gNl);
+    cf[COEF_YL] = v.member(m).yloss_rate / (Lf * gNl);
     cf[COEF_INV_N] = 1.f / gN;
     cf[COEF_PERT_PLAIN] = 1.f / (Lf * gNp);
     cf[COEF_YL_PLAIN] = 1.f / (Lf * gNl);
@@ -251,7 +251,7 @@ __global__ void __launch_bounds__(PREP_THREADS) prep_kernel(DevView v) {
           for (int k = 0; k < 4; ++k) {
             if (f + k < v.X) {
               x[k] = src[f + k];
-              if (noisy) x[k] += v.dyn->s.noise_std * (v.own_noise ? z[k] : eps[f + k]);
+              if (noisy) x[k] += v.member(m).noise_std * (v.own_noise ? z[k] : eps[f + k]);
             }
           }
         }
@@ -328,7 +328,7 @@ __device__ __forceinline__ void classifier_row(const DevView& v, int m, int r, i
       if (lb) {
         if (j == yi) yl = lq;
       } else {
-        ycat += -q * (v.dyn->s.log_prior[j] - lq);
+        ycat += -q * (v.member(m).log_prior[j] - lq);
       }
     }
   }
@@ -394,7 +394,7 @@ __device__ __forceinline__ void classifier_row_regs(const DevView& v, int m, int
       if (lb) {
         if (j == yi) yl = lq;
       } else {
-        ycat += -q * (v.dyn->s.log_prior[j] - lq);
+        ycat += -q * (v.member(m).log_prior[j] - lq);
       }
     }
   }
@@ -802,7 +802,7 @@ __device__ __forceinline__ void clf_dlogit_row(const DevView& v, const int m, co
         g[j] = (j == yi) ? -cf[COEF_YL] / q[j] : 0.f;
       } else {
         const float ke = v.has_fprop ? v.kfp_row.at(m)[l * Fl + v.ebase.at(m)[i] + j] : 0.f;
-        g[j] = cf[COEF_KLD] * (ke + logf(q[j]) - v.dyn->s.log_prior[j] + 1.f);
+        g[j] = cf[COEF_KLD] * (ke + logf(q[j]) - v.member(m).log_prior[j] + 1.f);
       }
       if (clamped) g[j] = 0.f;
       dot += q[j] * g[j];
@@ -1140,7 +1140,7 @@ __device__ __forceinline__ void clf_grad_reduce_elem(const DevView& v, const int
     float* M1 = v.adam_m.at(m);
     float* V2 = v.adam_v.at(m);
     float pv = P[idx], m1 = M1[idx], v1 = V2[idx];
-    adam_update(s, pv, m1, v1, v.dyn->s.adam);
+    adam_update(s, pv, m1, v1, v.member(m).adam);
     M1[idx] = m1;
     V2[idx] = v1;
     P[idx] = pv;
@@ -1338,8 +1338,9 @@ __device__ __forceinline__ void loss_final_model(const DevView& v, const int m) 
   const float PERT = cf[COEF_PERT_PLAIN] * a[1];
   const float KLD = cf[COEF_KLZ2] * a[2] + cf[COEF_KLD] * (a[5] + a[4]) + cf[COEF_INV_N] * a[6];
   const float YL = cf[COEF_YL_PLAIN] * a[3];
-  const float ELBO = RECL + v.dyn->s.beta_pert * v.dyn->s.pertloss_rate * PERT - KLD;
-  const float CMPL = -ELBO - v.dyn->s.yloss_rate * YL;
+  const MemberScalars& ms = v.member(m);
+  const float ELBO = RECL + v.dyn->s.beta_pert * ms.pertloss_rate * PERT - KLD;
+  const float CMPL = -ELBO - ms.yloss_rate * YL;
   float* o = v.losses.at(m);
   o[0] = RECL;
   o[1] = KLD;

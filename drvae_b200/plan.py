@@ -159,6 +159,38 @@ class Plan:
                 hp.log_prior_y[j] = math.log(float(prior_y[j])) if j < len(prior_y) else 0.0
         return hp
 
+    MEMBER_KEYS = ("yloss_rate", "pertloss_rate", "kl_qz2pz2_rate", "noise_std", "lr", "weight_decay", "prior_y")
+
+    def set_member_hparams(self, members):
+        """Per-member hyperparameters (drvae_set_member_hparams): `members` is a list of n_models dicts with the keys of
+        MEMBER_KEYS (prior_y: class probabilities, as in hparams()); these values then replace the same fields of the
+        hparams passed to every step, member by member.  None clears the table.  Takes effect from the next step
+        enqueued on the current stream."""
+        if members is None:
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.drvae_set_member_hparams(self.h, None, 0, self._stream()), "set_member_hparams")
+            return
+        members = list(members)
+        if len(members) != self.E:
+            raise ValueError("need one hyperparameter dict per member (%d), got %d" % (self.E, len(members)))
+        table = (_lib.MemberHParams * self.E)()
+        ny = max(1, self.dim_y)
+        for m, (row, d) in enumerate(zip(table, members)):
+            if set(d) != set(self.MEMBER_KEYS):
+                raise ValueError("member %d: keys must be %s, got %s" % (m, sorted(self.MEMBER_KEYS), sorted(d)))
+            for k in self.MEMBER_KEYS[:-1]:
+                x = float(d[k])
+                if not math.isfinite(x) or x < 0:
+                    raise ValueError("member %d: %s must be finite and >= 0, got %r" % (m, k, d[k]))
+                setattr(row, k, x)
+            prior = [float(p) for p in d["prior_y"]]
+            if len(prior) != ny or not all(math.isfinite(p) and p > 0 for p in prior):
+                raise ValueError("member %d: prior_y must be %d positive probabilities, got %r" % (m, ny, d["prior_y"]))
+            for j in range(8):
+                row.log_prior_y[j] = math.log(prior[j]) if j < ny else 0.0
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.drvae_set_member_hparams(self.h, table, self.E, self._stream()), "set_member_hparams")
+
     def _batch(self, x1, x2=None, y=None, has_x2=None, has_y=None, row_index=None):
         """Marshal one minibatch per model.  With row_index ([n_models, N] or [N] int32) the other fields are whole
         device-resident datasets ([n_models, D, ...]) and the minibatch is rows row_index of them — the step reads the

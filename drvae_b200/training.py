@@ -245,16 +245,45 @@ def validation_objective(model, perf):
     return perf["y_auroc"] + perf["y_aupr"] + perf["x1_pearr"]
 
 
+class SnapshotRule:
+    """The early-stopping rule of the reference's fit (DrVAE.py:822-860): the rolling mean over 3 epochs of the
+    validation objective, patience >= 50 epochs (40 for VFAE) extended to epoch + 15 at every 0.1 % improvement, a
+    snapshot at every improvement (early_stop) or once when patience runs out, and, without early_stop, training that
+    continues after patience with the patience pushed past the epoch cap.  Shared by fit() and sweep.fit_sweep()."""
+    patience_increase, improvement_threshold, memory_length = 15, 0.999, 3
+
+    def __init__(self, kind, epochs, early_stop=False, min_patience=None):
+        self.patience = min_patience if min_patience is not None else (40 if kind == "vfae" else 50)
+        self.epochs, self.early_stop = int(epochs), bool(early_stop)
+        self.best, self.rolling, self.mean = -np.inf, [], float("nan")
+        self.since_improvement, self.snapshotted = 0, False
+
+    def update(self, epoch, vobj):
+        """Record epoch `epoch`'s validation objective.  -> (snapshot, patience_reached, stop): take a snapshot now;
+        patience ran out this epoch; training stops (early_stop only)."""
+        self.since_improvement += 1
+        self.rolling = (self.rolling + [vobj])[-self.memory_length:]
+        self.mean = float(np.mean(self.rolling))
+        self.best_before = self.best
+        if self.mean * self.improvement_threshold > self.best:
+            self.patience = max(self.patience, epoch + self.patience_increase)
+            self.best, self.since_improvement = self.mean, 0
+        snapshot = (self.early_stop and self.since_improvement == 0) or (self.patience <= epoch and not self.snapshotted)
+        if snapshot:
+            self.snapshotted = True
+        reached = self.patience <= epoch
+        if reached and not self.early_stop:
+            self.patience, self.snapshotted = self.epochs + 1, False
+        return snapshot, reached, reached and self.early_stop
+
+
 def fit(model, train_loader, valid_loader, add_noise=False, verbose=False, early_stop=False, model_filename="best_model.pth",
         min_patience=None):
     """Train `model` (reference `fit`): epochs of run_on_batch(train_mode=True) over train_loader, evaluation of
     the full train / validation sets every epoch, early stopping on the rolling mean (3 rounds) of the validation
     objective with patience >= 50 epochs (40 for VFAE), extended by 15 epochs at every 0.1 % improvement, and a
-    state_dict snapshot at the best epoch."""
-    patience = min_patience if min_patience is not None else (40 if model.kind == "vfae" else 50)
-    patience_increase, improvement_threshold, memory_length = 15, 0.999, 3
-    best, rolling = -np.inf, []
-    since_improvement, snapshotted = 0, False
+    state_dict snapshot at the best epoch (SnapshotRule)."""
+    rule = SnapshotRule(model.kind, model.epochs, early_stop, min_patience)
     fields = train_loader.dataset.fields
     model.w2log("Starting training at: {}".format(time.strftime("%c")))
     epoch = 0
@@ -280,27 +309,20 @@ def fit(model, train_loader, valid_loader, add_noise=False, verbose=False, early
             vperf, vstr = evaluate_performance_on_dataset(model, valid_loader.dataset)
             vobj = validation_objective(model, vperf)
             model.w2log("Valid: sec/epoch: {:.2f}\tValid set loss: {:9.4f}\t{}".format(time.time() - t0, vobj, vstr))
-            since_improvement += 1
-            rolling = (rolling + [vobj])[-memory_length:]
-            cur = float(np.mean(rolling))
-            model.w2log("Valid rolling mem: {}\tmean: {:.4f}\tbest: {:.4f}".format(np.array(rolling), cur, best))
-            if cur * improvement_threshold > best:
-                patience = max(patience, epoch + patience_increase)
-                best, since_improvement = cur, 0
-            if (early_stop and since_improvement == 0) or (patience <= epoch and not snapshotted):
-                snapshotted = True
+            snapshot, reached, stop = rule.update(epoch, vobj)
+            model.w2log("Valid rolling mem: {}\tmean: {:.4f}\tbest: {:.4f}".format(np.array(rule.rolling), rule.mean, rule.best_before))
+            if snapshot:
                 model.save_to_file(model_filename)
                 model.w2log("* Snapshotting at epoch {}".format(epoch))
-            if patience <= epoch:
+            if reached:
                 model.w2log("Early stopping at: {} with train: {:.4f} valid: {:.4f} best_valid_obj: {:.4f}".format(
-                    epoch, train_loss, vobj, best))
-                if early_stop:
+                    epoch, train_loss, vobj, rule.best))
+                if stop:
                     break
                 model.w2log("Continuing")
-                patience, snapshotted = model.epochs + 1, False
     except KeyboardInterrupt:
         model.w2log("KeyboardInterrupt")
-        if not snapshotted:
+        if not rule.snapshotted:
             model.save_to_file(model_filename)
             model.w2log("* Snapshotting at epoch {}".format(epoch))
     model.w2log("Finished training at: {}".format(time.strftime("%c")))

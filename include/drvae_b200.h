@@ -101,6 +101,17 @@ typedef struct {
   const long long* global_counts_dev;
 } drvae_hparams_t;
 
+/* Per-member hyperparameters of an ensemble (heterogeneous ensembles: a learning-rate x loss-rate x fold grid in one
+ * plan).  With a table set, these fields of member m replace the same fields of drvae_hparams_t for that member;
+ * everything else (step, training, add_noise, beta_pert, kl_min, Adam betas and epsilon, global counts) still comes from
+ * drvae_hparams_t.  log_prior_y as in drvae_hparams_t. */
+typedef struct {
+  float yloss_rate, pertloss_rate, kl_qz2pz2_rate;
+  float noise_std;
+  float lr, weight_decay;
+  float log_prior_y[8];
+} drvae_member_hparams_t;
+
 /* Layout of the row-indexed eps block (floats, per model; Ncap = max_batch):
  *   x1   [Ncap][dim_x]            input noise of x1 rows
  *   x2   [Ncap][dim_x]            input noise of x2 rows (indexed by the row of the pair)
@@ -152,6 +163,15 @@ int drvae_loss_forward(drvae_plan_t* plan, const drvae_batch_t* batch, const drv
 int drvae_grad_step(drvae_plan_t* plan, const drvae_batch_t* batch, const drvae_noise_t* noise,
                     const drvae_hparams_t* hp, float* losses_out, void* stream);
 int drvae_adam_step(drvae_plan_t* plan, const drvae_hparams_t* hp, void* stream);
+
+/* Member table.  members: HOST array of n_models entries, or NULL with count 0 to clear the table.  Stream-ordered:
+ * the table is copied to the plan's device copy on `stream` and takes effect from the next step enqueued on `stream`,
+ * including graph replays (replacing one table by another keeps captured graphs; setting or clearing one drops them).
+ * Each step expands the table into per-member Adam and loss scalars on the device, so a member's update is
+ * bit-identical to that of a table-less plan whose drvae_hparams_t carries the member's values.  Errors: a count other
+ * than n_models or 0, a non-finite value, a negative rate, lr or noise_std, and a plan with drvae_dp_attach done
+ * (either order: drvae_dp_attach also refuses a plan with a table). */
+int drvae_set_member_hparams(drvae_plan_t* plan, const drvae_member_hparams_t* members, int count, void* stream);
 
 /* Gradient buckets for data-parallel overlap.  drvae_grad_step completes the flat gradient in
  * contiguous ranges ("buckets", one per network block, reported here in completion order) and
