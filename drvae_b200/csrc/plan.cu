@@ -413,7 +413,7 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
   if (a->dim_x < 1 || a->dim_z1 < 1 || a->L < 1 || a->max_batch < 1) return set_error("drvae_plan_create: bad dimensions");
   if (a->dim_z1 > 32 * MAXJ) return set_error("drvae_plan_create: dim_z1 > 256 is not supported");
   if (a->kind != DRVAE_KIND_PVAE && (a->dim_y < 2 || a->dim_y > MAXY)) return set_error("drvae_plan_create: dim_y must be in [2, 8]");
-  if (a->kind != DRVAE_KIND_PVAE && (a->dim_z3 < 1 || a->dim_z3 > 32 * MAXJ)) return set_error("drvae_plan_create: bad dim_z3");
+  if (a->kind != DRVAE_KIND_PVAE && (a->dim_z3 < 1 || a->dim_z3 > 32 * MAXJ)) return set_error("drvae_plan_create: dim_z3 must be in [1, 256]");
   if (a->n_enc_z1 < 1 || a->n_enc_z1 > DRVAE_MAX_HIDDEN || a->n_dec_x < 1 || a->n_dec_x > DRVAE_MAX_HIDDEN)
     return set_error("drvae_plan_create: enc_z1 / dec_x need between 1 and 4 hidden layers");
   if (a->kind != DRVAE_KIND_PVAE &&

@@ -477,6 +477,17 @@ __device__ __forceinline__ void sample_q1_row(const DevView& v, const int m, con
       }
       n1[k] = z;  // (kept for the classifier below)
     }
+    // features past the register slots (dim_z1 near 32 J): only constant columns, the ones column and the one-hot
+    // class columns, can lie there
+    for (int f = 32 * J + lane; f < v.Zc; f += 32) {
+      const float z = (f == v.Z) ? 1.f : 0.f;
+      st_c8(zdec, v.Zdec.rcap, r, f, z);
+      if (p >= 0) st_c8(zdec, v.Zdec.rcap, LN + l * Np + p, f, z);
+      for (int jj = 0; jj < ecnt; ++jj) {
+        const int cls = ecnt == 1 ? ycl : jj;
+        st_c8(z1e, v.Z1e.rcap, l * Fl + eb + jj, f, (f == v.Z + 1 + cls) ? 1.f : z);
+      }
+    }
     if (v.has_clf && !v.has_T) classifier_row_regs<J>(v, m, r, i, lane, n1, n1, false);
   }
   if (v.kind == KIND_PVAE) {  // KL(q1 || N(0,I)) and KL(q2 || N(0,I)) with free bits (PVAE.py:330-372)
@@ -555,6 +566,8 @@ __device__ __forceinline__ void T_post_row(const DevView& v, const int m, const 
       if (p >= 0) st_c8(zdec, v.Zdec.rcap, LN + LNp + l * Np + p, f, z2f);
       a_ef[k] = z2f;  // (kept for the classifier below)
     }
+    if (p >= 0)  // constant columns past the register slots (see sample_q1_row)
+      for (int f = 32 * J + lane; f < v.Zc; f += 32) st_c8(zdec, v.Zdec.rcap, LN + LNp + l * Np + p, f, (f == v.Z) ? 1.f : 0.f);
     kl = warp_sum(kl);
     if (lane == 0) v.klz2_row.at(m)[r] = q2 ? fmaxf(kl, v.dyn->s.kl_min) : 0.f;
     if (v.has_clf && !v.clf_split) classifier_row_regs<J>(v, m, r, i, lane, a_z1, a_ef, v.clf_in > v.Z);
@@ -635,6 +648,8 @@ __device__ __forceinline__ void z3_post_row(const DevView& v, const int m, const
     }
     st_c8(z3b, v.Z3b.rcap, e, f, z);
   }
+  for (int f = 32 * J + lane; f < v.Z3c; f += 32)  // constant columns past the register slots (see sample_q1_row)
+    st_c8(z3b, v.Z3b.rcap, e, f, (f == v.Z3 || f == v.Z3 + 1 + cls) ? 1.f : 0.f);
   kl = warp_sum(kl);
   if (lane == 0) v.kfp_row.at(m)[e] = fmaxf(kl, v.dyn->s.kl_min);
 }

@@ -23,6 +23,11 @@ import this module.  The product (drvae_b200/) never does.
 `emulate_bf16=True` reproduces the rounding points of the CUDA path (GEMM operands and stored
 activations / pre-activation gradients rounded to bf16, fp32 accumulation) so that kernel logic
 can be checked at a much tighter tolerance than the bf16-vs-fp32 budget of 1e-3.
+
+`OracleModel(..., dtype=torch.float64)` runs the same restatement in float64: parameters, Adam state, batch and tape
+draws are cast on entry.  With `emulate_bf16=True` that keeps the kernels' bf16 rounding points and makes every other
+operation (accumulation, transcendentals, reductions) exact to fp32 precision, so what is left of a difference is the
+kernel's own fp32 arithmetic.  float32 (the default) is what tests/golden pins.
 """
 from collections import OrderedDict
 
@@ -62,7 +67,7 @@ class Tape:
 # bf16 emulation of the CUDA path's rounding points
 # ------------------------------------------------------------------------------------------------
 def rb(t):
-    return t.to(torch.bfloat16).to(torch.float32)
+    return t.to(torch.bfloat16).to(t.dtype)
 
 
 class _LinearBF16(torch.autograd.Function):
@@ -169,7 +174,10 @@ def gauss_lv(ops, sd, prefix, x, yhot=None):
 
 def gauss_linear(ops, sd, prefix, z):
     """DiagGaussianModuleLinear (blocks.py:349-361): mu = z + z W_mu^T + bias_mu."""
-    mu = z + ops.lin(z, sd[prefix + ".W_mu"], None) + sd[prefix + ".bias_mu"]
+    if ops.emu:  # the CUDA path treats bias_mu as the GEMM's bias: its gradient sums the bf16-rounded output gradient
+        mu = z + ops.lin(z, sd[prefix + ".W_mu"], sd[prefix + ".bias_mu"])
+    else:
+        mu = z + ops.lin(z, sd[prefix + ".W_mu"], None) + sd[prefix + ".bias_mu"]
     lv = ops.lin(z, sd[prefix + ".encoder_lv.linear_lv.weight"], sd[prefix + ".encoder_lv.linear_lv.bias"]) - 2.0
     return mu, lv
 
@@ -211,8 +219,8 @@ def logn_sigma(x, mu, sg):
     return (-0.5 * torch.sum(LOG2PI + torch.log(sg ** 2) + ((x - mu) ** 2) / (sg ** 2), dim=1)).sum()  # blocks.py:234
 
 
-def one_hot(y, k):
-    return F.one_hot(y.long().view(-1), k).float()
+def one_hot(y, k, dtype=torch.float32):
+    return F.one_hot(y.long().view(-1), k).to(dtype)
 
 
 def free_bits(kl, kl_min):
@@ -241,14 +249,15 @@ def _y_terms(ops, sd, cfg, enc, z1, q1, qy, y, tape, n, L):
     YL = 0.0
     if y is not None:
         YL = torch.log(qy).gather(1, y.long().view(-1, 1)).sum() / L  # -nll_loss(log ps, y) summed
-        k = _fprop(ops, sd, cfg, enc, z1, q1, one_hot(y, dim_y), tape)
+        k = _fprop(ops, sd, cfg, enc, z1, q1, one_hot(y, dim_y, z1.dtype), tape)
     else:
         k = 0.0
         for j in range(dim_y):
-            yj = one_hot(torch.full((n,), j), dim_y)
+            yj = one_hot(torch.full((n,), j), dim_y, z1.dtype)
             k = k + qy[:, j] * _fprop(ops, sd, cfg, enc, z1, q1, yj, tape)
         prior = cfg.get("prior_y_vec")
-        pr = torch.full((n, dim_y), 1.0 / dim_y) if prior is None else torch.tensor(prior).float().expand(n, dim_y)
+        pr = (torch.full((n, dim_y), 1.0 / dim_y, dtype=qy.dtype) if prior is None
+              else torch.tensor(prior).float().to(qy.dtype).expand(n, dim_y))
         k = k + (-qy * (torch.log(pr) - torch.log(qy))).sum(1)  # blocks.py:479-480
     return YL, k.sum() / L
 
@@ -340,9 +349,26 @@ def _idx(mask):
     return torch.nonzero(mask).view(-1)
 
 
-def loss_function(sd, batch, tape, cfg, iters, train=True, emulate_bf16=False):
-    """Returns OrderedDict of 0-dim tensors with the reference's keys for cfg['kind']."""
+class _CastTape:
+    """Hands out a tape's draws in the oracle's dtype (the tape itself keeps what it drew, for the ε block)."""
+
+    def __init__(self, tape, dtype):
+        self.tape, self.dtype = tape, dtype
+
+    def draw(self, *shape):
+        return self.tape.draw(*shape).to(self.dtype)
+
+
+def _cast_batch(batch, dtype):
+    return {k: (v.to(dtype) if k in ("x1", "x2") else v) for k, v in batch.items()}
+
+
+def loss_function(sd, batch, tape, cfg, iters, train=True, emulate_bf16=False, dtype=torch.float32):
+    """Returns OrderedDict of 0-dim tensors with the reference's keys for cfg['kind'].  `dtype` is the arithmetic
+    type: `sd` must hold it; the batch and the tape draws are cast to it."""
     ops = Ops(emulate_bf16)
+    batch = _cast_batch(batch, dtype)
+    tape = _CastTape(tape, dtype)
     cfg = dict(cfg)
     cfg["noisy"] = bool(cfg["noisy"] and train)  # noise only when self.training and self.add_noise
     kind = cfg["kind"]
@@ -373,7 +399,7 @@ def loss_function(sd, batch, tape, cfg, iters, train=True, emulate_bf16=False):
         out["KLD"] = tot["KLD"] / N
         out["PERT"] = tot["PERT"] / max(1.0, Np)
         out["YL"] = tot["YL"] / max(1.0, Nl)
-        out["MMD"] = torch.zeros(())
+        out["MMD"] = torch.zeros((), dtype=dtype)
         out["ELBO"] = out["RECL"] + beta_pert * cfg["pertloss_rate"] * out["PERT"] - out["KLD"]
         out["CMPL"] = -out["ELBO"] - cfg["yloss_rate"] * out["YL"]
     elif kind == "pvae":
@@ -391,7 +417,7 @@ def loss_function(sd, batch, tape, cfg, iters, train=True, emulate_bf16=False):
         out["RECL"] = tot["RECL"] / N
         out["KLD"] = tot["KLD"] / N
         out["PERT"] = tot["PERT"] / max(1.0, Np)
-        out["MMD"] = torch.zeros(())
+        out["MMD"] = torch.zeros((), dtype=dtype)
         out["ELBO"] = out["RECL"] + beta_pert * cfg["pertloss_rate"] * out["PERT"] - out["KLD"]
         out["CMPL"] = -out["ELBO"]
     elif kind == "vfae":
@@ -409,35 +435,38 @@ def loss_function(sd, batch, tape, cfg, iters, train=True, emulate_bf16=False):
         out["RECL"] = tot["RECL"] / N
         out["KLD"] = tot["KLD"] / N
         out["YL"] = tot["YL"] / Nl  # no max(1, .) guard in the reference (VFAE.py:443)
-        out["MMD"] = torch.zeros(())
+        out["MMD"] = torch.zeros((), dtype=dtype)
         out["ELBO"] = out["RECL"] - out["KLD"]
         out["CMPL"] = -out["ELBO"] - cfg["yloss_rate"] * out["YL"]
     else:
         raise ValueError(kind)
     for k in out:
         if not torch.is_tensor(out[k]):
-            out[k] = torch.tensor(float(out[k]))
+            out[k] = torch.tensor(float(out[k]), dtype=dtype)
     return out
 
 
 class OracleModel:
     """Parameters + torch.optim.Adam, stepping like DGMMixin.run_on_batch (DGMMixin.py:91-126)."""
 
-    def __init__(self, state_dict, cfg):
+    def __init__(self, state_dict, cfg, dtype=torch.float32):
         self.cfg = dict(cfg)
-        self.sd = OrderedDict((k, v.detach().clone().float().requires_grad_(True)) for k, v in state_dict.items())
+        self.dtype = dtype
+        self.sd = OrderedDict((k, v.detach().clone().to(dtype).requires_grad_(True)) for k, v in state_dict.items())
         self.opt = torch.optim.Adam(list(self.sd.values()), lr=cfg["lr"], weight_decay=cfg["weight_decay"])
         self.iters = 0
 
     def loss(self, batch, tape, train=False, emulate_bf16=False):
         with torch.no_grad():
-            return loss_function(self.sd, batch, tape, self.cfg, self.iters, train=train, emulate_bf16=emulate_bf16)
+            return loss_function(self.sd, batch, tape, self.cfg, self.iters, train=train, emulate_bf16=emulate_bf16,
+                                 dtype=self.dtype)
 
     def grads(self, batch, tape, emulate_bf16=False):
         """forward + backward only; returns (losses, {name: grad}) without touching the optimizer."""
         for p in self.sd.values():
             p.grad = None
-        losses = loss_function(self.sd, batch, tape, self.cfg, self.iters, train=True, emulate_bf16=emulate_bf16)
+        losses = loss_function(self.sd, batch, tape, self.cfg, self.iters, train=True, emulate_bf16=emulate_bf16,
+                               dtype=self.dtype)
         losses["CMPL"].backward()
         g = OrderedDict((k, (p.grad.detach().clone() if p.grad is not None else torch.zeros_like(p)))
                         for k, p in self.sd.items())
@@ -445,7 +474,8 @@ class OracleModel:
 
     def step(self, batch, tape, emulate_bf16=False, grad_hook=None):
         self.opt.zero_grad()
-        losses = loss_function(self.sd, batch, tape, self.cfg, self.iters, train=True, emulate_bf16=emulate_bf16)
+        losses = loss_function(self.sd, batch, tape, self.cfg, self.iters, train=True, emulate_bf16=emulate_bf16,
+                               dtype=self.dtype)
         losses["CMPL"].backward()
         if grad_hook is not None:
             grad_hook(self.sd)
@@ -460,6 +490,7 @@ class OracleModel:
     def forward(self, x1, emulate_bf16=False):
         ops = Ops(emulate_bf16)
         sd, kind = self.sd, self.cfg["kind"]
+        x1 = x1.to(self.dtype)
         with torch.no_grad():
             q1 = gauss_lv(ops, sd, "encoder_z1", x1)
             res = {"z1": q1[0], "qz1": q1}

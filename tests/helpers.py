@@ -51,3 +51,46 @@ def rel_l2(a, b):
     a = a.detach().double().cpu()
     b = b.detach().double().cpu()
     return ((a - b).norm() / (b.norm() + 1e-30)).item()
+
+
+def _worst_line(d, r, dim):
+    """Largest ||d_i|| / (||r_i|| + 0.1 ||r|| / sqrt(lines)) over the lines i of `dim` (0: rows, 1: columns)."""
+    other = 1 - dim
+    lines = r.shape[dim]
+    allowed = r.norm(dim=other) + 0.1 * r.norm() / np.sqrt(lines)
+    ratio = d.norm(dim=other) / allowed.clamp_min(1e-300)
+    i = int(ratio.argmax())
+    return float(ratio[i]), i, float(d.norm(dim=other)[i]), float(allowed[i])
+
+
+def grad_errors(got, ref):
+    """Relative L2 of the whole tensor and, per output row / input column, the worst ||got_i - ref_i|| divided by
+    (||ref_i|| + 0.1 ||ref|| / sqrt(lines)).  A vector is checked element by element (its rows have one column).
+    The floor keeps rows whose reference is near zero from failing on rounding noise."""
+    g = got.detach().double().cpu()
+    r = ref.detach().double().cpu()
+    assert g.shape == r.shape, (tuple(g.shape), tuple(r.shape))
+    out = dict(l2=((g - r).norm() / (r.norm() + 1e-300)).item())
+    if r.norm() == 0:
+        out["l2"] = 0.0 if g.norm() == 0 else float("inf")
+    d = g - r
+    if r.dim() == 1:
+        d, r = d[:, None], r[:, None]
+    out["row"] = _worst_line(d, r, 0)
+    if r.shape[1] > 1:
+        out["col"] = _worst_line(d, r, 1)
+    return out
+
+
+def assert_grad_close(got, ref, tag, tol_l2=1e-2, tol_line=3e-2):
+    """Tensor-wide relative L2 <= tol_l2, and every row and every column within tol_line of its own reference norm
+    (see grad_errors).  A fault confined to one tile, row or column of a large matrix hides in the tensor-wide norm;
+    the line checks name where it is.  Returns the errors for reporting."""
+    e = grad_errors(got, ref)
+    assert e["l2"] <= tol_l2, "%s: relative L2 %.3e > %.1e" % (tag, e["l2"], tol_l2)
+    for what in ("row", "col"):
+        if what in e:
+            ratio, i, err, allowed = e[what]
+            assert ratio <= tol_line, "%s: %s %d of %s: |got - ref| = %.4e is %.3e of its reference scale %.4e (> %.1e)" % (
+                tag, what, i, tuple(ref.shape), err, ratio, allowed, tol_line)
+    return e
