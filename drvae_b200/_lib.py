@@ -77,7 +77,7 @@ EXPORTS = ["drvae_last_error", "drvae_plan_create", "drvae_plan_destroy", "drvae
            "drvae_profile_end", "drvae_plan_num_buckets", "drvae_plan_bucket_info", "drvae_stream_wait_bucket", "drvae_set_graph", "drvae_plan_graph_replays", "drvae_debug_wait_stats",
            "drvae_push_scalars", "drvae_set_external_scalars", "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_set_chains", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
            "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_adam_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
-           "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams"]
+           "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams", "drvae_plan_create_clf"]
 
 
 def load():
@@ -93,6 +93,8 @@ def load():
     lib.drvae_last_error.restype = ctypes.c_char_p
     lib.drvae_plan_create.restype = c_int
     lib.drvae_plan_create.argtypes = [P(Arch), c_int, P(c_void_p)]
+    lib.drvae_plan_create_clf.restype = c_int
+    lib.drvae_plan_create_clf.argtypes = [P(Arch), c_int, P(c_int), c_int, P(c_void_p)]
     lib.drvae_plan_destroy.restype = c_int
     lib.drvae_plan_destroy.argtypes = [c_void_p]
     lib.drvae_plan_param_count.restype = c_ll

@@ -233,6 +233,20 @@ def class_prior(kind, args, train_ds, dim_y=2):
     return list(prior / prior.sum())
 
 
+def sweep_arch(kind, args, dim_x):
+    """Plan's shape arguments of a sweep: the single-model driver's flags, --class-y included (DrVAE / VFAE)."""
+    if kind == 'drvae':
+        arch = dict(dim_z3=args.dim_z3, enc_z3=args.enc_z3, dec_z1=args.dec_z1)
+    elif kind == 'vfae':
+        arch = dict(dim_z3=args.dim_z2, enc_z3=args.enc_z2, dec_z1=args.dec_z1)
+    else:
+        arch = dict(dim_z3=0, enc_z3=[], dec_z1=[])
+    arch.update(dim_x=dim_x, dim_y=2, dim_z1=args.dim_z1, enc_z1=args.enc_z1, dec_x=args.dec_x)
+    if kind != 'pvae':
+        arch.update(clf_hidden=list(args.class_y))
+    return arch
+
+
 def sweep_main(argv):
     from . import checkpoint
     from .sweep import evaluate_members, fit_sweep, pad_members
@@ -245,7 +259,7 @@ def sweep_main(argv):
     assert args.data_mode in ['strictC2C'], 'Unsupported data mode'
     assert args.type_y == 'discrete', 'sweep: only type-y discrete is supported'
     assert args.useMF is False, 'use of mol.features not supported'
-    assert not (args.useS or args.useMMD or getattr(args, 'class_y', [])), 'sweep: use-s, use-mmd and class-y are not supported'
+    assert not (args.useS or args.useMMD), 'sweep: use-s and use-mmd are not supported'
     grid = sweep_grid(kind, args)
     data = {}  # the single-model driver loads the data with its --rseed
     for seed in args.rseeds:
@@ -259,14 +273,7 @@ def sweep_main(argv):
                   weight_decay=0.05, prior_y=class_prior(kind, args, train_ds))
         members.append(dict(seed=seed, hparams=hp))
         datasets.append((train_ds, valid_ds))
-    dim_x = datasets[0][0].x1.shape[1]
-    if kind == 'drvae':
-        arch = dict(dim_z3=args.dim_z3, enc_z3=args.enc_z3, dec_z1=args.dec_z1)
-    elif kind == 'vfae':
-        arch = dict(dim_z3=args.dim_z2, enc_z3=args.enc_z2, dec_z1=args.dec_z1)
-    else:
-        arch = dict(dim_z3=0, enc_z3=[], dec_z1=[])
-    arch.update(dim_x=dim_x, dim_y=2, dim_z1=args.dim_z1, enc_z1=args.enc_z1, dec_x=args.dec_x)
+    arch = sweep_arch(kind, args, datasets[0][0].x1.shape[1])
     epochs = args.epochs or (300 if kind == 'drvae' else 1000)
     out = fit_sweep(kind, arch, members, datasets, batch_size=args.batch_size, L=args.L, epochs=epochs,
                     early_stop=args.stopearly, add_noise=args.train_w_noise,

@@ -89,11 +89,25 @@ __global__ void __launch_bounds__(256) linear_f32_kernel(LinF32 a) {
   }
 }
 
+// u = [z1, z2 - z1] of DrVAE in fp32, [N][ld] (the input of the classifier's hidden layers).  grid (ceil(N 2Z / 256), models)
+__global__ void __launch_bounds__(256) clf_u_f32_kernel(const float* z1, const float* z2, long long z_ms, int Z, int N, float* u,
+                                                        long long u_ms, int ld) {
+  const int m = blockIdx.y;
+  const long long k = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (k >= (long long)N * 2 * Z) return;
+  const int r = (int)(k / (2 * Z)), f = (int)(k - (long long)r * 2 * Z);
+  const float* a = z1 + m * z_ms + (long long)r * Z;
+  const float* b = z2 + m * z_ms + (long long)r * Z;
+  u[m * u_ms + (long long)r * ld + f] = f < Z ? a[f] : b[f - Z] - a[f - Z];
+}
+
 // classifier q(y | u), u = [z1, z2 - z1] (DrVAE) or z1 (VFAE), on fp32 latents; writes proba / pred.  One warp per row.
+// With hidden layers z1 is the last hidden activation (Z = its width, z2 = null).
 struct ClfF32 {
-  const float* z1;  // [N][Z]
-  const float* z2;  // [N][Z] or null
+  const float* z1;  // [N][ldz]
+  const float* z2;  // [N][ldz] or null
   long long z_ms;
+  int ldz;
   const float* W;   // [Y][ldw]
   const float* b;
   long long p_ms;
@@ -106,8 +120,8 @@ __global__ void __launch_bounds__(256) clf_f32_kernel(ClfF32 a) {
   const int m = blockIdx.y, lane = threadIdx.x & 31;
   const int r = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (r >= a.N) return;
-  const float* z1 = a.z1 + m * a.z_ms + (long long)r * a.Z;
-  const float* z2 = a.z2 ? a.z2 + m * a.z_ms + (long long)r * a.Z : nullptr;
+  const float* z1 = a.z1 + m * a.z_ms + (long long)r * a.ldz;
+  const float* z2 = a.z2 ? a.z2 + m * a.z_ms + (long long)r * a.ldz : nullptr;
   const float* W = a.W + m * a.p_ms;
   const float* B = a.b + m * a.p_ms;
   float acc[MAXY];

@@ -55,6 +55,7 @@ struct drvae_plan {
   int E;
   int X, Y, Z, Z3, L, Ncap;
   int has_pair, has_T, has_clf, has_fprop, clf_in;
+  int clf_nh = 0, clf_pin = 0;  // classifier hidden layers (dim_h_clf) and the input width of linear_p
   // parameters
   std::vector<ParamInfo> tensors;
   std::vector<Seg> segs;
@@ -74,6 +75,9 @@ struct drvae_plan {
   long long shadow_elems = 0;   // bf16 per model
   long long derived_elems = 0;  // fp32 per model
   MlpBlock enc, dec, z3b, dz1b;
+  MlpBlock clfb;  // classifier hidden layers (no head: linear_p stays an fp32 row kernel)
+  ClfView clfv{};  // ... their buffers, and the device copy the row kernels read (DevView::clf)
+  ClfView* d_clfv = nullptr;
   Shadow Tsh;
   int dec_hb = 0;
   // workspace
@@ -320,9 +324,8 @@ Shadow make_shadow(drvae_plan* pl, int ntens, const int* w_tid, const int* b_tid
   return sh;
 }
 
-// blocks.DiagGaussianModule / DiagGaussianSigmaModule: hidden MLP + two heads.
-void build_gauss_block(drvae_plan* pl, MlpBlock& blk, const std::string& prefix, int in_dim, int class_cols, int nh,
-                       const int* widths, int out_dim, bool sigma_heads) {
+// blocks.MLP: `nh` Linear + ELU layers <prefix>.nnet.model.linear{1..nh}; returns the width of the last one.
+int build_hidden(drvae_plan* pl, MlpBlock& blk, const std::string& prefix, int in_dim, int class_cols, int nh, const int* widths) {
   blk.class_aug = class_cols > 0;
   int prev = in_dim;
   for (int i = 0; i < nh; ++i) {
@@ -338,6 +341,13 @@ void build_gauss_block(drvae_plan* pl, MlpBlock& blk, const std::string& prefix,
     blk.widths.push_back(widths[i]);
     prev = widths[i];
   }
+  return prev;
+}
+
+// blocks.DiagGaussianModule / DiagGaussianSigmaModule: hidden MLP + two heads.
+void build_gauss_block(drvae_plan* pl, MlpBlock& blk, const std::string& prefix, int in_dim, int class_cols, int nh,
+                       const int* widths, int out_dim, bool sigma_heads) {
+  const int prev = build_hidden(pl, blk, prefix, in_dim, class_cols, nh, widths);
   int wt[2], bt[2], gt[2] = {-1, -1};
   const char* second = sigma_heads ? "sg" : "lv";
   const std::string heads[2] = {prefix + ".encoder_mu.linear_mu", prefix + ".encoder_" + second + ".linear_" + second};
@@ -407,6 +417,10 @@ void drop_graphs(drvae_plan* pl) {
 // plan creation
 // =============================================================================================
 extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan_t** out) {
+  return drvae_plan_create_clf(a, 0, nullptr, n_models, out);
+}
+
+extern "C" int drvae_plan_create_clf(const drvae_arch_t* a, int n_clf, const int* clf_hidden, int n_models, drvae_plan_t** out) {
   if (!a || !out) return set_error("drvae_plan_create: null argument");
   if (n_models < 1) return set_error("drvae_plan_create: n_models must be >= 1");
   if (a->kind < 0 || a->kind > 2) return set_error("drvae_plan_create: unknown model kind");
@@ -419,6 +433,13 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
   if (a->kind != DRVAE_KIND_PVAE &&
       (a->n_enc_z3 < 1 || a->n_enc_z3 > DRVAE_MAX_HIDDEN || a->n_dec_z1 < 1 || a->n_dec_z1 > DRVAE_MAX_HIDDEN))
     return set_error("drvae_plan_create: enc_z3 / dec_z1 need between 1 and 4 hidden layers");
+  if (n_clf < 0 || n_clf > DRVAE_MAX_HIDDEN) return set_error("drvae_plan_create_clf: n_clf must be in [0, 4]");
+  if (n_clf > 0 && a->kind == DRVAE_KIND_PVAE)
+    return set_error("drvae_plan_create_clf: PVAE has no classifier, n_clf must be 0");
+  if (n_clf > 0 && !clf_hidden) return set_error("drvae_plan_create_clf: clf_hidden is null");
+  for (int i = 0; i < n_clf; ++i)
+    if (clf_hidden[i] < 1 || clf_hidden[i] > DRVAE_MAX_CLF_WIDTH)
+      return set_error("drvae_plan_create_clf: classifier hidden widths must be in [1, 4096]");
 
   drvae_plan* pl = new drvae_plan();
   pl->arch = *a;
@@ -435,6 +456,8 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
   pl->has_clf = a->kind != DRVAE_KIND_PVAE;
   pl->has_fprop = a->kind != DRVAE_KIND_PVAE;
   pl->clf_in = (a->kind == DRVAE_KIND_DRVAE) ? 2 * pl->Z : pl->Z;
+  pl->clf_nh = n_clf;
+  pl->clf_pin = n_clf > 0 ? clf_hidden[n_clf - 1] : pl->clf_in;
   const int X = pl->X, Y = pl->Y, Z = pl->Z, Z3 = pl->Z3, L = pl->L, E = pl->E;
 
   // ---- parameters in the reference's state_dict order (SURVEY.md Appendix C) ----
@@ -457,7 +480,9 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
     pl->T_range[0] = r_T[0], pl->T_range[1] = r_T[1];
   }
   if (pl->has_clf) {
-    int w = add_tensor(pl, "encoder_y.decoder_p.linear_p.weight", Y, pl->clf_in);
+    // CategoricalDecoder (blocks.py:456-463): its MLP (nnet) first, then linear_p
+    build_hidden(pl, pl->clfb, "encoder_y", pl->clf_in, 0, pl->clf_nh, clf_hidden);
+    int w = add_tensor(pl, "encoder_y.decoder_p.linear_p.weight", Y, pl->clf_pin);
     int b = add_tensor(pl, "encoder_y.decoder_p.linear_p.bias", Y, 0);
     pl->clf_w_off = pl->tensors[w].off;
     pl->clf_b_off = pl->tensors[b].off;
@@ -473,7 +498,7 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
         r.w_off = pl->clf_w_off + n * pl->tensors[w].ld;
         r.g_idx = pl->tensors[g].off + n;
         r.ld = pl->tensors[w].ld;
-        r.len = r.kin = pl->clf_in;
+        r.len = r.kin = pl->clf_pin;
         r.sh_off = -1;
         r.aux_off = pl->clf_eff_off + (long long)n * pl->tensors[w].ld;
         pl->wn_rows.push_back(r);
@@ -558,7 +583,7 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
   BufRec r_dZdec = F32("dZdec", (size_t)Rdcap * Z), r_dZ1T = F32("dZ1T", (size_t)LNcap * Z);
   BufRec r_DZ1 = F32("DZ1", (size_t)LNcap * Z), r_DZ2F = F32("DZ2F", (size_t)LNcap * Z);
   BufRec r_dlogit = F32("dlogit", (size_t)LNcap * Y);
-  BufRec r_clfp = F32("clf_part", (size_t)CLF_SPLITS_MAX * Y * (pl->clf_in + 1));
+  BufRec r_clfp = F32("clf_part", (size_t)CLF_SPLITS_MAX * Y * (std::max(pl->clf_in, pl->clf_pin) + 1));
   BufRec r_lossp = F32("loss_part", (size_t)LOSS_SLICES_MAX * 8);
   BufRec r_losses = F32("losses", 8);
   // per-block activations
@@ -567,7 +592,8 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
     const char* nm;
     int rcap;
   };
-  BlkAlloc blks[4] = {{&pl->enc, "enc", R0cap}, {&pl->dec, "dec", Rdcap}, {&pl->z3b, "z3", Fcap}, {&pl->dz1b, "dz1", Fcap}};
+  BlkAlloc blks[5] = {{&pl->enc, "enc", R0cap}, {&pl->dec, "dec", Rdcap}, {&pl->z3b, "z3", Fcap}, {&pl->dz1b, "dz1", Fcap},
+                      {&pl->clfb, "clf", LNcap}};
   std::vector<std::pair<C8Buf*, BufRec>> pend;
   for (auto& ba : blks) {
     ba.b->H.resize(ba.b->hidden.size());
@@ -577,6 +603,14 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
       pend.push_back({&ba.b->H[i], C8(std::string(ba.nm) + ".H" + std::to_string(i), ba.rcap, fcap)});
       pend.push_back({&ba.b->dPre[i], C8(std::string(ba.nm) + ".dPre" + std::to_string(i), ba.rcap, fcap)});
     }
+  }
+  // classifier hidden layers: DrVAE's operand u = [z1 | z2f - z1 | 1] and the fp32 gradient of u (VFAE: u is the z1
+  // rows of Zdec, its gradient goes straight to DZ1)
+  BufRec r_U{}, r_dU{};
+  const bool own_u = pl->clf_nh > 0 && a->kind == DRVAE_KIND_DRVAE;
+  if (own_u) {
+    r_U = C8("clf.U", LNcap, round_up(pl->clf_in + 1, 16));
+    r_dU = F32("clf.dU", (size_t)LNcap * pl->clf_in);
   }
   pl->arena_bytes = ab.total;
   cudaError_t err = cudaMalloc(&pl->arena, pl->arena_bytes);
@@ -645,7 +679,7 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
   v.Z3c = Z3c;
   v.Zs = Zs;
   v.Z3s = Z3s;
-  v.clf_ld = round_up(pl->clf_in, 4);
+  v.clf_ld = round_up(pl->clf_pin, 4);
   v.R0cap = R0cap;
   v.LNcap = LNcap;
   v.Rdcap = Rdcap;
@@ -704,6 +738,18 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
   v.losses = mbuf_of<float>(pl, r_losses);
   v.clf_w_off = pl->clf_w_off;
   v.clf_b_off = pl->clf_b_off;
+  if (pl->clf_nh > 0) {
+    ClfView& c = pl->clfv;
+    c.nh = pl->clf_nh;
+    c.pin = pl->clf_pin;
+    c.U = own_u ? c8_of(pl, r_U) : v.Zdec;
+    c.H = pl->clfb.H.back();
+    c.D = pl->clfb.dPre.back();
+    if (own_u) c.dU = mbuf_of<float>(pl, r_dU);
+    cudaMalloc(&pl->d_clfv, sizeof(ClfView));
+    cudaMemcpy(pl->d_clfv, &c, sizeof(ClfView), cudaMemcpyHostToDevice);
+    v.clf = pl->d_clfv;
+  }
   *out = pl;
   return 0;
 }
@@ -726,6 +772,7 @@ extern "C" int drvae_plan_destroy(drvae_plan_t* pl) {
   if (pl->d_stepk_bar) cudaFree(pl->d_stepk_bar);
   if (pl->d_sview) cudaFree(pl->d_sview);
   if (pl->d_member_hp) cudaFree(pl->d_member_hp);
+  if (pl->d_clfv) cudaFree(pl->d_clfv);
   if (pl->d_member) cudaFree(pl->d_member);
   if (pl->h_member_stage) cudaFreeHost(pl->h_member_stage);
   if (pl->member_ev) cudaEventDestroy(pl->member_ev);
@@ -835,6 +882,8 @@ int build_dwa(drvae_plan* pl) {
     add_block(pl->dz1b, &v.dY9, &v.Z3b, CNT_F);
   }
   if (pl->has_T) refs.push_back({&pl->Tsh, &v.dYT, &v.Zdec, CNT_LN, pl->arch.kind == DRVAE_KIND_PVAE ? CNT_NP : -1});
+  for (int i = 0; i < pl->clf_nh; ++i)
+    refs.push_back({&pl->clfb.hidden[i], &pl->clfb.dPre[i], i == 0 ? &pl->clfv.U : &pl->clfb.H[i - 1], CNT_LN, -1});
   if ((int)refs.size() > DWA_MAX_LAYERS) return 0;
   // heaviest layers first: the strided persistent grid then ends on the small ones
   std::stable_sort(refs.begin(), refs.end(), [](const Ref& a, const Ref& b) {
@@ -1236,6 +1285,13 @@ struct Exec {
       hook();
     }
     gemm_dw(dYh, b.H[n - 1], 0, b.head, dyn_which, row_bound);
+    block_bwd_hidden(b, in, in_row0, in_feat, dx_out, dx_ms, dyn_which, row_bound);
+  }
+  // backward of the hidden layers given dPre of the last one (written by the head's dX GEMM, or by a row kernel for a
+  // block without a GEMM head: the classifier)
+  void block_bwd_hidden(MlpBlock& b, const C8Buf& in, int in_row0, int in_feat, float* dx_out, long long dx_ms, int dyn_which,
+                        int row_bound) {
+    const int n = (int)b.hidden.size();
     for (int i = n - 1; i >= 0; --i) {
       const C8Buf& src = (i == 0) ? in : b.H[i - 1];
       sub = "h" + std::to_string(i);
@@ -1438,11 +1494,13 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
   ex.splitk = backward && !fused_adam && Rdb >= 2048;
   // DrVAE: the reparameterised draws of q(z1|x1) come out of the encoder-head GEMM's epilogue (no sample_q1 launch).
   // Needs both statistics of a feature in one tile (one N tile) and one model range (the device view is per step).
-  const bool fuse_sample = pl->fuse_sample && pl->has_T && pl->has_fprop && pl->has_clf && pl->enc.head.tiles_n == 1 &&
+  // (classifier hidden layers: the classifier cannot run inside a row stage or an epilogue, so every fusion that computes
+  // it there is off and q(y|.) comes from its own GEMMs + logits kernel, the clf_split placement)
+  const bool fuse_sample = pl->fuse_sample && pl->has_T && pl->has_fprop && pl->has_clf && pl->clf_nh == 0 && pl->enc.head.tiles_n == 1 &&
                            pl->view.Zc <= 256 && pl->d_sview != nullptr && (pl->chains <= 1 || pl->prof_on || (backward && !fused_adam));
   if (fuse_sample) v.sview_dev = pl->d_sview;
-  v.clf_back_fused = (pl->has_T && pl->has_clf && pl->clf_in > pl->Z && (pl->sched & 32) && !(pl->sched & 2)) ? 1 : 0;
-  v.clf_split = (pl->has_T && pl->has_clf && pl->has_fprop && (pl->sched & 16)) ? 1 : 0;
+  v.clf_back_fused = (pl->has_T && pl->has_clf && pl->clf_nh == 0 && pl->clf_in > pl->Z && (pl->sched & 32) && !(pl->sched & 2)) ? 1 : 0;
+  v.clf_split = ((pl->has_T && pl->has_clf && pl->has_fprop && (pl->sched & 16)) || pl->clf_nh > 0) ? 1 : 0;
   ex.defer_dw = backward && fused_adam && pl->dwa_ok && pl->dwa_enabled;
   if (ex.splitk) {
     cudaError_t e0 = cudaMemsetAsync(pl->grads, 0, sizeof(float) * (size_t)pl->P * E, st);
@@ -1639,18 +1697,40 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
       ex.gemm_nt(pl->dz1b.H.back(), 0, pl->dz1b.head, EPI_STORE_F32,
                  ex.epi_f32(v.PZ1.p, v.PZ1.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->dz1b.head), CNT_F, Fb);
     };
+    // the classifier's input gradient (DZ1, DZ2F): d loss / d logits and, with hidden layers, dPre of the last one
+    // (+ its zero padding rows), then their dX (+ dW) GEMMs and the split of d u into DZ1 / DZ2F
     auto clf_back = [&]() {
       ex.phase = "clf.bwd";
-      ex.row_op(SROW_CLF_BACK, "clf_back", row_items(LNb), 0,
-                [&]() { launch_k(clf_back_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
+      if (pl->clf_nh == 0)
+        ex.row_op(SROW_CLF_BACK, "clf_back", row_items(LNb), 0,
+                  [&]() { launch_k(clf_back_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
+      if (pl->clf_nh > 0) {
+        ex.row_op(SROW_CLF_BACK_H, "clf_back", row_items(round_up(LNb, 128)), 0,
+                  [&]() { launch_k(clf_back_h_kernel, rows_grid(round_up(LNb, 128)), dim3(ROW_THREADS), 0, ex.st, 2, v); });
+        const bool split_du = pl->clf_in > pl->Z;
+        float* du = split_du ? pl->clfv.dU.p : v.DZ1.p;
+        const long long du_ms = split_du ? pl->clfv.dU.ms : v.DZ1.ms;
+        // (their weight gradients stay on this stream: the classifier's gradient bucket is recorded here)
+        cudaStream_t keep_dw = ex.dw_stream;
+        ex.dw_stream = nullptr;
+        ex.block_bwd_hidden(pl->clfb, pl->clfv.U, 0, pl->clf_in, du, du_ms, CNT_LN, LNb);
+        ex.dw_stream = keep_dw;
+        if (split_du)
+          ex.row_op(SROW_CLF_DU, "clf_du", row_items(LNb), 0,
+                    [&]() { launch_k(clf_du_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
+      }
     };
     // classifier weight gradient (+ Adam in the fused step): feeds nothing but the optimizer
     auto clf_grad = [&]() {
       ex.phase = "clf.bwd";
-      ex.row_op(SROW_CLF_GRAD_PARTIAL, "clf_grad_partial", v.clf_splits, 0,
-                [&]() { launch_k(clf_grad_partial_kernel, dim3(v.clf_splits, Ec), dim3(256), 0, ex.st, 2, v); });
-      ex.row_op(SROW_CLF_GRAD_REDUCE, "clf_grad_reduce", row_items(pl->Y * (pl->clf_in + 1)), 0, [&]() {
-        launch_k(clf_grad_reduce_kernel, dim3(cdiv(pl->Y * (pl->clf_in + 1), 8), Ec), dim3(256), 0, ex.st, 2, v);
+      if (pl->clf_nh == 0)
+        ex.row_op(SROW_CLF_GRAD_PARTIAL, "clf_grad_partial", v.clf_splits, 0,
+                  [&]() { launch_k(clf_grad_partial_kernel, dim3(v.clf_splits, Ec), dim3(256), 0, ex.st, 2, v); });
+      else  // linear_p over the last hidden activation
+        ex.row_op(SROW_CLF_GRAD_PARTIAL_H, "clf_grad_partial", v.clf_splits, 0,
+                  [&]() { launch_k(clf_grad_partial_h_kernel, dim3(v.clf_splits, Ec), dim3(256), 0, ex.st, 2, v); });
+      ex.row_op(SROW_CLF_GRAD_REDUCE, "clf_grad_reduce", row_items(pl->Y * (pl->clf_pin + 1)), 0, [&]() {
+        launch_k(clf_grad_reduce_kernel, dim3(cdiv(pl->Y * (pl->clf_pin + 1), 8), Ec), dim3(256), 0, ex.st, 2, v);
       });
     };
     auto clf_bwd = [&]() {
@@ -1677,6 +1757,13 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
       on(side);
       if (v.clf_split) {
         ex.phase = "T.fwd";
+        if (pl->clf_nh > 0) {
+          ex.phase = "clf.fwd";
+          if (pl->clf_in > pl->Z)  // DrVAE: u = [z1 | z2f - z1 | 1] (VFAE reads the z1 rows of Zdec)
+            ex.row_op(SROW_CLF_U, "clf_u", row_items(LNb), 0,
+                      [&]() { launch_k(clf_u_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
+          ex.block_hidden_fwd(pl->clfb, pl->clfv.U, 0, CNT_LN, LNb);
+        }
         ex.row_op(SROW_CLF_FWD, "clf_fwd", row_items(LNb), 0,
                   [&]() { launch_k(clf_fwd_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
       }
@@ -2240,8 +2327,9 @@ namespace {
 int run_infer_fp32(drvae_plan* pl, const float* x1, int N, const drvae_infer_out_t* out, cudaStream_t st) {
   const int E = pl->E, X = pl->X, Z = pl->Z, Y = pl->Y;
   int maxw = Z;
-  for (const MlpBlock* b : {&pl->enc, &pl->dec})
+  for (const MlpBlock* b : {&pl->enc, &pl->dec, &pl->clfb})
     for (int w : b->widths) maxw = std::max(maxw, w);
+  if (pl->clf_nh > 0) maxw = std::max(maxw, pl->clf_in);  // u = [z1, z2 - z1] is staged in an activation buffer
   // scratch per model: two activation buffers [N][maxw], z1 / z2 / one spare [N][Z]
   const size_t per = (size_t)pl->Ncap * (2 * (size_t)maxw + 3 * (size_t)Z);
   if (pl->f32ws_floats < per * E) {
@@ -2301,9 +2389,24 @@ int run_infer_fp32(drvae_plan* pl, const float* x1, int N, const drvae_infer_out
   if (pl->has_clf && (out->proba || out->pred)) {
     if (pl->has_T && z2_ms != z1_ms) return set_error("drvae_infer: z1_mu and z2_mu must both be given or both be null");
     ClfF32 c{};
-    c.z1 = z1, c.z2 = pl->has_T ? z2 : nullptr, c.z_ms = z1_ms;
+    c.z1 = z1, c.z2 = pl->has_T ? z2 : nullptr, c.z_ms = z1_ms, c.ldz = Z;
+    if (pl->clf_nh > 0) {
+      // u in fp32 (DrVAE: [z1, z2 - z1] materialised, VFAE: z1 itself), the hidden layers, then linear_p on the last
+      const float* u = z1;
+      long long u_ms = z1_ms;
+      int u_ld = Z;
+      if (pl->has_T) {
+        clf_u_f32_kernel<<<dim3(cdiv(N * 2 * Z, 256), E), 256, 0, st>>>(z1, z2, z1_ms, Z, N, Ha, ws_ms, maxw);
+        pl->launches++;
+        if (lerr == cudaSuccess) lerr = cudaGetLastError();
+        u = Ha, u_ms = ws_ms, u_ld = maxw;
+      }
+      hidden(pl->clfb, u, u_ms, u_ld, h, h_ms, h_ld);
+      c.z1 = h, c.z2 = nullptr, c.z_ms = h_ms, c.ldz = h_ld;
+    }
     c.W = pl->params + pl->clf_w_off, c.b = pl->params + pl->clf_b_off, c.p_ms = pl->P;
-    c.ldw = pl->view.clf_ld, c.Z = Z, c.Y = Y, c.N = N;
+    c.ldw = pl->view.clf_ld, c.Y = Y, c.N = N;
+    c.Z = pl->clf_nh > 0 ? pl->clf_pin : Z;  // features per input half (DrVAE without hidden layers: z1 and z2 - z1)
     c.proba = out->proba, c.pred = out->pred;
     clf_f32_kernel<<<dim3(cdiv(N, 8), E), 256, 0, st>>>(c);
     pl->launches++;
@@ -2386,6 +2489,13 @@ extern "C" int drvae_infer(drvae_plan_t* pl, const float* x1, int N, const drvae
     ex.gemm_nt(v.Zdec, 0, pl->Tsh, EPI_STORE_F32, ex.epi_f32(v.PT.p, v.PT.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->Tsh), CNT_LN, N);
     ex.pre("infer_z2");
     infer_z2_kernel<<<rows_grid(N), ROW_THREADS, 0, st>>>(v, o);
+    ex.chk();
+  }
+  if (pl->clf_nh > 0 && (out->proba || out->pred)) {
+    // classifier hidden layers over u (written by infer_z2 / the z1 rows of Zdec), then the logits row kernel
+    ex.block_hidden_fwd(pl->clfb, pl->clfv.U, 0, CNT_LN, N);
+    ex.pre("infer_clf");
+    clf_h_infer_kernel<<<rows_grid(N), ROW_THREADS, 0, st>>>(v, o);
     ex.chk();
   }
   if (out->px1_mu || out->px2_mu) {

@@ -101,6 +101,17 @@ struct WnRow {
   int aux_ld;
 };
 
+// The classifier's hidden layers (dim_h_clf): u -> [Linear -> ELU] x nh -> linear_p.  Kept in device memory behind one
+// pointer of the row kernels' view, which the plans without them do not read.
+struct ClfView {
+  int nh;
+  int pin;        // input width of linear_p: the last hidden width
+  C8Buf U;        // u with its ones column as the first hidden GEMM's operand ([z1 | z2f - z1 | 1] rows of DrVAE, written by
+                  // clf_u_kernel; VFAE reads the z1 rows of Zdec)
+  C8Buf H, D;     // last hidden activation (read by the logits row kernel) and its pre-activation gradient
+  MBuf<float> dU; // DrVAE: [LNcap][clf_in] gradient of u, split into DZ1 / DZ2F by clf_du_kernel
+};
+
 struct MlpBlock {
   std::vector<Shadow> hidden;   // hidden[i]: layer i (ELU)
   Shadow head;                  // stacked (mu | lv) or interleaved (mu, sg) heads
@@ -231,6 +242,7 @@ struct DevView {
   SampleView* sview_dev;  // device copy of the sampling epilogue's view (written by rowmap_kernel; null: not used)
   unsigned long long* trace;  // kernel trace buffer (null: off) and this launch's slot
   int trace_id;
+  const ClfView* clf;  // classifier hidden layers (device memory); null: linear_p reads u itself
 };
 
 constexpr int CLF_SPLITS = 32;       // row splits of the classifier weight gradient (ensemble-sized batches)

@@ -280,25 +280,10 @@ __global__ void __launch_bounds__(PREP_THREADS) prep_kernel(DevView v) {
 // ---------------------------------------------------------------------------------------------
 // classifier q(y | u): u = [z1, z2f - z1] (DrVAE) or z1 (VFAE).  Warp-cooperative, fp32.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void classifier_row(const DevView& v, int m, int r, int i, int lane) {
-  const float* Wc = v.clf_w.at(m);
+// The classifier's output stage: acc[j] holds lane-partial logits (bias not yet added).  Shuffle-tree sum, softmax,
+// clamp (blocks.py:462), then q(y|.) and the row's label terms.
+__device__ __forceinline__ void classifier_tail(const DevView& v, int m, int r, int i, int lane, float (&acc)[MAXY]) {
   const float* bc = v.params.at(m) + v.clf_b_off;
-  const float* z1 = v.Z1f.at(m) + (long long)r * v.Z;
-  const float* z2f = (v.clf_in > v.Z) ? v.Z2Ff.at(m) + (long long)r * v.Z : nullptr;
-  float acc[MAXY];
-#pragma unroll
-  for (int j = 0; j < MAXY; ++j) acc[j] = 0.f;
-  for (int f = lane; f < v.Z; f += 32) {
-    const float a = z1[f];
-    const float d = z2f ? z2f[f] - a : 0.f;
-#pragma unroll
-    for (int j = 0; j < MAXY; ++j) {
-      if (j < v.Y) {
-        acc[j] = fmaf(Wc[j * v.clf_ld + f], a, acc[j]);
-        if (z2f) acc[j] = fmaf(Wc[j * v.clf_ld + v.Z + f], d, acc[j]);
-      }
-    }
-  }
   float mx = -INFINITY;
 #pragma unroll
   for (int j = 0; j < MAXY; ++j) {
@@ -338,6 +323,27 @@ __device__ __forceinline__ void classifier_row(const DevView& v, int m, int r, i
   }
 }
 
+__device__ __forceinline__ void classifier_row(const DevView& v, int m, int r, int i, int lane) {
+  const float* Wc = v.clf_w.at(m);
+  const float* z1 = v.Z1f.at(m) + (long long)r * v.Z;
+  const float* z2f = (v.clf_in > v.Z) ? v.Z2Ff.at(m) + (long long)r * v.Z : nullptr;
+  float acc[MAXY];
+#pragma unroll
+  for (int j = 0; j < MAXY; ++j) acc[j] = 0.f;
+  for (int f = lane; f < v.Z; f += 32) {
+    const float a = z1[f];
+    const float d = z2f ? z2f[f] - a : 0.f;
+#pragma unroll
+    for (int j = 0; j < MAXY; ++j) {
+      if (j < v.Y) {
+        acc[j] = fmaf(Wc[j * v.clf_ld + f], a, acc[j]);
+        if (z2f) acc[j] = fmaf(Wc[j * v.clf_ld + v.Z + f], d, acc[j]);
+      }
+    }
+  }
+  classifier_tail(v, m, r, i, lane, acc);
+}
+
 // The same classifier with its input taken from registers: feature f = lane + 32 k of z1 (and of z2f when the
 // classifier sees [z1, z2f - z1]).  Same accumulation order as classifier_row (k ascending per lane, then the shuffle
 // tree), so both give bit-identical results; this form has no global round trip for the row the caller has just
@@ -346,9 +352,6 @@ template <int J>
 __device__ __forceinline__ void classifier_row_regs(const DevView& v, int m, int r, int i, int lane, const float (&z1)[J],
                                                     const float (&z2f)[J], bool two) {
   const float* Wc = v.clf_w.at(m);
-  const float* bc = v.params.at(m) + v.clf_b_off;
-  const bool lb = v.lab.at(m)[i] != 0;
-  const int yi = v.ycls.at(m)[i];
   float acc[MAXY];
 #pragma unroll
   for (int j = 0; j < MAXY; ++j) acc[j] = 0.f;
@@ -367,41 +370,32 @@ __device__ __forceinline__ void classifier_row_regs(const DevView& v, int m, int
       }
     }
   }
-  float mx = -INFINITY;
+  classifier_tail(v, m, r, i, lane, acc);
+}
+
+// The classifier with hidden layers: linear_p (fp32 weights) over the last hidden activation of stacked row r (bf16
+// chunk8, ClfView::pin features); lane l takes the 8-feature chunks l, l + 32, ...
+__device__ __forceinline__ void classifier_row_h(const DevView& v, int m, int r, int i, int lane) {
+  const ClfView& cv = *v.clf;
+  const float* Wc = v.clf_w.at(m);
+  const uint4* hp = reinterpret_cast<const uint4*>(cv.H.at(m)) + r;
+  float acc[MAXY];
 #pragma unroll
-  for (int j = 0; j < MAXY; ++j) {
-    if (j < v.Y) {
-      acc[j] = warp_sum(acc[j]) + bc[j];
-      mx = fmaxf(mx, acc[j]);
-    }
-  }
-  float den = 0.f;
+  for (int j = 0; j < MAXY; ++j) acc[j] = 0.f;
+  for (int c = lane; c < (cv.pin + 7) >> 3; c += 32) {
+    float h[8];
+    unpack_bf16x8(hp[(long long)c * cv.H.rcap], h);
 #pragma unroll
-  for (int j = 0; j < MAXY; ++j) {
-    if (j < v.Y) {
-      acc[j] = expf(acc[j] - mx);
-      den += acc[j];
-    }
-  }
-  float yl = 0.f, ycat = 0.f;
+    for (int e = 0; e < 8; ++e) {
+      const int f = 8 * c + e;
+      if (f < cv.pin) {
 #pragma unroll
-  for (int j = 0; j < MAXY; ++j) {
-    if (j < v.Y) {
-      float q = acc[j] / den;
-      q = fminf(fmaxf(q, 1e-10f), 1.f - 1e-10f);
-      if (lane == 0) v.QY.at(m)[(long long)r * v.Y + j] = q;
-      const float lq = logf(q);
-      if (lb) {
-        if (j == yi) yl = lq;
-      } else {
-        ycat += -q * (v.member(m).log_prior[j] - lq);
+        for (int j = 0; j < MAXY; ++j)
+          if (j < v.Y) acc[j] = fmaf(Wc[j * v.clf_ld + f], h[e], acc[j]);
       }
     }
   }
-  if (lane == 0) {
-    v.yl_row.at(m)[r] = yl;
-    v.ycat_row.at(m)[r] = ycat;
-  }
+  classifier_tail(v, m, r, i, lane, acc);
 }
 
 __device__ __forceinline__ float kl_prior_term(float mu, float lv) { return 0.5f * (-lv - 1.f + mu * mu + expf(lv)); }
@@ -488,7 +482,7 @@ __device__ __forceinline__ void sample_q1_row(const DevView& v, const int m, con
         st_c8(z1e, v.Z1e.rcap, l * Fl + eb + jj, f, (f == v.Z + 1 + cls) ? 1.f : z);
       }
     }
-    if (v.has_clf && !v.has_T) classifier_row_regs<J>(v, m, r, i, lane, n1, n1, false);
+    if (v.has_clf && !v.has_T && !v.clf_split) classifier_row_regs<J>(v, m, r, i, lane, n1, n1, false);
   }
   if (v.kind == KIND_PVAE) {  // KL(q1 || N(0,I)) and KL(q2 || N(0,I)) with free bits (PVAE.py:330-372)
     float k1 = 0.f, k2 = 0.f;
@@ -566,6 +560,7 @@ __device__ __forceinline__ void T_post_row(const DevView& v, const int m, const 
       if (p >= 0) st_c8(zdec, v.Zdec.rcap, LN + LNp + l * Np + p, f, z2f);
       a_ef[k] = z2f;  // (kept for the classifier below)
     }
+
     if (p >= 0)  // constant columns past the register slots (see sample_q1_row)
       for (int f = 32 * J + lane; f < v.Zc; f += 32) st_c8(zdec, v.Zdec.rcap, LN + LNp + l * Np + p, f, (f == v.Z) ? 1.f : 0.f);
     kl = warp_sum(kl);
@@ -591,7 +586,10 @@ __device__ __forceinline__ void clf_fwd_row(const DevView& v, const int m, const
   const int* cnt = v.counts.at(m);
   const int N = cnt[CNT_N], LN = cnt[CNT_LN];
   if (r >= LN) return;
-  classifier_row(v, m, r, r % N, lane);
+  if (v.clf)
+    classifier_row_h(v, m, r, r % N, lane);
+  else
+    classifier_row(v, m, r, r % N, lane);
 }
 
 __global__ void __launch_bounds__(ROW_THREADS) clf_fwd_kernel(DevView v) {
@@ -599,6 +597,32 @@ __global__ void __launch_bounds__(ROW_THREADS) clf_fwd_kernel(DevView v) {
   pdl_launch_dependents();
   pdl_wait();
   clf_fwd_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+
+// clf_u (DrVAE, classifier hidden layers): the first hidden GEMM's operand u = [z1 | z2f - z1 | 1] of stacked row r, as
+// bf16 chunk8, from the fp32 samples sample_q1 / T_post have stored.  Runs next to the classifier's GEMMs, off the
+// main chain (T_post itself is the same as without hidden layers).
+__device__ __forceinline__ void clf_u_row(const DevView& v, const int m, const int r, const int lane) {
+  if (r >= v.counts.at(m)[CNT_LN]) return;
+  const C8Buf& U = v.clf->U;
+  bf16* u = U.at(m);
+  const float* z1 = v.Z1f.at(m) + (long long)r * v.Z;
+  const float* z2f = v.Z2Ff.at(m) + (long long)r * v.Z;
+  for (int f = lane; f < U.fcap; f += 32) {
+    float x = (f == 2 * v.Z) ? 1.f : 0.f;
+    if (f < v.Z)
+      x = z1[f];
+    else if (f < 2 * v.Z)
+      x = z2f[f - v.Z] - z1[f - v.Z];
+    st_c8(u, U.rcap, r, f, x);
+  }
+}
+
+__global__ void __launch_bounds__(ROW_THREADS) clf_u_kernel(DevView v) {
+  TraceScope trace_scope(v.trace, v.trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  clf_u_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -864,6 +888,67 @@ __global__ void __launch_bounds__(ROW_THREADS) clf_back_kernel(DevView v) {
   clf_back_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
+// The same with hidden layers: d loss / d logits, then dPre of the last hidden layer, (dl . W_p) * ELU'(H) as bf16
+// chunk8, with zero rows [LN, pad128(LN)) (the weight-gradient GEMMs contract over them).  The block's dX / dW GEMMs
+// and clf_du take it from there.  grid (ceil(pad128(LNcap) / ROW_WARPS), n_models)
+__device__ __forceinline__ void clf_back_h_row(const DevView& v, const int m, const int r, const int lane) {
+  const int* cnt = v.counts.at(m);
+  const int N = cnt[CNT_N], LN = cnt[CNT_LN], Fl = cnt[CNT_FL];
+  const ClfView& cv = *v.clf;
+  if (r >= LN) {
+    if (r < pad128(LN)) zero_c8_row(cv.D, m, r, lane);
+    return;
+  }
+  const int l = r / N, i = r - l * N;
+  float dl[MAXY];
+  clf_dlogit_row(v, m, r, l, i, Fl, lane, dl);
+  const float* Wc = v.clf_w.at(m);
+  const uint4* hp = reinterpret_cast<const uint4*>(cv.H.at(m)) + r;
+  uint4* dp = reinterpret_cast<uint4*>(cv.D.at(m)) + r;
+  for (int c = lane; c < (cv.D.fcap >> 3); c += 32) {
+    float h[8], d[8];
+    unpack_bf16x8(hp[(long long)c * cv.H.rcap], h);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const int f = 8 * c + e;
+      float g = 0.f;
+      if (f < cv.pin) {
+#pragma unroll
+        for (int j = 0; j < MAXY; ++j)
+          if (j < v.Y) g = fmaf(dl[j], Wc[j * v.clf_ld + f], g);
+      }
+      d[e] = f < cv.pin ? g * elu1_grad_from_out(h[e]) : 0.f;
+    }
+    dp[(long long)c * cv.D.rcap] = pack_bf16x8(d);
+  }
+}
+
+__global__ void __launch_bounds__(ROW_THREADS) clf_back_h_kernel(DevView v) {
+  TraceScope trace_scope(v.trace, v.trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  clf_back_h_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+
+// clf_du (DrVAE, hidden layers): d loss / d u = [dz1 part | dz2f part] from the first layer's dX GEMM ->
+// DZ1 = dU[:Z] - dU[Z:], DZ2F = dU[Z:] (what clf_back_row writes without hidden layers).  One warp per stacked row.
+__device__ __forceinline__ void clf_du_row(const DevView& v, const int m, const int r, const int lane) {
+  if (r >= v.counts.at(m)[CNT_LN]) return;
+  const float* du = v.clf->dU.at(m) + (long long)r * v.clf_in;
+  for (int f = lane; f < v.Z; f += 32) {
+    const float a = du[f], b = du[v.Z + f];
+    v.DZ1.at(m)[(long long)r * v.Z + f] = a - b;
+    v.DZ2F.at(m)[(long long)r * v.Z + f] = b;
+  }
+}
+
+__global__ void __launch_bounds__(ROW_THREADS) clf_du_kernel(DevView v) {
+  TraceScope trace_scope(v.trace, v.trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  clf_du_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+
 // ---------------------------------------------------------------------------------------------
 // T_back: gradient rows of the p(z2|z1) heads (dYT = [d p_mu | d p_lv]), the KL(q2||p) gradient
 // towards q2 (dQ2) and the residual / classifier contributions to d z1 (DZ1).
@@ -1099,10 +1184,35 @@ __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_QBACK) q_back_kernel(DevVi
 }
 
 // ---------------------------------------------------------------------------------------------
-// classifier weight gradient: dWc[j][t] = sum_r dlogit[r][j] * u[r][t], u = [z1, z2f - z1, 1]
+// classifier weight gradient: dWc[j][t] = sum_r dlogit[r][j] * u[r][t], u = [z1, z2f - z1, 1] (with hidden layers
+// u = [H_last, 1], the bf16 activation the logits were computed from)
 // two stages (row-split partials, then a fixed-order reduction) -> deterministic
 // ---------------------------------------------------------------------------------------------
 // (m, split): one row split of one model; thread t0 of nthreads cooperating threads
+// with hidden layers: u = [H_last, 1]
+__device__ __forceinline__ void clf_grad_partial_h_block(const DevView& v, const int m, const int split, const int t0, const int nthreads) {
+  const ClfView& cv = *v.clf;
+  const int LN = v.counts.at(m)[CNT_LN], splits = v.clf_splits, Y = v.Y;
+  const float* dlogit = v.dlogit.at(m);
+  float* part = v.clf_part.at(m);
+  const int width = cv.pin + 1;
+  for (int t = t0; t < width; t += nthreads) {
+    float acc[MAXY];
+#pragma unroll
+    for (int j = 0; j < MAXY; ++j) acc[j] = 0.f;
+    for (int r = split; r < LN; r += splits) {
+      const float u = t < cv.pin ? __bfloat162float(cv.H.at(m)[c8_index(r, t, cv.H.rcap)]) : 1.f;
+      const float* dl = dlogit + (long long)r * Y;
+#pragma unroll
+      for (int j = 0; j < MAXY; ++j)
+        if (j < Y) acc[j] = fmaf(dl[j], u, acc[j]);
+    }
+#pragma unroll
+    for (int j = 0; j < MAXY; ++j)
+      if (j < Y) part[((long long)split * Y + j) * width + t] = acc[j];
+  }
+}
+
 __device__ __forceinline__ void clf_grad_partial_block(const DevView& v, const int m, const int split, const int t0, const int nthreads) {
   const int LN = v.counts.at(m)[CNT_LN];
   const int width = v.clf_in + 1;
@@ -1136,17 +1246,25 @@ __global__ void __launch_bounds__(256) clf_grad_partial_kernel(DevView v) {
   clf_grad_partial_block(v, v.model0 + blockIdx.y, blockIdx.x, threadIdx.x, 256);
 }
 
+__global__ void __launch_bounds__(256) clf_grad_partial_h_kernel(DevView v) {
+  TraceScope trace_scope(v.trace, v.trace_id);
+  pdl_launch_dependents();
+  pdl_wait();
+  clf_grad_partial_h_block(v, v.model0 + blockIdx.y, blockIdx.x, threadIdx.x, 256);
+}
+
 // grid (ceil(Y * (clf_in + 1) / 8), n_models), block 256: one warp per gradient element, lanes over the row splits
 // (lane l sums splits l, l + 32, ... in order, then a fixed shuffle tree -> deterministic)
 __device__ __forceinline__ void clf_grad_reduce_elem(const DevView& v, const int m, const int k, const int lane) {
-  const int width = v.clf_in + 1;
+  const int pin = v.clf ? v.clf->pin : v.clf_in;  // input width of linear_p
+  const int width = pin + 1;
   if (k >= v.Y * width) return;
   const int j = k / width, t = k - j * width;
   float s = 0.f;
   for (int sp = lane; sp < v.clf_splits; sp += 32) s += v.clf_part.at(m)[((long long)sp * v.Y + j) * width + t];
   s = warp_sum(s);
   if (lane != 0) return;
-  const int idx = (t < v.clf_in) ? v.clf_w_off + j * v.clf_ld + t : v.clf_b_off + j;
+  const int idx = (t < pin) ? v.clf_w_off + j * v.clf_ld + t : v.clf_b_off + j;
   if (!v.dyn->s.fused_adam) {
     v.grads.at(m)[idx] = s;
   } else {
@@ -1234,7 +1352,7 @@ __global__ void __launch_bounds__(ROW_THREADS) infer_z1_kernel(DevView v, InferV
     }
     st_c8(zdec, v.Zdec.rcap, r, f, z);
   }
-  if (v.has_clf && !v.has_T) {
+  if (v.has_clf && !v.has_T && !v.clf) {
     __syncwarp();
     classifier_row(v, m, r, r, lane);
     __syncwarp();
@@ -1260,13 +1378,27 @@ __global__ void __launch_bounds__(ROW_THREADS) infer_z2_kernel(DevView v, InferV
       if (o.z2_lv) o.z2_lv[((long long)m * N + r) * v.Z + f] = pt[v.Zs + f];
     }
     st_c8(zdec, v.Zdec.rcap, N + r, f, z);
+    if (v.clf && f < v.Z) {  // u = [z1 | z2 - z1] for the classifier's hidden layers (clf_h_infer_kernel)
+      st_c8(v.clf->U.at(m), v.clf->U.rcap, r, f, z1[f]);
+      st_c8(v.clf->U.at(m), v.clf->U.rcap, r, v.Z + f, z - z1[f]);
+    }
   }
-  if (v.has_clf) {
+  if (v.has_clf && !v.clf) {
     __syncwarp();
     classifier_row(v, m, r, r, lane);
     __syncwarp();
     infer_emit_proba(v, o, m, r, lane);
   }
+}
+
+// classifier with hidden layers: logits from the last hidden activation (the block's GEMMs ran over u)
+__global__ void __launch_bounds__(ROW_THREADS) clf_h_infer_kernel(DevView v, InferView o) {
+  const int m = v.model0 + blockIdx.y, lane = threadIdx.x & 31;
+  const int r = blockIdx.x * ROW_WARPS + (threadIdx.x >> 5);
+  if (r >= v.N) return;
+  classifier_row_h(v, m, r, r, lane);
+  __syncwarp();
+  infer_emit_proba(v, o, m, r, lane);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -51,7 +51,11 @@ enum {
   SROW_CLF_GRAD_REDUCE,
   SROW_LOSS_PARTIAL,
   SROW_LOSS_FINAL,
-  SROW_CLF_FWD
+  SROW_CLF_FWD,
+  SROW_CLF_DU,
+  SROW_CLF_U,
+  SROW_CLF_BACK_H,
+  SROW_CLF_GRAD_PARTIAL_H
 };
 
 struct StepOp {
@@ -378,6 +382,10 @@ __global__ void __launch_bounds__(STEPK_THREADS, 1) step_kernel(const __grid_con
                 z3_back_row<MAXJ>(T.v, m, r, lane);
               break;
             case SROW_CLF_BACK: clf_back_row(T.v, m, r, lane); break;
+            case SROW_CLF_DU: clf_du_row(T.v, m, r, lane); break;
+            case SROW_CLF_U: clf_u_row(T.v, m, r, lane); break;
+            case SROW_CLF_BACK_H: clf_back_h_row(T.v, m, r, lane); break;
+            case SROW_CLF_GRAD_PARTIAL_H: clf_grad_partial_h_block(T.v, m, blk, threadIdx.x - GEMM_EPI_WARP0 * 32, GEMM_EPI_WARPS * 32); break;
             case SROW_T_BACK: 
               if (T.v.Zc <= 128)
                 T_back_row<4>(T.v, m, r, lane);

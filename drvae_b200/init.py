@@ -11,9 +11,12 @@ from collections import OrderedDict
 import torch
 
 
-def init_state_dict(kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=(), dec_z1=(), seed=12345, weight_norm=False):
+def init_state_dict(kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=(), dec_z1=(), seed=12345, weight_norm=False,
+                    clf_hidden=()):
     """weight_norm=True: every layer except decoder_z2Fz1 is a layers.WeightNormLinear, which adds a `.g`
-    vector initialised to ones without consuming random numbers (reference layers.py:17-23)."""
+    vector initialised to ones without consuming random numbers (reference layers.py:17-23).
+    clf_hidden (dim_h_clf): the classifier's MLP layers encoder_y.nnet.model.linear{i}, created before its linear_p
+    like every other block's MLP (CategoricalDecoder, blocks.py:456-463)."""
     torch.manual_seed(seed)
     sd = OrderedDict()
 
@@ -32,6 +35,13 @@ def init_state_dict(kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=()
         lin("%s.encoder_mu.linear_mu" % prefix, prev, out)
         lin("%s.encoder_%s.linear_%s" % (prefix, second, second), prev, out)
 
+    def categorical(prefix, in_dim, hidden, out):
+        prev = in_dim
+        for i, h in enumerate(hidden):
+            lin("%s.nnet.model.linear%d" % (prefix, i + 1), prev, h)
+            prev = h
+        lin(prefix + ".decoder_p.linear_p", prev, out)
+
     def gauss_linear(prefix, z):
         lin(prefix + ".encoder_lv.linear_lv", z, z, wn=False)
         sd[prefix + ".W_mu"] = torch.Tensor(z, z).uniform_(-0.0001, 0.0001)
@@ -41,11 +51,11 @@ def init_state_dict(kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=()
     if kind in ("drvae", "pvae"):
         gauss_linear("decoder_z2Fz1", dim_z1)
     if kind == "drvae":
-        lin("encoder_y.decoder_p.linear_p", 2 * dim_z1, dim_y)
+        categorical("encoder_y", 2 * dim_z1, clf_hidden, dim_y)
         gauss("encoder_z3", dim_z1 + dim_y, enc_z3, dim_z3)
         gauss("decoder_z1", dim_z3 + dim_y, dec_z1, dim_z1)
     elif kind == "vfae":
-        lin("encoder_y.decoder_p.linear_p", dim_z1, dim_y)
+        categorical("encoder_y", dim_z1, clf_hidden, dim_y)
         gauss("encoder_z2", dim_z1 + dim_y, enc_z3, dim_z3)
         gauss("decoder_z1", dim_z3 + dim_y, dec_z1, dim_z1)
     gauss("decoder_x", dim_z1, dec_x, dim_x, second="sg")

@@ -11,8 +11,8 @@ fused forward + ELBO + backward + Adam launch sequence.
 
 Options the reference advertises but that are broken as shipped (SURVEY.md §0 fact 7) or outside
 the hot path raise ValueError here instead of failing later: use_s=True, type_rec other than
-'diag_gaussian', MMD with use_s, continuous y, clf_1sig, hidden classifier layers, dropout,
-non-ELU nonlinearities, Adamax.
+'diag_gaussian', MMD with use_s, continuous y, clf_1sig, dropout, non-ELU nonlinearities, Adamax.
+The classifier's hidden layers (dim_h_clf, --class-y) are supported: ELU layers in front of linear_p.
 """
 import inspect
 import warnings
@@ -90,8 +90,6 @@ class _B200Model(nn.Module):
                 bad("type_y=%r" % (self.type_y,))
             if self.clf_1sig:
                 bad("clf_1sig")
-            if len(_as_list(self.dim_h_clf)) > 0:
-                bad("hidden classifier layers (--class-y)")
             if self.kind == 'drvae' and not self.clf_z1z2:
                 bad("clf_z1z2=False")
             if self.kind == 'vfae' and not self.semi_supervised:
@@ -105,6 +103,8 @@ class _B200Model(nn.Module):
         arch = dict(dim_x=self.dim_x, dim_y=self.dim_y, dim_z1=self.dim_z1, dim_z3=self._dim_top,
                     enc_z1=_as_list(self.dim_h_en_z1), dec_x=_as_list(self.dim_h_de_x),
                     enc_z3=self._enc_top, dec_z1=_as_list(getattr(self, 'dim_h_de_z1', [])))
+        if self.kind != 'pvae':
+            arch['clf_hidden'] = _as_list(self.dim_h_clf)
         self._arch = arch
         self.plan = Plan(self.kind, L=self.L, max_batch=max(int(self.batch_size), 1), n_models=1,
                          weight_norm=self.wn, **arch)

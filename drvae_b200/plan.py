@@ -35,7 +35,8 @@ def anneal_coef(iter_num, iter_max=1000, iter_offset=0):
 
 class Plan:
     def __init__(self, kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=(), dec_z1=(), L=1, max_batch=200,
-                 n_models=1, weight_norm=False, device=None):
+                 n_models=1, weight_norm=False, device=None, clf_hidden=()):
+        """clf_hidden: widths of the classifier's hidden ELU layers (dim_h_clf, --class-y), DrVAE / VFAE only."""
         if not torch.cuda.is_available():
             raise RuntimeError("drvae_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = _lib.load()
@@ -53,6 +54,10 @@ class Plan:
             arr = getattr(a, name)
             for i, h in enumerate(lst):
                 arr[i] = h
+        clf_hidden = [int(h) for h in clf_hidden]
+        if len(clf_hidden) > _lib.MAX_HIDDEN:
+            raise ValueError("at most %d classifier hidden layers are supported" % _lib.MAX_HIDDEN)
+        self.clf_hidden = tuple(clf_hidden)
         a.weight_norm = int(bool(weight_norm))
         a.L = int(L)
         a.max_batch = int(max_batch)
@@ -61,7 +66,9 @@ class Plan:
         self.dim_x, self.dim_y, self.dim_z1, self.dim_z3 = a.dim_x, a.dim_y, a.dim_z1, a.dim_z3
         h = ctypes.c_void_p()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.drvae_plan_create(ctypes.byref(a), self.E, ctypes.byref(h)), "plan_create")
+            widths = (ctypes.c_int * max(1, len(clf_hidden)))(*clf_hidden)
+            _lib.check(self.lib.drvae_plan_create_clf(ctypes.byref(a), len(clf_hidden), widths, self.E, ctypes.byref(h)),
+                       "plan_create")
         self.h = h
         self.P = int(self.lib.drvae_plan_param_count(h))
         self.tensors = []

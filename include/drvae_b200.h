@@ -33,13 +33,15 @@ extern "C" {
 #define DRVAE_KIND_PVAE 1
 #define DRVAE_KIND_VFAE 2
 #define DRVAE_MAX_HIDDEN 4
+#define DRVAE_MAX_CLF_WIDTH 4096
 
 typedef struct drvae_plan drvae_plan_t;
 
 /* Architecture = constructor arguments of the reference classes that shape tensors
  * (DrVAE.py:45-70, PVAE.py:45-63, VFAE.py:42-60) with the run_*.py fixed choices:
  * type_rec='diag_gaussian', nonlinearity='elu', type_y='discrete', clf_z1z2=True,
- * use_s=False, use_MMD=False, dropout 0, batch norm off, dim_h_clf=[]. */
+ * use_s=False, use_MMD=False, dropout 0, batch norm off.  The classifier's hidden layers (dim_h_clf, --class-y)
+ * are an argument of drvae_plan_create_clf; drvae_plan_create builds the classifier without them. */
 typedef struct {
   int kind;                /* DRVAE_KIND_* */
   int dim_x, dim_y;
@@ -136,6 +138,11 @@ typedef struct {
 const char* drvae_last_error(void);
 
 int drvae_plan_create(const drvae_arch_t* arch, int n_models, drvae_plan_t** out);
+/* The same with n_clf hidden ELU layers of widths clf_hidden[0..n_clf) in front of the classifier's linear_p
+ * (CategoricalDecoder = blocks.MLP + linear_p, dim_h_clf / --class-y): n_clf in [0, DRVAE_MAX_HIDDEN], every width in
+ * [1, DRVAE_MAX_CLF_WIDTH], n_clf = 0 on a PVAE plan (it has no classifier).  n_clf = 0 is drvae_plan_create.
+ * Their tensors come before linear_p: encoder_y.nnet.model.linear{1..n_clf}.{weight, bias[, g]}. */
+int drvae_plan_create_clf(const drvae_arch_t* arch, int n_clf, const int* clf_hidden, int n_models, drvae_plan_t** out);
 int drvae_plan_destroy(drvae_plan_t* plan);
 
 /* Parameter layout: tensors in the reference's state_dict order (SURVEY.md Appendix C), each row-major at `offset`
