@@ -75,7 +75,7 @@ EXPORTS = ["drvae_last_error", "drvae_plan_create", "drvae_plan_destroy", "drvae
            "drvae_loss_forward", "drvae_grad_step", "drvae_adam_step", "drvae_infer", "drvae_set_gemm_impl",
            "drvae_plan_launch_count", "drvae_debug_buffer", "drvae_debug_gemm", "drvae_profile_begin",
            "drvae_profile_end", "drvae_plan_num_buckets", "drvae_plan_bucket_info", "drvae_stream_wait_bucket", "drvae_set_graph", "drvae_plan_graph_replays", "drvae_debug_wait_stats",
-           "drvae_push_scalars", "drvae_set_external_scalars", "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_set_chains", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
+           "drvae_push_scalars", "drvae_set_external_scalars", "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
            "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_adam_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
            "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams", "drvae_plan_create_clf"]
 
@@ -169,8 +169,6 @@ def load():
     lib.drvae_trace_begin.argtypes = [c_void_p, c_int]
     lib.drvae_trace_end.restype = c_int
     lib.drvae_trace_end.argtypes = [c_void_p, ctypes.c_char_p, c_int]
-    lib.drvae_set_chains.restype = c_int
-    lib.drvae_set_chains.argtypes = [c_void_p, c_int]
     lib.drvae_debug_side_delay.restype = c_int
     lib.drvae_debug_side_delay.argtypes = [c_void_p, c_ll]
     lib.drvae_set_gemm_impl.restype = c_int

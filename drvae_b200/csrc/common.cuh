@@ -42,36 +42,14 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return (uint32_t)__cvta_generic_to_shared(p);
 }
 
-// ---------------------------------------------------------------------------------------------
-// Programmatic dependent launch.  Every kernel of the step sequence starts with pdl_launch_dependents() (the next
-// kernel of the stream may be scheduled as soon as every CTA of this one has started) and calls pdl_wait() before
-// its first access to global memory (returns once the kernels this one depends on have completed and flushed).
-// With the launch attribute set (launch_k below) a kernel's launch latency and prologue — barrier init, TMEM
-// allocation — overlap the tail of its predecessor; without it both instructions are no-ops.  Measured and NOT
-// enabled by default (DRVAE_B200_PDL, profiles/r01_experiments.md): early-resident CTAs of the next persistent GEMM
-// take SMs from the side-stream kernels, which costs more than the hidden launch latency gains.
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-inline int& pdl_mask() {  // bit 0: GEMM kernels, bit 1: row / element kernels launched with the attribute
-  static int mask = 0;  // measured on B200 (32-model step): 1.023 ms off, 1.022 ms with bit 1, 1.055 ms with bit 0 -> off by default
-  return mask;
-}
-// Kernel launch with the programmatic-stream-serialization attribute (see above) when `pdl` (1: GEMM, 2: other kernel)
-// is enabled in pdl_mask().
+// Kernel launch that returns the launch's error status.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int pdl, Args&&... args) {
+inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (pdl & pdl_mask()) ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 

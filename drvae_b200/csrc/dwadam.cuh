@@ -229,7 +229,6 @@ __global__ void __launch_bounds__(DWA_THREADS, DWA_MIN_BLOCKS) dwadam_kernel(con
   int* bidx = reinterpret_cast<int*>(bst + 3 * 256);                         // [256] flat offset of b[n] or -1
 
   TraceScope trace_scope(p.trace, p.trace_id);
-  pdl_launch_dependents();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
     for (int s = 0; s < DWA_OPS; ++s) {
@@ -257,7 +256,6 @@ __global__ void __launch_bounds__(DWA_THREADS, DWA_MIN_BLOCKS) dwadam_kernel(con
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_s;
-  pdl_wait();
   long long w_a = 0, w_b = 0;  // wait-cycle counters of this thread's role (p.stats)
   const long long cta_t0 = (STATS && p.stats) ? clock64() : 0;
 
@@ -562,8 +560,8 @@ inline cudaError_t dwadam_launch(const DwaParams& p, cudaStream_t st, int max_ct
   int grid = std::min(p.tile_end - p.tile_begin, gemm_num_sms());
   if (max_ctas > 0) grid = std::min(grid, max_ctas);
   if (grid < 1) return cudaSuccess;
-  if (p.stats) return launch_k(dwadam_kernel<true>, dim3(grid), dim3(DWA_THREADS), (size_t)DWA_SMEM, st, 1, p);
-  return launch_k(dwadam_kernel<false>, dim3(grid), dim3(DWA_THREADS), (size_t)DWA_SMEM, st, 1, p);
+  if (p.stats) return launch_k(dwadam_kernel<true>, dim3(grid), dim3(DWA_THREADS), (size_t)DWA_SMEM, st, p);
+  return launch_k(dwadam_kernel<false>, dim3(grid), dim3(DWA_THREADS), (size_t)DWA_SMEM, st, p);
 }
 
 }  // namespace drvae

@@ -44,10 +44,8 @@ enum {
   EPI_DECLOSS = 4,    // decoder heads: Gaussian log-density partials + d loss / d pre-activation
   EPI_DECOUT = 5,     // decoder heads at inference: mu and sigma as fp32 row-major
   EPI_LIN_C8 = 6,     // +bias -> bf16 chunk8 (no activation)
-  EPI_GRAD_ADAM = 7,  // as EPI_GRAD, but the gradient never leaves the SM: fused Adam update of p, m, v
+  EPI_GRAD_ADAM = 7   // as EPI_GRAD, but the gradient never leaves the SM: fused Adam update of p, m, v
                       // and refresh of the bf16 weight shadow / derived bias in the same epilogue
-  EPI_SAMPLE_Q1 = 8   // encoder heads of DrVAE: (mu | logvar) -> fp32 statistics AND the reparameterised draws z1 / z2 of every MC
-                      // sample, written straight to the decoder / evaluation operand rows (no sample_q1 launch)
 };
 
 constexpr int GEMM_BM = 128;
@@ -102,34 +100,13 @@ struct GemmProblem {
   int tiles_m;
   int nstages;
   int ksplit;       // >1: contraction split into ksplit tiles (EPI_GRAD accumulates atomically)
-  int n_models;     // models of this launch ...
-  int model0;       // ... starting at this ensemble member
+  int n_models;     // models of this launch
   int ens;          // ensemble members the operand buffers hold (extent of the tensor maps); 0: n_models
   int desc_variant; // debug knob for descriptor bring-up (0 = designed encoding)
   int max_ctas;     // > 0: cap on the persistent grid (the step reserves SMs for a concurrent launch)
   DebugWord* dbg;
   unsigned long long* trace;  // kernel trace (common.cuh TraceScope)
   int trace_id;
-};
-
-// What the sampling epilogue (EPI_SAMPLE_Q1) needs of the step's device view: written to device memory by
-// rowmap_kernel, the first kernel of every sequence, so that the GEMM parameter block only carries a pointer.
-struct SampleView {
-  int Z, Zs, Zc, L, Ncap, Y;
-  const int* counts;
-  int counts_stride;
-  const int *pair_of, *ebase, *lab, *ycls;
-  long long pair_ms, ebase_ms, lab_ms, ycls_ms;
-  const float *eps_z1, *eps_z2;
-  long long eps_z1_ms, eps_z2_ms;
-  float* Z1f;
-  long long z1f_ms;
-  bf16* zdec;
-  long long zdec_ms;
-  int zdec_rcap;
-  bf16* z1e;
-  long long z1e_ms;
-  int z1e_rcap;
 };
 
 struct EpiParams {
@@ -200,8 +177,6 @@ struct EpiParams {
   long long part_ms;
   int part_rcap;
   int write_dy;  // 0 in eval mode (loss only)
-  // EPI_SAMPLE_Q1
-  const SampleView* sview;  // device memory
 };
 
 // Offsets inside the per-model counts / coefficient blocks (written by rowmap_kernel).
@@ -549,90 +524,6 @@ __device__ __forceinline__ void epi_end(const EpiParams& e, RowCtx& rc, int tile
 }
 
 // ---------------------------------------------------------------------------------------------
-// EPI_SAMPLE_Q1.  The thread holds the (mu | logvar) pre-activations of features [c, c + 16) of encoder row `rc.row`.
-// Reference: blocks.py:170-174 (z = eps * exp(0.5 logvar) + mu), DrVAE.py:420-428 (z1 and z2 both drawn from q(z1|x1)).
-// Rows < N are x1 rows: for every MC sample l the draws go to Z1f (fp32), to decoder operand row l N + i (and
-// LN + l Np + p for the z2 of a pair) and to the evaluation-ordered rows of q(z_top | z1, y) with their one-hot class
-// column; feature Z is the ones column.  Same arithmetic as sample_q1_row (rowops.cuh): bit-identical results.
-// Rows >= N (x2 rows of pairs) only leave their statistics in Q.  Rows of tile 0 also zero the padding rows of Z1e.
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void epi_sample_chunk(const EpiParams& e, const RowCtx& rc, int c, bool in_stats, float (&mu)[16], float (&lv)[16]) {
-  const SampleView& v = *e.sview;
-  const int m = rc.model, i = rc.row;
-  const int* cnt = v.counts + (long long)m * v.counts_stride;
-  const int N = cnt[CNT_N], Np = cnt[CNT_NP], LN = cnt[CNT_LN], Fl = cnt[CNT_FL], F = cnt[CNT_F];
-  if (in_stats) {
-    const float* b = e.bias + m * e.bias_ms;
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 bm = *reinterpret_cast<const float4*>(b + c + j);
-      const float4 bl = *reinterpret_cast<const float4*>(b + v.Zs + c + j);
-      mu[j] += bm.x, mu[j + 1] += bm.y, mu[j + 2] += bm.z, mu[j + 3] += bm.w;
-      lv[j] += bl.x, lv[j + 1] += bl.y, lv[j + 2] += bl.z, lv[j + 3] += bl.w;
-    }
-    if (rc.valid) {
-      float* q = e.out_f32 + m * e.out_f32_ms + (long long)i * e.out_ld;
-#pragma unroll
-      for (int j = 0; j < 16; j += 4) {
-        *reinterpret_cast<float4*>(q + c + j) = make_float4(mu[j], mu[j + 1], mu[j + 2], mu[j + 3]);
-        *reinterpret_cast<float4*>(q + v.Zs + c + j) = make_float4(lv[j], lv[j + 1], lv[j + 2], lv[j + 3]);
-      }
-    }
-  }
-  const int a0 = c >> 3;           // chunk8 atoms of this feature chunk: a0, a0 + 1
-  const int natoms = v.Zc >> 3;
-  uint4* zdec = reinterpret_cast<uint4*>(v.zdec + m * v.zdec_ms);
-  uint4* z1e = reinterpret_cast<uint4*>(v.z1e + m * v.z1e_ms);
-  // padding rows of the evaluation operand (what sample_q1's pad-duty warps did): rows [F, pad128(F))
-  if (i < 128 && F + i < ((F + 127) & ~127)) {
-    const uint4 z = make_uint4(0, 0, 0, 0);
-    if (a0 < natoms) z1e[(long long)a0 * v.z1e_rcap + F + i] = z;
-    if (a0 + 1 < natoms) z1e[(long long)(a0 + 1) * v.z1e_rcap + F + i] = z;
-  }
-  if (!rc.valid || i >= N) return;
-  const int p = v.pair_of[(long long)m * v.pair_ms + i];
-  const int eb = v.ebase[(long long)m * v.ebase_ms + i];
-  const int ecnt = v.lab[(long long)m * v.lab_ms + i] ? 1 : v.Y;
-  const int ycl = v.ycls[(long long)m * v.ycls_ms + i];
-  float sd[16];
-#pragma unroll
-  for (int j = 0; j < 16; ++j) sd[j] = (in_stats && c + j < v.Z) ? expf(0.5f * lv[j]) : 0.f;
-  for (int l = 0; l < v.L; ++l) {
-    const int r = l * N + i;
-    const float* e1 = v.eps_z1 + m * v.eps_z1_ms + ((long long)l * v.Ncap + i) * v.Z;
-    const float* e2 = v.eps_z2 + m * v.eps_z2_ms + ((long long)l * v.Ncap + i) * v.Z;
-    float* z1f = v.Z1f + m * v.z1f_ms + (long long)r * v.Z;
-#pragma unroll
-    for (int hh = 0; hh < 2; ++hh) {  // two atoms of 8 features
-      const int a = a0 + hh;
-      if (a >= natoms) continue;
-      float z[8], z2[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int f = c + hh * 8 + j;
-        const int k = hh * 8 + j;
-        z[j] = (f == v.Z) ? 1.f : 0.f;  // ones column (bias gradients); class columns are set per evaluation below
-        z2[j] = z[j];
-        if (f < v.Z) {
-          z[j] = mu[k] + sd[k] * e1[f];
-          z1f[f] = z[j];
-          if (p >= 0) z2[j] = mu[k] + sd[k] * e2[f];
-        }
-      }
-      zdec[(long long)a * v.zdec_rcap + r] = pack_bf16x8(z);
-      if (p >= 0) zdec[(long long)a * v.zdec_rcap + LN + l * Np + p] = pack_bf16x8(z2);
-      for (int jj = 0; jj < ecnt; ++jj) {
-        const int cls = ecnt == 1 ? ycl : jj;
-        float ze[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) ze[j] = (c + hh * 8 + j == v.Z + 1 + cls) ? 1.f : z[j];
-        z1e[(long long)a * v.z1e_rcap + l * Fl + eb + jj] = pack_bf16x8(ze);
-      }
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
 // Tile geometry shared by both kernels
 // ---------------------------------------------------------------------------------------------
 struct TileInfo {
@@ -650,7 +541,7 @@ __device__ __forceinline__ TileInfo gemm_tile_info(const GemmProblem& p, int til
   const int mn = tile % tiles_mn;
   const int rest = tile / tiles_mn;
   const int ks = rest % p.ksplit;
-  t.model = p.model0 + rest / p.ksplit;
+  t.model = rest / p.ksplit;
   if (p.mode == GEMM_DW) {
     // weight-gradient tiles: consecutive tiles (running at the same time on neighbouring SMs) take
     // consecutive 128-feature segments of the SAME reference-weight rows
@@ -684,21 +575,7 @@ template <int EPI>
 __device__ __forceinline__ void run_epilogue_row(const GemmProblem& p, const EpiParams& e, const TileInfo& t, RowCtx& rc,
                                                  uint32_t taddr_row, bool have_acc, bool atomic) {
   epi_begin<EPI>(e, rc);
-  if (EPI == EPI_SAMPLE_Q1) {
-    const int Zs = e.sview->Zs;
-    const int cmax = max(Zs, e.sview->Zc);
-    for (int c = rc.cg * 16; c < cmax; c += 16 * EPI_GROUPS) {
-      float am[16], as[16];
-      const bool in_stats = c < Zs;
-      if (have_acc && in_stats) {
-        tmem_ld16x2(taddr_row + c, taddr_row + Zs + c, am, as);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) am[i] = as[i] = 0.f;
-      }
-      epi_sample_chunk(e, rc, c, in_stats, am, as);
-    }
-  } else if (EPI == EPI_DECLOSS || EPI == EPI_DECOUT) {
+  if (EPI == EPI_DECLOSS || EPI == EPI_DECOUT) {
     const int hb = p.BN >> 1;
     for (int c = rc.cg * 16; c < hb; c += 16 * EPI_GROUPS) {
       float am[16], as[16];
@@ -1061,7 +938,6 @@ __global__ void __launch_bounds__((GEMM_PROD_WARPS + 1 + EW) * 32, 1) gemm_tc_ke
   __shared__ uint32_t tmem_base_s;
 
   TraceScope trace_scope(p.trace, p.trace_id);
-  pdl_launch_dependents();
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int BN = p.BN;
@@ -1093,7 +969,6 @@ __global__ void __launch_bounds__((GEMM_PROD_WARPS + 1 + EW) * 32, 1) gemm_tc_ke
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_s;
-  pdl_wait();  // everything above (barriers, TMEM) overlapped the previous kernel's tail; global memory from here on
 #ifdef GEMM_PROFILE_WAITS
   const long long ws_cta_t0 = clock64();
 #endif
@@ -1337,21 +1212,7 @@ __global__ void __launch_bounds__(GEMM_SIMT_THREADS) gemm_simt_kernel(const Gemm
       }
     }
   };
-  if (EPI == EPI_SAMPLE_Q1) {
-    const int Zs = e.sview->Zs;
-    const int cmax = max(Zs, e.sview->Zc);
-    for (int c = rc.cg * 16; c < cmax; c += 16 * EPI_GROUPS) {
-      float am[16], as[16];
-      const bool in_stats = c < Zs;
-#pragma unroll
-      for (int i = 0; i < 16; ++i) am[i] = as[i] = 0.f;
-      if (in_stats) {
-        dot16(t.n0 + c, am);
-        dot16(t.n0 + Zs + c, as);
-      }
-      epi_sample_chunk(e, rc, c, in_stats, am, as);
-    }
-  } else if (EPI == EPI_DECLOSS || EPI == EPI_DECOUT) {
+  if (EPI == EPI_DECLOSS || EPI == EPI_DECOUT) {
     const int hb = p.BN >> 1;
     for (int c = rc.cg * 16; c < hb; c += 16 * EPI_GROUPS) {
       float am[16], as[16];
@@ -1493,7 +1354,7 @@ inline cudaError_t gemm_launch_t(GemmProblem p, const EpiParams& e, int n_models
   if (err != cudaSuccess) return err;
   int grid = total < gemm_num_sms() ? total : gemm_num_sms();  // persistent: one CTA per SM
   if (p.max_ctas > 0 && grid > p.max_ctas) grid = p.max_ctas;
-  return launch_k(gemm_tc_kernel<EPI, EW, VEC>, dim3(grid), dim3((GEMM_PROD_WARPS + 1 + EW) * 32), smem, st, 1, p, e, tmA, tmB, tmB2);
+  return launch_k(gemm_tc_kernel<EPI, EW, VEC>, dim3(grid), dim3((GEMM_PROD_WARPS + 1 + EW) * 32), smem, st, p, e, tmA, tmB, tmB2);
 }
 
 inline cudaError_t gemm_launch(int epi, const GemmProblem& p, const EpiParams& e, int n_models, int impl,
@@ -1509,7 +1370,6 @@ inline cudaError_t gemm_launch(int epi, const GemmProblem& p, const EpiParams& e
       return gemm_launch_t<EPI_GRAD_ADAM>(p, e, n_models, impl, st);
     case EPI_DECLOSS: return gemm_launch_t<EPI_DECLOSS>(p, e, n_models, impl, st);
     case EPI_DECOUT: return gemm_launch_t<EPI_DECOUT>(p, e, n_models, impl, st);
-    case EPI_SAMPLE_Q1: return gemm_launch_t<EPI_SAMPLE_Q1>(p, e, n_models, impl, st);
   }
   return cudaErrorInvalidValue;
 }

@@ -162,8 +162,6 @@ __global__ void spin_kernel(long long cycles) {
 // member table it also expands the table into this step's per-member scalars: lr / bc1 rounds like the host's float
 // division of adam_scalars(), so a member gets exactly the update of a table-less plan run with its lr.
 __global__ void set_dyn_kernel(StepDyn value, StepDyn* dst, MemberExpand mx) {
-  pdl_launch_dependents();
-  pdl_wait();
   if (threadIdx.x == 0) {
     if (value.counts_dev) {  // batch-global normalisers left in device memory by the caller's all-reduce
       value.s.gN = (int)value.counts_dev[0];
@@ -198,15 +196,13 @@ struct EpsSegs {
   int inner[6];      // floats per row
 };
 
-__global__ void __launch_bounds__(256) philox_normal_kernel(MBuf<float> out, EpsSegs sg, int N, int Ncap, const StepDyn* dyn, int model0,
+__global__ void __launch_bounds__(256) philox_normal_kernel(MBuf<float> out, EpsSegs sg, int N, int Ncap, const StepDyn* dyn,
                                                             unsigned long long* trace, int trace_id) {
   TraceScope trace_scope(trace, trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
   const long long row_offset = dyn->row_offset;
   const unsigned long long seed = dyn->noise_seed;
   const unsigned int step = dyn->noise_step;
-  const int m = model0 + blockIdx.y, seg = blockIdx.z;
+  const int m = blockIdx.y, seg = blockIdx.z;
   int inner = 0, outer = 0;
   long long seg_off = 0;
 #pragma unroll

@@ -62,7 +62,6 @@ struct drvae_plan {
   Seg* d_segs = nullptr;
   std::vector<int> h_tabs;  // gradient-epilogue tables of every weight (see make_shadow)
   int* d_tabs = nullptr;
-  int sched = 13;              // schedule knob (DRVAE_B200_SCHED): bit 0 = noise generator on the side stream, bit 2 = classifier weight gradient off the dX chain, bit 3 = stand-alone weight-gradient GEMMs (gradient path) on their own stream, bit 4 = DrVAE classifier forward as its own kernel on the side stream (measured: no gain, the side branch becomes the longer chain), bit 5 = classifier input gradient inside T_back (measured slower: T_back 15 -> 43-64 us), bit 1 = whole classifier backward on the side stream (measured: 1.037 / 1.027 / 1.048 / 1.048 ms for 0 / 1 / 2 / 3)
   int adam_vec_max = 4;       // debug knob (DRVAE_B200_ADAM_VEC): cap on the vector width of the fused Adam epilogue
   bool wn = false;            // layers.WeightNormLinear instead of nn.Linear
   std::vector<WnRow> wn_rows;
@@ -120,21 +119,16 @@ struct drvae_plan {
   long long graph_clock = 0;
   long long graph_replays = 0;
   long long graph_failures = 0;  // capture / instantiation failures (those combinations run as plain launches)
-  // streams of the step schedule (see run_step): per model range a main stream (range 0 uses the caller's) and a side
-  // stream for the label-dependent branch
-  static constexpr int MAX_CHAINS = 8;
-  struct Chain {
-    cudaStream_t main = nullptr, side = nullptr;
-    cudaEvent_t ev_fork = nullptr, ev_qy = nullptr, ev_side_fwd = nullptr, ev_side_bwd = nullptr, ev_begin = nullptr, ev_eps = nullptr,
-                ev_clf = nullptr, ev_kfp = nullptr, ev_end = nullptr, ev_side_end = nullptr, ev_dw = nullptr, ev_dw_end = nullptr;
-    static constexpr int N_EVENTS = 12;
-    cudaEvent_t* all() { return &ev_fork; }  // N_EVENTS consecutive events
-  };
-  Chain chain[MAX_CHAINS];
-  bool main_prio = true;      // main chain on the plan's high-priority stream (DRVAE_B200_PRIO=0: on the caller's stream)
-  int chains = 1;             // model ranges per step (DRVAE_B200_CHAINS; default chosen from n_models at creation)
-  cudaEvent_t ev_begin = nullptr;
-  bool overlap = true;
+  // streams and events of the step schedule (see run_step): the plan's high-priority main stream, the low-priority side
+  // stream of the label-dependent branch, and a low-priority stream for the early part of the grouped dW+Adam launch
+  cudaStream_t s_main = nullptr, s_side = nullptr, s_dwa = nullptr;
+  struct StepEvents {
+    cudaEvent_t begin = nullptr, fork = nullptr, qy = nullptr, side_fwd = nullptr, side_bwd = nullptr, noise = nullptr, eps = nullptr,
+                clf = nullptr, kfp = nullptr, end = nullptr, side_end = nullptr, dw = nullptr, dw_end = nullptr, dwa = nullptr,
+                dwa_end = nullptr;
+    static constexpr int N = 15;
+    cudaEvent_t* all() { return &begin; }  // N consecutive events
+  } ev;
   long long side_delay_cycles = 0;  // test knob (drvae_debug_side_delay): spin on the side stream before pz1_post
   // gradient buckets (data-parallel overlap): contiguous parameter ranges in backward completion order
   std::vector<std::pair<long long, long long>> buckets;  // (offset, count)
@@ -156,10 +150,6 @@ struct drvae_plan {
   bool stepk_enabled = false;          // drvae_set_step_kernel / DRVAE_B200_STEPK (measured slower than the graph of launches: profiles/r02_experiments.md)
   bool stepk_unsupported = false;      // a recorded sequence did not fit the kernel's tables: this plan launches kernel by kernel
   unsigned int* d_stepk_bar = nullptr; // {arrival count, generation}
-  SampleView* d_sview = nullptr;       // device view of the sampling epilogue (EPI_SAMPLE_Q1), written by rowmap_kernel
-  bool fuse_sample = false;            // DRVAE_B200_FUSE_SAMPLE=1: DrVAE's sample_q1 inside the encoder-head GEMM epilogue (bit-identical;
-                                       // measured slower: 64 tiles x 16 warps have less parallelism than one warp per row, and the whole
-                                       // GEMM then waits for the noise generator: profiles/r02_experiments.md)
   long long stepk_launches = 0;
   // data-parallel exchange over peer memory (dp_peer.cuh): attached by drvae_dp_attach
   bool dp_on = false;
@@ -622,30 +612,21 @@ extern "C" int drvae_plan_create_clf(const drvae_arch_t* a, int n_clf, const int
   cudaMalloc(&pl->d_dyn, sizeof(StepDyn));
   cudaMemset(pl->d_dyn, 0, sizeof(StepDyn));
   if (const char* knob = getenv("DRVAE_B200_ADAM_VEC")) pl->adam_vec_max = atoi(knob);  // measurement knob
-  if (const char* knob = getenv("DRVAE_B200_SCHED")) pl->sched = atoi(knob);
   if (const char* knob = getenv("DRVAE_B200_DWADAM")) pl->dwa_enabled = atoi(knob) != 0;
   if (const char* knob = getenv("DRVAE_B200_STEPK")) pl->stepk_enabled = atoi(knob) != 0;
   if (const char* knob = getenv("DRVAE_B200_DWA_EARLY_SMS")) pl->dwa_early_sms = std::max(0, atoi(knob));
-  if (const char* knob = getenv("DRVAE_B200_FUSE_SAMPLE")) pl->fuse_sample = atoi(knob) != 0;
-  cudaMalloc(&pl->d_sview, sizeof(SampleView));
-  cudaMemset(pl->d_sview, 0, sizeof(SampleView));
   cudaMalloc(&pl->d_stepk_bar, 2 * sizeof(unsigned int));
   cudaMemset(pl->d_stepk_bar, 0, 2 * sizeof(unsigned int));
-  if (const char* knob = getenv("DRVAE_B200_PDL")) pdl_mask() = atoi(knob);  // measurement knob: programmatic dependent launch
-  pl->chains = 1;  // measured (32 models): 0.970 / 1.002 / 1.020 / 1.054 ms for 1 / 2 / 4 / 8 ranges
-  if (const char* knob = getenv("DRVAE_B200_CHAINS")) pl->chains = std::max(1, atoi(knob));
-  if (const char* knob = getenv("DRVAE_B200_OVERLAP")) pl->overlap = atoi(knob) != 0;
-  if (const char* knob = getenv("DRVAE_B200_PRIO")) pl->main_prio = atoi(knob) != 0;
-  for (auto& ch : pl->chain) {
+  {
     // the main chain outranks the side branch: when both have CTAs waiting for an SM (the side stream's wide row kernels
     // vs the next GEMM of the critical path) the critical path goes first
     int prio_least = 0, prio_greatest = 0;
     cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest);
-    cudaStreamCreateWithPriority(&ch.main, cudaStreamNonBlocking, prio_greatest);
-    cudaStreamCreateWithPriority(&ch.side, cudaStreamNonBlocking, prio_least);
-    for (int i = 0; i < drvae_plan::Chain::N_EVENTS; ++i) cudaEventCreateWithFlags(ch.all() + i, cudaEventDisableTiming);
+    cudaStreamCreateWithPriority(&pl->s_main, cudaStreamNonBlocking, prio_greatest);
+    cudaStreamCreateWithPriority(&pl->s_side, cudaStreamNonBlocking, prio_least);
+    cudaStreamCreateWithPriority(&pl->s_dwa, cudaStreamNonBlocking, prio_least);
+    for (int i = 0; i < drvae_plan::StepEvents::N; ++i) cudaEventCreateWithFlags(pl->ev.all() + i, cudaEventDisableTiming);
   }
-  cudaEventCreateWithFlags(&pl->ev_begin, cudaEventDisableTiming);
   pl->bucket_ev.resize(pl->buckets.size());
   for (auto& ev : pl->bucket_ev) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
   cudaMalloc(&pl->dbg, sizeof(DebugWord));
@@ -770,20 +751,16 @@ extern "C" int drvae_plan_destroy(drvae_plan_t* pl) {
   if (pl->d_trace) cudaFree(pl->d_trace);
   if (pl->d_dwa_stats) cudaFree(pl->d_dwa_stats);
   if (pl->d_stepk_bar) cudaFree(pl->d_stepk_bar);
-  if (pl->d_sview) cudaFree(pl->d_sview);
   if (pl->d_member_hp) cudaFree(pl->d_member_hp);
   if (pl->d_clfv) cudaFree(pl->d_clfv);
   if (pl->d_member) cudaFree(pl->d_member);
   if (pl->h_member_stage) cudaFreeHost(pl->h_member_stage);
   if (pl->member_ev) cudaEventDestroy(pl->member_ev);
   for (auto& ev : pl->bucket_ev) cudaEventDestroy(ev);
-  for (auto& ch : pl->chain) {
-    for (int i = 0; i < drvae_plan::Chain::N_EVENTS; ++i)
-      if (ch.all()[i]) cudaEventDestroy(ch.all()[i]);
-    if (ch.main) cudaStreamDestroy(ch.main);
-    if (ch.side) cudaStreamDestroy(ch.side);
-  }
-  if (pl->ev_begin) cudaEventDestroy(pl->ev_begin);
+  for (int i = 0; i < drvae_plan::StepEvents::N; ++i)
+    if (pl->ev.all()[i]) cudaEventDestroy(pl->ev.all()[i]);
+  for (cudaStream_t s : {pl->s_main, pl->s_side, pl->s_dwa})
+    if (s) cudaStreamDestroy(s);
   delete pl;
   return 0;
 }
@@ -831,12 +808,6 @@ extern "C" int drvae_set_gemm_impl(drvae_plan_t* pl, int impl) {
   if (!pl || (impl != GEMM_IMPL_TC && impl != GEMM_IMPL_SIMT)) return set_error("drvae_set_gemm_impl: bad argument");
   if (pl->gemm_impl != impl) drop_graphs(pl);  // captured sequences replay the kernels of the old implementation
   pl->gemm_impl = impl;
-  return 0;
-}
-extern "C" int drvae_set_chains(drvae_plan_t* pl, int chains) {
-  if (!pl || chains < 1) return set_error("drvae_set_chains: bad argument");
-  pl->chains = std::min(chains, (int)drvae_plan::MAX_CHAINS);
-  drop_graphs(pl);
   return 0;
 }
 extern "C" int drvae_set_step_kernel(drvae_plan_t* pl, int enable) {
@@ -1017,7 +988,6 @@ struct Exec {
   std::string sub = "head";  // layer within the current block: h0, h1, ..., head
   bool fused = false;        // Adam inside the gradient epilogues (drvae_train_step)
   bool splitk = false;       // split-K weight gradients (large minibatches, unfused path)
-  int model0 = 0, Ec = 0;    // model range of the launches being enqueued (Ec = 0: the whole ensemble)
   bool defer_dw = false;     // weight gradients + Adam of every layer in ONE launch at the end of backward (dwadam.cuh)
   StepRecorder* rec = nullptr;  // non-null: launches are recorded as ops of the persistent step kernel (stepk.cuh)
   // stand-alone weight-gradient GEMMs (gradient path: they feed nothing but the optimizer / the gradient exchange) leave
@@ -1045,7 +1015,7 @@ struct Exec {
   void row_op(int kind, const char* name, int per_model, int arg, F&& real_launch) {
     if (!ok()) return;
     if (rec) {
-      rec->add_row(kind, per_model, model0, Ec > 0 ? Ec : pl->E, arg, st, std::string(phase) + ":" + name);
+      rec->add_row(kind, per_model, pl->E, arg, st, std::string(phase) + ":" + name);
       return;
     }
     pre(name);
@@ -1085,19 +1055,18 @@ struct Exec {
     p.dbg = pl->dbg;
     p.desc_variant = 0;
     if (p.ksplit < 1) p.ksplit = 1;
-    p.model0 = model0;
     p.ens = pl->E;
     p.max_ctas = cta_cap;
     if (rec) {
       p.trace = nullptr;
       p.trace_id = 0;
-      rec->add_gemm(epi, p, e, Ec > 0 ? Ec : pl->E, st, std::string(phase) + ":" + op);
+      rec->add_gemm(epi, p, e, pl->E, st, std::string(phase) + ":" + op);
       return;
     }
     pre(op);
     p.trace = v.trace;
     p.trace_id = v.trace_id;
-    cudaError_t r = gemm_launch(epi, p, e, Ec > 0 ? Ec : pl->E, pl->gemm_impl, st);
+    cudaError_t r = gemm_launch(epi, p, e, pl->E, pl->gemm_impl, st);
     post();
     if (r != cudaSuccess) err = r;
     pl->launches++;
@@ -1358,7 +1327,6 @@ int fill_view(drvae_plan* pl, Exec& ex, const drvae_batch_t* b, const drvae_nois
   v.dyn = pl->d_dyn;
   v.mem = member_base(pl);
   v.mem_stride = pl->member_table ? 1 : 0;
-  v.sview_dev = nullptr;
   v.params = MBuf<float>{pl->params, pl->P};
   v.clf_w = pl->wn ? MBuf<const float>{pl->derived.p + pl->clf_eff_off, pl->derived.ms}
                    : MBuf<const float>{pl->params + pl->clf_w_off, pl->P};
@@ -1396,7 +1364,7 @@ StepDyn make_dyn(const drvae_noise_t* nz, const drvae_hparams_t* hp, bool fused_
 int push_dyn(drvae_plan* pl, const StepDyn& d, cudaStream_t st) {
   prof_pre(pl, st, ":set_dyn");
   const MemberExpand mx = member_expand(pl);
-  launch_k(set_dyn_kernel, dim3(1), dim3(set_dyn_threads(mx)), 0, st, 2, d, pl->d_dyn, mx);
+  launch_k(set_dyn_kernel, dim3(1), dim3(set_dyn_threads(mx)), 0, st, d, pl->d_dyn, mx);
   prof_post(pl, st);
   pl->launches++;
   cudaError_t err = cudaGetLastError();
@@ -1464,11 +1432,16 @@ int run_wn_grad(drvae_plan* pl, cudaStream_t st) {
 
 // forward (+ optional backward) of one minibatch per model
 //
-// Schedule.  The ensemble is cut into `chains` contiguous model ranges; each range runs its whole forward + dX chain
-// on its own pair of streams (main + side, the side stream taking the label-dependent branch as before), so the
-// latency-bound small kernels of one range overlap those of the others.  The ranges fork from the caller's stream
-// after the per-step scalars and join before the grouped dW+Adam launch, which covers every model and layer at once.
-// Captured into a CUDA graph the forks and joins become graph edges.
+// Schedule.  One launch sequence covers every member of the ensemble.  The main chain (encoder, p(z2|z1), decoder and
+// the dX GEMMs back to the encoder) runs on the plan's high-priority stream: it forks from the caller's stream after
+// the per-step scalars and joins it again before the grouped dW+Adam launch.  What is off that chain runs on the
+// low-priority side stream: the latent-noise generator (next to the encoder GEMMs), the label-dependent branch
+// (forward and backward) and the loss reduction.  The classifier weight gradient runs on the caller's stream, idle
+// until the join, and the early part of the dW+Adam launch on a low-priority stream of its own.  Captured into a CUDA
+// graph the forks and joins become graph edges.  The main chain stays on the caller's stream under per-launch
+// profiling, under the step kernel and on the gradient path, whose bucket events the caller waits for on that stream
+// (the stand-alone weight-gradient GEMMs then take the plan's main stream); profiling and plans without the
+// label-dependent branch run on one stream.
 int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, const drvae_hparams_t* hp, float* losses_out,
              cudaStream_t st, bool backward, bool fused_adam) {
   if (!hp) return set_error("drvae: hparams is null");
@@ -1492,15 +1465,6 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
   v.clf_splits = std::max(CLF_SPLITS, std::min(CLF_SPLITS_MAX, cdiv(LNb, 64)));
   v.loss_slices = std::max(1, std::min(LOSS_SLICES_MAX, cdiv(Rdb, 512)));
   ex.splitk = backward && !fused_adam && Rdb >= 2048;
-  // DrVAE: the reparameterised draws of q(z1|x1) come out of the encoder-head GEMM's epilogue (no sample_q1 launch).
-  // Needs both statistics of a feature in one tile (one N tile) and one model range (the device view is per step).
-  // (classifier hidden layers: the classifier cannot run inside a row stage or an epilogue, so every fusion that computes
-  // it there is off and q(y|.) comes from its own GEMMs + logits kernel, the clf_split placement)
-  const bool fuse_sample = pl->fuse_sample && pl->has_T && pl->has_fprop && pl->has_clf && pl->clf_nh == 0 && pl->enc.head.tiles_n == 1 &&
-                           pl->view.Zc <= 256 && pl->d_sview != nullptr && (pl->chains <= 1 || pl->prof_on || (backward && !fused_adam));
-  if (fuse_sample) v.sview_dev = pl->d_sview;
-  v.clf_back_fused = (pl->has_T && pl->has_clf && pl->clf_nh == 0 && pl->clf_in > pl->Z && (pl->sched & 32) && !(pl->sched & 2)) ? 1 : 0;
-  v.clf_split = ((pl->has_T && pl->has_clf && pl->has_fprop && (pl->sched & 16)) || pl->clf_nh > 0) ? 1 : 0;
   ex.defer_dw = backward && fused_adam && pl->dwa_ok && pl->dwa_enabled;
   if (ex.splitk) {
     cudaError_t e0 = cudaMemsetAsync(pl->grads, 0, sizeof(float) * (size_t)pl->P * E, st);
@@ -1520,12 +1484,9 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
                          !(backward && fused_adam && !ex.defer_dw) && pl->d_stepk_bar != nullptr;
   StepRecorder recorder;
 
-  // model ranges: separate chains only where the gradient buckets are not consumed outside (drvae_grad_step records
-  // one event per bucket on ONE stream) and not under per-launch profiling
-  int K = 1;
-  if (!use_stepk && !pl->prof_on && !(backward && !fused_adam)) K = std::max(1, std::min({pl->chains, E, (int)drvae_plan::MAX_CHAINS}));
-  const bool own_main = !use_stepk && pl->main_prio && !pl->prof_on && !(backward && !fused_adam) && pl->has_fprop && pl->overlap;
-  if (K > 1 || own_main) cudaEventRecord(pl->ev_begin, st);
+  // the main chain on the plan's high-priority stream (see above)
+  const bool own_main = !use_stepk && !pl->prof_on && !(backward && !fused_adam) && pl->has_fprop;
+  if (own_main) cudaEventRecord(pl->ev.begin, st);
 
   // grouped weight-gradient + Adam launch over the tiles [t0, t1) (dwadam.cuh)
   auto launch_dwadam = [&](int t0, int t1, cudaStream_t stream, int max_ctas, const char* tag) {
@@ -1570,413 +1531,358 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
   // the chain are capped to the other SMs while it runs.
   bool dwa_early_done = false;
   const int nsm = gemm_num_sms();
-  const bool dwa_early = backward && ex.defer_dw && !use_stepk && !pl->prof_on && pl->overlap && K == 1 &&
+  const bool dwa_early = backward && ex.defer_dw && !use_stepk && !pl->prof_on &&
                          pl->dwa_early_tiles > 0 && pl->dwa_early_tiles < pl->dwa_tiles && pl->dwa_early_sms >= 8 &&
                          pl->dwa_early_sms <= nsm - 16;
 
-  for (int c = 0; c < K && ex.ok(); ++c) {
-    drvae_plan::Chain& ch = pl->chain[c];
-    const int m0 = (int)((long long)E * c / K), Ec = (int)((long long)E * (c + 1) / K) - m0;
-    // range 0 stays on the caller's stream unless the plan's own high-priority stream is used for the main chain
-    const bool forked = c > 0 || own_main;
-    cudaStream_t cm = forked ? ch.main : st;
-    if (forked) cudaStreamWaitEvent(cm, pl->ev_begin, 0);
-    v.model0 = m0;
-    ex.phase = "";
-    ex.model0 = m0;
-    ex.Ec = Ec;
-    ex.st = cm;
-    auto rows_grid = [&](int rows) { return dim3(cdiv(rows, ROW_WARPS), Ec); };
-    auto row_items = [&](int rows) { return cdiv(rows, STEPK_ROWS); };
-    // Two-stream schedule inside a range: everything that is not on the longest dependency chain runs on the range's
-    // side stream — the latent-noise generator (next to rowmap / prep / the encoder), the label-dependent branch and
-    // the loss reduction.  (While recording for the step kernel the two "streams" only define the levels.)
-    const bool overlap = pl->has_fprop && pl->overlap && !pl->prof_on;
-    cudaStream_t side = overlap ? ch.side : cm;
-    auto on = [&](cudaStream_t s) { ex.st = s; };
-    auto after = [&](cudaStream_t waiter, cudaEvent_t ev, cudaStream_t producer) {
-      if (!overlap || waiter == producer) return;
-      if (ex.rec) {
-        ex.rec->after(waiter, producer);
-        return;
-      }
-      cudaEventRecord(ev, producer);
-      cudaStreamWaitEvent(waiter, ev, 0);
-    };
-    // gradient path (stand-alone weight-gradient GEMMs inside the chain): they run on the range's otherwise unused main
-    // stream, next to the dX chain on the caller's stream
-    const bool dw_aside = backward && !fused_adam && !forked && overlap && (pl->sched & 8);
-    ex.dw_stream = dw_aside ? ch.main : nullptr;
-    ex.dw_event = ch.ev_dw;
-    if (dw_aside && !use_stepk) {
-      cudaEventRecord(ch.ev_dw, cm);  // (the split-K path zeroes the gradient buffer on the caller's stream first)
-      cudaStreamWaitEvent(ch.main, ch.ev_dw, 0);
+  ex.phase = "";
+  cudaStream_t cm = own_main ? pl->s_main : st;
+  if (own_main) cudaStreamWaitEvent(cm, pl->ev.begin, 0);
+  ex.st = cm;
+  auto rows_grid = [&](int rows) { return dim3(cdiv(rows, ROW_WARPS), E); };
+  auto row_items = [&](int rows) { return cdiv(rows, STEPK_ROWS); };
+  // (While recording for the step kernel the streams only define the levels.)
+  const bool overlap = pl->has_fprop && !pl->prof_on;
+  cudaStream_t side = overlap ? pl->s_side : cm;
+  auto on = [&](cudaStream_t s) { ex.st = s; };
+  auto after = [&](cudaStream_t waiter, cudaEvent_t ev, cudaStream_t producer) {
+    if (!overlap || waiter == producer) return;
+    if (ex.rec) {
+      ex.rec->after(waiter, producer);
+      return;
     }
-    auto launch_noise = [&]() {
-      const drvae_eps_layout_t& el = pl->epsl;
-      EpsSegs sg{};
-      const long long offs[6] = {el.off_x1, el.off_x2, el.off_z1, el.off_z2, el.off_z2f, el.off_z3};
-      const int outer[6] = {1, 1, L, L, L, L};
-      // the input noise (segments 0, 1) is drawn inside prep_kernel with the same keys
-      const int inner[6] = {0, 0, pl->Z, pl->has_pair ? pl->Z : 0, pl->has_T ? pl->Z : 0, pl->has_fprop ? pl->Y * pl->Z3 : 0};
-      long long most = 0;
-      for (int i = 0; i < 6; ++i) {
-        sg.off[i] = offs[i];
-        sg.outer[i] = outer[i];
-        sg.inner[i] = inner[i];
-        most = std::max(most, (long long)outer[i] * N * ((inner[i] + 3) / 4));
-      }
-      dim3 g((unsigned)((most + 255) / 256), Ec, 6);
-      ex.pre("philox_normal");
-      launch_k(philox_normal_kernel, g, dim3(256), 0, ex.st, 2, pl->eps_own, sg, N, pl->Ncap, pl->d_dyn, m0, v.trace, v.trace_id);
-      ex.chk();
-    };
-    // step kernel: the noise generator needs only this step's scalars, so it is forked first and overlaps rowmap / prep
-    if (use_stepk && own_eps) {
-      if (overlap) {
-        after(side, ch.ev_begin, cm);
-        on(side);
-      }
-      launch_noise();
-      on(cm);
+    cudaEventRecord(ev, producer);
+    cudaStreamWaitEvent(waiter, ev, 0);
+  };
+  // gradient path (stand-alone weight-gradient GEMMs inside the chain): they run on the plan's main stream, unused
+  // there, next to the dX chain on the caller's stream
+  const bool dw_aside = backward && !fused_adam && overlap;
+  ex.dw_stream = dw_aside ? pl->s_main : nullptr;
+  ex.dw_event = pl->ev.dw;
+  if (dw_aside && !use_stepk) {
+    cudaEventRecord(pl->ev.dw, cm);  // (the split-K path zeroes the gradient buffer on the caller's stream first)
+    cudaStreamWaitEvent(pl->s_main, pl->ev.dw, 0);
+  }
+  auto launch_noise = [&]() {
+    const drvae_eps_layout_t& el = pl->epsl;
+    EpsSegs sg{};
+    const long long offs[6] = {el.off_x1, el.off_x2, el.off_z1, el.off_z2, el.off_z2f, el.off_z3};
+    const int outer[6] = {1, 1, L, L, L, L};
+    // the input noise (segments 0, 1) is drawn inside prep_kernel with the same keys
+    const int inner[6] = {0, 0, pl->Z, pl->has_pair ? pl->Z : 0, pl->has_T ? pl->Z : 0, pl->has_fprop ? pl->Y * pl->Z3 : 0};
+    long long most = 0;
+    for (int i = 0; i < 6; ++i) {
+      sg.off[i] = offs[i];
+      sg.outer[i] = outer[i];
+      sg.inner[i] = inner[i];
+      most = std::max(most, (long long)outer[i] * N * ((inner[i] + 3) / 4));
     }
-    ex.pre("rowmap");
-    launch_k(rowmap_kernel, dim3(Ec), dim3(ROWMAP_THREADS), 0, cm, 2, v);
+    dim3 g((unsigned)((most + 255) / 256), E, 6);
+    ex.pre("philox_normal");
+    launch_k(philox_normal_kernel, g, dim3(256), 0, ex.st, pl->eps_own, sg, N, pl->Ncap, pl->d_dyn, v.trace, v.trace_id);
     ex.chk();
-    ex.pre("prep");
-    launch_k(prep_kernel, dim3(round_up(R0b, 128) / PREP_ROWS, cdiv(pl->view.Xc, PREP_SLAB), Ec), dim3(PREP_THREADS), 0, cm, 2, v);
-    ex.chk();
-    // latent noise: on the side stream, forked AFTER prep so that it fills the SMs next to the encoder GEMMs instead of
-    // running in front of prep (it is first needed by sample_q1)
-    if (own_eps && !use_stepk) {
-      if (pl->sched & 1) {
-        after(side, ch.ev_begin, cm);  // after this step's scalars (set_dyn), rowmap and prep
-        on(side);
-      }
-      launch_noise();
-      on(cm);
-    }
-    if (use_stepk) {
-      if (own_eps) after(cm, ch.ev_eps, side);  // the step kernel starts after the noise generator
-      ex.rec = &recorder;
-    }
-
-    // ---- encoder q(z1|x1), shared with q(z2|x2) (DrVAE.py:408,418) ----
-    ex.phase = "enc.fwd";
-    ex.block_hidden_fwd(pl->enc, v.Ain, 0, CNT_R0, R0b);
-    if (fuse_sample) {
-      if (own_eps && (pl->sched & 1) && !use_stepk) after(cm, ch.ev_eps, side);  // latent noise of this step
-      EpiParams es = ex.epi_f32(v.Q.p, v.Q.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->enc.head);
-      es.sview = pl->d_sview;
-      ex.sub = "head+sample";
-      ex.gemm_nt(pl->enc.H.back(), 0, pl->enc.head, EPI_SAMPLE_Q1, es, CNT_R0, R0b);
-      ex.sub = "head";
-    } else {
-      ex.gemm_nt(pl->enc.H.back(), 0, pl->enc.head, EPI_STORE_F32,
-                 ex.epi_f32(v.Q.p, v.Q.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->enc.head), CNT_R0, R0b);
-      if (own_eps && (pl->sched & 1) && !use_stepk) after(cm, ch.ev_eps, side);  // latent noise of this step
-      ex.row_op(SROW_SAMPLE_Q1, "sample_q1", row_items(N + PAD_WARPS), 0, [&]() {
-        launch_k(pl->view.Zc <= 128 ? sample_q1_kernel<4> : sample_q1_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, cm, 2, v);
-      });
-    }
-    // The label-dependent branch (q(z_top|z1,y) -> p(z1|z_top,y), forward and backward dX: small GEMMs + row kernels
-    // that leave most SMs idle) is independent of the decoder branch: side stream between a fork here and a join
-    // before the encoder backward.
-    after(side, ch.ev_fork, cm);
-
-    auto fprop_fwd_gemms = [&]() {
-      // ---- label-dependent part: q(z_top|z1,y), p(z1|z_top,y) per (row, class) evaluation ----
-      ex.phase = "z3.fwd";
-      ex.block_hidden_fwd(pl->z3b, v.Z1e, 0, CNT_F, Fb);
-      ex.gemm_nt(pl->z3b.H.back(), 0, pl->z3b.head, EPI_STORE_F32,
-                 ex.epi_f32(v.Q3.p, v.Q3.ms, 2 * pl->view.Z3s, 2 * pl->view.Z3s, &pl->z3b.head), CNT_F, Fb);
-      ex.row_op(SROW_Z3_POST, "z3_post", row_items(round_up(Fb, 128)), 0,
-                [&]() { launch_k(pl->view.Z3c <= 128 ? z3_post_kernel<4> : z3_post_kernel<MAXJ>, rows_grid(round_up(Fb, 128)), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-      ex.phase = "dz1.fwd";
-      ex.block_hidden_fwd(pl->dz1b, v.Z3b, 0, CNT_F, Fb);
-      ex.gemm_nt(pl->dz1b.H.back(), 0, pl->dz1b.head, EPI_STORE_F32,
-                 ex.epi_f32(v.PZ1.p, v.PZ1.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->dz1b.head), CNT_F, Fb);
-    };
-    // the classifier's input gradient (DZ1, DZ2F): d loss / d logits and, with hidden layers, dPre of the last one
-    // (+ its zero padding rows), then their dX (+ dW) GEMMs and the split of d u into DZ1 / DZ2F
-    auto clf_back = [&]() {
-      ex.phase = "clf.bwd";
-      if (pl->clf_nh == 0)
-        ex.row_op(SROW_CLF_BACK, "clf_back", row_items(LNb), 0,
-                  [&]() { launch_k(clf_back_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-      if (pl->clf_nh > 0) {
-        ex.row_op(SROW_CLF_BACK_H, "clf_back", row_items(round_up(LNb, 128)), 0,
-                  [&]() { launch_k(clf_back_h_kernel, rows_grid(round_up(LNb, 128)), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-        const bool split_du = pl->clf_in > pl->Z;
-        float* du = split_du ? pl->clfv.dU.p : v.DZ1.p;
-        const long long du_ms = split_du ? pl->clfv.dU.ms : v.DZ1.ms;
-        // (their weight gradients stay on this stream: the classifier's gradient bucket is recorded here)
-        cudaStream_t keep_dw = ex.dw_stream;
-        ex.dw_stream = nullptr;
-        ex.block_bwd_hidden(pl->clfb, pl->clfv.U, 0, pl->clf_in, du, du_ms, CNT_LN, LNb);
-        ex.dw_stream = keep_dw;
-        if (split_du)
-          ex.row_op(SROW_CLF_DU, "clf_du", row_items(LNb), 0,
-                    [&]() { launch_k(clf_du_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-      }
-    };
-    // classifier weight gradient (+ Adam in the fused step): feeds nothing but the optimizer
-    auto clf_grad = [&]() {
-      ex.phase = "clf.bwd";
-      if (pl->clf_nh == 0)
-        ex.row_op(SROW_CLF_GRAD_PARTIAL, "clf_grad_partial", v.clf_splits, 0,
-                  [&]() { launch_k(clf_grad_partial_kernel, dim3(v.clf_splits, Ec), dim3(256), 0, ex.st, 2, v); });
-      else  // linear_p over the last hidden activation
-        ex.row_op(SROW_CLF_GRAD_PARTIAL_H, "clf_grad_partial", v.clf_splits, 0,
-                  [&]() { launch_k(clf_grad_partial_h_kernel, dim3(v.clf_splits, Ec), dim3(256), 0, ex.st, 2, v); });
-      ex.row_op(SROW_CLF_GRAD_REDUCE, "clf_grad_reduce", row_items(pl->Y * (pl->clf_pin + 1)), 0, [&]() {
-        launch_k(clf_grad_reduce_kernel, dim3(cdiv(pl->Y * (pl->clf_pin + 1), 8), Ec), dim3(256), 0, ex.st, 2, v);
-      });
-    };
-    auto clf_bwd = [&]() {
-      clf_back();
-      clf_grad();
-    };
-    if (pl->has_fprop) {
+  };
+  // step kernel: the noise generator needs only this step's scalars, so it is forked first and overlaps rowmap / prep
+  if (use_stepk && own_eps) {
+    if (overlap) {
+      after(side, pl->ev.noise, cm);
       on(side);
-      fprop_fwd_gemms();
-      on(cm);
     }
-    // ---- p(z2|z1) ----
-    ex.phase = "T.fwd";
-    if (pl->has_T) {
-      ex.gemm_nt(v.Zdec, 0, pl->Tsh, EPI_STORE_F32, ex.epi_f32(v.PT.p, v.PT.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->Tsh), CNT_LN, LNb);
-      ex.row_op(SROW_T_POST, "T_post", row_items(N + PAD_WARPS), 0, [&]() {
-        launch_k(pl->view.Zc <= 128 ? T_post_kernel<4> : T_post_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, 2, v);
-      });
-    }
-    if (pl->has_fprop) {
-      // pz1_post weighs unlabeled evaluations by q(y|.), which the classifier (T_post or clf_fwd for DrVAE,
-      // sample_q1 for VFAE) produces
-      after(side, ch.ev_qy, cm);
-      on(side);
-      if (v.clf_split) {
-        ex.phase = "T.fwd";
-        if (pl->clf_nh > 0) {
-          ex.phase = "clf.fwd";
-          if (pl->clf_in > pl->Z)  // DrVAE: u = [z1 | z2f - z1 | 1] (VFAE reads the z1 rows of Zdec)
-            ex.row_op(SROW_CLF_U, "clf_u", row_items(LNb), 0,
-                      [&]() { launch_k(clf_u_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-          ex.block_hidden_fwd(pl->clfb, pl->clfv.U, 0, CNT_LN, LNb);
-        }
-        ex.row_op(SROW_CLF_FWD, "clf_fwd", row_items(LNb), 0,
-                  [&]() { launch_k(clf_fwd_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-      }
-      if (pl->side_delay_cycles > 0 && !ex.rec) spin_kernel<<<1, 1, 0, ex.st>>>(pl->side_delay_cycles);
-      ex.row_op(SROW_PZ1_POST, "pz1_post", row_items(round_up(Fb, 128)), 0,
-                [&]() { launch_k(pl->view.Zc <= 128 ? pz1_post_kernel<4> : pz1_post_kernel<MAXJ>, rows_grid(round_up(Fb, 128)), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-      // clf_back (main stream) reads the per-class KL terms pz1_post has just written (kfp_row)
-      if (overlap && backward && pl->has_clf && !(pl->sched & 2)) ex.ev_record(ch.ev_kfp, ex.st);
-      if (backward) {
-        if (pl->has_clf && (pl->sched & 2)) {
-          // classifier backward: needs only q(y|.) (T_post / sample_q1) and the per-class terms pz1_post has just
-          // written, so it leaves the main stream's chain; T_back / q_back wait for ev_clf
-          clf_bwd();
-          if (!ex.rec) cudaEventRecord(pl->bucket_ev[3], ex.st);  // buckets: dz1, z3 (this stream), dec, clf, ...
-          if (overlap) ex.ev_record(ch.ev_clf, ex.st);
-        }
-        if (dwa_early) ex.cta_cap = nsm - pl->dwa_early_sms;  // (they run next to the early dW+Adam launch)
-        ex.phase = "dz1.bwd";
-        ex.block_bwd(pl->dz1b, v.dY9, v.Z3b, 0, pl->Z3, v.dZ3.p, v.dZ3.ms, CNT_F, Fb);
-        if (!ex.rec) cudaEventRecord(pl->bucket_ev[0], ex.dw_stream ? ex.dw_stream : ex.st);
-        ex.row_op(SROW_Z3_BACK, "z3_back", row_items(round_up(Fb, 128)), 0,
-                  [&]() { launch_k(pl->view.Z3c <= 128 ? z3_back_kernel<4> : z3_back_kernel<MAXJ>, rows_grid(round_up(Fb, 128)), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-        ex.phase = "z3.bwd";
-        ex.block_bwd(pl->z3b, v.dY7, v.Z1e, 0, pl->Z, v.dZ1e.p, v.dZ1e.ms, CNT_F, Fb);
-        if (!ex.rec) cudaEventRecord(pl->bucket_ev[1], ex.dw_stream ? ex.dw_stream : ex.st);
-        ex.cta_cap = 0;
-        // what q_back needs from this stream; the loss reduction that follows here is joined at the end of the step only
-        if (overlap) ex.ev_record(ch.ev_side_bwd, ex.st);
-      }
-      on(cm);
-    }
-    // ---- decoder p(x|z) on the stacked rows [z1 | z2 | z2f], fused log-density + gradient ----
-    ex.phase = "dec.fwd";
-    ex.block_hidden_fwd(pl->dec, v.Zdec, 0, CNT_RD, Rdb);
-    {
-      EpiParams e = ex.epi_base();
-      e.out_c8 = pl->dY5.p;
-      e.out_c8_ms = pl->dY5.ms;
-      e.out_c8_rcap = pl->dY5.rcap;
-      e.bias = pl->derived.p + pl->dec.head.bias_off;
-      e.bias_ms = pl->derived.ms;
-      e.tgt4 = v.tgt4.p;
-      e.tgt_ms = v.tgt4.ms;
-      e.tgt_rcap = pl->view.R0cap;
-      e.X = pl->X;
-      e.Xc = pl->view.Xc;
-      e.counts = v.counts.p;
-      e.counts_stride = (int)v.counts.ms;
-      e.coefs = v.coefs.p;
-      e.coefs_stride = (int)v.coefs.ms;
-      e.L = L;
-      e.part = v.dec_part.p;
-      e.part_ms = v.dec_part.ms;
-      e.part_rcap = pl->view.Rdcap;
-      e.write_dy = backward ? 1 : 0;
-      ex.gemm_nt(pl->dec.H.back(), 0, pl->dec.head, EPI_DECLOSS, e, CNT_RD, Rdb);
-    }
-    // The loss reduction is off the backward's critical path: it runs at the tail of the side stream
-    // (after that branch's backward), once the decoder log-density partials of the main stream exist.
-    after(side, ch.ev_side_fwd, cm);
-    on(side);
-    ex.phase = "";
-    ex.row_op(SROW_LOSS_PARTIAL, "loss", v.loss_slices, v.loss_slices,
-              [&]() { launch_k(loss_partial_kernel, dim3(v.loss_slices, Ec), dim3(256), 0, ex.st, 2, v); });
-    ex.row_op(SROW_LOSS_FINAL, "loss_final", 1, 0, [&]() { launch_k(loss_final_kernel, dim3(Ec), dim3(32), 0, ex.st, 2, v); });
-    if (losses_out && ex.ok() && !ex.rec) {
-      // losses buffer per model is padded to 256 B in the arena; the caller's is dense [E][8]
-      ex.err = cudaMemcpy2DAsync(losses_out + 8 * (size_t)m0, 8 * sizeof(float), v.losses.at(m0), v.losses.ms * sizeof(float),
-                                 8 * sizeof(float), Ec, cudaMemcpyDeviceToDevice, ex.st);
-    }
-    if (overlap) ex.ev_record(ch.ev_side_end, side);  // everything the side stream does in this step
+    launch_noise();
     on(cm);
+  }
+  ex.pre("rowmap");
+  launch_k(rowmap_kernel, dim3(E), dim3(ROWMAP_THREADS), 0, cm, v);
+  ex.chk();
+  ex.pre("prep");
+  launch_k(prep_kernel, dim3(round_up(R0b, 128) / PREP_ROWS, cdiv(pl->view.Xc, PREP_SLAB), E), dim3(PREP_THREADS), 0, cm, v);
+  ex.chk();
+  // latent noise: on the side stream, forked AFTER prep so that it fills the SMs next to the encoder GEMMs instead of
+  // running in front of prep (it is first needed by sample_q1)
+  if (own_eps && !use_stepk) {
+    after(side, pl->ev.noise, cm);  // after this step's scalars (set_dyn), rowmap and prep
+    on(side);
+    launch_noise();
+    on(cm);
+  }
+  if (use_stepk) {
+    if (own_eps) after(cm, pl->ev.eps, side);  // the step kernel starts after the noise generator
+    ex.rec = &recorder;
+  }
 
-    if (backward && ex.ok()) {
-      size_t bk = pl->has_fprop ? 2 : 0;  // buckets 0, 1 (decoder_z1, encoder_z3) were recorded by the side branch
-      auto bucket_done = [&](bool weight_gemm = true) {
-        if (!ex.rec) cudaEventRecord(pl->bucket_ev[bk], (weight_gemm && ex.dw_stream) ? ex.dw_stream : ex.st);
-        ++bk;
+  // ---- encoder q(z1|x1), shared with q(z2|x2) (DrVAE.py:408,418) ----
+  ex.phase = "enc.fwd";
+  ex.block_hidden_fwd(pl->enc, v.Ain, 0, CNT_R0, R0b);
+  ex.gemm_nt(pl->enc.H.back(), 0, pl->enc.head, EPI_STORE_F32,
+             ex.epi_f32(v.Q.p, v.Q.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->enc.head), CNT_R0, R0b);
+  if (own_eps && !use_stepk) after(cm, pl->ev.eps, side);  // latent noise of this step
+  ex.row_op(SROW_SAMPLE_Q1, "sample_q1", row_items(N + PAD_WARPS), 0, [&]() {
+    launch_k(pl->view.Zc <= 128 ? sample_q1_kernel<4> : sample_q1_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, cm, v);
+  });
+  // The label-dependent branch (q(z_top|z1,y) -> p(z1|z_top,y), forward and backward dX: small GEMMs + row kernels
+  // that leave most SMs idle) is independent of the decoder branch: side stream between a fork here and a join
+  // before the encoder backward.
+  after(side, pl->ev.fork, cm);
+
+  auto fprop_fwd_gemms = [&]() {
+    // ---- label-dependent part: q(z_top|z1,y), p(z1|z_top,y) per (row, class) evaluation ----
+    ex.phase = "z3.fwd";
+    ex.block_hidden_fwd(pl->z3b, v.Z1e, 0, CNT_F, Fb);
+    ex.gemm_nt(pl->z3b.H.back(), 0, pl->z3b.head, EPI_STORE_F32,
+               ex.epi_f32(v.Q3.p, v.Q3.ms, 2 * pl->view.Z3s, 2 * pl->view.Z3s, &pl->z3b.head), CNT_F, Fb);
+    ex.row_op(SROW_Z3_POST, "z3_post", row_items(round_up(Fb, 128)), 0,
+              [&]() { launch_k(pl->view.Z3c <= 128 ? z3_post_kernel<4> : z3_post_kernel<MAXJ>, rows_grid(round_up(Fb, 128)), dim3(ROW_THREADS), 0, ex.st, v); });
+    ex.phase = "dz1.fwd";
+    ex.block_hidden_fwd(pl->dz1b, v.Z3b, 0, CNT_F, Fb);
+    ex.gemm_nt(pl->dz1b.H.back(), 0, pl->dz1b.head, EPI_STORE_F32,
+               ex.epi_f32(v.PZ1.p, v.PZ1.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->dz1b.head), CNT_F, Fb);
+  };
+  // the classifier's input gradient (DZ1, DZ2F): d loss / d logits and, with hidden layers, dPre of the last one
+  // (+ its zero padding rows), then their dX (+ dW) GEMMs and the split of d u into DZ1 / DZ2F
+  auto clf_back = [&]() {
+    ex.phase = "clf.bwd";
+    if (pl->clf_nh == 0)
+      ex.row_op(SROW_CLF_BACK, "clf_back", row_items(LNb), 0,
+                [&]() { launch_k(clf_back_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, v); });
+    if (pl->clf_nh > 0) {
+      ex.row_op(SROW_CLF_BACK_H, "clf_back", row_items(round_up(LNb, 128)), 0,
+                [&]() { launch_k(clf_back_h_kernel, rows_grid(round_up(LNb, 128)), dim3(ROW_THREADS), 0, ex.st, v); });
+      const bool split_du = pl->clf_in > pl->Z;
+      float* du = split_du ? pl->clfv.dU.p : v.DZ1.p;
+      const long long du_ms = split_du ? pl->clfv.dU.ms : v.DZ1.ms;
+      // (their weight gradients stay on this stream: the classifier's gradient bucket is recorded here)
+      cudaStream_t keep_dw = ex.dw_stream;
+      ex.dw_stream = nullptr;
+      ex.block_bwd_hidden(pl->clfb, pl->clfv.U, 0, pl->clf_in, du, du_ms, CNT_LN, LNb);
+      ex.dw_stream = keep_dw;
+      if (split_du)
+        ex.row_op(SROW_CLF_DU, "clf_du", row_items(LNb), 0,
+                  [&]() { launch_k(clf_du_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, v); });
+    }
+  };
+  // classifier weight gradient (+ Adam in the fused step): feeds nothing but the optimizer
+  auto clf_grad = [&]() {
+    ex.phase = "clf.bwd";
+    if (pl->clf_nh == 0)
+      ex.row_op(SROW_CLF_GRAD_PARTIAL, "clf_grad_partial", v.clf_splits, 0,
+                [&]() { launch_k(clf_grad_partial_kernel, dim3(v.clf_splits, E), dim3(256), 0, ex.st, v); });
+    else  // linear_p over the last hidden activation
+      ex.row_op(SROW_CLF_GRAD_PARTIAL_H, "clf_grad_partial", v.clf_splits, 0,
+                [&]() { launch_k(clf_grad_partial_h_kernel, dim3(v.clf_splits, E), dim3(256), 0, ex.st, v); });
+    ex.row_op(SROW_CLF_GRAD_REDUCE, "clf_grad_reduce", row_items(pl->Y * (pl->clf_pin + 1)), 0, [&]() {
+      launch_k(clf_grad_reduce_kernel, dim3(cdiv(pl->Y * (pl->clf_pin + 1), 8), E), dim3(256), 0, ex.st, v);
+    });
+  };
+  auto clf_bwd = [&]() {
+    clf_back();
+    clf_grad();
+  };
+  if (pl->has_fprop) {
+    on(side);
+    fprop_fwd_gemms();
+    on(cm);
+  }
+  // ---- p(z2|z1) ----
+  ex.phase = "T.fwd";
+  if (pl->has_T) {
+    ex.gemm_nt(v.Zdec, 0, pl->Tsh, EPI_STORE_F32, ex.epi_f32(v.PT.p, v.PT.ms, 2 * pl->view.Zs, 2 * pl->view.Zs, &pl->Tsh), CNT_LN, LNb);
+    ex.row_op(SROW_T_POST, "T_post", row_items(N + PAD_WARPS), 0, [&]() {
+      launch_k(pl->view.Zc <= 128 ? T_post_kernel<4> : T_post_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, v);
+    });
+  }
+  if (pl->has_fprop) {
+    // pz1_post weighs unlabeled evaluations by q(y|.), which the classifier (T_post for DrVAE, sample_q1 for VFAE,
+    // clf_fwd with hidden layers) produces
+    after(side, pl->ev.qy, cm);
+    on(side);
+    if (pl->clf_nh > 0) {
+      ex.phase = "clf.fwd";
+      if (pl->clf_in > pl->Z)  // DrVAE: u = [z1 | z2f - z1 | 1] (VFAE reads the z1 rows of Zdec)
+        ex.row_op(SROW_CLF_U, "clf_u", row_items(LNb), 0,
+                  [&]() { launch_k(clf_u_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, v); });
+      ex.block_hidden_fwd(pl->clfb, pl->clfv.U, 0, CNT_LN, LNb);
+      ex.row_op(SROW_CLF_FWD, "clf_fwd", row_items(LNb), 0,
+                [&]() { launch_k(clf_fwd_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, v); });
+    }
+    if (pl->side_delay_cycles > 0 && !ex.rec) spin_kernel<<<1, 1, 0, ex.st>>>(pl->side_delay_cycles);
+    ex.row_op(SROW_PZ1_POST, "pz1_post", row_items(round_up(Fb, 128)), 0,
+              [&]() { launch_k(pl->view.Zc <= 128 ? pz1_post_kernel<4> : pz1_post_kernel<MAXJ>, rows_grid(round_up(Fb, 128)), dim3(ROW_THREADS), 0, ex.st, v); });
+    // clf_back (main stream) reads the per-class KL terms pz1_post has just written (kfp_row)
+    if (overlap && backward && pl->has_clf) ex.ev_record(pl->ev.kfp, ex.st);
+    if (backward) {
+      if (dwa_early) ex.cta_cap = nsm - pl->dwa_early_sms;  // (they run next to the early dW+Adam launch)
+      ex.phase = "dz1.bwd";
+      ex.block_bwd(pl->dz1b, v.dY9, v.Z3b, 0, pl->Z3, v.dZ3.p, v.dZ3.ms, CNT_F, Fb);
+      if (!ex.rec) cudaEventRecord(pl->bucket_ev[0], ex.dw_stream ? ex.dw_stream : ex.st);
+      ex.row_op(SROW_Z3_BACK, "z3_back", row_items(round_up(Fb, 128)), 0,
+                [&]() { launch_k(pl->view.Z3c <= 128 ? z3_back_kernel<4> : z3_back_kernel<MAXJ>, rows_grid(round_up(Fb, 128)), dim3(ROW_THREADS), 0, ex.st, v); });
+      ex.phase = "z3.bwd";
+      ex.block_bwd(pl->z3b, v.dY7, v.Z1e, 0, pl->Z, v.dZ1e.p, v.dZ1e.ms, CNT_F, Fb);
+      if (!ex.rec) cudaEventRecord(pl->bucket_ev[1], ex.dw_stream ? ex.dw_stream : ex.st);
+      ex.cta_cap = 0;
+      // what q_back needs from this stream; the loss reduction that follows here is joined at the end of the step only
+      if (overlap) ex.ev_record(pl->ev.side_bwd, ex.st);
+    }
+    on(cm);
+  }
+  // ---- decoder p(x|z) on the stacked rows [z1 | z2 | z2f], fused log-density + gradient ----
+  ex.phase = "dec.fwd";
+  ex.block_hidden_fwd(pl->dec, v.Zdec, 0, CNT_RD, Rdb);
+  {
+    EpiParams e = ex.epi_base();
+    e.out_c8 = pl->dY5.p;
+    e.out_c8_ms = pl->dY5.ms;
+    e.out_c8_rcap = pl->dY5.rcap;
+    e.bias = pl->derived.p + pl->dec.head.bias_off;
+    e.bias_ms = pl->derived.ms;
+    e.tgt4 = v.tgt4.p;
+    e.tgt_ms = v.tgt4.ms;
+    e.tgt_rcap = pl->view.R0cap;
+    e.X = pl->X;
+    e.Xc = pl->view.Xc;
+    e.counts = v.counts.p;
+    e.counts_stride = (int)v.counts.ms;
+    e.coefs = v.coefs.p;
+    e.coefs_stride = (int)v.coefs.ms;
+    e.L = L;
+    e.part = v.dec_part.p;
+    e.part_ms = v.dec_part.ms;
+    e.part_rcap = pl->view.Rdcap;
+    e.write_dy = backward ? 1 : 0;
+    ex.gemm_nt(pl->dec.H.back(), 0, pl->dec.head, EPI_DECLOSS, e, CNT_RD, Rdb);
+  }
+  // The loss reduction is off the backward's critical path: it runs at the tail of the side stream
+  // (after that branch's backward), once the decoder log-density partials of the main stream exist.
+  after(side, pl->ev.side_fwd, cm);
+  on(side);
+  ex.phase = "";
+  ex.row_op(SROW_LOSS_PARTIAL, "loss", v.loss_slices, v.loss_slices,
+            [&]() { launch_k(loss_partial_kernel, dim3(v.loss_slices, E), dim3(256), 0, ex.st, v); });
+  ex.row_op(SROW_LOSS_FINAL, "loss_final", 1, 0, [&]() { launch_k(loss_final_kernel, dim3(E), dim3(32), 0, ex.st, v); });
+  if (losses_out && ex.ok() && !ex.rec) {
+    // losses buffer per model is padded to 256 B in the arena; the caller's is dense [E][8]
+    ex.err = cudaMemcpy2DAsync(losses_out, 8 * sizeof(float), v.losses.p, v.losses.ms * sizeof(float),
+                               8 * sizeof(float), E, cudaMemcpyDeviceToDevice, ex.st);
+  }
+  if (overlap) ex.ev_record(pl->ev.side_end, side);  // everything the side stream does in this step
+  on(cm);
+
+  if (backward && ex.ok()) {
+    size_t bk = pl->has_fprop ? 2 : 0;  // buckets 0, 1 (decoder_z1, encoder_z3) were recorded by the side branch
+    auto bucket_done = [&](bool weight_gemm = true) {
+      if (!ex.rec) cudaEventRecord(pl->bucket_ev[bk], (weight_gemm && ex.dw_stream) ? ex.dw_stream : ex.st);
+      ++bk;
+    };
+    ex.phase = "dec.bwd";
+    if (dwa_early) {
+      ex.after_head_dx = [&]() {
+        cudaEventRecord(pl->ev.dwa, cm);
+        cudaStreamWaitEvent(pl->s_dwa, pl->ev.dwa, 0);
+        launch_dwadam(0, pl->dwa_early_tiles, pl->s_dwa, pl->dwa_early_sms, "dw_adam_early");
+        ex.phase = "dec.bwd";
+        ex.cta_cap = nsm - pl->dwa_early_sms;
+        dwa_early_done = true;
       };
-      ex.phase = "dec.bwd";
-      if (dwa_early) {
-        ex.after_head_dx = [&]() {
-          cudaStream_t es = pl->chain[1].side;
-          cudaEventRecord(pl->chain[1].ev_dw, cm);
-          cudaStreamWaitEvent(es, pl->chain[1].ev_dw, 0);
-          launch_dwadam(0, pl->dwa_early_tiles, es, pl->dwa_early_sms, "dw_adam_early");
-          ex.phase = "dec.bwd";
-          ex.cta_cap = nsm - pl->dwa_early_sms;
-          dwa_early_done = true;
-        };
-      }
-      ex.block_bwd(pl->dec, pl->dY5, v.Zdec, 0, pl->Z, v.dZdec.p, v.dZdec.ms, CNT_RD, Rdb);
-      bucket_done();
-      if (pl->has_clf) {
-        if (pl->has_fprop && (pl->sched & 2)) {
-          ++bk;  // ran on the side stream right after pz1_post (bucket event recorded there)
-          if (overlap) ex.ev_wait(cm, ch.ev_clf);
-        } else {
-          if (overlap && pl->has_fprop) ex.ev_wait(cm, ch.ev_kfp);
-          if (v.clf_back_fused) {
-            // T_back (next) computes d loss / d logits and the classifier's input gradient for its own rows; only the
-            // weight gradient remains, after T_back
-          } else if (overlap && forked && (pl->sched & 4)) {
-            // only the input gradient (clf_back) is on the chain towards T_back / q_back; the weight gradient runs on
-            // the caller's stream, which is otherwise idle until this range joins it in front of the dW+Adam launch
-            clf_back();
-            after(st, ch.ev_clf, cm);
-            on(st);
-            clf_grad();
-            bucket_done(false);
-            on(cm);
-          } else {
-            clf_bwd();
-            bucket_done(false);
-          }
-        }
-      }
-      if (pl->has_T) {
-        ex.phase = "T.bwd";
-        ex.row_op(SROW_T_BACK, "T_back", row_items(N + PAD_WARPS), 0,
-                  [&]() { launch_k(pl->view.Zc <= 128 ? T_back_kernel<4> : T_back_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-        if (pl->has_clf && v.clf_back_fused) {
-          if (overlap && forked && (pl->sched & 4)) {
-            after(st, ch.ev_clf, cm);
-            on(st);
-            clf_grad();
-            bucket_done(false);
-            on(cm);
-          } else {
-            clf_grad();
-            bucket_done(false);
-          }
-        }
-        ex.gemm_dx(v.dYT, pl->Tsh, EPI_STORE_F32, ex.epi_f32(v.dZ1T.p, v.dZ1T.ms, pl->Z, pl->Z, nullptr), CNT_LN, LNb);
-        ex.gemm_dw(v.dYT, v.Zdec, 0, pl->Tsh, CNT_LN, LNb, pl->arch.kind == DRVAE_KIND_PVAE ? CNT_NP : -1);
-        bucket_done();
-      }
-      if (overlap) ex.ev_wait(cm, ch.ev_side_bwd);  // join: q_back sums the side branch's gradients into q(z1|x1)
-      ex.phase = "enc.bwd";
-      ex.row_op(SROW_Q_BACK, "q_back", row_items(N + PAD_WARPS), 0,
-                [&]() { launch_k(pl->view.Zc <= 128 ? q_back_kernel<4> : q_back_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, 2, v); });
-      ex.block_bwd(pl->enc, v.dY2, v.Ain, 0, pl->X, nullptr, 0, CNT_R0, R0b);
-      bucket_done();
     }
-    ex.cta_cap = 0;
-    if (overlap) ex.ev_wait(cm, ch.ev_side_end);
-    if (ex.dw_stream) {  // join the weight-gradient stream
-      if (ex.rec) {
-        ex.rec->after(cm, ex.dw_stream);
+    ex.block_bwd(pl->dec, pl->dY5, v.Zdec, 0, pl->Z, v.dZdec.p, v.dZdec.ms, CNT_RD, Rdb);
+    bucket_done();
+    if (pl->has_clf) {
+      if (overlap && pl->has_fprop) ex.ev_wait(cm, pl->ev.kfp);
+      if (own_main) {
+        // only the input gradient (clf_back) is on the chain towards T_back / q_back; the weight gradient runs on
+        // the caller's stream, which is otherwise idle until the main chain joins it in front of the dW+Adam launch
+        clf_back();
+        after(st, pl->ev.clf, cm);
+        on(st);
+        clf_grad();
+        bucket_done(false);
+        on(cm);
       } else {
-        cudaEventRecord(ch.ev_dw_end, ex.dw_stream);
-        cudaStreamWaitEvent(cm, ch.ev_dw_end, 0);
+        clf_bwd();
+        bucket_done(false);
       }
     }
-    if (ex.rec && ex.ok()) {
-      // ---- the recorded chain as one cooperative launch ----
-      ex.rec = nullptr;
-      ex.st = cm;
-      ex.phase = "step";
-      StepParams* sp = new StepParams();
-      std::vector<std::string> tags;
-      int max_items = 1;
-      cudaError_t ferr = recorder.finalize(*sp, tags, max_items);
-      if (ferr == cudaErrorNotSupported) {
-        // more ops than the kernel's tables hold (very deep blocks): this plan keeps the launch-per-kernel schedule.
-        // What has been issued so far (noise, rowmap, prep) is idempotent, so the sequence is simply enqueued again.
-        delete sp;
-        cudaGetLastError();
-        pl->stepk_unsupported = true;
-        return run_step(pl, b, nz, hp, losses_out, st, backward, fused_adam);
-      }
-      if (ferr != cudaSuccess) {
-        delete sp;
-        return set_cuda_error("drvae step kernel tables", ferr);
-      }
-      sp->t.v = v;
-      sp->t.v.trace = nullptr;
-      sp->bar = pl->d_stepk_bar;
-      sp->dbg = pl->dbg;
-      sp->trace = nullptr;
-      sp->trace_id0 = 0;
-      prof_pre(pl, cm, "step:chain");
-      if (pl->trace_on && pl->trace_next + sp->t.n_levels <= pl->trace_cap) {
-        sp->trace = pl->d_trace;
-        sp->trace_id0 = pl->trace_next;
-        pl->trace_next += sp->t.n_levels;
-        for (int l = 0; l < sp->t.n_levels; ++l) pl->trace_tags.push_back("L" + std::to_string(l) + "|" + tags[l]);
-      }
-      cudaError_t lerr = step_kernel_launch(*sp, max_items, cm);
-      delete sp;
-      prof_post(pl, cm);
-      if (lerr != cudaSuccess) ex.err = lerr;
-      pl->launches++;
-      pl->stepk_launches++;
-      if (losses_out && ex.ok()) {
-        ex.err = cudaMemcpy2DAsync(losses_out + 8 * (size_t)m0, 8 * sizeof(float), v.losses.at(m0), v.losses.ms * sizeof(float),
-                                   8 * sizeof(float), Ec, cudaMemcpyDeviceToDevice, cm);
-      }
-      if (backward)
-        for (auto& ev : pl->bucket_ev) cudaEventRecord(ev, cm);  // every gradient bucket is complete when the kernel ends
+    if (pl->has_T) {
+      ex.phase = "T.bwd";
+      ex.row_op(SROW_T_BACK, "T_back", row_items(N + PAD_WARPS), 0,
+                [&]() { launch_k(pl->view.Zc <= 128 ? T_back_kernel<4> : T_back_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, v); });
+      ex.gemm_dx(v.dYT, pl->Tsh, EPI_STORE_F32, ex.epi_f32(v.dZ1T.p, v.dZ1T.ms, pl->Z, pl->Z, nullptr), CNT_LN, LNb);
+      ex.gemm_dw(v.dYT, v.Zdec, 0, pl->Tsh, CNT_LN, LNb, pl->arch.kind == DRVAE_KIND_PVAE ? CNT_NP : -1);
+      bucket_done();
     }
-    if (forked) {  // join this range into the caller's stream
-      cudaEventRecord(ch.ev_end, cm);
-      cudaStreamWaitEvent(st, ch.ev_end, 0);
+    if (overlap) ex.ev_wait(cm, pl->ev.side_bwd);  // join: q_back sums the side branch's gradients into q(z1|x1)
+    ex.phase = "enc.bwd";
+    ex.row_op(SROW_Q_BACK, "q_back", row_items(N + PAD_WARPS), 0,
+              [&]() { launch_k(pl->view.Zc <= 128 ? q_back_kernel<4> : q_back_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, v); });
+    ex.block_bwd(pl->enc, v.dY2, v.Ain, 0, pl->X, nullptr, 0, CNT_R0, R0b);
+    bucket_done();
+  }
+  ex.cta_cap = 0;
+  if (overlap) ex.ev_wait(cm, pl->ev.side_end);
+  if (ex.dw_stream) {  // join the weight-gradient stream
+    if (ex.rec) {
+      ex.rec->after(cm, ex.dw_stream);
+    } else {
+      cudaEventRecord(pl->ev.dw_end, ex.dw_stream);
+      cudaStreamWaitEvent(cm, pl->ev.dw_end, 0);
     }
   }
+  if (ex.rec && ex.ok()) {
+    // ---- the recorded chain as one cooperative launch ----
+    ex.rec = nullptr;
+    ex.st = cm;
+    ex.phase = "step";
+    StepParams* sp = new StepParams();
+    std::vector<std::string> tags;
+    int max_items = 1;
+    cudaError_t ferr = recorder.finalize(*sp, tags, max_items);
+    if (ferr == cudaErrorNotSupported) {
+      // more ops than the kernel's tables hold (very deep blocks): this plan keeps the launch-per-kernel schedule.
+      // What has been issued so far (noise, rowmap, prep) is idempotent, so the sequence is simply enqueued again.
+      delete sp;
+      cudaGetLastError();
+      pl->stepk_unsupported = true;
+      return run_step(pl, b, nz, hp, losses_out, st, backward, fused_adam);
+    }
+    if (ferr != cudaSuccess) {
+      delete sp;
+      return set_cuda_error("drvae step kernel tables", ferr);
+    }
+    sp->t.v = v;
+    sp->t.v.trace = nullptr;
+    sp->bar = pl->d_stepk_bar;
+    sp->dbg = pl->dbg;
+    sp->trace = nullptr;
+    sp->trace_id0 = 0;
+    prof_pre(pl, cm, "step:chain");
+    if (pl->trace_on && pl->trace_next + sp->t.n_levels <= pl->trace_cap) {
+      sp->trace = pl->d_trace;
+      sp->trace_id0 = pl->trace_next;
+      pl->trace_next += sp->t.n_levels;
+      for (int l = 0; l < sp->t.n_levels; ++l) pl->trace_tags.push_back("L" + std::to_string(l) + "|" + tags[l]);
+    }
+    cudaError_t lerr = step_kernel_launch(*sp, max_items, cm);
+    delete sp;
+    prof_post(pl, cm);
+    if (lerr != cudaSuccess) ex.err = lerr;
+    pl->launches++;
+    pl->stepk_launches++;
+    if (losses_out && ex.ok()) {
+      ex.err = cudaMemcpy2DAsync(losses_out, 8 * sizeof(float), v.losses.p, v.losses.ms * sizeof(float),
+                                 8 * sizeof(float), E, cudaMemcpyDeviceToDevice, cm);
+    }
+    if (backward)
+      for (auto& ev : pl->bucket_ev) cudaEventRecord(ev, cm);  // every gradient bucket is complete when the kernel ends
+  }
+  if (own_main) {  // join the main chain into the caller's stream
+    cudaEventRecord(pl->ev.end, cm);
+    cudaStreamWaitEvent(st, pl->ev.end, 0);
+  }
   ex.st = st;
-  ex.model0 = 0;
-  ex.Ec = E;
   if (backward && ex.defer_dw && ex.ok()) {
     if (dwa_early_done) {  // the early part runs on its own stream: the rest starts when both are complete
-      cudaEventRecord(pl->chain[1].ev_dw_end, pl->chain[1].side);
-      cudaStreamWaitEvent(st, pl->chain[1].ev_dw_end, 0);
+      cudaEventRecord(pl->ev.dwa_end, pl->s_dwa);
+      cudaStreamWaitEvent(st, pl->ev.dwa_end, 0);
     }
     ex.st = st;
     launch_dwadam(dwa_early_done ? pl->dwa_early_tiles : 0, pl->dwa_tiles, st, 0, dwa_early_done ? "dw_adam_rest" : "dw_adam_all");
@@ -2461,7 +2367,6 @@ extern "C" int drvae_infer(drvae_plan_t* pl, const float* x1, int N, const drvae
   v.dyn = pl->d_dyn;
   v.mem = member_base(pl);
   v.mem_stride = pl->member_table ? 1 : 0;
-  v.sview_dev = nullptr;
   v.own_noise = 0;
   {
     drvae_hparams_t ihp{};  // eval mode: training = 0, add_noise = 0

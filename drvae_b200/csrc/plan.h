@@ -167,7 +167,6 @@ struct MemberExpand {
 
 struct DevView {
   int kind, X, Y, Z, Z3, L, N, Ncap;
-  int model0;        // first ensemble member of this launch (a step may run sub-ranges of the ensemble as separate chains)
   int Xc;            // round_up(X, 16)
   int Zc, Z3c;       // chunk8 feature capacities of the latent buffers
   int Zs, Z3s;       // column of the logvar half in (mu | logvar) rows: round_up(Z, 16) / round_up(Z3, 16).  The two
@@ -177,8 +176,6 @@ struct DevView {
   int R0cap, LNcap, Rdcap, Fcap, Flcap;
   int has_pair, has_T, has_clf, has_fprop, clf_in;
   int need_grad;
-  int clf_back_fused;  // 1: T_back computes the classifier's input gradient itself (no clf_back launch; DrVAE)
-  int clf_split;     // 1: the classifier q(y|z1, z2f) runs as its own kernel (clf_fwd_kernel) off the main chain instead of inside T_post
   // batch (caller memory)
   MBuf<const float> x1, x2;
   MBuf<const int> y, has_x2, has_y;
@@ -239,10 +236,10 @@ struct DevView {
   const MemberScalars* mem;  // per-member scalars of global model m: mem[m * mem_stride] (stride 0: the copy in dyn)
   int mem_stride;
   __host__ __device__ __forceinline__ const MemberScalars& member(int m) const { return mem[(long long)m * mem_stride]; }
-  SampleView* sview_dev;  // device copy of the sampling epilogue's view (written by rowmap_kernel; null: not used)
   unsigned long long* trace;  // kernel trace buffer (null: off) and this launch's slot
   int trace_id;
-  const ClfView* clf;  // classifier hidden layers (device memory); null: linear_p reads u itself
+  const ClfView* clf;  // classifier hidden layers (device memory), which run as their own GEMMs + clf_fwd_kernel; null:
+                       // no hidden layers, linear_p reads u itself inside sample_q1 (VFAE) / T_post (DrVAE)
 };
 
 constexpr int CLF_SPLITS = 32;       // row splits of the classifier weight gradient (ensemble-sized batches)

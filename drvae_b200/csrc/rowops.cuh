@@ -94,9 +94,7 @@ __device__ __forceinline__ int block_exclusive_scan(int x, int* warp_tot, int& t
 
 __global__ void __launch_bounds__(ROWMAP_THREADS) rowmap_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  const int m = v.model0 + blockIdx.x, t = threadIdx.x, N = v.N;
+  const int m = blockIdx.x, t = threadIdx.x, N = v.N;
   __shared__ int s_tot[33];
   const int* hx = v.has_pair ? v.has_x2.at(m) : nullptr;
   const int* hy = (v.has_clf && v.has_y.p) ? v.has_y.at(m) : nullptr;
@@ -117,22 +115,6 @@ __global__ void __launch_bounds__(ROWMAP_THREADS) rowmap_kernel(DevView v) {
   int p = block_exclusive_scan(np, s_tot, Np);
   int e = block_exclusive_scan(ne, s_tot, Fl);
   (void)block_exclusive_scan(nl, s_tot, Nlab);
-  if (t == 0 && blockIdx.x == 0 && v.sview_dev) {
-    // view of the sampling epilogue of the encoder-head GEMM (gemm.cuh EPI_SAMPLE_Q1): pointers of model 0 + strides
-    SampleView s;
-    s.Z = v.Z, s.Zs = v.Zs, s.Zc = v.Zc, s.L = v.L, s.Ncap = v.Ncap, s.Y = v.Y;
-    s.counts = v.counts.p, s.counts_stride = (int)v.counts.ms;
-    s.pair_of = v.pair_of.p, s.pair_ms = v.pair_of.ms;
-    s.ebase = v.ebase.p, s.ebase_ms = v.ebase.ms;
-    s.lab = v.lab.p, s.lab_ms = v.lab.ms;
-    s.ycls = v.ycls.p, s.ycls_ms = v.ycls.ms;
-    s.eps_z1 = v.eps_z1.p, s.eps_z1_ms = v.eps_z1.ms;
-    s.eps_z2 = v.eps_z2.p, s.eps_z2_ms = v.eps_z2.ms;
-    s.Z1f = v.Z1f.p, s.z1f_ms = v.Z1f.ms;
-    s.zdec = v.Zdec.p, s.zdec_ms = v.Zdec.ms, s.zdec_rcap = v.Zdec.rcap;
-    s.z1e = v.Z1e.p, s.z1e_ms = v.Z1e.ms, s.z1e_rcap = v.Z1e.rcap;
-    *v.sview_dev = s;
-  }
   if (t == 0) {
     int* cnt = v.counts.at(m);
     cnt[CNT_N] = N;
@@ -211,10 +193,8 @@ constexpr int PREP_SLAB = 256;
 
 __global__ void __launch_bounds__(PREP_THREADS) prep_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float tile[PREP_ROWS][PREP_SLAB + 1];
-  const int m = v.model0 + blockIdx.z, r0 = blockIdx.x * PREP_ROWS;
+  const int m = blockIdx.z, r0 = blockIdx.x * PREP_ROWS;
   const int* cnt = v.counts.at(m);
   const int N = cnt[CNT_N], R0 = cnt[CNT_R0];
   if (r0 >= pad128(R0)) return;
@@ -482,7 +462,7 @@ __device__ __forceinline__ void sample_q1_row(const DevView& v, const int m, con
         st_c8(z1e, v.Z1e.rcap, l * Fl + eb + jj, f, (f == v.Z + 1 + cls) ? 1.f : z);
       }
     }
-    if (v.has_clf && !v.has_T && !v.clf_split) classifier_row_regs<J>(v, m, r, i, lane, n1, n1, false);
+    if (v.has_clf && !v.has_T && !v.clf) classifier_row_regs<J>(v, m, r, i, lane, n1, n1, false);
   }
   if (v.kind == KIND_PVAE) {  // KL(q1 || N(0,I)) and KL(q2 || N(0,I)) with free bits (PVAE.py:330-372)
     float k1 = 0.f, k2 = 0.f;
@@ -503,9 +483,7 @@ __device__ __forceinline__ void sample_q1_row(const DevView& v, const int m, con
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_SAMPLE) sample_q1_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  sample_q1_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  sample_q1_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -565,38 +543,31 @@ __device__ __forceinline__ void T_post_row(const DevView& v, const int m, const 
       for (int f = 32 * J + lane; f < v.Zc; f += 32) st_c8(zdec, v.Zdec.rcap, LN + LNp + l * Np + p, f, (f == v.Z) ? 1.f : 0.f);
     kl = warp_sum(kl);
     if (lane == 0) v.klz2_row.at(m)[r] = q2 ? fmaxf(kl, v.dyn->s.kl_min) : 0.f;
-    if (v.has_clf && !v.clf_split) classifier_row_regs<J>(v, m, r, i, lane, a_z1, a_ef, v.clf_in > v.Z);
+    if (v.has_clf && !v.clf) classifier_row_regs<J>(v, m, r, i, lane, a_z1, a_ef, v.clf_in > v.Z);
   }
 }
 
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_TPOST) T_post_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  T_post_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  T_post_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
-// clf_fwd: the classifier q(y | z1, z2f - z1) of DrVAE as its own kernel, one warp per stacked row r = l * N + i.
-// Only the label-dependent branch and the backward need q(y|.), the decoder does not: split from T_post it leaves
-// the main chain (sample z2f -> decoder) for the side stream (DevView::clf_split).
+// clf_fwd: the output layer linear_p of a classifier with hidden layers (DevView::clf), one warp per stacked row
+// r = l * N + i, after the hidden layers' GEMMs.  Only the label-dependent branch and the backward need q(y|.), the
+// decoder does not: it runs on the side stream, and sample_q1 / T_post stay as without hidden layers.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void clf_fwd_row(const DevView& v, const int m, const int r, const int lane) {
   const int* cnt = v.counts.at(m);
   const int N = cnt[CNT_N], LN = cnt[CNT_LN];
   if (r >= LN) return;
-  if (v.clf)
-    classifier_row_h(v, m, r, r % N, lane);
-  else
-    classifier_row(v, m, r, r % N, lane);
+  classifier_row_h(v, m, r, r % N, lane);
 }
 
 __global__ void __launch_bounds__(ROW_THREADS) clf_fwd_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_fwd_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_fwd_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // clf_u (DrVAE, classifier hidden layers): the first hidden GEMM's operand u = [z1 | z2f - z1 | 1] of stacked row r, as
@@ -620,9 +591,7 @@ __device__ __forceinline__ void clf_u_row(const DevView& v, const int m, const i
 
 __global__ void __launch_bounds__(ROW_THREADS) clf_u_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_u_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_u_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -681,9 +650,7 @@ __device__ __forceinline__ void z3_post_row(const DevView& v, const int m, const
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_EVAL) z3_post_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  z3_post_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  z3_post_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // weight of evaluation e in the batch KLD: 1 for the true class of a labeled row, q(y=j) otherwise
@@ -754,9 +721,7 @@ __device__ __forceinline__ void pz1_post_row(const DevView& v, const int m, cons
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_EVAL) pz1_post_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  pz1_post_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  pz1_post_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -810,9 +775,7 @@ __device__ __forceinline__ void z3_back_row(const DevView& v, const int m, const
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_EVAL) z3_back_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  z3_back_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  z3_back_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -883,9 +846,7 @@ __device__ __forceinline__ void clf_back_row(const DevView& v, const int m, cons
 
 __global__ void __launch_bounds__(ROW_THREADS) clf_back_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_back_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_back_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // The same with hidden layers: d loss / d logits, then dPre of the last hidden layer, (dl . W_p) * ELU'(H) as bf16
@@ -925,9 +886,7 @@ __device__ __forceinline__ void clf_back_h_row(const DevView& v, const int m, co
 
 __global__ void __launch_bounds__(ROW_THREADS) clf_back_h_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_back_h_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_back_h_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // clf_du (DrVAE, hidden layers): d loss / d u = [dz1 part | dz2f part] from the first layer's dX GEMM ->
@@ -944,9 +903,7 @@ __device__ __forceinline__ void clf_du_row(const DevView& v, const int m, const 
 
 __global__ void __launch_bounds__(ROW_THREADS) clf_du_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_du_row(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_du_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -983,10 +940,7 @@ __device__ __forceinline__ void T_back_row(const DevView& v, const int m, const 
     const float* dzd = p >= 0 ? v.dZdec.at(m) + (long long)(LN + LNp + l * Np + p) * v.Z : nullptr;
     const bool act = q2 && v.klz2_row.at(m)[r] > v.dyn->s.kl_min;
     float* dz1 = v.DZ1.at(m) + (long long)r * v.Z;
-    const bool clf_here = v.has_clf && v.clf_back_fused;  // the classifier's input gradient computed right here
-    const float* dz2f_c = (v.has_clf && !clf_here) ? v.DZ2F.at(m) + (long long)r * v.Z : nullptr;
-    float dl[MAXY];
-    if (clf_here) clf_dlogit_row(v, m, r, l, i, cnt[CNT_FL], lane, dl);
+    const float* dz2f_c = v.has_clf ? v.DZ2F.at(m) + (long long)r * v.Z : nullptr;
     float b_pmu[J], b_plv[J], b_g[J], b_c[J], b_ef[J], b_dz1[J];
 #pragma unroll
     for (int k = 0; k < J; ++k) {  // every load of this sample before the first store
@@ -997,21 +951,7 @@ __device__ __forceinline__ void T_back_row(const DevView& v, const int m, const 
       b_g[k] = (in && dzd) ? dzd[f] : 0.f;
       b_c[k] = (in && dz2f_c) ? dz2f_c[f] : 0.f;
       b_ef[k] = in ? ef[f] : 0.f;
-      b_dz1[k] = (in && v.has_clf && !clf_here) ? dz1[f] : 0.f;
-      if (clf_here && in) {
-        // d loss / d [z1, z2f - z1] = dlogit . Wc (same sums as clf_back_row): z2f gets b, z1 gets a - b
-        const float* Wc = v.clf_w.at(m);
-        float a = 0.f, b = 0.f;
-#pragma unroll
-        for (int j = 0; j < MAXY; ++j) {
-          if (j < v.Y) {
-            a = fmaf(dl[j], Wc[j * v.clf_ld + f], a);
-            b = fmaf(dl[j], Wc[j * v.clf_ld + v.Z + f], b);
-          }
-        }
-        b_c[k] = b;
-        b_dz1[k] = a - b;
-      }
+      b_dz1[k] = (in && v.has_clf) ? dz1[f] : 0.f;
     }
 #pragma unroll
     for (int k = 0; k < J; ++k) {
@@ -1052,9 +992,7 @@ __device__ __forceinline__ void T_back_row(const DevView& v, const int m, const 
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_TBACK) T_back_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  T_back_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  T_back_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1178,9 +1116,7 @@ __device__ __forceinline__ void q_back_row(const DevView& v, const int m, const 
 template <int J>
 __global__ void __launch_bounds__(ROW_THREADS, ROW_LB_QBACK) q_back_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  q_back_row<J>(v, v.model0 + blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  q_back_row<J>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1241,16 +1177,12 @@ __device__ __forceinline__ void clf_grad_partial_block(const DevView& v, const i
 
 __global__ void __launch_bounds__(256) clf_grad_partial_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_grad_partial_block(v, v.model0 + blockIdx.y, blockIdx.x, threadIdx.x, 256);
+  clf_grad_partial_block(v, blockIdx.y, blockIdx.x, threadIdx.x, 256);
 }
 
 __global__ void __launch_bounds__(256) clf_grad_partial_h_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_grad_partial_h_block(v, v.model0 + blockIdx.y, blockIdx.x, threadIdx.x, 256);
+  clf_grad_partial_h_block(v, blockIdx.y, blockIdx.x, threadIdx.x, 256);
 }
 
 // grid (ceil(Y * (clf_in + 1) / 8), n_models), block 256: one warp per gradient element, lanes over the row splits
@@ -1282,9 +1214,7 @@ __device__ __forceinline__ void clf_grad_reduce_elem(const DevView& v, const int
 
 __global__ void __launch_bounds__(256) clf_grad_reduce_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  clf_grad_reduce_elem(v, v.model0 + blockIdx.y, blockIdx.x * 8 + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_grad_reduce_elem(v, blockIdx.y, blockIdx.x * 8 + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 
@@ -1330,7 +1260,7 @@ __device__ __forceinline__ void infer_emit_proba(const DevView& v, const InferVi
 
 // z1 = mu(q(z1|x1)); stage it for the p(z2|z1) and decoder GEMMs.  One warp per row.
 __global__ void __launch_bounds__(ROW_THREADS) infer_z1_kernel(DevView v, InferView o, int rows_dec) {
-  const int m = v.model0 + blockIdx.y, lane = threadIdx.x & 31;
+  const int m = blockIdx.y, lane = threadIdx.x & 31;
   const int r = blockIdx.x * ROW_WARPS + (threadIdx.x >> 5);
   const int N = v.N;
   if (r >= N) {
@@ -1362,7 +1292,7 @@ __global__ void __launch_bounds__(ROW_THREADS) infer_z1_kernel(DevView v, InferV
 
 // z2 = mu(p(z2|z1)) = z1 + z1 W^T + b; classifier on [z1, z2 - z1].
 __global__ void __launch_bounds__(ROW_THREADS) infer_z2_kernel(DevView v, InferView o) {
-  const int m = v.model0 + blockIdx.y, lane = threadIdx.x & 31;
+  const int m = blockIdx.y, lane = threadIdx.x & 31;
   const int r = blockIdx.x * ROW_WARPS + (threadIdx.x >> 5);
   const int N = v.N;
   if (r >= N) return;
@@ -1393,7 +1323,7 @@ __global__ void __launch_bounds__(ROW_THREADS) infer_z2_kernel(DevView v, InferV
 
 // classifier with hidden layers: logits from the last hidden activation (the block's GEMMs ran over u)
 __global__ void __launch_bounds__(ROW_THREADS) clf_h_infer_kernel(DevView v, InferView o) {
-  const int m = v.model0 + blockIdx.y, lane = threadIdx.x & 31;
+  const int m = blockIdx.y, lane = threadIdx.x & 31;
   const int r = blockIdx.x * ROW_WARPS + (threadIdx.x >> 5);
   if (r >= v.N) return;
   classifier_row_h(v, m, r, r, lane);
@@ -1468,10 +1398,8 @@ __device__ __forceinline__ void loss_partial_block(const DevView& v, const int m
 
 __global__ void __launch_bounds__(256) loss_partial_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
   __shared__ float sm[256];
-  loss_partial_block(v, v.model0 + blockIdx.y, blockIdx.x, gridDim.x, threadIdx.x, sm, SyncBlock());
+  loss_partial_block(v, blockIdx.y, blockIdx.x, gridDim.x, threadIdx.x, sm, SyncBlock());
 }
 
 // grid n_models, one warp: fixed-order sum of the slices, then the reference's normalisation
@@ -1501,9 +1429,7 @@ __device__ __forceinline__ void loss_final_model(const DevView& v, const int m) 
 
 __global__ void __launch_bounds__(32) loss_final_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  pdl_launch_dependents();
-  pdl_wait();
-  if (threadIdx.x == 0) loss_final_model(v, v.model0 + blockIdx.x);
+  if (threadIdx.x == 0) loss_final_model(v, blockIdx.x);
 }
 
 }  // namespace drvae

@@ -65,7 +65,6 @@ struct StepOp {
   int item_begin;  // first item of this op inside its level
   int items;
   int per_model;   // row op: items per ensemble member
-  int model0;
   int arg;         // row op: kernel-specific (loss slices)
 };
 
@@ -338,7 +337,6 @@ __global__ void __launch_bounds__(STEPK_THREADS, 1) step_kernel(const __grid_con
             case EPI_DACT_C8: step_gemm_epilogue<EPI_DACT_C8>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
             case EPI_DECLOSS: step_gemm_epilogue<EPI_DECLOSS>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
             case EPI_GRAD: step_gemm_epilogue<EPI_GRAD>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
-            case EPI_SAMPLE_Q1: step_gemm_epilogue<EPI_SAMPLE_Q1>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
             default: break;
           }
           tc_fence_before();
@@ -346,7 +344,7 @@ __global__ void __launch_bounds__(STEPK_THREADS, 1) step_kernel(const __grid_con
           if (lane == 0) mbar_arrive(&acc_empty[a]);
           ++acc_j;
         } else {
-          const int m = op.model0 + local / op.per_model;
+          const int m = local / op.per_model;
           const int blk = local - (local / op.per_model) * op.per_model;
           const int r = blk * STEPK_ROWS + w;
           switch (op.sub) {
@@ -469,7 +467,7 @@ struct StepRecorder {
     cur[w] = std::max(cur[w], cur[p]);
   }
   void add_gemm(int epi, const GemmProblem& p, const EpiParams& e, int n_models, cudaStream_t s, const std::string& tag) {
-    if (epi != EPI_STORE_F32 && epi != EPI_ELU_C8 && epi != EPI_DACT_C8 && epi != EPI_DECLOSS && epi != EPI_GRAD && epi != EPI_SAMPLE_Q1) unsupported = true;
+    if (epi != EPI_STORE_F32 && epi != EPI_ELU_C8 && epi != EPI_DACT_C8 && epi != EPI_DECLOSS && epi != EPI_GRAD) unsupported = true;
     if (p.BN > 256) unsupported = true;
     Rec r{};
     r.op.kind = SOP_GEMM;
@@ -480,19 +478,17 @@ struct StepRecorder {
     r.g.p.trace = nullptr;
     r.g.e = e;
     r.op.items = p.tiles_m * p.tiles_n * p.ksplit * n_models;
-    r.op.model0 = p.model0;
     const int i = sid(s);
     r.level = ++cur[i];
     r.tag = tag;
     recs.push_back(r);
   }
-  void add_row(int kind, int per_model, int model0, int n_models, int arg, cudaStream_t s, const std::string& tag) {
+  void add_row(int kind, int per_model, int n_models, int arg, cudaStream_t s, const std::string& tag) {
     Rec r{};
     r.op.kind = SOP_ROW;
     r.op.sub = kind;
     r.op.per_model = per_model < 1 ? 1 : per_model;
     r.op.items = r.op.per_model * n_models;
-    r.op.model0 = model0;
     r.op.arg = arg;
     const int i = sid(s);
     r.level = ++cur[i];

@@ -361,7 +361,7 @@ class Plan:
         return int(self.lib.drvae_plan_graph_failures(self.h))
 
     def set_step_kernel(self, enable):
-        """Persistent step kernel on (default) / off (one launch per GEMM and row operation)."""
+        """Persistent step kernel on / off (default: one launch per GEMM and row operation)."""
         _lib.check(self.lib.drvae_set_step_kernel(self.h, 1 if enable else 0))
 
     def step_kernel_launches(self):
@@ -369,9 +369,6 @@ class Plan:
 
     def set_gemm_impl(self, impl):
         _lib.check(self.lib.drvae_set_gemm_impl(self.h, {"tc": 0, "simt": 1}[impl]))
-
-    def set_chains(self, chains):
-        _lib.check(self.lib.drvae_set_chains(self.h, int(chains)), "set_chains")
 
     def debug_side_delay(self, cycles):
         _lib.check(self.lib.drvae_debug_side_delay(self.h, int(cycles)), "debug_side_delay")

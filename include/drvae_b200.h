@@ -244,16 +244,13 @@ int drvae_set_external_scalars(drvae_plan_t* plan, int enable);
 long long drvae_plan_graph_replays(const drvae_plan_t* plan);
 /* Captures that failed (that call shape then runs as plain launches; other shapes still capture): 0 on a healthy plan. */
 long long drvae_plan_graph_failures(const drvae_plan_t* plan);
-/* Persistent step kernel (default on): the forward + ELBO + input-gradient chain of a step runs as ONE cooperative
- * launch whose dependent stages are separated by grid barriers instead of kernel boundaries; 0 restores one launch per
- * GEMM / row operation.  Results do not depend on it (bit-identical).  drvae_plan_step_kernel_launches counts the
- * launches of that kernel (0: the plan fell back to the launch-per-operation schedule). */
+/* Persistent step kernel (default off: measured slower than the captured graph of launches, DESIGN.md §4): the
+ * forward + ELBO + input-gradient chain of a step runs as ONE cooperative launch whose dependent stages are separated
+ * by grid barriers instead of kernel boundaries; 0 keeps one launch per GEMM / row operation.  Results do not depend
+ * on it (bit-identical).  drvae_plan_step_kernel_launches counts the launches of that kernel (0: the plan fell back to
+ * the launch-per-operation schedule). */
 int drvae_set_step_kernel(drvae_plan_t* plan, int enable);
 long long drvae_plan_step_kernel_launches(const drvae_plan_t* plan);
-/* Step schedule: the ensemble is cut into `chains` contiguous model ranges whose forward + input-gradient chains run on
- * separate streams (their latency-bound kernels overlap); the grouped weight-gradient + Adam launch at the end covers
- * all of them.  Default 1.  Results do not depend on it (bit-identical). */
-int drvae_set_chains(drvae_plan_t* plan, int chains);
 
 /* Introspection for tests and bench.py */
 int drvae_set_gemm_impl(drvae_plan_t* plan, int impl);   /* 0 tcgen05 (default), 1 SIMT validation kernel */

@@ -35,7 +35,7 @@ CASES = {
     "z125": (_arch(40, 2, 125, 125, [32]), 64, 2),
     # <MAXJ> row kernels; 126 + 1 + 2 = 129 > 128: per-layer EPI_GRAD_ADAM; LN = 130
     "z126": (_arch(40, 2, 126, 126, [32]), 65, 2),
-    # (mu | logvar) head: one tile exactly 256 wide (the whole TMEM accumulator); <MAXJ>; sampling epilogue allowed
+    # (mu | logvar) head: one tile exactly 256 wide (the whole TMEM accumulator); <MAXJ>
     "z128": (_arch(40, 2, 128, 9, [48]), 40, 2),
     # <MAXJ> lanes all populated; heads over two N tiles 256 wide; classifier over 512 inputs; README widths
     "z256": (_arch(978, 2, 256, 256, [800], [600], [200], [200]), 150, 2),
@@ -125,7 +125,6 @@ def geometry(case, kind):
         Y=Y, Zc=Zc, Z3c=Z3c if fprop else 0, maxj=Zc > 128 or (fprop and Z3c > 128), enc_head=heads["enc"],
         heads=heads, hb=hb, dec_tiles=cdiv(X, hb), dec_last=X - (cdiv(X, hb) - 1) * hb, Xc=round_up(X + 1, 16),
         hidden=hidden, per_layer_adam=per_layer, dwa_layers=layers,
-        fuse_sample=kind == "drvae" and heads["enc"][1] == 1 and Zc <= 256,
         rows=runtime_rows(case, kind),
         n_hidden=max(len(arch[b]) for b in blocks))
 
@@ -350,33 +349,6 @@ def test_step_kernel_equals_one_launch_per_operation(case):
     for a, b in zip(res[True][:5], res[False][:5]):
         assert torch.equal(a, b)
     assert bool(torch.isfinite(res[True][1]).all())
-
-
-@pytest.mark.parametrize("case", ("z128", "z256"))
-def test_sampling_epilogue_equals_the_row_kernel(case, monkeypatch):
-    """DRVAE_B200_FUSE_SAMPLE=1 fuses q(z1|x1) sampling into the encoder-head GEMM only when mu and logvar share one
-    N tile: at z128 (one tile 256 wide) it must fuse, at z256 (two tiles) fall back.  Bit-identical either way."""
-    kind, E = "drvae", 2
-    arch, N, L = CASES[case]
-    batches = [batch_fields(kind, case_batch(case, kind, 40 + m)) for m in range(E)]
-    big = {k: torch.stack([b[k] for b in batches]).contiguous().cuda() for k in batches[0]}
-    res = {}
-    for fuse in ("0", "1"):
-        monkeypatch.setenv("DRVAE_B200_FUSE_SAMPLE", fuse)
-        plan = make_plan(case, kind, n_models=E)
-        l0 = plan.launch_count()
-        losses = [plan.train_step(big, plan.hparams(step=it), seed=6).cpu().clone() for it in range(3)]
-        ev = plan.loss_forward(big, plan.hparams(step=3, training=False), seed=6).cpu().clone()
-        torch.cuda.synchronize()
-        res[fuse] = (torch.stack(losses), plan.params.cpu().clone(), ev, plan.launch_count() - l0)
-    fuses = geometry(case, kind)["fuse_sample"]
-    assert fuses == (case == "z128")
-    if fuses:
-        assert res["1"][3] < res["0"][3], (res["0"][3], res["1"][3])
-    else:
-        assert res["1"][3] == res["0"][3], (res["0"][3], res["1"][3])
-    for a, b in zip(res["0"][:3], res["1"][:3]):
-        assert torch.equal(a, b)
 
 
 @pytest.mark.parametrize("kind", KINDS)

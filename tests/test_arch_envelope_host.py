@@ -48,7 +48,6 @@ def test_grouped_and_per_layer_optimizer_on_both_sides():
 def test_head_tiles():
     _covers(lambda g: g["enc_head"] == (256, 1), "a (mu | logvar) head in one tile exactly 256 wide")
     _covers(lambda g: g["enc_head"][1] == 2, "a (mu | logvar) head over two N tiles")
-    _covers(lambda g: g["fuse_sample"] and g["enc_head"] == (256, 1), "the sampling epilogue on a 256-wide head")
     _covers(lambda g: g["dec_tiles"] >= 2 and g["dec_last"] == 1, "a decoder-head tile holding one feature")
     _covers(lambda g: g["dec_tiles"] == 2 and g["dec_last"] == 128 and g["Xc"] == 272, "two full decoder-head tiles")
     _covers(lambda g: g["dec_tiles"] == 8 and g["hb"] == 128, "the README decoder head (978 = 7 x 128 + 82)")

@@ -198,16 +198,11 @@ def test_table_swap_replays_without_recapture_and_clear_restores():
     _assert_same(a, b, "cleared table vs no table")
 
 
-@pytest.mark.parametrize("schedule", ("chains2", "step_kernel", "fuse_sample"))
-def test_table_under_other_schedules(schedule, monkeypatch):
+@pytest.mark.parametrize("schedule", ("step_kernel",))
+def test_table_under_other_schedules(schedule):
     kind, (arch, wn, N) = "drvae", CASES["readme"]
     base = _distinct_vs_reference(kind, arch, wn, N)
-    if schedule == "fuse_sample":
-        monkeypatch.setenv("DRVAE_B200_FUSE_SAMPLE", "1")  # read at plan creation; the fused sampler needs one chain
-        configure = lambda p: p.set_chains(1)
-    else:
-        configure = (lambda p: p.set_chains(2)) if schedule == "chains2" else (lambda p: p.set_step_kernel(True))
-    other = _distinct_vs_reference(kind, arch, wn, N, configure=configure)
+    other = _distinct_vs_reference(kind, arch, wn, N, configure=lambda p: p.set_step_kernel(True))
     _assert_same(base[3] + base[4], other[3] + other[4], schedule)
 
 

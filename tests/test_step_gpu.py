@@ -745,31 +745,6 @@ def test_pvae_without_pairs_leaves_the_perturbation_block_untouched(path):
 
 
 @pytest.mark.parametrize("kind", KINDS)
-def test_model_range_chains_do_not_change_results(kind):
-    """The step may run sub-ranges of the ensemble as separate stream chains (drvae_set_chains); the grouped
-    weight-gradient + Adam launch at the end covers all models.  1, 2 and 3 ranges over 6 models (distinct weights and
-    batches), plain launches and graph replays: losses and parameters are bit-identical."""
-    arch, N, E = ARCH["tiny"], 36, 6
-    sds = [init_state_dict(kind, seed=SEED_MODEL + m, **arch) for m in range(E)]
-    batches = [batch_fields(kind, orc.synthetic_batch(N, arch["dim_x"], seed=20 + m)) for m in range(E)]
-    big = {k: torch.stack([b[k] for b in batches]).contiguous().cuda() for k in batches[0]}
-    res = {}
-    for chains in (1, 2, 3):
-        plan = Plan(kind, L=L, max_batch=N, n_models=E, **arch)
-        plan.set_chains(chains)
-        for m in range(E):
-            plan.load_state_dict(sds[m], model=m)
-        out = [plan.train_step(big, plan.hparams(step=it, beta_pert=anneal_coef(it, 1, 0)), seed=11).cpu().clone() for it in range(5)]
-        ev = plan.loss_forward(big, plan.hparams(step=5, training=False), seed=11).cpu().clone()
-        res[chains] = (torch.stack(out), plan.params.cpu().clone(), ev)
-        assert plan.graph_replays() >= 2
-    for chains in (2, 3):
-        for a, b in zip(res[1], res[chains]):
-            assert torch.equal(a, b), chains
-    assert not torch.equal(res[1][0][0, 0], res[1][0][0, 1])  # members really differ
-
-
-@pytest.mark.parametrize("kind", KINDS)
 def test_device_resident_dataset_indexing_equals_gathered_batches(kind):
     """drvae_batch_t.row_index: the minibatch as indices into datasets that stay on the device (what the reference's
     fit() does on the host with a sampler + DataLoader) gives bit-identical steps to passing the gathered rows."""
@@ -894,32 +869,3 @@ def test_early_part_of_the_grouped_optimizer_launch_changes_nothing(kind, monkey
         for a, b in zip(res["0"][0], res[sms][0]):
             assert torch.equal(a, b)
         assert torch.equal(res["0"][1], res[sms][1]) and torch.equal(res["0"][2], res[sms][2])
-
-
-@pytest.mark.parametrize("arch_name", ("tiny", "deep"))
-def test_sampling_epilogue_of_the_encoder_head_gemm_equals_the_row_kernel(arch_name, monkeypatch):
-    """EPI_SAMPLE_Q1 (gemm.cuh): DrVAE's reparameterised draws of q(z1|x1) written by the encoder-head GEMM's epilogue
-    instead of sample_q1_kernel (DRVAE_B200_FUSE_SAMPLE=1; off by default, measured slower).  Same arithmetic per element:
-    bit-identical losses and parameters, tensor-core and SIMT mainloops, tape noise and Philox noise."""
-    kind, arch, N, E = "drvae", ARCH[arch_name], 40, 3
-    sds = [init_state_dict(kind, seed=SEED_MODEL + m, **arch) for m in range(E)]
-    batches = [batch_fields(kind, orc.synthetic_batch(N, arch["dim_x"], seed=40 + m)) for m in range(E)]
-    big = {k: torch.stack([b[k] for b in batches]).contiguous().cuda() for k in batches[0]}
-    res = {}
-    for fuse in ("0", "1"):
-        monkeypatch.setenv("DRVAE_B200_FUSE_SAMPLE", fuse)
-        for impl in ("tc", "simt"):
-            plan = Plan(kind, L=L, max_batch=N, n_models=E, **arch)
-            plan.set_gemm_impl(impl)
-            for m in range(E):
-                plan.load_state_dict(sds[m], model=m)
-            l0 = plan.launch_count()
-            losses = [plan.train_step(big, plan.hparams(step=it, beta_pert=anneal_coef(it, 1, 0)), seed=6).cpu().clone() for it in range(4)]
-            ev = plan.loss_forward(big, plan.hparams(step=4, training=False), seed=6).cpu().clone()
-            torch.cuda.synchronize()
-            res[fuse, impl] = (losses, plan.params.cpu().clone(), ev, plan.launch_count() - l0)
-    for impl in ("tc", "simt"):
-        assert res["1", impl][3] < res["0", impl][3]  # fewer launches
-        for a, b in zip(res["0", impl][0], res["1", impl][0]):
-            assert torch.equal(a, b)
-        assert torch.equal(res["0", impl][1], res["1", impl][1]) and torch.equal(res["0", impl][2], res["1", impl][2])

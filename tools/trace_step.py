@@ -2,7 +2,7 @@
 """Timeline of ONE training step as it really ran on the GPU (drvae_trace_begin / _end: every kernel stamps the
 global timer at its first CTA's start and its last CTA's end).  Workload: bench.py's default ensemble shard.
 
-    python tools/trace_step.py [--models 32] [--kind drvae] [--chains K] > profiles/rNN_trace.txt
+    python tools/trace_step.py [--models 32] [--kind drvae] > profiles/rNN_trace.txt
 """
 import argparse
 import os
@@ -25,12 +25,9 @@ def main():
     ap.add_argument("--models", type=int, default=32)
     ap.add_argument("--kind", default="drvae")
     ap.add_argument("--batch", type=int, default=150)
-    ap.add_argument("--chains", type=int, default=0)
     args = ap.parse_args()
     M = args.models
     plan = Plan(args.kind, L=2, max_batch=args.batch, n_models=M, **README)
-    if args.chains:
-        plan.set_chains(args.chains)
     fields = {"drvae": ("x1", "x2", "y", "has_x2", "has_y"), "pvae": ("x1", "x2", "has_x2"), "vfae": ("x1", "y", "has_y")}[args.kind]
     host = {k: [] for k in fields}
     for m in range(M):
