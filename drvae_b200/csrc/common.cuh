@@ -169,12 +169,6 @@ __device__ __forceinline__ void tma_prefetch_map(const void* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"((unsigned long long)map) : "memory");
 }
 
-// L2 prefetch of the cache line holding `p` (per-lane address, no destination register).  Used to
-// pull optimizer state towards L2 ahead of the fused Adam epilogue.
-__device__ __forceinline__ void prefetch_l2(const void* p) {
-  asm volatile("prefetch.global.L2 [%0];" ::"l"(p) : "memory");
-}
-
 // ---------------------------------------------------------------------------------------------
 // tcgen05: TMEM allocation, UMMA issue, commit, TMEM loads
 // ---------------------------------------------------------------------------------------------
@@ -265,19 +259,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-// 32 lanes x 8 consecutive fp32 columns.
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  __syncwarp();
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-
 // Two 16-column loads in flight before one wait (decoder heads: mu and sigma halves of a tile).
 __device__ __forceinline__ void tmem_ld16x2(uint32_t taddr0, uint32_t taddr1, float (&v0)[16], float (&v1)[16]) {
   uint32_t r[16], q[16];
@@ -346,7 +327,7 @@ __device__ __forceinline__ float sigmoid_sp(float x) { return x > 20.f ? 1.f : 1
 // torch.optim.Adam with coupled weight decay (SURVEY.md Appendix A.6; reference DGMMixin.py:31-40):
 //   g <- g + wd p ; m <- b1 m + (1-b1) g ; v <- b2 v + (1-b2) g^2 ;
 //   p <- p - (lr / (1-b1^t)) * m / (sqrt(v) / sqrt(1-b2^t) + eps)
-// One definition for the stand-alone optimizer kernel and the fused gradient epilogues, so both
+// One definition for the stand-alone optimizer kernel and the grouped dW+Adam kernel, so both
 // apply bit-identical updates.  sqrt / divide use the hardware approximations (<= 2 ulp): the
 // update is ~lr in magnitude, so the absolute effect is ~1e-10 per step.
 struct AdamHyper {

@@ -9,8 +9,7 @@
 //   GEMM_DW  weight grad    D[in, out]    = X[rows, in]^T . dY[rows, out]    (A, B MN-major)
 // The weight gradient is produced TRANSPOSED (D row = input feature, D column = output feature)
 // so that the 32 lanes of an epilogue warp (32 consecutive D rows) touch 32 consecutive elements
-// of a row of the reference's [out, in] weight tensor: gradient stores — and, in the fused
-// variant, the whole Adam read-modify-write of p, m, v — are 128-byte coalesced.  Every GEMM
+// of a row of the reference's [out, in] weight tensor: gradient stores are 128-byte coalesced.  Every GEMM
 // input carries a ones column (and the one-hot class columns of [z, onehot(y)] inputs) after its
 // last real feature, so the bias and class-column gradients are rows of the same D tile.
 // Operand tiles are moved global->shared by TMA tensor loads (one box per operand tile and
@@ -18,7 +17,8 @@
 // 8-byte elements, so a box lands in shared memory as the no-swizzle UMMA canonical layout),
 // multiplied with tcgen05.mma (bf16 in, fp32 accumulate in TMEM) by one elected thread, and the
 // accumulator tile is read back with tcgen05.ld by the epilogue warps that apply the layer's
-// epilogue (bias/ELU, ELU', Gaussian log-density + its gradient, Adam, ...).
+// epilogue (bias/ELU, ELU', Gaussian log-density + its gradient, weight gradient, ...).  The weight gradients and
+// Adam of a fused train step are not computed here but in the grouped launch of dwadam.cuh.
 //
 // A slow SIMT kernel with the *same* operand format and the *same* epilogue code is kept as a
 // validation reference for the tensor-core mainloop (tests only; never selected implicitly).
@@ -43,9 +43,7 @@ enum {
   EPI_GRAD = 3,       // weight (+bias, +class column) gradient -> flat fp32 grad buffer, reference tensor layout
   EPI_DECLOSS = 4,    // decoder heads: Gaussian log-density partials + d loss / d pre-activation
   EPI_DECOUT = 5,     // decoder heads at inference: mu and sigma as fp32 row-major
-  EPI_LIN_C8 = 6,     // +bias -> bf16 chunk8 (no activation)
-  EPI_GRAD_ADAM = 7   // as EPI_GRAD, but the gradient never leaves the SM: fused Adam update of p, m, v
-                      // and refresh of the bf16 weight shadow / derived bias in the same epilogue
+  EPI_LIN_C8 = 6      // +bias -> bf16 chunk8 (no activation)
 };
 
 constexpr int GEMM_BM = 128;
@@ -60,8 +58,6 @@ constexpr int GEMM_PROD_WARPS = 3;                     // warps before the MMA w
 constexpr int GEMM_MMA_WARP = GEMM_PROD_WARPS;         // warp 3: MMA issuer; warps 4.. epilogue
 constexpr int GEMM_EPI_WARP0 = GEMM_PROD_WARPS + 1;
 constexpr int GEMM_THREADS = (GEMM_PROD_WARPS + 1 + GEMM_EPI_WARPS) * 32;
-constexpr int GEMM_ADAM_EPI_WARPS = 24;                // the fused dW+Adam epilogue is an HBM stream whose bandwidth scales with
-                                                       // resident warps (profiles/r01_experiments.md): 24 warps at <= 72 registers
 constexpr int GEMM_SIMT_THREADS = 128 * EPI_GROUPS;    // validation kernel: thread = (row, column group)
 constexpr int GEMM_ACC_STAGES = 2;                     // accumulator tiles in TMEM (epilogue of tile i overlaps mainloop of i+1)
 constexpr int GEMM_SMEM_BUDGET = 208 * 1024;           // operand ring per CTA (one CTA per SM)
@@ -94,7 +90,6 @@ struct GemmProblem {
   int M, N, K;      // static upper bounds of D rows / D cols / contraction length
   const int* dyn;   // per-model dynamic extent: rows of D (NT, DX) or contraction rows (DW); may be null
   int dyn_stride;   // ints between models in `dyn`
-  const int* skip;  // optional per-model count (same stride): when it is zero the model's tiles do nothing at all
   int BN;           // N tile (multiple of 16, <= 256)
   int tiles_n;
   int tiles_m;
@@ -137,31 +132,16 @@ struct EpiParams {
   long long act_ms;
   int act_rcap;
   int act_row0;
-  // EPI_GRAD / EPI_GRAD_ADAM: D row = input feature k (k == g_kin: ones column -> bias gradient,
+  // EPI_GRAD: D row = input feature k (k == g_kin: ones column -> bias gradient,
   // k > g_kin: one-hot class columns), D col = shadow row s.  g_tab holds three int tables of
   // g_tab_n entries each, indexed by s: flat offset of W[n(s)][0] (or -1: padding row), flat
   // offset of b[n(s)], and the constant folded into the derived bias (float bits).
   float* grad;
-  long long grad_ms;  // also the model stride of params / adam_m / adam_v
+  long long grad_ms;
   const int* g_tab;
   int g_tab_n;
   int g_kin;      // true input features
   int g_kaug;     // g_kin + 1 + class columns
-  int g_vec;      // EPI_GRAD_ADAM: 4 / 2 = weight rows are 16- / 8-byte aligned (vector epilogue), 1 = scalar epilogue
-  // EPI_GRAD_ADAM
-  float* adam_p;
-  float* adam_m;
-  float* adam_v;
-  bf16* sh;           // this layer's bf16 chunk8 shadow (model 0)
-  long long sh_ms;
-  int sh_rcap;
-  float* drv;         // derived fp32 arena (model 0)
-  long long drv_ms;
-  long long drv_bias_off;
-  long long drv_clsb_off;
-  int drv_clsb_ld;
-  const AdamHyper* adam;  // device memory (StepDyn or the member table): changes every step
-  int adam_ms;            // bytes between the Adam scalars of consecutive models (0: shared)
   // EPI_DECLOSS / EPI_DECOUT
   const float4* tgt4;  // fp32 targets, chunk4 layout [Xc/4][tgt_rcap] float4
   long long tgt_ms;    // float4 elements between models
@@ -323,7 +303,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
                ((long long)(col0 >> 3) * e.out_c8_rcap + e.out_c8_row0 + rc.row);
     o[0] = pack_bf16x8(v);
     o[e.out_c8_rcap] = pack_bf16x8(v + 8);
-  } else if (EPI == EPI_GRAD || EPI == EPI_GRAD_ADAM) {
+  } else if (EPI == EPI_GRAD) {
     const int k = rc.row;  // input feature (or ones / class column)
     if (k >= e.g_kaug || col0 >= e.g_tab_n) return;  // (weight-gradient tiles need not divide the shadow rows)
     // flat parameter index of column i: weight W[n][k], bias b[n] or class column W[n][kin + j]
@@ -336,61 +316,14 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
       const int4 t = tw[i >> 2];
       idx[i] = t.x, idx[i + 1] = t.y, idx[i + 2] = t.z, idx[i + 3] = t.w;
     }
-    if (EPI == EPI_GRAD) {
-      float* g = e.grad + rc.model * e.grad_ms + kofs;
+    float* g = e.grad + rc.model * e.grad_ms + kofs;
 #pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        if (idx[i] >= 0) {
-          if (atomic)
-            atomicAdd(g + idx[i], acc[i]);
-          else
-            g[idx[i]] = acc[i];
-        }
-      }
-    } else {
-      // generic (unpipelined) form, used by the SIMT validation kernel; the tensor-core kernel runs
-      // adam_epilogue_row below.  All 48 loads of the chunk are issued back to back.
-      float* P = e.adam_p + rc.model * e.grad_ms + kofs;
-      float* M1 = e.adam_m + rc.model * e.grad_ms + kofs;
-      float* V2 = e.adam_v + rc.model * e.grad_ms + kofs;
-      const AdamHyper h = adam_of(e.adam, e.adam_ms, rc.model);
-      float pv[16], mv[16], vv[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        pv[i] = mv[i] = vv[i] = 0.f;
-        if (idx[i] >= 0) {
-          pv[i] = ld_global_f32(P + idx[i]);
-          mv[i] = ld_global_f32(M1 + idx[i]);
-          vv[i] = ld_global_f32(V2 + idx[i]);
-        }
-      }
-#pragma unroll
-      for (int i = 0; i < 16; ++i) adam_update(acc[i], pv[i], mv[i], vv[i], h);
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        if (idx[i] >= 0) {
-          P[idx[i]] = pv[i];
-          M1[idx[i]] = mv[i];
-          V2[idx[i]] = vv[i];
-        }
-      }
-      // kernel-facing copies
-      if (k < e.g_kin) {
-        bf16* sh = e.sh + rc.model * e.sh_ms + ((long long)(k >> 3) * e.sh_rcap + col0) * 8 + (k & 7);
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          if (idx[i] >= 0) sh[i * 8] = __float2bfloat16_rn(pv[i]);
-      } else if (k == e.g_kin) {
-        float* d = e.drv + rc.model * e.drv_ms + e.drv_bias_off + col0;
-        const float* bc = reinterpret_cast<const float*>(e.g_tab + 2 * e.g_tab_n + col0);
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          if (idx[i] >= 0) d[i] = pv[i] + bc[i];
-      } else {
-        float* d = e.drv + rc.model * e.drv_ms + e.drv_clsb_off + (long long)(k - e.g_kin - 1) * e.drv_clsb_ld + col0;
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          if (idx[i] >= 0) d[i] = pv[i];
+    for (int i = 0; i < 16; ++i) {
+      if (idx[i] >= 0) {
+        if (atomic)
+          atomicAdd(g + idx[i], acc[i]);
+        else
+          g[idx[i]] = acc[i];
       }
     }
   }
@@ -567,7 +500,6 @@ __device__ __forceinline__ TileInfo gemm_tile_info(const GemmProblem& p, int til
   t.kb_begin = min(nkb, ks * per);
   t.kb_end = min(nkb, t.kb_begin + per);
   t.active = t.m0 < t.Mrows && (t.kb_end > t.kb_begin || ks == 0);
-  if (p.skip && p.skip[(long long)t.model * p.dyn_stride] == 0) t.active = false;
   return t;
 }
 
@@ -603,333 +535,19 @@ __device__ __forceinline__ void run_epilogue_row(const GemmProblem& p, const Epi
 }
 
 // ---------------------------------------------------------------------------------------------
-// Fused weight-gradient + Adam epilogue of the tensor-core kernel, software-pipelined.
-// A thread owns D row k (one input feature) and the columns of its group in half-chunks of 8
-// shadow rows.  For each half-chunk it streams p, m, v of 8 reference-weight elements W[n][k]
-// (lanes = consecutive k: 128-byte coalesced), applies Adam to the accumulator column and writes
-// p, m, v, the bf16 shadow and the derived bias back.  The loads of half-chunk h+1 are in flight
-// while h is computed and stored, and the first half-chunk is requested BEFORE the wait on the
-// accumulator barrier, i.e. while the MMA mainloop is still running.
-// ---------------------------------------------------------------------------------------------
-struct AdamBuf {
-  int idx[8];
-  float p[8], m[8], v[8];
-};
-
-__device__ __forceinline__ void adam_pipe_load(const EpiParams& e, int model, int k, int kofs, int col, AdamBuf& b) {
-  if (k >= e.g_kaug) return;
-  const int4* tw = reinterpret_cast<const int4*>(e.g_tab + (k == e.g_kin ? e.g_tab_n : 0) + col);
-  const int4 t0 = tw[0], t1 = tw[1];
-  b.idx[0] = t0.x, b.idx[1] = t0.y, b.idx[2] = t0.z, b.idx[3] = t0.w;
-  b.idx[4] = t1.x, b.idx[5] = t1.y, b.idx[6] = t1.z, b.idx[7] = t1.w;
-  const float* P = e.adam_p + model * e.grad_ms + kofs;
-  const float* M1 = e.adam_m + model * e.grad_ms + kofs;
-  const float* V2 = e.adam_v + model * e.grad_ms + kofs;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    b.p[i] = b.m[i] = b.v[i] = 0.f;
-    if (b.idx[i] >= 0) {
-      b.p[i] = ld_global_f32(P + b.idx[i]);
-      b.m[i] = ld_global_f32(M1 + b.idx[i]);
-      b.v[i] = ld_global_f32(V2 + b.idx[i]);
-    }
-  }
-}
-
-__device__ __forceinline__ void adam_pipe_apply(const EpiParams& e, int model, int k, int kofs, int col, uint32_t taddr,
-                                                bool have_acc, AdamBuf& b) {
-  float acc[8];
-  if (have_acc) {
-    tmem_ld8(taddr, acc);  // warp-collective: executed by every lane, including rows beyond kaug
-  } else {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) acc[i] = 0.f;
-  }
-  if (k >= e.g_kaug) return;
-  const AdamHyper h = adam_of(e.adam, e.adam_ms, model);
-#pragma unroll
-  for (int i = 0; i < 8; ++i) adam_update(acc[i], b.p[i], b.m[i], b.v[i], h);
-  float* P = e.adam_p + model * e.grad_ms + kofs;
-  float* M1 = e.adam_m + model * e.grad_ms + kofs;
-  float* V2 = e.adam_v + model * e.grad_ms + kofs;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    if (b.idx[i] >= 0) {
-      P[b.idx[i]] = b.p[i];
-      M1[b.idx[i]] = b.m[i];
-      V2[b.idx[i]] = b.v[i];
-    }
-  }
-  if (k < e.g_kin) {
-    bf16* sh = e.sh + model * e.sh_ms + ((long long)(k >> 3) * e.sh_rcap + col) * 8 + (k & 7);
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-      if (b.idx[i] >= 0) sh[i * 8] = __float2bfloat16_rn(b.p[i]);
-  } else if (k == e.g_kin) {
-    float* d = e.drv + model * e.drv_ms + e.drv_bias_off + col;
-    const float* bc = reinterpret_cast<const float*>(e.g_tab + 2 * e.g_tab_n + col);
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-      if (b.idx[i] >= 0) d[i] = b.p[i] + bc[i];
-  } else {
-    float* d = e.drv + model * e.drv_ms + e.drv_clsb_off + (long long)(k - e.g_kin - 1) * e.drv_clsb_ld + col;
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-      if (b.idx[i] >= 0) d[i] = b.p[i];
-  }
-}
-
-constexpr int ADAM_PREFETCH_DIST = 4;  // half-chunks of optimizer state requested into L2 ahead of their loads
-
-// GROUPS column groups share the tile's half-chunks (8 shadow rows each) round-robin.  With 4 groups
-// (16 epilogue warps, 96 registers) the loads are double-buffered in registers; with more groups
-// (24 warps, 72 registers) each warp keeps one half-chunk in flight and the extra warps provide the
-// memory-level parallelism.
-template <int GROUPS>
-__device__ __forceinline__ void adam_epilogue_row(const GemmProblem& p, const EpiParams& e, const TileInfo& t, int cg, int k,
-                                                  uint32_t taddr_row, bool have_acc, uint64_t* acc_bar, uint32_t acc_parity) {
-  const int nhc = min(p.BN, e.g_tab_n - t.n0) >> 3;                // half-chunks of shadow rows that exist in the tile
-  const int nh = nhc > cg ? (nhc - cg + GROUPS - 1) / GROUPS : 0;  // half-chunks of this column group
-  const int kofs = (k < e.g_kin) ? k : (k == e.g_kin ? 0 : k - 1);
-  auto lcol = [&](int h) { return (cg + h * GROUPS) * 8; };  // tile-local column of this group's h-th half-chunk
-  // L2 prefetch of half-chunk h for the whole warp: lane j < 24 requests the warp's 32-feature
-  // (128-byte) segment of array j % 3 (p, m, v) in weight row j / 3 — first and last byte, the
-  // segment may straddle two lines — so the later per-thread loads find their lines in L2 instead
-  // of paying the loaded DRAM latency with registers held
-  const int lane = threadIdx.x & 31;
-  const int k0 = k - lane;  // first feature of this warp
-  auto prefetch = [&](int h) {
-    if (h >= nh || lane >= 24 || k0 >= e.g_kin) return;
-    const int widx = e.g_tab[t.n0 + lcol(h) + lane / 3];
-    if (widx < 0) return;
-    const int a = lane % 3;
-    const float* base = (a == 0 ? e.adam_p : (a == 1 ? e.adam_m : e.adam_v)) + t.model * e.grad_ms + widx + k0;
-    prefetch_l2(base);
-    prefetch_l2(base + min(32, e.g_kin - k0) - 1);
-  };
-  if (GROUPS == EPI_GROUPS) {
-    AdamBuf A, B;
-    if (nh > 0) adam_pipe_load(e, t.model, k, kofs, t.n0 + lcol(0), A);
-#pragma unroll
-    for (int d = 1; d <= ADAM_PREFETCH_DIST; ++d) prefetch(d);
-    if (lane == 0) mbar_wait(acc_bar, acc_parity, p.dbg, 0xA0000000u);  // one poller per warp
-    __syncwarp();
-    tc_fence_after();
-    for (int h = 0; h < nh; h += 2) {
-      prefetch(h + 1 + ADAM_PREFETCH_DIST);
-      if (h + 1 < nh) adam_pipe_load(e, t.model, k, kofs, t.n0 + lcol(h + 1), B);
-      adam_pipe_apply(e, t.model, k, kofs, t.n0 + lcol(h), taddr_row + lcol(h), have_acc, A);
-      prefetch(h + 2 + ADAM_PREFETCH_DIST);
-      if (h + 2 < nh) adam_pipe_load(e, t.model, k, kofs, t.n0 + lcol(h + 2), A);
-      if (h + 1 < nh) adam_pipe_apply(e, t.model, k, kofs, t.n0 + lcol(h + 1), taddr_row + lcol(h + 1), have_acc, B);
-    }
-  } else {
-    AdamBuf A;
-    if (nh > 0) adam_pipe_load(e, t.model, k, kofs, t.n0 + lcol(0), A);
-#pragma unroll
-    for (int d = 1; d <= ADAM_PREFETCH_DIST; ++d) prefetch(d);
-    if (lane == 0) mbar_wait(acc_bar, acc_parity, p.dbg, 0xA0000000u);
-    __syncwarp();
-    tc_fence_after();
-    for (int h = 0; h < nh; ++h) {
-      prefetch(h + 1 + ADAM_PREFETCH_DIST);
-      adam_pipe_apply(e, t.model, k, kofs, t.n0 + lcol(h), taddr_row + lcol(h), have_acc, A);
-      if (h + 1 < nh) adam_pipe_load(e, t.model, k, kofs, t.n0 + lcol(h + 1), A);
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Vectorised form of the fused weight-gradient + Adam epilogue (the default; the scalar form above
-// remains for layers whose weight rows are not 16-byte aligned).  After tcgen05.ld a thread
-// holds 8 columns (weight rows) of ONE input feature k; a 4x4 transpose inside each lane quad
-// (4 shuffles per 4 columns) turns that into 4 CONSECUTIVE k of 2 weight rows, so the optimizer
-// state streams as 16-byte accesses: 6 LDG.128 + 6 STG.128 (+ 2 x 8-byte bf16 shadow stores) per
-// thread and half-chunk instead of 24 + 24 (+ 8) scalar ones for the same bytes.  Memory-level
-// parallelism per resident warp is 4x that of the scalar form, which is what the HBM stream of
-// this kernel is limited by (tools/adam_pattern_bench.cu: 3.6-4.2 -> 4.8 TB/s in this geometry).
-// Used when the weight rows are 16-byte aligned (ld % 4 == 0).  Measured on B200 (32 models,
-// profiles/r01_experiments.md): decoder heads 261 -> 226 us; with 8-byte aligned rows (ld = 978 or
-// 102) an 8-byte variant of this epilogue was slower than the scalar one (166 -> 183 us), so those
-// layers keep the scalar epilogue.  The ragged end of the feature range (k4 + 3 >= kin:
-// last partial quad, the bias row k == kin and the class columns k > kin) is loaded / stored
-// element-wise into the same registers.
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void quad_transpose4(const float (&x)[4], float (&y)[4], int lane) {
-  const bool hi2 = lane & 2, hi1 = lane & 1;
-  const float r0 = __shfl_xor_sync(0xffffffffu, hi2 ? x[0] : x[2], 2);
-  const float r1 = __shfl_xor_sync(0xffffffffu, hi2 ? x[1] : x[3], 2);
-  const float z0 = hi2 ? r0 : x[0], z1 = hi2 ? r1 : x[1], z2 = hi2 ? x[2] : r0, z3 = hi2 ? x[3] : r1;
-  const float u0 = __shfl_xor_sync(0xffffffffu, hi1 ? z0 : z1, 1);
-  const float u1 = __shfl_xor_sync(0xffffffffu, hi1 ? z2 : z3, 1);
-  const float k0 = hi1 ? z1 : z0, k1 = hi1 ? z3 : z2;
-  y[0] = hi1 ? u0 : k0;
-  y[1] = hi1 ? k0 : u0;
-  y[2] = hi1 ? u1 : k1;
-  y[3] = hi1 ? k1 : u1;
-}
-
-struct AdamVecBuf {
-  int idx[2];  // flat offset of W[n][0] for this thread's two weight rows (or -1)
-  float4 p[2], m[2], v[2];
-};
-
-__device__ __forceinline__ float4 ld_state(const float* a) { return *reinterpret_cast<const float4*>(a); }
-__device__ __forceinline__ void st_state(float* a, const float4& x) { *reinterpret_cast<float4*>(a) = x; }
-
-// Ragged end of the feature range (quads with k4 + 3 >= kin: last weights, the bias row k == kin, class columns
-// k > kin): element offset inside the flat per-model vector, or -1.  s = shadow row.
-__device__ __forceinline__ int adam_edge_off(const EpiParams& e, int k, int s) {
-  if (k >= e.g_kaug) return -1;
-  const int idx = e.g_tab[(k == e.g_kin ? e.g_tab_n : 0) + s];
-  if (idx < 0) return -1;
-  return idx + ((k < e.g_kin) ? k : (k == e.g_kin ? 0 : k - 1));
-}
-__device__ __forceinline__ float& f4c(float4& x, int r) { return r == 0 ? x.x : (r == 1 ? x.y : (r == 2 ? x.z : x.w)); }
-
-// request p, m, v of this thread's two weight rows, features [k4, k4 + 4); col = first shadow row of the half-chunk.
-// Ragged quads fill the same registers with scalar loads, so they are pipelined like the vector path.
-__device__ __forceinline__ void adam_vec_load(const EpiParams& e, int model, int k4, int col, int ci, AdamVecBuf& b) {
-  const float* P = e.adam_p + model * e.grad_ms;
-  const float* M1 = e.adam_m + model * e.grad_ms;
-  const float* V2 = e.adam_v + model * e.grad_ms;
-#pragma unroll
-  for (int j = 0; j < 2; ++j) b.p[j] = b.m[j] = b.v[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (k4 + 3 < e.g_kin) {
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      b.idx[j] = e.g_tab[col + 4 * j + ci];
-      if (b.idx[j] >= 0) {
-        const int o = b.idx[j] + k4;
-        b.p[j] = ld_state(P + o);
-        b.m[j] = ld_state(M1 + o);
-        b.v[j] = ld_state(V2 + o);
-      }
-    }
-  } else if (k4 < e.g_kaug) {
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        const int o = adam_edge_off(e, k4 + r, col + 4 * j + ci);
-        if (o >= 0) {
-          f4c(b.p[j], r) = ld_global_f32(P + o);
-          f4c(b.m[j], r) = ld_global_f32(M1 + o);
-          f4c(b.v[j], r) = ld_global_f32(V2 + o);
-        }
-      }
-    }
-  }
-}
-
-__device__ __forceinline__ void adam_vec_apply(const EpiParams& e, int model, int k4, int col, int ci, int lane, uint32_t taddr,
-                                               bool have_acc, AdamVecBuf& b) {
-  float acc[8];
-  if (have_acc) {
-    tmem_ld8(taddr, acc);  // warp-collective
-  } else {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) acc[i] = 0.f;
-  }
-  float g[2][4];
-  {
-    const float x0[4] = {acc[0], acc[1], acc[2], acc[3]}, x1[4] = {acc[4], acc[5], acc[6], acc[7]};
-    quad_transpose4(x0, g[0], lane);
-    quad_transpose4(x1, g[1], lane);
-  }
-  if (k4 >= e.g_kaug) return;
-  const AdamHyper h = adam_of(e.adam, e.adam_ms, model);
-#pragma unroll
-  for (int j = 0; j < 2; ++j) {
-    adam_update(g[j][0], b.p[j].x, b.m[j].x, b.v[j].x, h);
-    adam_update(g[j][1], b.p[j].y, b.m[j].y, b.v[j].y, h);
-    adam_update(g[j][2], b.p[j].z, b.m[j].z, b.v[j].z, h);
-    adam_update(g[j][3], b.p[j].w, b.m[j].w, b.v[j].w, h);
-  }
-  float* P = e.adam_p + model * e.grad_ms;
-  float* M1 = e.adam_m + model * e.grad_ms;
-  float* V2 = e.adam_v + model * e.grad_ms;
-  if (k4 + 3 < e.g_kin) {
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      if (b.idx[j] < 0) continue;
-      const int o = b.idx[j] + k4;
-      st_state(P + o, b.p[j]);
-      st_state(M1 + o, b.m[j]);
-      st_state(V2 + o, b.v[j]);
-      const int s = col + 4 * j + ci;
-      uint2 pk;
-      pk.x = pack_bf16x2(b.p[j].x, b.p[j].y);
-      pk.y = pack_bf16x2(b.p[j].z, b.p[j].w);
-      *reinterpret_cast<uint2*>(e.sh + model * e.sh_ms + ((long long)(k4 >> 3) * e.sh_rcap + s) * 8 + (k4 & 7)) = pk;
-    }
-  } else {
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      const int s = col + 4 * j + ci;
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        const int k = k4 + r;
-        const int o = adam_edge_off(e, k, s);
-        if (o < 0) continue;
-        const float pv = f4c(b.p[j], r);
-        P[o] = pv;
-        M1[o] = f4c(b.m[j], r);
-        V2[o] = f4c(b.v[j], r);
-        if (k < e.g_kin) {
-          e.sh[model * e.sh_ms + ((long long)(k >> 3) * e.sh_rcap + s) * 8 + (k & 7)] = __float2bfloat16_rn(pv);
-        } else if (k == e.g_kin) {
-          e.drv[model * e.drv_ms + e.drv_bias_off + s] = pv + reinterpret_cast<const float*>(e.g_tab + 2 * e.g_tab_n)[s];
-        } else {
-          e.drv[model * e.drv_ms + e.drv_clsb_off + (long long)(k - e.g_kin - 1) * e.drv_clsb_ld + s] = pv;
-        }
-      }
-    }
-  }
-}
-
-template <int GROUPS>
-__device__ __forceinline__ void adam_epilogue_vec(const GemmProblem& p, const EpiParams& e, const TileInfo& t, int cg, int kbase,
-                                                  uint32_t taddr_row, bool have_acc, uint64_t* acc_bar, uint32_t acc_parity) {
-  const int lane = threadIdx.x & 31;
-  const int ci = lane & 3, k4 = kbase + (lane >> 2) * 4;
-  const int nhc = min(p.BN, e.g_tab_n - t.n0) >> 3;  // half-chunks of shadow rows that exist (the last tile may be ragged)
-  const int nh = nhc > cg ? (nhc - cg + GROUPS - 1) / GROUPS : 0;
-  auto lcol = [&](int h) { return (cg + h * GROUPS) * 8; };
-  AdamVecBuf A;
-  if (nh > 0) adam_vec_load(e, t.model, k4, t.n0 + lcol(0), ci, A);
-  if (lane == 0) {
-    constexpr int EPI = EPI_GRAD_ADAM;
-    (void)EPI;
-    WS_T0();
-    mbar_wait(acc_bar, acc_parity, p.dbg, 0xA0000000u);
-    if ((threadIdx.x >> 5) == GEMM_EPI_WARP0) WS_ADD(WS_EPI_ACC_FULL);
-  }
-  __syncwarp();
-  tc_fence_after();
-  // one half-chunk in flight per warp: 24 warps x 72 registers provide the memory-level parallelism (a 16-warp,
-  // 96-register variant with double-buffered loads measured slower: 254 vs 226 us on the decoder heads)
-  for (int h = 0; h < nh; ++h) {
-    adam_vec_apply(e, t.model, k4, t.n0 + lcol(h), ci, lane, taddr_row + lcol(h), have_acc, A);
-    if (h + 1 < nh) adam_vec_load(e, t.model, k4, t.n0 + lcol(h + 1), ci, A);
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
 // Tensor-core kernel: persistent (one CTA per SM, tiles strided by gridDim.x) and warp-specialised.
 //   warp 0        producer: TMA tensor loads of the operand tiles -> shared-memory ring (full/empty mbarriers)
 //   warps 1..2    idle
 //   warp 3        one elected lane issues tcgen05.mma into one of two TMEM accumulator tiles; owns TMEM
-//   warps 4..     epilogue (16, or 24 for the fused Adam): warp w reads TMEM lanes [32(w%4), +32), columns of group (w-4)/4
-// The accumulator is double-buffered (acc_full / acc_empty mbarriers), so the epilogue of tile i —
-// for the weight gradients a long HBM-bound Adam stream — overlaps the mainloop of tile i+1.
+//   warps 4..     epilogue (GEMM_EPI_WARPS): warp w reads TMEM lanes [32(w%4), +32), columns of group (w-4)/4
+// The accumulator is double-buffered (acc_full / acc_empty mbarriers), so the epilogue of tile i overlaps the
+// mainloop of tile i+1.
 // ---------------------------------------------------------------------------------------------
-// VEC (EPI_GRAD_ADAM only): vector width of the optimizer-state accesses, 4 (adam_epilogue_vec) or 1 (adam_epilogue_row)
-template <int EPI, int EW, int VEC>
-__global__ void __launch_bounds__((GEMM_PROD_WARPS + 1 + EW) * 32, 1) gemm_tc_kernel(const GemmProblem p, const EpiParams e,
-                                                                                     const __grid_constant__ CUtensorMap tmA,
-                                                                                     const __grid_constant__ CUtensorMap tmB,
-                                                                                     const __grid_constant__ CUtensorMap tmB2) {
+template <int EPI>
+__global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const GemmProblem p, const EpiParams e,
+                                                                 const __grid_constant__ CUtensorMap tmA,
+                                                                 const __grid_constant__ CUtensorMap tmB,
+                                                                 const __grid_constant__ CUtensorMap tmB2) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t full_bar[GEMM_MAX_STAGES];
   __shared__ __align__(8) uint64_t empty_bar[GEMM_MAX_STAGES];
@@ -957,7 +575,7 @@ __global__ void __launch_bounds__((GEMM_PROD_WARPS + 1 + EW) * 32, 1) gemm_tc_ke
     }
     for (int a = 0; a < GEMM_ACC_STAGES; ++a) {
       mbar_init(&acc_full[a], 1);
-      mbar_init(&acc_empty[a], EW);
+      mbar_init(&acc_empty[a], GEMM_EPI_WARPS);
     }
     mbar_fence_init();
   }
@@ -1133,26 +751,19 @@ __global__ void __launch_bounds__((GEMM_PROD_WARPS + 1 + EW) * 32, 1) gemm_tc_ke
       const uint32_t a = j & 1, aph = (j >> 1) & 1;
       const bool have_acc = t.kb_end > t.kb_begin;
       const uint32_t taddr_row = tmem_base + a * ncols + ((uint32_t)(q * 32) << 16);
-      if (EPI == EPI_GRAD_ADAM) {
-        if (VEC == 4)
-          adam_epilogue_vec<EW / 4>(p, e, t, cg, t.m0 + q * 32, taddr_row, have_acc, &acc_full[a], aph);
-        else
-          adam_epilogue_row<EW / 4>(p, e, t, cg, t.m0 + q * 32 + lane, taddr_row, have_acc, &acc_full[a], aph);
-      } else {
-        if (lane == 0) {
-          WS_T0();
-          mbar_wait(&acc_full[a], aph, p.dbg, 0xA0000000u | tile);  // one poller per warp
-          if (warp == GEMM_EPI_WARP0) WS_ADD(WS_EPI_ACC_FULL);
-        }
-        __syncwarp();
-        tc_fence_after();
-        RowCtx rc;
-        rc.model = t.model;
-        rc.row = t.m0 + q * 32 + lane;
-        rc.cg = cg;
-        rc.valid = rc.row < t.Mrows;
-        run_epilogue_row<EPI>(p, e, t, rc, taddr_row, have_acc, p.ksplit > 1);
+      if (lane == 0) {
+        WS_T0();
+        mbar_wait(&acc_full[a], aph, p.dbg, 0xA0000000u | tile);  // one poller per warp
+        if (warp == GEMM_EPI_WARP0) WS_ADD(WS_EPI_ACC_FULL);
       }
+      __syncwarp();
+      tc_fence_after();
+      RowCtx rc;
+      rc.model = t.model;
+      rc.row = t.m0 + q * 32 + lane;
+      rc.cg = cg;
+      rc.valid = rc.row < t.Mrows;
+      run_epilogue_row<EPI>(p, e, t, rc, taddr_row, have_acc, p.ksplit > 1);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&acc_empty[a]);
@@ -1322,7 +933,7 @@ inline cudaError_t gemm_make_maps(const GemmProblem& p, int n_models, CUtensorMa
   return err;
 }
 
-template <int EPI, int VEC = 1>
+template <int EPI>
 inline cudaError_t gemm_launch_t(GemmProblem p, const EpiParams& e, int n_models, int impl, cudaStream_t st) {
   p.n_models = n_models;
   const int total = p.tiles_n * p.tiles_m * p.ksplit * n_models;
@@ -1331,20 +942,13 @@ inline cudaError_t gemm_launch_t(GemmProblem p, const EpiParams& e, int n_models
     return cudaGetLastError();
   }
   p.nstages = gemm_pick_stages(p.BN);
-  // weight-gradient tiles have short contractions (batch rows) and a long HBM-bound epilogue whose
-  // streaming loads/stores go through L1: a shallow operand ring leaves the rest of the 256 KB as L1.
-  // Only when a CTA runs several tiles, though: with at most one tile per CTA (small layers) nothing hides the
-  // mainloop, and a deeper ring shortens its exposed TMA latency chain.
-  if (EPI == EPI_GRAD_ADAM && p.nstages > 2 && total > gemm_num_sms()) p.nstages = 2;
   size_t smem = (size_t)p.nstages * (GEMM_A_STAGE_BYTES + p.BN * GEMM_BK * 2);
-  // fused Adam epilogue (scalar and vector form): 24 warps x 72 registers, its HBM stream scales with resident warps
-  constexpr int EW = (EPI == EPI_GRAD_ADAM) ? GEMM_ADAM_EPI_WARPS : GEMM_EPI_WARPS;
   // (function attributes are per device: one process may drive several GPUs)
   static bool attr_set[64] = {};
   const int dev = gemm_current_device();
   if (!attr_set[dev]) {
     cudaError_t err =
-        cudaFuncSetAttribute(gemm_tc_kernel<EPI, EW, VEC>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BUDGET + 4096);
+        cudaFuncSetAttribute(gemm_tc_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BUDGET + 4096);
     if (err != cudaSuccess) return err;
     attr_set[dev] = true;
   }
@@ -1354,7 +958,7 @@ inline cudaError_t gemm_launch_t(GemmProblem p, const EpiParams& e, int n_models
   if (err != cudaSuccess) return err;
   int grid = total < gemm_num_sms() ? total : gemm_num_sms();  // persistent: one CTA per SM
   if (p.max_ctas > 0 && grid > p.max_ctas) grid = p.max_ctas;
-  return launch_k(gemm_tc_kernel<EPI, EW, VEC>, dim3(grid), dim3((GEMM_PROD_WARPS + 1 + EW) * 32), smem, st, p, e, tmA, tmB, tmB2);
+  return launch_k(gemm_tc_kernel<EPI>, dim3(grid), dim3(GEMM_THREADS), smem, st, p, e, tmA, tmB, tmB2);
 }
 
 inline cudaError_t gemm_launch(int epi, const GemmProblem& p, const EpiParams& e, int n_models, int impl,
@@ -1365,9 +969,6 @@ inline cudaError_t gemm_launch(int epi, const GemmProblem& p, const EpiParams& e
     case EPI_LIN_C8: return gemm_launch_t<EPI_LIN_C8>(p, e, n_models, impl, st);
     case EPI_DACT_C8: return gemm_launch_t<EPI_DACT_C8>(p, e, n_models, impl, st);
     case EPI_GRAD: return gemm_launch_t<EPI_GRAD>(p, e, n_models, impl, st);
-    case EPI_GRAD_ADAM:
-      if (impl != GEMM_IMPL_SIMT && e.g_vec == 4) return gemm_launch_t<EPI_GRAD_ADAM, 4>(p, e, n_models, impl, st);
-      return gemm_launch_t<EPI_GRAD_ADAM>(p, e, n_models, impl, st);
     case EPI_DECLOSS: return gemm_launch_t<EPI_DECLOSS>(p, e, n_models, impl, st);
     case EPI_DECOUT: return gemm_launch_t<EPI_DECOUT>(p, e, n_models, impl, st);
   }

@@ -62,7 +62,6 @@ struct drvae_plan {
   Seg* d_segs = nullptr;
   std::vector<int> h_tabs;  // gradient-epilogue tables of every weight (see make_shadow)
   int* d_tabs = nullptr;
-  int adam_vec_max = 4;       // debug knob (DRVAE_B200_ADAM_VEC): cap on the vector width of the fused Adam epilogue
   bool wn = false;            // layers.WeightNormLinear instead of nn.Linear
   std::vector<WnRow> wn_rows;
   WnRow* d_wn_rows = nullptr;
@@ -140,7 +139,6 @@ struct drvae_plan {
   int dwa_tiles = 0;
   bool dwa_ok = false;       // every layer fits the kernel's layout conditions and the state is bound
   unsigned long long* d_dwa_stats = nullptr;  // drvae_debug_dwa_stats
-  bool dwa_enabled = true;   // measurement knob (DRVAE_B200_DWADAM=0: per-layer fused kernels of round 1)
   // Early part of the grouped launch: the decoder heads (half of the optimizer state) have all their inputs once the
   // decoder's dX GEMM has run; their tiles start then, on dwa_early_sms SMs, next to the latency-bound rest of the
   // backward chain (whose persistent GEMMs are capped to the remaining SMs).  0: one launch at the end.
@@ -182,8 +180,9 @@ int add_tensor(drvae_plan* pl, const std::string& name, int rows, int cols) {
   t.name = name;
   t.rows = rows;
   t.cols = cols;
-  // every tensor starts on a 16-byte boundary of the flat vector (vector accesses of the fused Adam epilogue); the
-  // padding elements are zero parameters with zero gradients and stay zero
+  // every tensor starts on a 16-byte boundary of the flat vector (TMA boxes of the grouped dW+Adam launch address
+  // the optimizer state from 16-byte aligned tensor starts); the padding elements are zero parameters with zero
+  // gradients and stay zero
   pl->P = round_up(pl->P, 4);
   t.off = pl->P;
   // matrix rows are 16-byte aligned as well (row stride = cols rounded up to 4 floats): the optimizer state of a
@@ -611,8 +610,6 @@ extern "C" int drvae_plan_create_clf(const drvae_arch_t* a, int n_clf, const int
   cudaMemset(pl->arena, 0, pl->arena_bytes);
   cudaMalloc(&pl->d_dyn, sizeof(StepDyn));
   cudaMemset(pl->d_dyn, 0, sizeof(StepDyn));
-  if (const char* knob = getenv("DRVAE_B200_ADAM_VEC")) pl->adam_vec_max = atoi(knob);  // measurement knob
-  if (const char* knob = getenv("DRVAE_B200_DWADAM")) pl->dwa_enabled = atoi(knob) != 0;
   if (const char* knob = getenv("DRVAE_B200_STEPK")) pl->stepk_enabled = atoi(knob) != 0;
   if (const char* knob = getenv("DRVAE_B200_DWA_EARLY_SMS")) pl->dwa_early_sms = std::max(0, atoi(knob));
   cudaMalloc(&pl->d_stepk_bar, 2 * sizeof(unsigned int));
@@ -826,9 +823,10 @@ extern "C" int drvae_debug_side_delay(drvae_plan_t* pl, long long cycles) {
 
 namespace {
 
-// Layer table + tensor maps of the grouped dW+Adam launch.  Leaves pl->dwa_ok false (-> per-layer kernels) when the
-// optimizer state is not bound, with weight norm (the update acts on (v, g)), or when a layer does not meet the
-// kernel's layout conditions (class columns must share the 128-feature tile of the ones column).
+// Layer table + tensor maps of the grouped dW+Adam launch.  Leaves pl->dwa_ok false (-> train steps run gradient +
+// stand-alone Adam) when the optimizer state is not bound, with weight norm (the update acts on (v, g)), with more
+// than DWA_MAX_LAYERS layers, or when a layer does not meet the kernel's layout conditions (class columns must share
+// the 128-feature tile of the ones column).
 int build_dwa(drvae_plan* pl) {
   pl->dwa_ok = false;
   pl->dwa_layers.clear();
@@ -986,9 +984,9 @@ struct Exec {
   cudaError_t err = cudaSuccess;
   const char* phase = "";
   std::string sub = "head";  // layer within the current block: h0, h1, ..., head
-  bool fused = false;        // Adam inside the gradient epilogues (drvae_train_step)
-  bool splitk = false;       // split-K weight gradients (large minibatches, unfused path)
-  bool defer_dw = false;     // weight gradients + Adam of every layer in ONE launch at the end of backward (dwadam.cuh)
+  bool splitk = false;       // split-K weight gradients (large minibatches, gradient path)
+  bool defer_dw = false;     // fused train step: weight gradients + Adam of every layer in ONE launch at the end of
+                             // backward (dwadam.cuh) instead of the per-layer gradient GEMMs
   StepRecorder* rec = nullptr;  // non-null: launches are recorded as ops of the persistent step kernel (stepk.cuh)
   // stand-alone weight-gradient GEMMs (gradient path: they feed nothing but the optimizer / the gradient exchange) leave
   // the dX chain for this stream; each waits for what has been enqueued on the chain's stream so far (its dY and input)
@@ -1105,11 +1103,10 @@ struct Exec {
     launch(epi, p, e, ("gemm_dx." + sub).c_str());
   }
   // grad W^T[kaug, nout] = Xin[rows, kaug]^T . dY[rows, nout]: weight, bias (ones column) and class-column
-  // gradients of one layer; with `fused` the epilogue applies Adam instead of storing the gradient.
-  void gemm_dw(const C8Buf& dY, const C8Buf& Xin, int x_row0, const Shadow& W, int dyn_which, int row_bound, int skip_which = -1) {
+  // gradients of one layer into the gradient buffer.
+  void gemm_dw(const C8Buf& dY, const C8Buf& Xin, int x_row0, const Shadow& W, int dyn_which, int row_bound) {
     if (defer_dw) return;
     GemmProblem p{};
-    if (skip_which >= 0 && fused) p.skip = cnt(skip_which);  // (unfused: the zero gradient is stored, adam_kernel skips)
     p.A = op_c8(Xin, x_row0);
     p.B = op_c8(dY, 0);
     p.mode = GEMM_DW;
@@ -1122,24 +1119,7 @@ struct Exec {
     p.tiles_n = W.tiles_n;
     p.tiles_m = cdiv(W.kaug, GEMM_BM);
     p.ksplit = 1;
-    if (fused) {
-      // Small layers: a 128 x 208 tile per model leaves most SMs idle and makes every epilogue warp walk its
-      // half-chunks one HBM round trip at a time.  Pick the tile width that minimises (waves of the persistent
-      // grid) x (time of one tile ~ fixed mainloop / latency part + epilogue part proportional to the width);
-      // constants from the measured 25 us of a full 128 x 256 tile.
-      const int nsm = gemm_num_sms();
-      int best_bn = p.BN;
-      float best = 1e30f;
-      for (int bn : {W.BN, 128, 64}) {
-        if (bn > W.BN) continue;
-        const int tiles = p.tiles_m * cdiv(W.rcap, bn) * pl->E;
-        const float cost = (float)cdiv(tiles, nsm) * (6.f + 20.f * (float)bn / 256.f);
-        if (cost < best * 0.97f) best = cost, best_bn = bn;
-      }
-      p.BN = best_bn;
-      p.tiles_n = cdiv(W.rcap, best_bn);
-    }
-    if (splitk && !fused) {
+    if (splitk) {
       // large minibatch, few weight tiles: split the contraction (rows) so the persistent grid is filled;
       // partial tiles accumulate with red.global.add into the gradient buffer zeroed at the start of the step
       const int nkb = cdiv(row_bound, GEMM_BK);
@@ -1154,27 +1134,7 @@ struct Exec {
     e.g_tab_n = W.rcap;
     e.g_kin = W.kin;
     e.g_kaug = W.kaug;
-    if (fused) {
-      // vector width of the optimizer-state accesses: weight rows W[n][:] start at w_off + n * ld floats
-      // (16-byte accesses when every row is 16-byte aligned, else the scalar epilogue: gemm.cuh, adam_epilogue_vec)
-      bool al4 = W.ld % 4 == 0 && v.params.ms % 4 == 0;
-      for (int w = 0; w < W.ntens; ++w) al4 = al4 && W.w_off[w] % 4 == 0;
-      e.g_vec = (al4 && pl->adam_vec_max >= 4) ? 4 : 1;
-      e.adam_p = v.params.p;
-      e.adam_m = v.adam_m.p;
-      e.adam_v = v.adam_v.p;
-      e.sh = pl->shadow.p + W.off;
-      e.sh_ms = pl->shadow.ms;
-      e.sh_rcap = W.rcap;
-      e.drv = pl->derived.p;
-      e.drv_ms = pl->derived.ms;
-      e.drv_bias_off = W.bias_off;
-      e.drv_clsb_off = W.clsb_off;
-      e.drv_clsb_ld = W.rcap;
-      e.adam = member_adam(pl);
-      e.adam_ms = member_adam_ms(pl);
-    }
-    const bool aside = dw_stream && !fused && dw_stream != st;
+    const bool aside = dw_stream && dw_stream != st;
     cudaStream_t chain_st = st;
     if (aside) {
       if (rec) {
@@ -1185,7 +1145,7 @@ struct Exec {
       }
       st = dw_stream;
     }
-    launch(fused ? EPI_GRAD_ADAM : EPI_GRAD, p, e, ((fused ? "gemm_dw_adam." : "gemm_dw.") + sub).c_str());
+    launch(EPI_GRAD, p, e, ("gemm_dw." + sub).c_str());
     st = chain_st;
   }
 
@@ -1241,8 +1201,8 @@ struct Exec {
     sub = "head";
   }
   // backward of a block given the head gradient rows dYh; optionally the input gradient as fp32.
-  // Per layer the input gradient (which reads the layer's weight shadow) is launched BEFORE the
-  // weight gradient, because the fused-Adam epilogue of the latter overwrites that shadow.
+  // Per layer the input gradient (the next layer's input, on the critical path) is launched before the
+  // weight gradient (which feeds nothing but the optimizer).
   void block_bwd(MlpBlock& b, const C8Buf& dYh, const C8Buf& in, int in_row0, int in_feat, float* dx_out, long long dx_ms,
                  int dyn_which, int row_bound) {
     const int n = (int)b.hidden.size();
@@ -1275,7 +1235,7 @@ struct Exec {
   }
 };
 
-// Step-dependent Adam scalars, computed once on the host so that the fused epilogue and the
+// Step-dependent Adam scalars, computed once on the host so that the grouped dW+Adam launch and the
 // stand-alone kernel apply bit-identical updates.  bc1_out: the bias correction lr is divided by (member tables).
 AdamHyper adam_scalars(const drvae_hparams_t* hp, float* bc1_out) {
   const double t = (double)hp->step + 1.0;
@@ -1299,7 +1259,7 @@ int fill_view(drvae_plan* pl, Exec& ex, const drvae_batch_t* b, const drvae_nois
   if (b->N < 1 || b->N > pl->Ncap) return set_error("drvae: batch.N exceeds the plan's max_batch");
   if (pl->has_pair && (!b->x2 || !b->has_x2)) return set_error("drvae: this model needs x2 and has_x2");
   if (pl->has_clf && (!b->y || !b->has_y)) return set_error("drvae: this model needs y and has_y");
-  if (need_grad && !ex.fused && !pl->grads) return set_error("drvae: no gradient buffer bound");
+  if (need_grad && !ex.defer_dw && !pl->grads) return set_error("drvae: no gradient buffer bound");
   DevView& v = ex.v;
   v = pl->view;
   const int N = b->N;
@@ -1445,11 +1405,12 @@ int run_wn_grad(drvae_plan* pl, cudaStream_t st) {
 int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, const drvae_hparams_t* hp, float* losses_out,
              cudaStream_t st, bool backward, bool fused_adam) {
   if (!hp) return set_error("drvae: hparams is null");
-  if (fused_adam && (!pl->adam_m || !pl->adam_v)) return set_error("drvae: Adam needs bound moment buffers");
+  // (train_is_fused chooses the fused step only when the grouped launch is built, i.e. the moments are bound)
+  if (fused_adam && !pl->dwa_ok) return set_error("drvae: the fused train step needs the grouped dW+Adam launch");
   Exec ex;
   ex.pl = pl;
   ex.st = st;
-  ex.fused = fused_adam;
+  ex.defer_dw = backward && fused_adam;
   int rc = fill_view(pl, ex, b, nz, hp, backward);
   if (rc) return rc;
   if (!pl->shadows_valid) {
@@ -1465,7 +1426,6 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
   v.clf_splits = std::max(CLF_SPLITS, std::min(CLF_SPLITS_MAX, cdiv(LNb, 64)));
   v.loss_slices = std::max(1, std::min(LOSS_SLICES_MAX, cdiv(Rdb, 512)));
   ex.splitk = backward && !fused_adam && Rdb >= 2048;
-  ex.defer_dw = backward && fused_adam && pl->dwa_ok && pl->dwa_enabled;
   if (ex.splitk) {
     cudaError_t e0 = cudaMemsetAsync(pl->grads, 0, sizeof(float) * (size_t)pl->P * E, st);
     if (e0 != cudaSuccess) return set_cuda_error("drvae: zeroing the gradient buffer", e0);
@@ -1481,7 +1441,7 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
   // Persistent step kernel (stepk.cuh): everything between the input preparation and the grouped dW+Adam launch is
   // recorded (same code below, same dependencies) and runs as ONE cooperative launch.
   const bool use_stepk = pl->stepk_enabled && !pl->stepk_unsupported && pl->gemm_impl == GEMM_IMPL_TC &&
-                         !(backward && fused_adam && !ex.defer_dw) && pl->d_stepk_bar != nullptr;
+                         pl->d_stepk_bar != nullptr;
   StepRecorder recorder;
 
   // the main chain on the plan's high-priority stream (see above)
@@ -1531,7 +1491,7 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
   // the chain are capped to the other SMs while it runs.
   bool dwa_early_done = false;
   const int nsm = gemm_num_sms();
-  const bool dwa_early = backward && ex.defer_dw && !use_stepk && !pl->prof_on &&
+  const bool dwa_early = ex.defer_dw && !use_stepk && !pl->prof_on &&
                          pl->dwa_early_tiles > 0 && pl->dwa_early_tiles < pl->dwa_tiles && pl->dwa_early_sms >= 8 &&
                          pl->dwa_early_sms <= nsm - 16;
 
@@ -1807,7 +1767,7 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
       ex.row_op(SROW_T_BACK, "T_back", row_items(N + PAD_WARPS), 0,
                 [&]() { launch_k(pl->view.Zc <= 128 ? T_back_kernel<4> : T_back_kernel<MAXJ>, rows_grid(N + PAD_WARPS), dim3(ROW_THREADS), 0, ex.st, v); });
       ex.gemm_dx(v.dYT, pl->Tsh, EPI_STORE_F32, ex.epi_f32(v.dZ1T.p, v.dZ1T.ms, pl->Z, pl->Z, nullptr), CNT_LN, LNb);
-      ex.gemm_dw(v.dYT, v.Zdec, 0, pl->Tsh, CNT_LN, LNb, pl->arch.kind == DRVAE_KIND_PVAE ? CNT_NP : -1);
+      ex.gemm_dw(v.dYT, v.Zdec, 0, pl->Tsh, CNT_LN, LNb);
       bucket_done();
     }
     if (overlap) ex.ev_wait(cm, pl->ev.side_bwd);  // join: q_back sums the side branch's gradients into q(z1|x1)
@@ -1879,7 +1839,7 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
     cudaStreamWaitEvent(st, pl->ev.end, 0);
   }
   ex.st = st;
-  if (backward && ex.defer_dw && ex.ok()) {
+  if (ex.defer_dw && ex.ok()) {
     if (dwa_early_done) {  // the early part runs on its own stream: the rest starts when both are complete
       cudaEventRecord(pl->ev.dwa_end, pl->s_dwa);
       cudaStreamWaitEvent(st, pl->ev.dwa_end, 0);
@@ -1897,12 +1857,12 @@ namespace {
 
 enum { SEQ_TRAIN = 0, SEQ_LOSS = 1, SEQ_GRAD = 2 };
 
-// does this train step run with Adam fused into the weight-gradient epilogues?
+// does this train step run the grouped dW+Adam launch (dwadam.cuh) instead of gradient + stand-alone Adam?
 bool train_is_fused(const drvae_plan* pl, const drvae_batch_t* b) {
-  // weight norm: the update acts on (v, g), not on the effective weights the GEMMs produce gradients for.
+  // Not when build_dwa left it out (weight norm, unbound moments, a layer outside its layout conditions).
   // One (or a few) models on a large minibatch: the weight gradients need split-K to fill the GPU, which the
-  // fused epilogue cannot do (it needs the complete sum).  Both -> gradient buffer + stand-alone optimizer.
-  if (pl->wn) return false;
+  // grouped launch does not do (its tiles take the complete sum).  Both -> gradient buffer + stand-alone optimizer.
+  if (!pl->dwa_ok) return false;
   if (b && (long long)b->N * pl->L >= 1024 && pl->E < 8) return false;
   return true;
 }
@@ -1920,8 +1880,8 @@ int enqueue_sequence(drvae_plan* pl, int seq, const drvae_batch_t* b, const drva
     return rc;
   }
   if (fused) {
-    // forward + ELBO + backward with Adam fused into the gradient epilogues: no gradient buffer traffic and
-    // no separate optimizer pass (the bound gradient buffer is left untouched)
+    // forward + ELBO + backward with the weight gradients and Adam of every layer in the grouped launch: no gradient
+    // buffer traffic and no separate optimizer pass (the bound gradient buffer is left untouched)
     return run_step(pl, b, nz, hp, losses_out, st, 2, true);
   }
   int rc = run_step(pl, b, nz, hp, losses_out, st, 2, false);

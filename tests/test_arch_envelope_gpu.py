@@ -1,6 +1,6 @@
 """Parity at the edges of the architecture range drvae_plan_create accepts (dim_z1 / dim_z3 up to 256, 2 to 8 classes,
 1 to 4 hidden layers per MLP, any widths).  Several code paths are chosen from the shape alone: the <MAXJ> row kernels,
-the per-layer fused dW+Adam GEMMs, (mu | logvar) heads over two N tiles, decoder-head and hidden-layer tile edges,
+the optimizer path of a train step (grouped dW+Adam launch or gradient + stand-alone Adam), (mu | logvar) heads over two N tiles, decoder-head and hidden-layer tile edges,
 stacked row counts on the 128-row M tile.  Each case of CASES sits on one side of one of these thresholds;
 tests/test_arch_envelope_host.py recomputes the geometry with plan.cu's formulas and checks that the table covers both
 sides of every threshold.
@@ -33,7 +33,7 @@ CASES = {
     # Zc = 128: the last <4> row-kernel case; class columns end exactly at row 128 (grouped dW+Adam).  Every row paired
     # and labelled: R0 = LN = F = 128, Rd = 384
     "z125": (_arch(40, 2, 125, 125, [32]), 64, 2),
-    # <MAXJ> row kernels; 126 + 1 + 2 = 129 > 128: per-layer EPI_GRAD_ADAM; LN = 130
+    # <MAXJ> row kernels; 126 + 1 + 2 = 129 > 128: train steps run gradient + stand-alone Adam; LN = 130
     "z126": (_arch(40, 2, 126, 126, [32]), 65, 2),
     # (mu | logvar) head: one tile exactly 256 wide (the whole TMEM accumulator); <MAXJ>
     "z128": (_arch(40, 2, 128, 9, [48]), 40, 2),
@@ -41,7 +41,7 @@ CASES = {
     "z256": (_arch(978, 2, 256, 256, [800], [600], [200], [200]), 150, 2),
     # MAXY classes: every acc[MAXY] loop full; no labels (DrVAE): F = 8 L N = 528 marginalised rows
     "y8": (_arch(60, 8, 100, 13, [64]), 33, 2),
-    # 120 + 1 + 8 = 129: per-layer Adam with 8 class columns
+    # 120 + 1 + 8 = 129: gradient + stand-alone Adam with 8 class columns
     "y8dwa": (_arch(60, 8, 120, 13, [64]), 33, 1),
     # DRVAE_MAX_HIDDEN layers per MLP (21 grouped dW+Adam layers); hidden tiles 1 x 256 and 2 x 144; decoder head
     # over two tiles, the second holding one feature
@@ -119,12 +119,12 @@ def geometry(case, kind):
         blocks.update(enc_z3=(Z, Y), dec_z1=(Z3, Y))
     hidden = [tile_cap(w + 1) for b in blocks for w in arch[b]]
     # build_dwa: class columns must share the 128-row tile of the ones column (first hidden layer of z3 / dz1 blocks)
-    per_layer = any(cc > 0 and (kin % 128) + 1 + cc > 128 for kin, cc in blocks.values())
+    split = any(cc > 0 and (kin % 128) + 1 + cc > 128 for kin, cc in blocks.values())
     layers = sum(len(arch[b]) + 1 for b in blocks) + (1 if pair else 0)
     return dict(
         Y=Y, Zc=Zc, Z3c=Z3c if fprop else 0, maxj=Zc > 128 or (fprop and Z3c > 128), enc_head=heads["enc"],
         heads=heads, hb=hb, dec_tiles=cdiv(X, hb), dec_last=X - (cdiv(X, hb) - 1) * hb, Xc=round_up(X + 1, 16),
-        hidden=hidden, per_layer_adam=per_layer, dwa_layers=layers,
+        hidden=hidden, split_optimizer=split, dwa_layers=layers,
         rows=runtime_rows(case, kind),
         n_hidden=max(len(arch[b]) for b in blocks))
 
@@ -251,8 +251,8 @@ def test_eval_loss_and_inference_match_the_float64_oracle(oracle, case, kind):
 
 @pytest.mark.parametrize("case,kind", CASE_KIND, ids=IDS)
 def test_fused_optimizer_equals_gradient_then_adam(case, kind):
-    """Two steps of train_step (grouped or per-layer dW+Adam, whichever the shape selects) against grad_step +
-    adam_step."""
+    """Two steps of train_step (grouped dW+Adam launch, or gradient + stand-alone Adam when the shape rules the grouped
+    launch out) against grad_step + adam_step."""
     arch, N, L = CASES[case]
     fields = batch_fields(kind, case_batch(case, kind, SEED_BATCH))
     res = {}
@@ -302,27 +302,36 @@ def test_second_member_equals_a_single_model_plan(case):
     assert torch.equal(single.grads[0].cpu(), grads[1])
 
 
-def _steady_launches(plan, fields):
-    plan.set_graph(False)
-    plan.train_step(fields, plan.hparams(step=0), seed=3)
-    n0 = plan.launch_count()
-    plan.train_step(fields, plan.hparams(step=1), seed=3)
-    torch.cuda.synchronize()
-    return plan.launch_count() - n0
-
-
-@pytest.mark.parametrize("case,per_layer", (("z125", False), ("z126", True), ("y8dwa", True)))
-def test_the_table_reaches_the_per_layer_optimizer(case, per_layer, monkeypatch):
-    """A train step launches the same kernels as with the grouped dW+Adam switched off (DRVAE_B200_DWADAM=0) exactly
-    when the class columns do not fit the ones column's 128-row tile."""
+@pytest.mark.parametrize("case,split", (("z125", False), ("z126", True), ("y8dwa", True)))
+def test_the_table_reaches_the_split_optimizer(case, split):
+    """A train step runs the grouped dW+Adam launch unless the class columns do not fit the ones column's 128-row tile;
+    then it is grad_step + adam_step, bit for bit: parameters, moments, bf16 shadows and derived copies."""
     kind = "drvae"
-    arch, N, L = CASES[case]
     fields = batch_fields(kind, case_batch(case, kind, SEED_BATCH))
-    default = _steady_launches(make_plan(case, kind), fields)
-    monkeypatch.setenv("DRVAE_B200_DWADAM", "0")
-    forced = _steady_launches(make_plan(case, kind), fields)
-    assert (default == forced) == per_layer, (case, default, forced)
-    assert geometry(case, kind)["per_layer_adam"] == per_layer
+    res = {}
+    for mode in ("train", "grad_adam"):
+        plan = make_plan(case, kind)
+        for it in range(2):
+            hp = plan.hparams(step=it)
+            if mode == "train":
+                if it == 0:
+                    plan.profile_begin()
+                plan.train_step(fields, hp, seed=3)
+                if it == 0:
+                    tags = plan.profile_end()
+            else:
+                plan.grad_step(fields, hp, seed=3)
+                plan.adam_step(hp)
+        sh, _, _ = plan.debug_buffer("shadow", torch.bfloat16)
+        dv, _, _ = plan.debug_buffer("derived")
+        torch.cuda.synchronize()
+        res[mode] = [t.cpu().clone() for t in (plan.params, plan.adam_m, plan.adam_v, sh, dv)]
+    assert ("bwd:dw_adam_all" in tags) == (not split), (case, sorted(tags))
+    assert ("opt:adam" in tags) == split, (case, sorted(tags))
+    assert geometry(case, kind)["split_optimizer"] == split
+    if split:
+        for name, a, b in zip(("params", "adam_m", "adam_v", "shadow", "derived"), res["train"], res["grad_adam"]):
+            assert torch.equal(a, b), "%s %s" % (case, name)
 
 
 @pytest.mark.parametrize("case", ("z128", "z256"))

@@ -36,11 +36,11 @@ def test_row_kernel_width_on_both_sides():
     _covers(lambda g: g["Z3c"] > 128, "<MAXJ> chosen by Z3c (z3_post / z3_back)")
 
 
-def test_grouped_and_per_layer_optimizer_on_both_sides():
-    _covers(lambda g: g["per_layer_adam"] and g["Y"] == 2, "per-layer dW+Adam with two classes (126 + 1 + 2 = 129)")
-    _covers(lambda g: g["per_layer_adam"] and g["Y"] == 8, "per-layer dW+Adam with eight classes (120 + 1 + 8 = 129)")
+def test_grouped_and_split_optimizer_on_both_sides():
+    _covers(lambda g: g["split_optimizer"] and g["Y"] == 2, "gradient + stand-alone Adam with two classes (126 + 1 + 2 = 129)")
+    _covers(lambda g: g["split_optimizer"] and g["Y"] == 8, "gradient + stand-alone Adam with eight classes (120 + 1 + 8 = 129)")
     # the grouped launch is still used when the class columns end exactly at row 128
-    _covers(lambda g: not g["per_layer_adam"] and g["Zc"] == 128 and g["Y"] == 2, "class columns ending at row 128")
+    _covers(lambda g: not g["split_optimizer"] and g["Zc"] == 128 and g["Y"] == 2, "class columns ending at row 128")
     _covers(lambda g: g["dwa_layers"] == 21, "21 layers in the grouped dW+Adam table")
     assert max(g["dwa_layers"] for g in GEO.values()) <= 24
 

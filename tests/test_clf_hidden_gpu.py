@@ -22,6 +22,8 @@ pytestmark = pytest.mark.gpu
 README = dict(dim_x=978, dim_y=2, dim_z1=100, dim_z3=100, enc_z1=[800], dec_x=[600], enc_z3=[200], dec_z1=[200])
 Z256 = dict(README, dim_z1=256, dim_z3=256)
 SMALL = dict(dim_x=40, dim_y=2, dim_z1=128, dim_z3=9, enc_z1=[48], dec_x=[48], enc_z3=[48], dec_z1=[48])
+DEEP4 = dict(dim_x=40, dim_y=2, dim_z1=16, dim_z3=9, enc_z1=[48, 32, 24, 40], dec_x=[32, 48, 40, 24], enc_z3=[24, 32, 16, 48],
+             dec_z1=[40, 16, 32, 24])
 CLF = {"c16": [16], "c200": [200], "c64_32": [64, 32], "c4l": [24, 48, 16, 40], "c256": [256]}
 # id -> (kind, arch, class_y, weight_norm, N, L)
 CASES = {"%s-readme-%s" % (k, c): (k, README, w, False, 150, 2) for k in ("drvae", "vfae") for c, w in CLF.items()}
@@ -146,6 +148,12 @@ def test_bf16_inference_path_matches_the_oracle():
         assert float((res["proba"][0].cpu().double() - ref).abs().max()) < 2e-3, kind
 
 
+# Inputs of the fused-optimizer checks: (architecture, classifier hidden layers).  deep4 has 4 hidden layers in every MLP
+# and in the classifier: 25 weight layers for DrVAE, one more than the grouped dW+Adam launch takes (its train step runs
+# gradient + stand-alone Adam), and 24 for VFAE, the most the grouped launch takes.
+STEP_CASES = {"readme": (README, [64, 32]), "deep4": (DEEP4, [8, 8, 8, 8])}
+
+
 def _split_vs_fused(kind, arch, clf, N, L):
     fields = batch_fields(kind, orc.synthetic_batch(N, arch["dim_x"], seed=SEED_BATCH))
     res = {}
@@ -169,22 +177,20 @@ def _split_vs_fused(kind, arch, clf, N, L):
     assert torch.allclose(f[0][1], s[0][1], rtol=1e-5, atol=1e-6), "second-step losses differ"
 
 
-@pytest.mark.parametrize("dwa", ("grouped", "per_layer"))
+@pytest.mark.parametrize("case", list(STEP_CASES))
 @pytest.mark.parametrize("kind", ("drvae", "vfae"))
-def test_fused_adam_equals_grad_then_adam(kind, dwa, monkeypatch):
-    if dwa == "per_layer":
-        monkeypatch.setenv("DRVAE_B200_DWADAM", "0")
-    _split_vs_fused(kind, README, [64, 32], 150, 2)
+def test_fused_adam_equals_grad_then_adam(kind, case):
+    arch, clf = STEP_CASES[case]
+    _split_vs_fused(kind, arch, clf, 150, 2)
 
 
-@pytest.mark.parametrize("dwa", ("grouped", "per_layer"))
+@pytest.mark.parametrize("case", list(STEP_CASES))
 @pytest.mark.parametrize("kind", ("drvae", "vfae"))
-def test_train_steps_track_the_oracle(kind, dwa, monkeypatch):
-    if dwa == "per_layer":
-        monkeypatch.setenv("DRVAE_B200_DWADAM", "0")
-    clf, N, L = [64, 32], 150, 2
-    batch = orc.synthetic_batch(N, README["dim_x"], seed=SEED_BATCH)
-    plan = make_plan(kind, README, clf, N=N, L=L)
+def test_train_steps_track_the_oracle(kind, case):
+    arch, clf = STEP_CASES[case]
+    N, L = 150, 2
+    batch = orc.synthetic_batch(N, arch["dim_x"], seed=SEED_BATCH)
+    plan = make_plan(kind, arch, clf, N=N, L=L)
     for it in range(3):
         cur = plan.state_dict()
         o = orc.OracleModel({k: v.cpu() for k, v in cur.items()}, orc.default_cfg(kind, L=L), dtype=torch.float64)

@@ -141,22 +141,11 @@ def test_adam_kernel_matches_torch_adam():
             assert torch.allclose(pv[name].cpu(), p.detach(), rtol=2e-5, atol=2e-7), (t, name)
 
 
-DWA_MODES = ("grouped", "per_layer")
-
-
-def set_dwa_mode(monkeypatch, dwa):
-    """grouped: one dW+Adam launch for every layer (the default); per_layer: one fused EPI_GRAD_ADAM GEMM per layer,
-    what plans whose class columns do not fit the ones column's 128-row tile run.  Read at plan creation."""
-    monkeypatch.setenv("DRVAE_B200_DWADAM", "1" if dwa == "grouped" else "0")
-
-
-@pytest.mark.parametrize("dwa", DWA_MODES)
 @pytest.mark.parametrize("kind", KINDS)
-def test_train_steps_track_the_oracle(kind, dwa, monkeypatch):
+def test_train_steps_track_the_oracle(kind):
     """Three fused steps (fwd+bwd+Adam).  After each step the GPU's own parameters are read back
     and the oracle evaluates the NEXT loss from them: this checks Adam -> shadow refresh -> next
     forward without accumulating the sign-sensitivity of Adam's first updates."""
-    set_dwa_mode(monkeypatch, dwa)
     arch, N, sd, batch, om, plan = setup(kind, "tiny")
     for it in range(3):
         cur = plan.state_dict()
@@ -396,15 +385,12 @@ def test_model_class_surface():
             assert np.isfinite(float(ev2["CMPL"]))
 
 
-@pytest.mark.parametrize("dwa", DWA_MODES)
 @pytest.mark.parametrize("case", ("tiny", "deep", "readme"))
 @pytest.mark.parametrize("kind", KINDS)
-def test_fused_adam_equals_grad_then_adam(kind, case, dwa, monkeypatch):
-    """drvae_train_step applies Adam inside the weight-gradient epilogues (the gradient never reaches
+def test_fused_adam_equals_grad_then_adam(kind, case):
+    """drvae_train_step applies Adam inside the grouped weight-gradient launch (the gradient never reaches
     HBM); drvae_grad_step + drvae_adam_step materialise it and run the stand-alone optimizer kernel.
-    Same gradients, same formula: parameters, moments and the refreshed bf16 shadows must agree.
-    Both fused forms: the grouped dW+Adam launch and the per-layer EPI_GRAD_ADAM GEMMs."""
-    set_dwa_mode(monkeypatch, dwa)
+    Same gradients, same formula: parameters, moments and the refreshed bf16 shadows must agree."""
     res = {}
     for mode in ("fused", "split"):
         arch, N, sd, batch, om, plan = setup(kind, case)
