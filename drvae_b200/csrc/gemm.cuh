@@ -42,8 +42,7 @@ enum {
   EPI_DACT_C8 = 2,    // * ELU'(stored activation) -> bf16 chunk8
   EPI_GRAD = 3,       // weight (+bias, +class column) gradient -> flat fp32 grad buffer, reference tensor layout
   EPI_DECLOSS = 4,    // decoder heads: Gaussian log-density partials + d loss / d pre-activation
-  EPI_DECOUT = 5,     // decoder heads at inference: mu and sigma as fp32 row-major
-  EPI_LIN_C8 = 6      // +bias -> bf16 chunk8 (no activation)
+  EPI_DECOUT = 5      // decoder heads at inference: mu and sigma as fp32 row-major
 };
 
 constexpr int GEMM_BM = 128;
@@ -250,7 +249,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
         if (c < e.n_valid) o[c] = acc[i] + (b ? b[c] : 0.f);
       }
     }
-  } else if (EPI == EPI_ELU_C8 || EPI == EPI_LIN_C8 || EPI == EPI_DACT_C8) {
+  } else if (EPI == EPI_ELU_C8 || EPI == EPI_DACT_C8) {
     float v[16];
     if (EPI == EPI_DACT_C8) {
       const uint4* a =
@@ -293,8 +292,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
         int c = col0 + i;
-        float x = acc[i] + bb[i];
-        if (EPI == EPI_ELU_C8) x = elu1(x);
+        const float x = elu1(acc[i] + bb[i]);
         // column n_valid is the ones column the next layer's dW turns into its bias gradient
         v[i] = !rc.valid ? 0.f : (c < e.n_valid ? x : (c == e.n_valid ? 1.f : 0.f));
       }
@@ -966,7 +964,6 @@ inline cudaError_t gemm_launch(int epi, const GemmProblem& p, const EpiParams& e
   switch (epi) {
     case EPI_STORE_F32: return gemm_launch_t<EPI_STORE_F32>(p, e, n_models, impl, st);
     case EPI_ELU_C8: return gemm_launch_t<EPI_ELU_C8>(p, e, n_models, impl, st);
-    case EPI_LIN_C8: return gemm_launch_t<EPI_LIN_C8>(p, e, n_models, impl, st);
     case EPI_DACT_C8: return gemm_launch_t<EPI_DACT_C8>(p, e, n_models, impl, st);
     case EPI_GRAD: return gemm_launch_t<EPI_GRAD>(p, e, n_models, impl, st);
     case EPI_DECLOSS: return gemm_launch_t<EPI_DECLOSS>(p, e, n_models, impl, st);

@@ -799,7 +799,9 @@ __device__ __forceinline__ void clf_dlogit_row(const DevView& v, const int m, co
     g[j] = 0.f;
     if (j < v.Y) {
       q[j] = qy[j];
-      const bool clamped = !(q[j] > 1e-10f && q[j] < 1.f - 1e-10f);
+      // (the clamp's upper bound 1 - 1e-10 rounds to 1.0f, which no probability exceeds: only the lower bound can
+      // cut a class's gradient, as in the reference's float32 clamp backward)
+      const bool clamped = !(q[j] > 1e-10f);
       if (lb) {
         g[j] = (j == yi) ? -cf[COEF_YL] / q[j] : 0.f;
       } else {
