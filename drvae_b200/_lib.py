@@ -75,8 +75,8 @@ EXPORTS = ["drvae_last_error", "drvae_plan_create", "drvae_plan_destroy", "drvae
            "drvae_loss_forward", "drvae_grad_step", "drvae_adam_step", "drvae_infer", "drvae_set_gemm_impl",
            "drvae_plan_launch_count", "drvae_debug_buffer", "drvae_debug_gemm", "drvae_profile_begin",
            "drvae_profile_end", "drvae_plan_num_buckets", "drvae_plan_bucket_info", "drvae_stream_wait_bucket", "drvae_set_graph", "drvae_plan_graph_replays", "drvae_debug_wait_stats",
-           "drvae_push_scalars", "drvae_set_external_scalars", "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
-           "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_adam_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
+           "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
+           "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_train_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
            "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams", "drvae_plan_create_clf"]
 
 
@@ -115,7 +115,7 @@ def load():
     lib.drvae_plan_bind.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.drvae_sync_shadows.restype = c_int
     lib.drvae_sync_shadows.argtypes = [c_void_p, c_void_p]
-    for name in ("drvae_train_step", "drvae_loss_forward", "drvae_grad_step"):
+    for name in ("drvae_train_step", "drvae_loss_forward", "drvae_grad_step", "drvae_dp_train_step"):
         fn = getattr(lib, name)
         fn.restype = c_int
         fn.argtypes = [c_void_p, P(Batch), P(Noise), P(HParams), c_void_p, c_void_p]
@@ -143,12 +143,8 @@ def load():
     lib.drvae_plan_graph_replays.argtypes = [c_void_p]
     lib.drvae_infer.restype = c_int
     lib.drvae_infer.argtypes = [c_void_p, c_void_p, c_int, P(InferOut), c_void_p]
-    lib.drvae_push_scalars.restype = c_int
-    lib.drvae_push_scalars.argtypes = [c_void_p, P(Noise), P(HParams), c_int, c_void_p]
     lib.drvae_set_member_hparams.restype = c_int
     lib.drvae_set_member_hparams.argtypes = [c_void_p, P(MemberHParams), c_int, c_void_p]
-    lib.drvae_set_external_scalars.restype = c_int
-    lib.drvae_set_external_scalars.argtypes = [c_void_p, c_int]
     lib.drvae_debug_wait_stats.restype = c_int
     lib.drvae_debug_wait_stats.argtypes = [c_void_p, c_int]
     lib.drvae_debug_dwa_stats.restype = c_int
@@ -161,8 +157,6 @@ def load():
     lib.drvae_dp_counts_ptr.argtypes = [c_void_p]
     lib.drvae_dp_exchange_counts.restype = c_int
     lib.drvae_dp_exchange_counts.argtypes = [c_void_p, c_ll, c_ll, c_ll, c_ll, c_void_p]
-    lib.drvae_dp_adam_step.restype = c_int
-    lib.drvae_dp_adam_step.argtypes = [c_void_p, P(HParams), c_void_p, c_void_p]
     lib.drvae_set_infer_precision.restype = c_int
     lib.drvae_set_infer_precision.argtypes = [c_void_p, c_int]
     lib.drvae_trace_begin.restype = c_int

@@ -104,7 +104,6 @@ struct drvae_plan {
   drvae_member_hparams_t* h_member_stage = nullptr;
   cudaEvent_t member_ev = nullptr;
   bool graph_enabled = true;
-  bool external_dyn = false;  // the caller pushes the per-step scalars (drvae_push_scalars) and captures the sequence itself
   struct GraphEntry {
     int seen = 0;
     cudaGraph_t graph = nullptr;  // kept alive: node handles used for parameter updates belong to it
@@ -1855,7 +1854,48 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
 
 namespace {
 
-enum { SEQ_TRAIN = 0, SEQ_LOSS = 1, SEQ_GRAD = 2 };
+enum { SEQ_TRAIN = 0, SEQ_LOSS = 1, SEQ_GRAD = 2, SEQ_DP = 3 };
+
+// data-parallel optimizer over peer memory (dp_peer.cuh): cross-GPU barrier (tag from the per-step scalars), then ONE
+// kernel that sums every rank's gradient and loss shares in rank order and applies Adam; global losses -> losses_out
+int run_dp_adam(drvae_plan* pl, float* losses_out, cudaStream_t st) {
+  prof_pre(pl, st, "opt:dp_barrier");
+  dp_barrier_kernel<<<1, 32, 0, st>>>(pl->dp, pl->d_dyn, pl->dbg);
+  prof_post(pl, st);
+  AdamArgs a{};
+  a.params = MBuf<float>{pl->params, pl->P};
+  a.grads = MBuf<float>{pl->grads, pl->P};
+  a.m = MBuf<float>{pl->adam_m, pl->P};
+  a.v = MBuf<float>{pl->adam_v, pl->P};
+  a.shadow = pl->shadow;
+  a.derived = pl->derived;
+  a.segs = pl->d_segs;
+  a.nseg = (int)pl->segs.size();
+  a.P = pl->P;
+  a.update = 1;
+  a.h = &pl->d_dyn->s.mem.adam;
+  a.skip_lo = a.skip_hi = 0;
+  if (pl->arch.kind == DRVAE_KIND_PVAE && pl->has_T) a.skip_lo = (int)pl->T_range[0], a.skip_hi = (int)(pl->T_range[0] + pl->T_range[1]);
+  a.dyn = pl->d_dyn;
+  a.counts = pl->view.counts.p;
+  a.counts_stride = (int)pl->view.counts.ms;
+  const int nred = pl->P + 8;
+  prof_pre(pl, st, "opt:adam_peer");
+  adam_peer_kernel<<<cdiv(nred, 1024), 256, 0, st>>>(a, pl->dp, nred, losses_out);
+  prof_post(pl, st);
+  pl->launches += 2;
+  cudaError_t err = cudaGetLastError();
+  if (err != cudaSuccess) return set_cuda_error("adam_peer_kernel", err);
+  if (pl->wn) {
+    WnArgs w{pl->d_wn_rows, (int)pl->wn_rows.size(), a.params, a.grads, pl->shadow, pl->derived};
+    wn_refresh_kernel<<<dim3(cdiv(w.nrows, 8), pl->E), 256, 0, st>>>(w);
+    pl->launches++;
+    err = cudaGetLastError();
+    if (err != cudaSuccess) return set_cuda_error("wn_refresh_kernel", err);
+  }
+  pl->shadows_valid = true;
+  return 0;
+}
 
 // does this train step run the grouped dW+Adam launch (dwadam.cuh) instead of gradient + stand-alone Adam?
 bool train_is_fused(const drvae_plan* pl, const drvae_batch_t* b) {
@@ -1884,11 +1924,14 @@ int enqueue_sequence(drvae_plan* pl, int seq, const drvae_batch_t* b, const drva
     // buffer traffic and no separate optimizer pass (the bound gradient buffer is left untouched)
     return run_step(pl, b, nz, hp, losses_out, st, 2, true);
   }
-  int rc = run_step(pl, b, nz, hp, losses_out, st, 2, false);
+  // split train step and data-parallel step: gradient buffer, weight-norm conversion, stand-alone optimizer.  With
+  // peers attached the loss shares go right behind the gradient, where the peer optimizer reduces them with it.
+  const bool peers = seq == SEQ_DP && pl->dp_on;
+  int rc = run_step(pl, b, nz, hp, peers ? pl->grads + pl->P : losses_out, st, 2, false);
   if (rc) return rc;
   rc = run_wn_grad(pl, st);
   if (rc) return rc;
-  return run_adam(pl, hp, 1, st);
+  return peers ? run_dp_adam(pl, losses_out, st) : run_adam(pl, hp, 1, st);
 }
 
 // One call = [set_dyn_kernel(per-step scalars)] + a launch sequence that is identical for every step of the same
@@ -1896,13 +1939,13 @@ int enqueue_sequence(drvae_plan* pl, int seq, const drvae_batch_t* b, const drva
 // captured into a CUDA graph (the side-stream fork/join becomes graph edges); afterwards a step is one graph launch
 // with the arguments of the set_dyn node updated.  Not captured: parity runs with a caller-provided eps block,
 // drvae_grad_step (its bucket events are consumed outside), profiling passes, and the legacy default stream.
+// drvae_dp_train_step is captured whole: its peer barrier and optimizer are plan launches, and no NCCL call is in it.
 int step_entry(drvae_plan* pl, int seq, const drvae_batch_t* b, const drvae_noise_t* nz, const drvae_hparams_t* hp,
                float* losses_out, cudaStream_t st) {
   if (!hp) return set_error("drvae: hparams is null");
   if (!b) return set_error("drvae: batch is null");
   const bool fused = seq == SEQ_TRAIN && train_is_fused(pl, b);
   const StepDyn dyn = make_dyn(nz, hp, fused);
-  if (pl->external_dyn) return enqueue_sequence(pl, seq, b, nz, hp, losses_out, st, fused);
   const bool graphable = pl->graph_enabled && !pl->prof_on && !(nz && nz->eps) && seq != SEQ_GRAD && pl->shadows_valid &&
                          st != nullptr && st != cudaStreamLegacy && st != cudaStreamPerThread;
   if (graphable) {
@@ -2020,11 +2063,15 @@ extern "C" int drvae_grad_step(drvae_plan_t* pl, const drvae_batch_t* b, const d
 
 extern "C" int drvae_adam_step(drvae_plan_t* pl, const drvae_hparams_t* hp, void* stream) {
   if (!pl || !hp) return set_error("drvae_adam_step: null argument");
-  if (!pl->external_dyn) {
-    int rc = push_dyn(pl, make_dyn(nullptr, hp, false), (cudaStream_t)stream);
-    if (rc) return rc;
-  }
+  int rc = push_dyn(pl, make_dyn(nullptr, hp, false), (cudaStream_t)stream);
+  if (rc) return rc;
   return run_adam(pl, hp, 1, (cudaStream_t)stream);
+}
+
+extern "C" int drvae_dp_train_step(drvae_plan_t* pl, const drvae_batch_t* b, const drvae_noise_t* nz, const drvae_hparams_t* hp,
+                                   float* losses_out, void* stream) {
+  if (!pl || !losses_out) return set_error("drvae_dp_train_step: null argument");
+  return step_entry(pl, SEQ_DP, b, nz, hp, losses_out, (cudaStream_t)stream);
 }
 
 // ---- data parallelism over NVLink peer memory (dp_peer.cuh) ----
@@ -2064,57 +2111,6 @@ extern "C" int drvae_dp_exchange_counts(drvae_plan_t* pl, long long N, long long
   if (err != cudaSuccess) return set_cuda_error("dp_counts_kernel", err);
   return 0;
 }
-extern "C" int drvae_dp_adam_step(drvae_plan_t* pl, const drvae_hparams_t* hp, float* losses_out, void* stream) {
-  if (!pl || !hp || !losses_out) return set_error("drvae_dp_adam_step: null argument");
-  if (!pl->dp_on) return set_error("drvae_dp_adam_step: no peers attached");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (!pl->external_dyn) {
-    int rc = push_dyn(pl, make_dyn(nullptr, hp, false), st);
-    if (rc) return rc;
-  }
-  prof_pre(pl, st, "opt:dp_barrier");
-  dp_barrier_kernel<<<1, 32, 0, st>>>(pl->dp, pl->d_dyn, pl->dbg);
-  prof_post(pl, st);
-  AdamArgs a{};
-  a.params = MBuf<float>{pl->params, pl->P};
-  a.grads = MBuf<float>{pl->grads, pl->P};
-  a.m = MBuf<float>{pl->adam_m, pl->P};
-  a.v = MBuf<float>{pl->adam_v, pl->P};
-  a.shadow = pl->shadow;
-  a.derived = pl->derived;
-  a.segs = pl->d_segs;
-  a.nseg = (int)pl->segs.size();
-  a.P = pl->P;
-  a.update = 1;
-  a.h = &pl->d_dyn->s.mem.adam;
-  a.skip_lo = a.skip_hi = 0;
-  if (pl->arch.kind == DRVAE_KIND_PVAE && pl->has_T) a.skip_lo = (int)pl->T_range[0], a.skip_hi = (int)(pl->T_range[0] + pl->T_range[1]);
-  a.dyn = pl->d_dyn;
-  a.counts = pl->view.counts.p;
-  a.counts_stride = (int)pl->view.counts.ms;
-  const int nred = pl->P + 8;
-  prof_pre(pl, st, "opt:adam_peer");
-  adam_peer_kernel<<<cdiv(nred, 1024), 256, 0, st>>>(a, pl->dp, nred, losses_out);
-  prof_post(pl, st);
-  pl->launches += 2;
-  cudaError_t err = cudaGetLastError();
-  if (err != cudaSuccess) return set_cuda_error("adam_peer_kernel", err);
-  if (pl->wn) {
-    WnArgs w{pl->d_wn_rows, (int)pl->wn_rows.size(), a.params, a.grads, pl->shadow, pl->derived};
-    wn_refresh_kernel<<<dim3(cdiv(w.nrows, 8), pl->E), 256, 0, st>>>(w);
-    pl->launches++;
-    err = cudaGetLastError();
-    if (err != cudaSuccess) return set_cuda_error("wn_refresh_kernel", err);
-  }
-  pl->shadows_valid = true;
-  return 0;
-}
-
-extern "C" int drvae_push_scalars(drvae_plan_t* pl, const drvae_noise_t* nz, const drvae_hparams_t* hp, int fused_adam,
-                                  void* stream) {
-  if (!pl || !hp) return set_error("drvae_push_scalars: null argument");
-  return push_dyn(pl, make_dyn(nz, hp, fused_adam != 0), (cudaStream_t)stream);
-}
 extern "C" int drvae_set_member_hparams(drvae_plan_t* pl, const drvae_member_hparams_t* members, int count, void* stream) {
   if (!pl) return set_error("drvae_set_member_hparams: null plan");
   if (pl->dp_on) return set_error("drvae_set_member_hparams: a data-parallel plan cannot take a member table");
@@ -2153,12 +2149,6 @@ extern "C" int drvae_set_member_hparams(drvae_plan_t* pl, const drvae_member_hpa
   pl->member_table = true;
   return 0;
 }
-extern "C" int drvae_set_external_scalars(drvae_plan_t* pl, int enable) {
-  if (!pl) return set_error("drvae_set_external_scalars: null plan");
-  pl->external_dyn = enable != 0;
-  return 0;
-}
-
 // Instrumented builds only (-DGEMM_PROFILE_WAITS): copy out (and optionally clear) the per-(mode, epilogue) barrier
 // wait counters of gemm.cuh; a normal build reports that the counters are not compiled in.
 extern "C" int drvae_debug_wait_stats(unsigned long long* out, int reset) {

@@ -11,6 +11,10 @@ produces an additive share of every loss term and of the gradient:
                backward pass has produced that bucket, overlapping the rest of backward
     drvae_adam_step(...)                                                 (replicated optimizer: 28 MB of state)
 
+That is the NCCL path of a multi-rank step, launched eagerly.  With NVLink peer memory (PeerBackend) a step is
+drvae_dp_exchange_counts + drvae_dp_train_step, which sums the gradients inside the optimizer kernel; on one rank it is
+drvae_dp_train_step alone.  The plan replays drvae_dp_train_step as a CUDA graph like its other steps.
+
 ε is keyed by the global row index (drvae_noise_t.row_offset), so the result does not depend on
 the number of ranks.  The communication backend is torch.distributed (NCCL over NVLink on the
 GPU box; gloo in the CPU tests of the host logic, with the oracle as the compute backend).
@@ -56,24 +60,22 @@ def global_counts_device(counts, device, group=None):
 class PlanBackend:
     """Compute backend over the C ABI: one single-model Plan on this rank's GPU.
 
-    graph=True (default; DRVAE_B200_DP_GRAPH=0 disables): DataParallel.step captures the whole step — gradient
-    kernels, the optimizer — as ONE CUDA graph per set of batch buffers and replays it; only the per-step scalars
-    (drvae_push_scalars) stay outside (1 GPU, batch 8192: 1.03 -> 0.96 ms).  Used on a single rank only for now:
-    capturing the per-bucket NCCL all-reduces as well is what a multi-rank step needs (a shard of a few hundred rows
-    finishes faster than the host can enqueue ~50 launches and 7 collectives), but that capture deadlocked when
-    tried and is left for the next round."""
+    On one rank DataParallel.step is one drvae_dp_train_step, replayed by the plan as a CUDA graph.  With more ranks
+    it is the eager NCCL path of the module docstring: capturing the per-bucket NCCL all-reduces as well is what a
+    multi-rank step needs (a shard of a few hundred rows finishes faster than the host can enqueue ~50 launches and 7
+    collectives), but that capture deadlocked when tried."""
 
-    def __init__(self, plan, graph=None):
+    def __init__(self, plan):
         if plan.E != 1:
             raise ValueError("data-parallel training shards ONE model; ensembles shard by model instead")
         self.plan = plan
         self.device = plan.device
         self.comm_stream = torch.cuda.Stream(device=plan.device)
-        self.graph = (os.environ.get("DRVAE_B200_DP_GRAPH", "1") != "0") if graph is None else bool(graph)
-        self.graphs = {}  # batch buffers -> (CUDAGraph, static losses)
-        self.seen = {}
-        self.counts_pin = torch.zeros(3, dtype=torch.int64).pin_memory()
-        self.counts_dev = torch.zeros(3, dtype=torch.int64, device=plan.device)
+
+    @property
+    def graphs(self):
+        """CUDA-graph replays of the plan's steps so far."""
+        return self.plan.graph_replays()
 
     def flat_grads(self):
         return self.plan.grads[0]
@@ -97,11 +99,11 @@ class PeerBackend(PlanBackend):
     mapped (torch.distributed._symmetric_memory is used for the allocation and the pointer exchange only), and the
     all-reduce is fused into the optimizer kernel (csrc/dp_peer.cuh): cross-GPU flag barrier + ONE kernel that sums the
     ranks' gradients over NVLink in rank order and applies Adam.  The whole step — gradient kernels, barrier, optimizer —
-    is one CUDA graph per set of batch buffers on every rank; per step the host launches the counts exchange, the
-    per-step scalars and the graph."""
+    is one drvae_dp_train_step, replayed as one CUDA graph per set of batch buffers on every rank; per step the host
+    launches the counts exchange and the step."""
 
-    def __init__(self, plan, group=None, graph=None, multicast=None):
-        super().__init__(plan, graph=graph)
+    def __init__(self, plan, group=None, multicast=None):
+        super().__init__(plan)
         import torch.distributed._symmetric_memory as symm_mem
         self.group = group if group is not None else dist.group.WORLD
         self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
@@ -124,12 +126,8 @@ class PeerBackend(PlanBackend):
         self.multicast = bool(mc)
         plan.dp_attach(self.rank, self.world, list(gh.buffer_ptrs), list(ch.buffer_ptrs), mc)
         self._handles = (gh, ch)
-        self.loss_share = self.gbuf[plan.P:plan.P + 8]  # this rank's additive loss shares, reduced with the gradient
         self.global_losses = torch.zeros(8, dtype=torch.float32, device=dev)
         self.peer = True
-
-    def flat_grads(self):
-        return self.gbuf[:self.plan.P]
 
 
 class DataParallel:
@@ -147,102 +145,6 @@ class DataParallel:
         if self.world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
 
-    def _enqueue(self, be, batch, hp_kwargs, counts, eps, seed, row_offset):
-        """grad_step -> per-bucket all-reduce on the communication stream -> optimizer, on the current stream."""
-        losses, events = be.grad_step(batch, hp_kwargs, counts, self.finished_training_iters, eps=eps, seed=seed,
-                                      row_offset=row_offset)
-        flat = be.flat_grads()
-        comm = be.comm_stream
-        # bucket k is complete when events[k] fires; its all-reduce runs on the side stream while
-        # the compute stream is still inside the backward pass of the remaining blocks
-        with torch.cuda.stream(comm):
-            for (off, cnt), wait in zip(be.buckets(), events):
-                wait(comm)
-                self._all_reduce(flat[off:off + cnt])
-            self._all_reduce(losses)
-        torch.cuda.current_stream(be.device).wait_stream(comm)
-        be.adam_step()
-        return losses
-
-    def _step_graph(self, be, batch, hp_kwargs, local, seed, row_offset):
-        """Replay (or, the third time a set of batch buffers is seen, capture) the step as one CUDA graph."""
-        plan = be.plan
-        # a graph bakes in the addresses (and dtypes) of the caller's batch buffers
-        key = (int(batch["x1"].shape[-2]),) + tuple((k, v.data_ptr(), str(v.dtype)) for k, v in sorted(batch.items()))
-        # batch-global normalisers: summed on the device, read by set_dyn (no host round trip)
-        if self.world > 1:
-            be.counts_pin.copy_(torch.tensor(local, dtype=torch.int64))
-            be.counts_dev.copy_(be.counts_pin, non_blocking=True)
-            dist.all_reduce(be.counts_dev, op=dist.ReduceOp.SUM, group=self.group)
-            counts = be.counts_dev
-        else:
-            counts = local
-        entry = be.graphs.get(key)
-        if entry is None:
-            if len(be.seen) > 64:  # callers that allocate a new batch every step never reach a capture
-                be.seen.clear()
-            be.seen[key] = be.seen.get(key, 0) + 1
-            if be.seen[key] < 3:  # warm-up: communicators, function attributes, tensor maps
-                return self._enqueue(be, batch, hp_kwargs, counts, None, seed, row_offset)
-            cur = torch.cuda.current_stream(be.device)
-            cur.synchronize()
-            plan.set_external_scalars(True)
-            try:
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                    losses = self._enqueue(be, batch, hp_kwargs, counts, None, seed, row_offset)
-            finally:
-                plan.set_external_scalars(False)
-            if len(be.graphs) >= 8:
-                be.graphs.clear()
-            entry = be.graphs[key] = (g, losses, dict(batch))  # keep the captured buffers alive
-        g, losses, _ = entry
-        hp = plan.hparams(step=self.finished_training_iters, global_counts=counts, **hp_kwargs)
-        plan.push_scalars(hp, seed=seed, row_offset=row_offset, fused=False)
-        g.replay()
-        return losses
-
-    def _step_peer(self, be, batch, hp_kwargs, local, eps, seed, row_offset):
-        """PeerBackend: counts exchange (doubles as the cross-step barrier) -> [graph: gradient kernels -> peer barrier ->
-        fused all-reduce + Adam]."""
-        plan = be.plan
-        it = self.finished_training_iters
-        plan.dp_exchange_counts(local, it + 1)
-        hp = plan.hparams(step=it, global_counts_ptr=plan.dp_counts_ptr, **hp_kwargs)
-
-        def enqueue():
-            plan.grad_step(batch, hp, eps=eps, seed=seed, row_offset=row_offset, losses_out=be.loss_share)
-            plan.dp_adam_step(hp, be.global_losses)
-
-        graphable = be.graph and eps is None and all(torch.is_tensor(v) and v.is_cuda for v in batch.values())
-        if not graphable:
-            enqueue()
-            return be.global_losses
-        key = (int(batch["x1"].shape[-2]),) + tuple((k, v.data_ptr(), str(v.dtype)) for k, v in sorted(batch.items()))
-        entry = be.graphs.get(key)
-        if entry is None:
-            if len(be.seen) > 64:
-                be.seen.clear()
-            be.seen[key] = be.seen.get(key, 0) + 1
-            if be.seen[key] < 3:  # warm-up: function attributes, tensor maps
-                enqueue()
-                return be.global_losses
-            cur = torch.cuda.current_stream(be.device)
-            cur.synchronize()
-            plan.set_external_scalars(True)
-            try:
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                    enqueue()
-            finally:
-                plan.set_external_scalars(False)
-            if len(be.graphs) >= 8:
-                be.graphs.clear()
-            entry = be.graphs[key] = (g, dict(batch))
-        plan.push_scalars(hp, seed=seed, row_offset=row_offset, fused=False)
-        entry[0].replay()
-        return be.global_losses
-
     def step(self, batch, hp_kwargs=None, eps=None, seed=0, row_offset=0, host_flags=None):
         """batch: this rank's shard (same fields as Plan.train_step).  Returns the GLOBAL losses as
         an 8-vector (RECL, KLD, PERT, YL, MMD, ELBO, CMPL, 0) identical on every rank.
@@ -252,23 +154,26 @@ class DataParallel:
         n = batch["x1"].shape[-2]
         flags = host_flags if host_flags is not None else batch
         local = local_counts(n, flags.get("has_x2"), flags.get("has_y"))
+        hp_kwargs = dict(hp_kwargs or {})
+        it = self.finished_training_iters
         if getattr(be, "peer", False):
-            losses = self._step_peer(be, batch, dict(hp_kwargs or {}), local, eps, seed, row_offset)
+            # the counts exchange is also the barrier that keeps a fast rank from overwriting a gradient a slow rank
+            # still reads
+            be.plan.dp_exchange_counts(local, it + 1)
+            hp = be.plan.hparams(step=it, global_counts_ptr=be.plan.dp_counts_ptr, **hp_kwargs)
+            losses = be.plan.dp_train_step(batch, hp, be.global_losses, eps=eps, seed=seed, row_offset=row_offset)
             self.finished_training_iters += 1
             return losses
-        # (single rank only: with NCCL collectives inside the capture the one 2-rank attempt of this round deadlocked,
-        #  so ranks > 1 keep the eager, event-overlapped path below)
-        if getattr(be, "graph", False) and self.world == 1 and eps is None and \
-                all(torch.is_tensor(v) and v.is_cuda for v in batch.values()):
-            losses = self._step_graph(be, batch, dict(hp_kwargs or {}), local, seed, row_offset)
+        if self.world == 1 and isinstance(be, PlanBackend):
+            hp = be.plan.hparams(step=it, global_counts=local, **hp_kwargs)
+            losses = be.plan.dp_train_step(batch, hp, be.plan.losses[0], eps=eps, seed=seed, row_offset=row_offset)
             self.finished_training_iters += 1
             return losses
         if self.world > 1 and getattr(be, "comm_stream", None) is not None:
             counts = global_counts_device(local, be.device, self.group)  # GPU backend: no host round trip
         else:
             counts = global_counts(local, self.group, device=getattr(be, "device", "cpu"))
-        losses, events = be.grad_step(batch, dict(hp_kwargs or {}), counts, self.finished_training_iters, eps=eps, seed=seed,
-                                      row_offset=row_offset)
+        losses, events = be.grad_step(batch, hp_kwargs, counts, it, eps=eps, seed=seed, row_offset=row_offset)
         flat = be.flat_grads()
         comm = getattr(be, "comm_stream", None)
         if comm is None:  # CPU backend (tests): no streams, one reduce per bucket in the same order

@@ -271,17 +271,6 @@ class Plan:
     def loss_forward(self, batch, hp, eps=None, seed=0, row_offset=0):
         return self._run(self.lib.drvae_loss_forward, "loss_forward", batch, hp, eps, seed, row_offset)
 
-    def push_scalars(self, hp, seed=0, row_offset=0, fused=False):
-        """Write one call's per-step scalars to the plan's device block without running a step (caller-side graph
-        capture: see drvae_b200/dp.py)."""
-        nz, _ = self._noise(None, seed, row_offset)
-        with torch.cuda.device(self.device):
-            _lib.check(self.lib.drvae_push_scalars(self.h, ctypes.byref(nz), ctypes.byref(hp), int(bool(fused)), self._stream()),
-                       "push_scalars")
-
-    def set_external_scalars(self, enable):
-        _lib.check(self.lib.drvae_set_external_scalars(self.h, int(bool(enable))), "set_external_scalars")
-
     def adam_step(self, hp):
         with torch.cuda.device(self.device):
             _lib.check(self.lib.drvae_adam_step(self.h, ctypes.byref(hp), self._stream()), "adam_step")
@@ -305,9 +294,10 @@ class Plan:
             _lib.check(self.lib.drvae_dp_exchange_counts(self.h, int(counts[0]), int(counts[1]), int(counts[2]), int(tag), self._stream()),
                        "dp_exchange_counts")
 
-    def dp_adam_step(self, hp, losses_out):
-        with torch.cuda.device(self.device):
-            _lib.check(self.lib.drvae_dp_adam_step(self.h, ctypes.byref(hp), _ptr(losses_out), self._stream()), "dp_adam_step")
+    def dp_train_step(self, batch, hp, losses_out, eps=None, seed=0, row_offset=0):
+        """One data-parallel optimisation step (drvae_dp_train_step): with peers attached gradient, NVLink reduction and
+        Adam, the global losses written to losses_out (8 floats); without, this plan's rows alone ([n_models, 8])."""
+        return self._run(self.lib.drvae_dp_train_step, "dp_train_step", batch, hp, eps, seed, row_offset, losses_out)
 
     def infer(self, x1):
         x1 = x1.to(self.device, torch.float32).contiguous()

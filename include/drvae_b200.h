@@ -194,9 +194,9 @@ int drvae_stream_wait_bucket(drvae_plan_t* plan, int index, void* stream);
  *   drvae_dp_exchange_counts   batch-global normalisers {N, Np, Nlab}: posted to all peers, summed into
  *                              drvae_dp_counts_ptr() (pass it as drvae_hparams_t.global_counts_dev); also the barrier
  *                              that keeps a fast rank from overwriting a gradient a slow rank still reads
- *   drvae_grad_step            with losses_out = own gradient vector + param_count (loss shares join the reduction)
- *   drvae_dp_adam_step         cross-GPU barrier (tag = step + 1, read from the per-step scalars so it replays inside a
- *                              CUDA graph) + ONE kernel that sums every rank's gradient over NVLink in rank order and
+ *   drvae_dp_train_step        forward + backward into the own gradient vector, the loss shares right behind it (they
+ *                              join the reduction), then a cross-GPU barrier (tag = step + 1, read from the per-step
+ *                              scalars) + ONE kernel that sums every rank's gradient over NVLink in rank order and
  *                              applies Adam and the shadow refresh; global losses -> losses_out (device, 8 floats)
  * grads_multicast (optional): NVLS multicast mapping of the gradient vectors; the sum is then formed inside the
  * switch (multimem.ld_reduce).  No NCCL call is involved; results are bit-identical on all ranks. */
@@ -210,7 +210,12 @@ int drvae_dp_attach(drvae_plan_t* plan, const drvae_dp_peers_t* peers);
 long long drvae_dp_grad_floats(const drvae_plan_t* plan);
 const long long* drvae_dp_counts_ptr(const drvae_plan_t* plan);
 int drvae_dp_exchange_counts(drvae_plan_t* plan, long long N, long long Np, long long Nlab, long long tag, void* stream);
-int drvae_dp_adam_step(drvae_plan_t* plan, const drvae_hparams_t* hp, float* losses_out, void* stream);
+/* One data-parallel optimisation step, always through the gradient buffer and the stand-alone optimizer (never the
+ * grouped dW+Adam launch of drvae_train_step).  With peers attached: the exchange above.  Without: this rank's rows
+ * alone, drvae_grad_step + drvae_adam_step in one call, losses -> losses_out [n_models][8].  Replayed as a CUDA graph
+ * like drvae_train_step. */
+int drvae_dp_train_step(drvae_plan_t* plan, const drvae_batch_t* batch, const drvae_noise_t* noise,
+                        const drvae_hparams_t* hp, float* losses_out, void* stream);
 int drvae_infer(drvae_plan_t* plan, const float* x1, int N, const drvae_infer_out_t* out, void* stream);
 /* Inference arithmetic.  fp32 != 0 (default): the mu-path is evaluated with fp32 operands and fp32 accumulation from
  * the master parameters, so that class probabilities agree with the reference to ~1e-6 and thresholded predictions
@@ -228,19 +233,12 @@ long long drvae_eval_workspace_bytes(int N, int X);
 int drvae_eval_x_reconstruction(const float* x, const float* x_rec, const float* x_sigma, const int* mask, int N, int X,
                                 double* out, void* workspace, void* stream);
 
-/* Launch mechanism.  With graphs enabled (default) drvae_train_step / drvae_loss_forward replay their launch
- * sequence as a CUDA graph from the third call with the same (N, batch buffers, output buffer, stream) on;
- * per-step scalars live in device memory, so only one kernel node's arguments change between steps.  Calls on
- * the legacy default stream, with a caller-provided eps block, or under profiling are launched kernel by kernel. */
+/* Launch mechanism.  With graphs enabled (default) drvae_train_step / drvae_loss_forward / drvae_dp_train_step
+ * replay their launch sequence as a CUDA graph from the second call with the same (N, batch buffers, output buffer,
+ * stream) on; per-step scalars live in device memory, so only one kernel node's arguments change between steps.
+ * Calls on the legacy default stream, with a caller-provided eps block, or under profiling are launched kernel by
+ * kernel, and so is drvae_grad_step.  drvae_plan_launch_count counts the launches of a replayed graph too. */
 int drvae_set_graph(drvae_plan_t* plan, int enable);
-/* Caller-side graph capture (drvae_b200/dp.py captures grad_step + its NCCL all-reduces + adam_step as one CUDA
- * graph): drvae_push_scalars writes a call's per-step scalars (step number, Adam bias corrections, beta_pert, noise
- * seed / row offset, global counts) to the plan's device block WITHOUT running a step; while external scalars are
- * enabled the step entry points do not write that block themselves, so a captured launch sequence can be replayed
- * with fresh scalars pushed before each replay. */
-int drvae_push_scalars(drvae_plan_t* plan, const drvae_noise_t* noise, const drvae_hparams_t* hp, int fused_adam,
-                       void* stream);
-int drvae_set_external_scalars(drvae_plan_t* plan, int enable);
 long long drvae_plan_graph_replays(const drvae_plan_t* plan);
 /* Captures that failed (that call shape then runs as plain launches; other shapes still capture): 0 on a healthy plan. */
 long long drvae_plan_graph_failures(const drvae_plan_t* plan);

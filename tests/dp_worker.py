@@ -68,7 +68,8 @@ def main():
         res = {"backend": backend, "world": world, "worst_rel_loss_err": worst,
                "param_rel_l2": float((params - pref).norm() / pref.norm()),
                "max_param_abs_diff": float((params - pref).abs().max()),
-               "ranks_identical": True, "graphs": len(getattr(be, "graphs", {})),
+               "ranks_identical": True, "graph_replays": plan.graph_replays(),
+               "graph_failures": plan.graph_failures(),
                "multicast": bool(getattr(be, "multicast", False))}
     if rank == 0:
         print("DPRESULT " + json.dumps(res), flush=True)

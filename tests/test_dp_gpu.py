@@ -32,5 +32,5 @@ def test_two_rank_data_parallel_step_equals_single_gpu_step(backend, arch, N):
     print(r)
     assert r["worst_rel_loss_err"] < 2e-5 if arch == "tiny" else r["worst_rel_loss_err"] < 1e-4, r
     assert r["param_rel_l2"] < 1e-4, r
-    if backend == "peer":
-        assert r["graphs"] == 1
+    if backend == "peer":  # the plan captures the step on its second call and replays it from then on
+        assert r["graph_replays"] >= 4 and r["graph_failures"] == 0, r
