@@ -411,8 +411,12 @@ extern "C" int drvae_plan_create(const drvae_arch_t* a, int n_models, drvae_plan
 extern "C" int drvae_plan_create_clf(const drvae_arch_t* a, int n_clf, const int* clf_hidden, int n_models, drvae_plan_t** out) {
   if (!a || !out) return set_error("drvae_plan_create: null argument");
   if (n_models < 1) return set_error("drvae_plan_create: n_models must be >= 1");
+  // the Philox counter has 20 bits for the model and 8 for the MC sample (drvae_noise_t): beyond them two models or two
+  // samples would draw the same normals
+  if (n_models > DRVAE_MAX_MODELS) return set_error("drvae_plan_create: n_models must be <= 1048576 (2^20)");
   if (a->kind < 0 || a->kind > 2) return set_error("drvae_plan_create: unknown model kind");
   if (a->dim_x < 1 || a->dim_z1 < 1 || a->L < 1 || a->max_batch < 1) return set_error("drvae_plan_create: bad dimensions");
+  if (a->L > DRVAE_MAX_L) return set_error("drvae_plan_create: L must be <= 256 Monte-Carlo samples");
   if (a->dim_z1 > 32 * MAXJ) return set_error("drvae_plan_create: dim_z1 > 256 is not supported");
   if (a->kind != DRVAE_KIND_PVAE && (a->dim_y < 2 || a->dim_y > MAXY)) return set_error("drvae_plan_create: dim_y must be in [2, 8]");
   if (a->kind != DRVAE_KIND_PVAE && (a->dim_z3 < 1 || a->dim_z3 > 32 * MAXJ)) return set_error("drvae_plan_create: dim_z3 must be in [1, 256]");
@@ -1944,6 +1948,10 @@ int step_entry(drvae_plan* pl, int seq, const drvae_batch_t* b, const drvae_nois
                float* losses_out, cudaStream_t st) {
   if (!hp) return set_error("drvae: hparams is null");
   if (!b) return set_error("drvae: batch is null");
+  // own noise is keyed by the global row row_offset + r in 40 bits (drvae_noise_t): outside [0, 2^40) rows would wrap
+  // onto other rows' normals
+  if (nz && !nz->eps && (nz->row_offset < 0 || nz->row_offset > DRVAE_MAX_ROWS - (long long)b->N))
+    return set_error("drvae: noise.row_offset must be >= 0 and row_offset + N <= 2^40");
   const bool fused = seq == SEQ_TRAIN && train_is_fused(pl, b);
   const StepDyn dyn = make_dyn(nz, hp, fused);
   const bool graphable = pl->graph_enabled && !pl->prof_on && !(nz && nz->eps) && seq != SEQ_GRAD && pl->shadows_valid &&

@@ -34,6 +34,9 @@ extern "C" {
 #define DRVAE_KIND_VFAE 2
 #define DRVAE_MAX_HIDDEN 4
 #define DRVAE_MAX_CLF_WIDTH 4096
+#define DRVAE_MAX_L 256                 /* Monte-Carlo samples per row (drvae_arch_t.L) */
+#define DRVAE_MAX_MODELS (1 << 20)      /* n_models of one plan */
+#define DRVAE_MAX_ROWS (1LL << 40)      /* global rows addressable by own noise (drvae_noise_t.row_offset + N) */
 
 typedef struct drvae_plan drvae_plan_t;
 
@@ -78,7 +81,10 @@ typedef struct {
 /* Noise.  eps != NULL: parity mode, a row-indexed block of standard normals per model laid out
  * as drvae_eps_layout() reports.  eps == NULL: the step draws its own with Philox4x32-10 keyed by
  * (seed, step, model, draw kind, MC sample, row_offset + row, feature): a data-parallel shard that
- * passes the global index of its first row draws the noise of the unsharded minibatch. */
+ * passes the global index of its first row draws the noise of the unsharded minibatch.  The counter holds the
+ * model in 20 bits, the MC sample in 8 and the global row in 40, so every key is distinct only inside these ranges,
+ * which the library enforces: n_models <= 2^20 and L <= 256 (drvae_plan_create), and with eps == NULL
+ * 0 <= row_offset and row_offset + N <= 2^40 (each step entry point). */
 typedef struct {
   const float* eps;
   unsigned long long seed;
