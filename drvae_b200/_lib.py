@@ -63,6 +63,16 @@ class DpPeers(ctypes.Structure):
                 ("grads_multicast", c_void_p)]
 
 
+class EvalMembersIn(ctypes.Structure):
+    _fields_ = [(n, c_void_p) for n in ("valid", "x1", "px1_mu", "px1_sg", "x2", "px2_mu", "px2_sg", "has_x2", "proba",
+                                        "pred", "y", "has_y")]
+
+
+# the output columns of drvae_eval_members, in the header's order
+EVAL_MEMBER_COLUMNS = ("y_acc", "y_auroc", "y_aupr", "x1_rmse", "x1_r2", "x1_pearr", "x1_ll", "x2_rmse", "x2_r2",
+                       "x2_pearr", "x2_ll")
+
+
 class InferOut(ctypes.Structure):
     _fields_ = [(n, c_void_p) for n in ("z1_mu", "z1_lv", "z2_mu", "z2_lv", "proba", "pred", "px1_mu", "px1_sg",
                                         "px2_mu", "px2_sg")]
@@ -77,7 +87,8 @@ EXPORTS = ["drvae_last_error", "drvae_plan_create", "drvae_plan_destroy", "drvae
            "drvae_profile_end", "drvae_plan_num_buckets", "drvae_plan_bucket_info", "drvae_stream_wait_bucket", "drvae_set_graph", "drvae_plan_graph_replays", "drvae_debug_wait_stats",
            "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
            "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_train_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
-           "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams", "drvae_plan_create_clf"]
+           "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams", "drvae_plan_create_clf",
+           "drvae_eval_members_workspace_bytes", "drvae_eval_members"]
 
 
 def load():
@@ -135,6 +146,10 @@ def load():
     lib.drvae_eval_workspace_bytes.argtypes = [c_int, c_int]
     lib.drvae_eval_x_reconstruction.restype = c_int
     lib.drvae_eval_x_reconstruction.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]
+    lib.drvae_eval_members_workspace_bytes.restype = c_ll
+    lib.drvae_eval_members_workspace_bytes.argtypes = [c_int, c_int, c_int, c_int]
+    lib.drvae_eval_members.restype = c_int
+    lib.drvae_eval_members.argtypes = [P(EvalMembersIn), c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]
     lib.drvae_set_step_kernel.restype = c_int
     lib.drvae_set_step_kernel.argtypes = [c_void_p, c_int]
     lib.drvae_plan_step_kernel_launches.restype = c_ll

@@ -13,7 +13,8 @@ import torch
 from . import checkpoint
 from .init import init_state_dict
 from .plan import Plan, anneal_coef
-from .training import SnapshotRule, eval_x_reconstruction, eval_y_prediction, validation_objective
+from ._lib import EVAL_MEMBER_COLUMNS
+from .training import SnapshotRule, eval_members, validation_objective
 
 FIELDS = {"drvae": ("x1", "x2", "y", "has_x2", "has_y"), "pvae": ("x1", "x2", "has_x2"), "vfae": ("x1", "y", "has_y")}
 MODEL_CLASS = {"drvae": "DrVAE", "pvae": "PVAE", "vfae": "VFAE"}
@@ -45,27 +46,25 @@ def steps_per_epoch(sizes, batch_size):
 
 def evaluate_members(plan, kind, fields, mask):
     """Per-member metrics of evaluate_performance (training.py) on padded device data: one ensemble inference in
-    chunks of the plan's row capacity, then the reference's metrics over each member's real rows.  -> [perf dict]."""
+    chunks of the plan's row capacity, one drvae_eval_members call over every member's real rows, and one [E, 11] read
+    back.  -> [perf dict]."""
     D = fields["x1"].shape[1]
     outs = [plan.infer(fields["x1"][:, c0:c0 + plan.Ncap]) for c0 in range(0, D, plan.Ncap)]
     res = {k: torch.cat([o[k] for o in outs], 1) for k in outs[0]}
+    groups = dict(x1=fields["x1"], px1_mu=res["px1_mu"], px1_sg=res["px1_sg"])
+    keys = ["x1_rmse", "x1_r2", "x1_pearr", "x1_ll"]
+    if kind != "pvae":
+        groups.update(proba=res["proba"], pred=res["pred"], y=fields["y"], has_y=fields["has_y"])
+        keys = ["y_acc", "y_auroc", "y_aupr"] + keys
+    if kind != "vfae":
+        groups.update(x2=fields["x2"], px2_mu=res["px2_mu"], px2_sg=res["px2_sg"], has_x2=fields["has_x2"])
+        keys += ["x2_rmse", "x2_r2", "x2_pearr", "x2_ll"]
+    table = eval_members(mask, **groups).cpu().tolist()
     perfs = []
-    for m in range(plan.E):
-        valid = mask[m] != 0
+    for row in table:
+        v = dict(zip(EVAL_MEMBER_COLUMNS, row))
         perf = OrderedDict(losses=None)
-        if kind != "pvae":
-            idx = torch.nonzero(valid & (fields["has_y"][m] != 0)).view(-1)
-            y = eval_y_prediction(res["pred"][m][idx].long(), res["proba"][m][idx], fields["y"][m][idx], plan.dim_y)
-            perf.update(("y_" + k, v) for k, v in y.items())
-        x1 = eval_x_reconstruction(fields["x1"][m], res["px1_mu"][m], res["px1_sg"][m], mask=valid)
-        perf.update(("x1_" + k, v) for k, v in x1.items())
-        if kind != "vfae":
-            pair = valid & (fields["has_x2"][m] != 0)
-            if bool(pair.any()):
-                x2 = eval_x_reconstruction(fields["x2"][m], res["px2_mu"][m], res["px2_sg"][m], mask=pair)
-                perf.update(("x2_" + k, v) for k, v in x2.items())
-            else:
-                perf.update(("x2_" + k, float("nan")) for k in ("rmse", "r2", "pearr", "ll"))
+        perf.update((k, v[k]) for k in keys)
         perf["model_class"] = MODEL_CLASS[kind]
         perfs.append(perf)
     return perfs

@@ -8,8 +8,9 @@ DrVAE.py:880-963, `VFAEDataset` / `wrap_in_VFAEDataset` VFAE.py:658-721, `eval_x
 components next to the hot path: they stay host-side Python, but everything per-sample runs on
 the GPU — the forward pass through `drvae_infer`, and the reconstruction metrics (RMSE, variance-
 weighted R², the per-row Pearson correlation the reference computes in a Python loop over
-scipy.stats.pearsonr, Gaussian log-likelihood) as batched device reductions.  Only AUROC / AUPR
-go through sklearn on the (N,)-sized probability vector, as in the reference.
+scipy.stats.pearsonr, Gaussian log-likelihood) as batched device reductions, and accuracy, AUROC and
+AUPR from exact rank counts (drvae_eval_members, one call for every member of an ensemble).  The
+sklearn form of the y metrics stays as the host path for CPU tensors and as the tests' reference.
 """
 import math
 import time
@@ -168,7 +169,60 @@ def eval_x_reconstruction(x, x_rec, x_rec_sigma=None, mask=None):
     return out
 
 
+def eval_members(valid, x1=None, px1_mu=None, px1_sg=None, x2=None, px2_mu=None, px2_sg=None, has_x2=None, proba=None,
+                 pred=None, y=None, has_y=None):
+    """drvae_eval_members: the metrics of E models on padded device data in one call, no host synchronisation.
+
+    valid: int [E, D], the rows of each member; x1 / px1_mu / px1_sg, x2 / px2_mu / px2_sg: float [E, D, X]; has_x2,
+    pred, y, has_y: int [E, D]; proba: float [E, D, dim_y].  x2 metrics use the rows with valid and has_x2, y metrics
+    those with valid and has_y.  A group left out (x1, x2 or y) gives nan.  -> float64 [E, 11] device tensor, columns
+    _lib.EVAL_MEMBER_COLUMNS."""
+    import ctypes
+    from . import _lib
+    lib = _lib.load()
+    if not valid.is_cuda or valid.dim() != 2:
+        raise ValueError("eval_members: valid must be a CUDA tensor [E, D]")
+    dev = valid.device
+    E, D = valid.shape
+    X = x1.shape[2] if x1 is not None else (x2.shape[2] if x2 is not None else 1)
+    Y = proba.shape[2] if proba is not None else 0
+    keep = []
+
+    def ptr(t, dtype, width=None):
+        if t is None:
+            return None
+        if tuple(t.shape) != ((E, D) if width is None else (E, D, width)):
+            raise ValueError("eval_members: a tensor of shape %s, expected [%d, %d%s]" % (
+                tuple(t.shape), E, D, "" if width is None else ", %d" % width))
+        t = t.detach().to(dev, dtype).contiguous()
+        keep.append(t)
+        return t.data_ptr()
+
+    f, i = torch.float32, torch.int32
+    args = _lib.EvalMembersIn(valid=ptr(valid, i), x1=ptr(x1, f, X), px1_mu=ptr(px1_mu, f, X), px1_sg=ptr(px1_sg, f, X),
+                              x2=ptr(x2, f, X), px2_mu=ptr(px2_mu, f, X), px2_sg=ptr(px2_sg, f, X), has_x2=ptr(has_x2, i),
+                              proba=ptr(proba, f, Y), pred=ptr(pred, i), y=ptr(y, i), has_y=ptr(has_y, i))
+    ws = torch.empty(int(lib.drvae_eval_members_workspace_bytes(E, D, X, Y)), dtype=torch.uint8, device=dev)
+    out = torch.empty(E, len(_lib.EVAL_MEMBER_COLUMNS), dtype=torch.float64, device=dev)
+    _lib.check(lib.drvae_eval_members(ctypes.byref(args), E, D, X, Y, ctypes.c_void_p(out.data_ptr()),
+                                      ctypes.c_void_p(ws.data_ptr()), ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
+               "eval_members")
+    return out
+
+
 def eval_y_prediction(pred, proba, ylab, dim_y=2):
+    """acc, auroc, aupr (DGMMixin.py:160-190) over all given rows.  CUDA tensors go through drvae_eval_members (one
+    3-double read back); CPU tensors through sklearn, as the reference does."""
+    if proba.is_cuda:
+        n = int(ylab.shape[0])
+        if n == 0:
+            return {"acc": float("nan"), "auroc": float("nan"), "aupr": float("nan")}
+        if proba.dim() != 2 or proba.shape[1] != dim_y:
+            raise ValueError("eval_y_prediction: proba must be [N, dim_y]")
+        ones = torch.ones(1, n, dtype=torch.int32, device=proba.device)
+        v = eval_members(ones, proba=proba.unsqueeze(0), pred=pred.reshape(1, n), y=ylab.long().reshape(1, n),
+                         has_y=ones)[0, :3].cpu().tolist()
+        return {"acc": v[0], "auroc": v[1], "aupr": v[2]}
     import sklearn.metrics
     out = {}
     y = ylab.long().cpu().numpy()

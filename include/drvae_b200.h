@@ -239,6 +239,32 @@ long long drvae_eval_workspace_bytes(int N, int X);
 int drvae_eval_x_reconstruction(const float* x, const float* x_rec, const float* x_sigma, const int* mask, int N, int X,
                                 double* out, void* workspace, void* stream);
 
+/* Every metric of the evaluation path for E models (ensemble members) in one call: the reconstruction metrics above
+ * for x1 and x2, and the y metrics of DeepGenerativeModelMixin.eval_y_prediction (src/DGMMixin.py:160-190): accuracy,
+ * sklearn roc_auc_score and average_precision_score, binary on proba[:, 1] for Y == 2, one-vs-rest with a macro
+ * average for Y > 2.  Member m's rows are its D rows with valid != 0; x2 metrics use those with has_x2 != 0 too, y
+ * metrics those with has_y != 0 too.  Padding rows (valid == 0) have no effect, whatever they hold.
+ *
+ * All buffers are [E][D](...) row-major device buffers.  A group left entirely NULL gives NaN in its output columns;
+ * px1_sg / px2_sg NULL give ll = NaN.  out: device [E][11] doubles, columns in this fixed order:
+ *   0 y_acc, 1 y_auroc, 2 y_aupr, 3 x1_rmse, 4 x1_r2, 5 x1_pearr, 6 x1_ll, 7 x2_rmse, 8 x2_r2, 9 x2_pearr, 10 x2_ll
+ * A member without a selected row gets NaN for that group.  auroc / aupr are NaN when a selected row has a label outside
+ * [0, Y) or a non-finite score (binary: column 1; Y > 2: any column); a score column whose rows are all of one class
+ * gives auroc NaN and ap 1 (all positive) or 0 (none positive), as sklearn 1.9 does.  AUROC and AP are computed from
+ * exact integer counts (no sort), fp64 sums in a fixed order: two calls give bit-identical results, and E = 1 with
+ * only x1 equals drvae_eval_x_reconstruction bit for bit.  workspace: drvae_eval_members_workspace_bytes(E, D, X, Y)
+ * bytes (Y < 2: no y group). */
+typedef struct {            /* all [E][D](...) row-major device buffers; a NULL group gives nan in its outputs */
+  const int* valid;                                      /* [E][D], required */
+  const float* x1; const float* px1_mu; const float* px1_sg;   /* [E][D][X]; px1_sg may be NULL */
+  const float* x2; const float* px2_mu; const float* px2_sg;   /* [E][D][X]; NULL for VFAE */
+  const int* has_x2;                                     /* [E][D] */
+  const float* proba; const int* pred; const int* y; const int* has_y;   /* [E][D][Y], [E][D] x3; NULL for PVAE */
+} drvae_eval_members_in_t;
+long long drvae_eval_members_workspace_bytes(int E, int D, int X, int Y);
+int drvae_eval_members(const drvae_eval_members_in_t* in, int E, int D, int X, int Y,
+                       double* out /* device [E][11] */, void* workspace, void* stream);
+
 /* Launch mechanism.  With graphs enabled (default) drvae_train_step / drvae_loss_forward / drvae_dp_train_step
  * replay their launch sequence as a CUDA graph from the second call with the same (N, batch buffers, output buffer,
  * stream) on; per-step scalars live in device memory, so only one kernel node's arguments change between steps.
