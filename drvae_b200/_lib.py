@@ -19,6 +19,8 @@ c_float = ctypes.c_float
 MAX_HIDDEN = 4
 
 KIND = {"drvae": 0, "pvae": 1, "vfae": 2}
+# hidden-layer activations (DRVAE_ACT_*, drvae_set_activation)
+ACTIVATION = {"elu": 0, "softplus": 1}
 
 
 class Arch(ctypes.Structure):
@@ -88,7 +90,7 @@ EXPORTS = ["drvae_last_error", "drvae_plan_create", "drvae_plan_destroy", "drvae
            "drvae_debug_side_delay", "drvae_plan_tensor_ld", "drvae_trace_begin", "drvae_trace_end", "drvae_debug_dwa_stats", "drvae_set_infer_precision", "drvae_dp_attach", "drvae_dp_grad_floats",
            "drvae_dp_counts_ptr", "drvae_dp_exchange_counts", "drvae_dp_train_step", "drvae_plan_graph_failures", "drvae_set_step_kernel", "drvae_plan_step_kernel_launches",
            "drvae_eval_workspace_bytes", "drvae_eval_x_reconstruction", "drvae_set_member_hparams", "drvae_plan_create_clf",
-           "drvae_eval_members_workspace_bytes", "drvae_eval_members"]
+           "drvae_eval_members_workspace_bytes", "drvae_eval_members", "drvae_set_activation"]
 
 
 def load():
@@ -172,6 +174,8 @@ def load():
     lib.drvae_dp_counts_ptr.argtypes = [c_void_p]
     lib.drvae_dp_exchange_counts.restype = c_int
     lib.drvae_dp_exchange_counts.argtypes = [c_void_p, c_ll, c_ll, c_ll, c_ll, c_void_p]
+    lib.drvae_set_activation.restype = c_int
+    lib.drvae_set_activation.argtypes = [c_void_p, c_int]
     lib.drvae_set_infer_precision.restype = c_int
     lib.drvae_set_infer_precision.argtypes = [c_void_p, c_int]
     lib.drvae_trace_begin.restype = c_int

@@ -320,6 +320,26 @@ __device__ __forceinline__ uint32_t umma_idesc_bf16(int bn, int a_mn_major, int 
 __device__ __forceinline__ float elu1(float x) { return x > 0.f ? x : __expf(x) - 1.f; }
 // d ELU / d pre, recovered from the stored (bf16-rounded) activation h: 1 if h > 0 else h + 1.
 __device__ __forceinline__ float elu1_grad_from_out(float h) { return h > 0.f ? 1.f : h + 1.f; }
+// Softplus hidden layers (torch.nn.Softplus(): log1p(exp(x)), x for x > 20), stored as bf16.  The result has to keep
+// bf16's RELATIVE precision for x << 0, where softplus(x) ~ exp(x) is tiny: exp(x) without flush-to-zero (exact down to
+// the denormal range), then log1p(e) as e (1 - e (1/2 - e (1/3 - e/4))) for e < 1/16 (relative error < e^4 / 5 < 4e-6)
+// and as lg2(1 + e) ln 2 above (1 + e rounds e to 2^-24 absolute, < 3e-7 relative there).  One ex2 and one lg2 per
+// element.
+__device__ __forceinline__ float softplus_act(float x) {
+  const float LOG2E = 1.4426950408889634f, LN2 = 0.6931471805599453f;
+  float e, l;
+  asm("ex2.approx.f32 %0, %1;" : "=f"(e) : "f"(fminf(x, 20.f) * LOG2E));
+  asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"(1.f + e));
+  const float small = e * fmaf(e, fmaf(e, fmaf(e, -0.25f, 1.f / 3.f), -0.5f), 1.f);
+  return x > 20.f ? x : (e < 0.0625f ? small : l * LN2);
+}
+// d softplus / d pre = sigmoid(x), recovered from the stored (bf16-rounded) activation h as -expm1(-h): h (1 - h (1/2 -
+// h (1/6 - h/24))) for h < 1/16, where 1 - exp(-h) would cancel (h ~ exp(x) is tiny for x << 0 but carries bf16
+// relative precision; series error < h^4 / 120), 1 - exp(-h) above, 1 for h > 20.
+__device__ __forceinline__ float softplus_grad_from_out(float h) {
+  const float small = h * fmaf(h, fmaf(h, fmaf(h, -1.f / 24.f, 1.f / 6.f), -0.5f), 1.f);
+  return h > 20.f ? 1.f : (h < 0.0625f ? small : 1.f - __expf(-h));
+}
 // torch.nn.Softplus(beta=1, threshold=20)
 __device__ __forceinline__ float softplus20(float x) { return x > 20.f ? x : log1pf(expf(x)); }
 __device__ __forceinline__ float sigmoid_sp(float x) { return x > 20.f ? 1.f : 1.f / (1.f + expf(-x)); }

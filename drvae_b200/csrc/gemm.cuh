@@ -17,7 +17,7 @@
 // 8-byte elements, so a box lands in shared memory as the no-swizzle UMMA canonical layout),
 // multiplied with tcgen05.mma (bf16 in, fp32 accumulate in TMEM) by one elected thread, and the
 // accumulator tile is read back with tcgen05.ld by the epilogue warps that apply the layer's
-// epilogue (bias/ELU, ELU', Gaussian log-density + its gradient, weight gradient, ...).  The weight gradients and
+// epilogue (bias/activation, activation', Gaussian log-density + its gradient, weight gradient, ...).  The weight gradients and
 // Adam of a fused train step are not computed here but in the grouped launch of dwadam.cuh.
 //
 // A slow SIMT kernel with the *same* operand format and the *same* epilogue code is kept as a
@@ -42,8 +42,14 @@ enum {
   EPI_DACT_C8 = 2,    // * ELU'(stored activation) -> bf16 chunk8
   EPI_GRAD = 3,       // weight (+bias, +class column) gradient -> flat fp32 grad buffer, reference tensor layout
   EPI_DECLOSS = 4,    // decoder heads: Gaussian log-density partials + d loss / d pre-activation
-  EPI_DECOUT = 5      // decoder heads at inference: mu and sigma as fp32 row-major
+  EPI_DECOUT = 5,     // decoder heads at inference: mu and sigma as fp32 row-major
+  EPI_SP_C8 = 6,      // EPI_ELU_C8 with softplus hidden layers
+  EPI_DSP_C8 = 7      // EPI_DACT_C8 with softplus hidden layers: * softplus'(stored activation)
 };
+// The hidden-layer activation is a compile-time property of the epilogue: the ELU instances are the code they were
+// before softplus existed, and a softplus plan launches its own instances (plan.cu act_fwd_epi / act_bwd_epi).
+constexpr bool epi_is_act_fwd(int epi) { return epi == EPI_ELU_C8 || epi == EPI_SP_C8; }
+constexpr bool epi_is_act_bwd(int epi) { return epi == EPI_DACT_C8 || epi == EPI_DSP_C8; }
 
 constexpr int GEMM_BM = 128;
 constexpr int GEMM_BK = 64;
@@ -194,7 +200,7 @@ __device__ __forceinline__ void epi_begin(const EpiParams& e, RowCtx& rc) {
   rc.lsum = 0.f;
   rc.trow = -1;
   rc.coef = 0.f;
-  if (EPI == EPI_ELU_C8) {
+  if (epi_is_act_fwd(EPI)) {
     if (e.row_cls && rc.valid) rc.cls = e.row_cls[rc.model * e.row_cls_ms + rc.row];
   }
   if (EPI == EPI_DECLOSS) {
@@ -249,9 +255,9 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
         if (c < e.n_valid) o[c] = acc[i] + (b ? b[c] : 0.f);
       }
     }
-  } else if (EPI == EPI_ELU_C8 || EPI == EPI_DACT_C8) {
+  } else if (epi_is_act_fwd(EPI) || epi_is_act_bwd(EPI)) {
     float v[16];
-    if (EPI == EPI_DACT_C8) {
+    if (epi_is_act_bwd(EPI)) {
       const uint4* a =
           reinterpret_cast<const uint4*>(e.act + rc.model * e.act_ms) + ((long long)(col0 >> 3) * e.act_rcap + e.act_row0 + rc.row);
       uint4 q0 = a[0];
@@ -268,7 +274,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
         bool ok = rc.valid && (col0 + i) < e.n_valid;
-        v[i] = ok ? acc[i] * elu1_grad_from_out(h[i]) : 0.f;
+        v[i] = ok ? acc[i] * (EPI == EPI_DSP_C8 ? softplus_grad_from_out(h[i]) : elu1_grad_from_out(h[i])) : 0.f;
       }
     } else {
       const float* b = e.bias + rc.model * e.bias_ms + col0;
@@ -292,7 +298,7 @@ __device__ __forceinline__ void epi_chunk(const EpiParams& e, RowCtx& rc, int co
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
         int c = col0 + i;
-        const float x = elu1(acc[i] + bb[i]);
+        const float x = EPI == EPI_SP_C8 ? softplus_act(acc[i] + bb[i]) : elu1(acc[i] + bb[i]);
         // column n_valid is the ones column the next layer's dW turns into its bias gradient
         v[i] = !rc.valid ? 0.f : (c < e.n_valid ? x : (c == e.n_valid ? 1.f : 0.f));
       }
@@ -968,6 +974,8 @@ inline cudaError_t gemm_launch(int epi, const GemmProblem& p, const EpiParams& e
     case EPI_GRAD: return gemm_launch_t<EPI_GRAD>(p, e, n_models, impl, st);
     case EPI_DECLOSS: return gemm_launch_t<EPI_DECLOSS>(p, e, n_models, impl, st);
     case EPI_DECOUT: return gemm_launch_t<EPI_DECOUT>(p, e, n_models, impl, st);
+    case EPI_SP_C8: return gemm_launch_t<EPI_SP_C8>(p, e, n_models, impl, st);
+    case EPI_DSP_C8: return gemm_launch_t<EPI_DSP_C8>(p, e, n_models, impl, st);
   }
   return cudaErrorInvalidValue;
 }

@@ -14,7 +14,7 @@
 
 namespace drvae {
 
-enum { ACT_NONE = 0, ACT_ELU = 1, ACT_SOFTPLUS_EPS = 2 };
+enum { ACT_NONE = 0, ACT_ELU = 1, ACT_SOFTPLUS_EPS = 2, ACT_SOFTPLUS = 3 };  // ACT_SOFTPLUS: softplus hidden layers
 
 struct LinF32 {
   const float* X;   // [rows][ldx]
@@ -84,6 +84,7 @@ __global__ void __launch_bounds__(256) linear_f32_kernel(LinF32 a) {
       if (a.resid) y += a.resid[m * a.r_ms + (long long)r * a.ldr + n];
       if (a.act == ACT_ELU) y = y > 0.f ? y : expm1f(y);
       if (a.act == ACT_SOFTPLUS_EPS) y = (y > 20.f ? y : log1pf(expf(y))) + 1e-3f;
+      if (a.act == ACT_SOFTPLUS) y = y > 20.f ? y : log1pf(expf(y));
       a.out[m * a.o_ms + (long long)r * a.ldo + n] = y;
     }
   }

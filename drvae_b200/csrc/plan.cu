@@ -92,6 +92,7 @@ struct drvae_plan {
   // bound state
   float *params = nullptr, *adam_m = nullptr, *adam_v = nullptr, *grads = nullptr;
   int gemm_impl = GEMM_IMPL_TC;
+  int act = DRVAE_ACT_ELU;  // hidden-layer activation of every MLP (drvae_set_activation)
   long long launches = 0;
   bool shadows_valid = false;
   // per-step scalars in device memory + CUDA-graph replay of the launch sequence (see step_entry)
@@ -817,6 +818,16 @@ extern "C" int drvae_set_step_kernel(drvae_plan_t* pl, int enable) {
   return 0;
 }
 extern "C" long long drvae_plan_step_kernel_launches(const drvae_plan_t* pl) { return pl ? pl->stepk_launches : -1; }
+extern "C" int drvae_set_activation(drvae_plan_t* pl, int act) {
+  if (!pl) return set_error("drvae_set_activation: null plan");
+  if (act != DRVAE_ACT_ELU && act != DRVAE_ACT_SOFTPLUS)
+    return set_error("drvae_set_activation: act must be DRVAE_ACT_ELU (0) or DRVAE_ACT_SOFTPLUS (1)");
+  // captured sequences (and the step kernel's op tables inside them) launch the old activation's epilogue instances;
+  // an uncaptured step records its tables afresh
+  if (pl->act != act) drop_graphs(pl);
+  pl->act = act;
+  return 0;
+}
 extern "C" int drvae_debug_side_delay(drvae_plan_t* pl, long long cycles) {
   if (!pl || cycles < 0) return set_error("drvae_debug_side_delay: bad argument");
   pl->side_delay_cycles = cycles;
@@ -1152,7 +1163,10 @@ struct Exec {
     st = chain_st;
   }
 
-  EpiParams epi_elu(const Shadow& W, const C8Buf& out, int width, bool class_aug) const {
+  // the hidden-layer activation's forward (bias + activation -> bf16 chunk8) and backward (* activation') epilogues
+  int act_fwd_epi() const { return pl->act == DRVAE_ACT_SOFTPLUS ? EPI_SP_C8 : EPI_ELU_C8; }
+  int act_bwd_epi() const { return pl->act == DRVAE_ACT_SOFTPLUS ? EPI_DSP_C8 : EPI_DACT_C8; }
+  EpiParams epi_act(const Shadow& W, const C8Buf& out, int width, bool class_aug) const {
     EpiParams e = epi_base();
     e.out_c8 = out.p;
     e.out_c8_ms = out.ms;
@@ -1198,7 +1212,7 @@ struct Exec {
     for (size_t i = 0; i < b.hidden.size(); ++i) {
       const C8Buf& src = (i == 0) ? in : b.H[i - 1];
       sub = "h" + std::to_string(i);
-      gemm_nt(src, i == 0 ? in_row0 : 0, b.hidden[i], EPI_ELU_C8, epi_elu(b.hidden[i], b.H[i], b.widths[i], b.class_aug && i == 0),
+      gemm_nt(src, i == 0 ? in_row0 : 0, b.hidden[i], act_fwd_epi(), epi_act(b.hidden[i], b.H[i], b.widths[i], b.class_aug && i == 0),
               dyn_which, row_bound);
     }
     sub = "head";
@@ -1210,7 +1224,7 @@ struct Exec {
                  int dyn_which, int row_bound) {
     const int n = (int)b.hidden.size();
     sub = "head";
-    gemm_dx(dYh, b.head, EPI_DACT_C8, epi_dact(b.H[n - 1], b.dPre[n - 1], b.widths[n - 1]), dyn_which, row_bound);
+    gemm_dx(dYh, b.head, act_bwd_epi(), epi_dact(b.H[n - 1], b.dPre[n - 1], b.widths[n - 1]), dyn_which, row_bound);
     if (after_head_dx) {
       auto hook = std::move(after_head_dx);
       after_head_dx = nullptr;
@@ -1228,7 +1242,7 @@ struct Exec {
       const C8Buf& src = (i == 0) ? in : b.H[i - 1];
       sub = "h" + std::to_string(i);
       if (i > 0) {
-        gemm_dx(b.dPre[i], b.hidden[i], EPI_DACT_C8, epi_dact(b.H[i - 1], b.dPre[i - 1], b.widths[i - 1]), dyn_which, row_bound);
+        gemm_dx(b.dPre[i], b.hidden[i], act_bwd_epi(), epi_dact(b.H[i - 1], b.dPre[i - 1], b.widths[i - 1]), dyn_which, row_bound);
       } else if (dx_out) {
         gemm_dx(b.dPre[0], b.hidden[0], EPI_STORE_F32, epi_f32(dx_out, dx_ms, in_feat, in_feat, nullptr), dyn_which, row_bound);
       }
@@ -1608,8 +1622,14 @@ int run_step(drvae_plan* pl, const drvae_batch_t* b, const drvae_noise_t* nz, co
       ex.row_op(SROW_CLF_BACK, "clf_back", row_items(LNb), 0,
                 [&]() { launch_k(clf_back_kernel, rows_grid(LNb), dim3(ROW_THREADS), 0, ex.st, v); });
     if (pl->clf_nh > 0) {
-      ex.row_op(SROW_CLF_BACK_H, "clf_back", row_items(round_up(LNb, 128)), 0,
-                [&]() { launch_k(clf_back_h_kernel, rows_grid(round_up(LNb, 128)), dim3(ROW_THREADS), 0, ex.st, v); });
+      if (pl->act == DRVAE_ACT_SOFTPLUS)
+        ex.row_op(SROW_CLF_BACK_H_SP, "clf_back", row_items(round_up(LNb, 128)), 0, [&]() {
+          launch_k(clf_back_h_kernel<EPI_DSP_C8>, rows_grid(round_up(LNb, 128)), dim3(ROW_THREADS), 0, ex.st, v);
+        });
+      else
+        ex.row_op(SROW_CLF_BACK_H, "clf_back", row_items(round_up(LNb, 128)), 0, [&]() {
+          launch_k(clf_back_h_kernel<EPI_DACT_C8>, rows_grid(round_up(LNb, 128)), dim3(ROW_THREADS), 0, ex.st, v);
+        });
       const bool split_du = pl->clf_in > pl->Z;
       float* du = split_du ? pl->clfv.dU.p : v.DZ1.p;
       const long long du_ms = split_du ? pl->clfv.dU.ms : v.DZ1.ms;
@@ -2222,12 +2242,13 @@ int run_infer_fp32(drvae_plan* pl, const float* x1, int N, const drvae_infer_out
     if (lerr == cudaSuccess) lerr = cudaGetLastError();
   };
   // hidden layers of a block: leaves (h, h_ms, h_ld) on the last activation
+  const int hidden_act = pl->act == DRVAE_ACT_SOFTPLUS ? ACT_SOFTPLUS : ACT_ELU;
   auto hidden = [&](const MlpBlock& b, const float* in, long long in_ms, int in_ld, const float*& h, long long& h_ms, int& h_ld) {
     h = in, h_ms = in_ms, h_ld = in_ld;
     for (size_t i = 0; i < b.hidden.size(); ++i) {
       const Shadow& W = b.hidden[i];
       float* dst = (h == Ha) ? Hb : Ha;
-      lin(h, h_ms, h_ld, W.w_off[0], W.b_off[0], W.ld, b.widths[i], W.kin, 0.f, ACT_ELU, nullptr, 0, 0, dst, ws_ms, maxw);
+      lin(h, h_ms, h_ld, W.w_off[0], W.b_off[0], W.ld, b.widths[i], W.kin, 0.f, hidden_act, nullptr, 0, 0, dst, ws_ms, maxw);
       h = dst, h_ms = ws_ms, h_ld = maxw;
     }
   };

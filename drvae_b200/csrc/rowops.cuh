@@ -851,9 +851,11 @@ __global__ void __launch_bounds__(ROW_THREADS) clf_back_kernel(DevView v) {
   clf_back_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
-// The same with hidden layers: d loss / d logits, then dPre of the last hidden layer, (dl . W_p) * ELU'(H) as bf16
+// The same with hidden layers: d loss / d logits, then dPre of the last hidden layer, (dl . W_p) * act'(H) as bf16
 // chunk8, with zero rows [LN, pad128(LN)) (the weight-gradient GEMMs contract over them).  The block's dX / dW GEMMs
-// and clf_du take it from there.  grid (ceil(pad128(LNcap) / ROW_WARPS), n_models)
+// and clf_du take it from there.  DACT: the activation's backward epilogue id (EPI_DACT_C8: ELU, EPI_DSP_C8: softplus).
+// grid (ceil(pad128(LNcap) / ROW_WARPS), n_models)
+template <int DACT>
 __device__ __forceinline__ void clf_back_h_row(const DevView& v, const int m, const int r, const int lane) {
   const int* cnt = v.counts.at(m);
   const int N = cnt[CNT_N], LN = cnt[CNT_LN], Fl = cnt[CNT_FL];
@@ -880,15 +882,16 @@ __device__ __forceinline__ void clf_back_h_row(const DevView& v, const int m, co
         for (int j = 0; j < MAXY; ++j)
           if (j < v.Y) g = fmaf(dl[j], Wc[j * v.clf_ld + f], g);
       }
-      d[e] = f < cv.pin ? g * elu1_grad_from_out(h[e]) : 0.f;
+      d[e] = f < cv.pin ? g * (DACT == EPI_DSP_C8 ? softplus_grad_from_out(h[e]) : elu1_grad_from_out(h[e])) : 0.f;
     }
     dp[(long long)c * cv.D.rcap] = pack_bf16x8(d);
   }
 }
 
+template <int DACT>
 __global__ void __launch_bounds__(ROW_THREADS) clf_back_h_kernel(DevView v) {
   TraceScope trace_scope(v.trace, v.trace_id);
-  clf_back_h_row(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+  clf_back_h_row<DACT>(v, blockIdx.y, blockIdx.x * ROW_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // clf_du (DrVAE, hidden layers): d loss / d u = [dz1 part | dz2f part] from the first layer's dX GEMM ->

@@ -55,7 +55,8 @@ enum {
   SROW_CLF_DU,
   SROW_CLF_U,
   SROW_CLF_BACK_H,
-  SROW_CLF_GRAD_PARTIAL_H
+  SROW_CLF_GRAD_PARTIAL_H,
+  SROW_CLF_BACK_H_SP  // SROW_CLF_BACK_H with softplus hidden layers
 };
 
 struct StepOp {
@@ -337,6 +338,8 @@ __global__ void __launch_bounds__(STEPK_THREADS, 1) step_kernel(const __grid_con
             case EPI_DACT_C8: step_gemm_epilogue<EPI_DACT_C8>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
             case EPI_DECLOSS: step_gemm_epilogue<EPI_DECLOSS>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
             case EPI_GRAD: step_gemm_epilogue<EPI_GRAD>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
+            case EPI_SP_C8: step_gemm_epilogue<EPI_SP_C8>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
+            case EPI_DSP_C8: step_gemm_epilogue<EPI_DSP_C8>(p, e, t, tmem_base, a, q, cg, lane, have_acc); break;
             default: break;
           }
           tc_fence_before();
@@ -382,7 +385,8 @@ __global__ void __launch_bounds__(STEPK_THREADS, 1) step_kernel(const __grid_con
             case SROW_CLF_BACK: clf_back_row(T.v, m, r, lane); break;
             case SROW_CLF_DU: clf_du_row(T.v, m, r, lane); break;
             case SROW_CLF_U: clf_u_row(T.v, m, r, lane); break;
-            case SROW_CLF_BACK_H: clf_back_h_row(T.v, m, r, lane); break;
+            case SROW_CLF_BACK_H: clf_back_h_row<EPI_DACT_C8>(T.v, m, r, lane); break;
+            case SROW_CLF_BACK_H_SP: clf_back_h_row<EPI_DSP_C8>(T.v, m, r, lane); break;
             case SROW_CLF_GRAD_PARTIAL_H: clf_grad_partial_h_block(T.v, m, blk, threadIdx.x - GEMM_EPI_WARP0 * 32, GEMM_EPI_WARPS * 32); break;
             case SROW_T_BACK: 
               if (T.v.Zc <= 128)
@@ -467,7 +471,7 @@ struct StepRecorder {
     cur[w] = std::max(cur[w], cur[p]);
   }
   void add_gemm(int epi, const GemmProblem& p, const EpiParams& e, int n_models, cudaStream_t s, const std::string& tag) {
-    if (epi != EPI_STORE_F32 && epi != EPI_ELU_C8 && epi != EPI_DACT_C8 && epi != EPI_DECLOSS && epi != EPI_GRAD) unsupported = true;
+    if (epi != EPI_STORE_F32 && !epi_is_act_fwd(epi) && !epi_is_act_bwd(epi) && epi != EPI_DECLOSS && epi != EPI_GRAD) unsupported = true;
     if (p.BN > 256) unsupported = true;
     Rec r{};
     r.op.kind = SOP_GEMM;

@@ -12,11 +12,13 @@ import torch
 
 
 def init_state_dict(kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=(), dec_z1=(), seed=12345, weight_norm=False,
-                    clf_hidden=()):
+                    clf_hidden=(), activation=None):
     """weight_norm=True: every layer except decoder_z2Fz1 is a layers.WeightNormLinear, which adds a `.g`
     vector initialised to ones without consuming random numbers (reference layers.py:17-23).
     clf_hidden (dim_h_clf): the classifier's MLP layers encoder_y.nnet.model.linear{i}, created before its linear_p
-    like every other block's MLP (CategoricalDecoder, blocks.py:456-463)."""
+    like every other block's MLP (CategoricalDecoder, blocks.py:456-463).
+    activation: ignored (the initial weights do not depend on the nonlinearity); accepted so that a Plan's shape
+    arguments, activation included, can be passed to both."""
     torch.manual_seed(seed)
     sd = OrderedDict()
 

@@ -11,8 +11,11 @@ fused forward + ELBO + backward + Adam launch sequence.
 
 Options the reference advertises but that are broken as shipped (SURVEY.md §0 fact 7) or outside
 the hot path raise ValueError here instead of failing later: use_s=True, type_rec other than
-'diag_gaussian', MMD with use_s, continuous y, clf_1sig, dropout, non-ELU nonlinearities, Adamax.
-The classifier's hidden layers (dim_h_clf, --class-y) are supported: ELU layers in front of linear_p.
+'diag_gaussian', MMD with use_s, continuous y, clf_1sig, dropout, nonlinearities other than ELU and
+softplus, Adamax.  `nonlinearity` is 'elu' (what the run_*.py drivers pass) or 'softplus' (the
+constructors' default, nn.Softplus in the reference's table, src/blocks.py:21-24): it is the activation of
+every hidden layer, the classifier's included.  The classifier's hidden layers (dim_h_clf, --class-y) are
+supported: hidden layers in front of linear_p.
 """
 import inspect
 import warnings
@@ -75,8 +78,8 @@ class _B200Model(nn.Module):
                              % (type(self).__name__, msg))
         if self.type_rec != 'diag_gaussian':
             bad("type_rec=%r (the reference only ships DiagGaussianSigmaModule)" % (self.type_rec,))
-        if self.nonlinearity != 'elu':
-            bad("nonlinearity=%r (run_*.py fix 'elu')" % (self.nonlinearity,))
+        if self.nonlinearity not in ('elu', 'softplus'):
+            bad("nonlinearity=%r (only 'elu' and 'softplus')" % (self.nonlinearity,))
         if self.use_s:
             bad("use_s=True (crashes in the reference, SURVEY.md fact 7)")
         if self.dropout_rate or self.input_x_dropout:
@@ -107,7 +110,7 @@ class _B200Model(nn.Module):
             arch['clf_hidden'] = _as_list(self.dim_h_clf)
         self._arch = arch
         self.plan = Plan(self.kind, L=self.L, max_batch=max(int(self.batch_size), 1), n_models=1,
-                         weight_norm=self.wn, **arch)
+                         weight_norm=self.wn, activation=self.nonlinearity, **arch)
         self._max_batch = self.plan.Ncap
         sd = init_state_dict(self.kind, seed=self.random_seed, weight_norm=self.wn, **arch)
         self.plan.load_state_dict(sd)
@@ -131,7 +134,8 @@ class _B200Model(nn.Module):
         if n > self._max_batch:
             # re-plan with a larger row capacity, keeping parameters and optimizer state
             old = self.plan
-            self.plan = Plan(self.kind, L=self.L, max_batch=int(n), n_models=1, weight_norm=self.wn, **self._arch)
+            self.plan = Plan(self.kind, L=self.L, max_batch=int(n), n_models=1, weight_norm=self.wn,
+                             activation=old.activation, **self._arch)
             self.plan.params.copy_(old.params)
             self.plan.adam_m.copy_(old.adam_m)
             self.plan.adam_v.copy_(old.adam_v)

@@ -35,8 +35,12 @@ def anneal_coef(iter_num, iter_max=1000, iter_offset=0):
 
 class Plan:
     def __init__(self, kind, dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x, enc_z3=(), dec_z1=(), L=1, max_batch=200,
-                 n_models=1, weight_norm=False, device=None, clf_hidden=()):
-        """clf_hidden: widths of the classifier's hidden ELU layers (dim_h_clf, --class-y), DrVAE / VFAE only."""
+                 n_models=1, weight_norm=False, device=None, clf_hidden=(), activation="elu"):
+        """clf_hidden: widths of the classifier's hidden layers (dim_h_clf, --class-y), DrVAE / VFAE only.
+        activation: hidden-layer nonlinearity of every MLP, "elu" (the run_*.py drivers' choice) or "softplus" (the
+        reference constructors' default), see drvae_set_activation."""
+        if activation not in _lib.ACTIVATION:
+            raise ValueError("activation must be one of %s, got %r" % (sorted(_lib.ACTIVATION), activation))
         if not torch.cuda.is_available():
             raise RuntimeError("drvae_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = _lib.load()
@@ -70,6 +74,9 @@ class Plan:
             _lib.check(self.lib.drvae_plan_create_clf(ctypes.byref(a), len(clf_hidden), widths, self.E, ctypes.byref(h)),
                        "plan_create")
         self.h = h
+        self.activation = "elu"  # a new plan's default (DRVAE_ACT_ELU)
+        if activation != "elu":
+            self.set_activation(activation)
         self.P = int(self.lib.drvae_plan_param_count(h))
         self.tensors = []
         nm = ctypes.create_string_buffer(256)
@@ -323,6 +330,13 @@ class Plan:
         with torch.cuda.device(self.device):
             _lib.check(self.lib.drvae_infer(self.h, _ptr(x1), int(N), ctypes.byref(out), self._stream()), "infer")
         return res
+
+    def set_activation(self, activation):
+        """Hidden-layer nonlinearity, "elu" or "softplus" (drvae_set_activation); takes effect from the next call."""
+        if activation not in _lib.ACTIVATION:
+            raise ValueError("activation must be one of %s, got %r" % (sorted(_lib.ACTIVATION), activation))
+        _lib.check(self.lib.drvae_set_activation(self.h, _lib.ACTIVATION[activation]), "set_activation")
+        self.activation = activation
 
     def set_infer_precision(self, fp32=True):
         """fp32 (default): exact thresholded predictions; False: bf16 tensor-core inference."""

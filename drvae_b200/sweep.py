@@ -76,9 +76,10 @@ def fit_sweep(kind, arch, members, datasets, batch_size=200, L=1, epochs=300, ea
     """Train E members in one plan.
 
     kind: "drvae" | "pvae" | "vfae"; arch: Plan's shape arguments (dim_x, dim_y, dim_z1, dim_z3, enc_z1, dec_x,
-    enc_z3, dec_z1).  members: E dicts {"seed": int, "hparams": dict of Plan.MEMBER_KEYS}.  datasets: E pairs
-    (train, valid) of DrVAEDataset / VFAEDataset.  anneal_perturb: (itermax, offset) of the perturbation-loss anneal,
-    or None for a constant 1 (VFAE).  weights: optional E sampling-weight tensors over each training split.
+    enc_z3, dec_z1, clf_hidden) and optionally its activation ("elu" | "softplus"; init_state_dict ignores it).
+    members: E dicts {"seed": int, "hparams": dict of Plan.MEMBER_KEYS}.  datasets: E pairs (train, valid) of
+    DrVAEDataset / VFAEDataset.  anneal_perturb: (itermax, offset) of the perturbation-loss anneal, or None for a
+    constant 1 (VFAE).  weights: optional E sampling-weight tensors over each training split.
 
     Per epoch one device multinomial over [E, D] weights (zero on padding rows) draws every member's minibatches;
     max_m floor(n_m / batch) steps follow, each one CUDA-graph replay.  After every epoch each member is validated and

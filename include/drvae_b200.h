@@ -42,7 +42,7 @@ typedef struct drvae_plan drvae_plan_t;
 
 /* Architecture = constructor arguments of the reference classes that shape tensors
  * (DrVAE.py:45-70, PVAE.py:45-63, VFAE.py:42-60) with the run_*.py fixed choices:
- * type_rec='diag_gaussian', nonlinearity='elu', type_y='discrete', clf_z1z2=True,
+ * type_rec='diag_gaussian', nonlinearity='elu' (drvae_set_activation: 'softplus'), type_y='discrete', clf_z1z2=True,
  * use_s=False, use_MMD=False, dropout 0, batch norm off.  The classifier's hidden layers (dim_h_clf, --class-y)
  * are an argument of drvae_plan_create_clf; drvae_plan_create builds the classifier without them. */
 typedef struct {
@@ -228,6 +228,15 @@ int drvae_infer(drvae_plan_t* plan, const float* x1, int N, const drvae_infer_ou
  * match it exactly; 0: the bf16 tensor-core GEMMs of the training step (faster, probabilities within ~1e-3).  Plans
  * with weight norm always use the tensor-core path. */
 int drvae_set_infer_precision(drvae_plan_t* plan, int fp32);
+
+/* Hidden-layer activation of every MLP of the model (blocks.MLP's `nonlinearity`, src/blocks.py:21-24): the encoders,
+ * the decoders and the classifier's hidden layers; the Gaussian heads, p(z2|z1), the decoder sigma and linear_p are
+ * unchanged.  DRVAE_ACT_ELU (the default of a new plan, the run_*.py drivers' choice): nn.ELU(); DRVAE_ACT_SOFTPLUS
+ * (the reference constructors' default): nn.Softplus() = log1p(exp(x)), x for x > 20.  Training steps, losses and
+ * drvae_infer all follow it.  Any other value is an error.  A change drops the plan's captured graphs. */
+#define DRVAE_ACT_ELU 0
+#define DRVAE_ACT_SOFTPLUS 1
+int drvae_set_activation(drvae_plan_t* plan, int act);
 
 /* Reconstruction metrics of the evaluation path: DeepGenerativeModelMixin.eval_x_reconstruction, src/DGMMixin.py:128-158
  * (numpy RMSE, sklearn r2_score(multioutput='variance_weighted'), the Python loop of scipy.stats.pearsonr over rows, the
